@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port; MATLAB absent)
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/<name>.npy
 
 One *step* = one pass of the hot path over one batch: the whole closed loop NTM_MPC_Sim.m:63-131
 (k_sim = 20 MPC steps, i_sim = 10 re-linearisations each under the default `fixed` inner policy) for
@@ -50,6 +51,7 @@ WORKLOADS = {  # name -> (BASELINE config id, TOTAL scenarios of the config as B
     "config2": (2, 1024), "config3": (3, 65536), "config4": (4, 1048576), "config5": (5, 16384),
 }
 HORIZON = {2: 10, 3: 20, 4: 20, 5: 100}
+DUMP_BYTES = 63_000_000      # --dump-outputs stays below 64 MB with the .npy headers; larger batches are sampled
 
 
 def host_threads() -> int:
@@ -109,6 +111,26 @@ def pct(xs, q):
     """q-quantile (nearest rank) of a list."""
     ys = sorted(xs)
     return ys[min(len(ys) - 1, max(0, int(round(q * (len(ys) - 1)))))]
+
+
+def dump_outputs(path: str, rec: np.ndarray, inner: np.ndarray, qp: np.ndarray) -> None:
+    """--dump-outputs: what the timed path returned in its last step, one <path>/<name>.npy per array, scenario-major.
+    The packed record [xk | uk | cost | status] is split into xk [S, K+1, 2], uk [S, K], cost [S] and status [S]
+    (float64, as the kernel stores them); inner_iters and qp_iters [S, K] are float32 (exact for these counts);
+    scenario [S] is each row's index in the batch.  A batch larger than DUMP_BYTES is written as a fixed seeded sample
+    of its scenarios, in index order, so that two builds can be compared row for row."""
+    S, K = inner.shape
+    idx = np.arange(S)
+    per_scenario = 8 * rec.shape[1] + 2 * 4 * K + 8
+    if S * per_scenario > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(S, DUMP_BYTES // per_scenario, replace=False))
+    rec = rec[idx]
+    arrays = dict(xk=rec[:, :2 * (K + 1)].reshape(-1, K + 1, 2), uk=rec[:, 2 * (K + 1):3 * K + 2], cost=rec[:, 3 * K + 2],
+                  status=rec[:, 3 * K + 3], inner_iters=inner[idx].astype(np.float32), qp_iters=qp[idx].astype(np.float32),
+                  scenario=idx.astype(np.float64))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a))
 
 
 class ClockSampler(threading.Thread):
@@ -241,7 +263,13 @@ def main():
     ap.add_argument("--scenarios", type=int, default=0, help="override the TOTAL scenario count of the workload")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary measurements (condense roofline, latency, eps_break)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (native path; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to the native path (the reference arm's batch size depends on its timing)")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -351,6 +379,12 @@ def main():
     flops = loop_flops(N, inner_loc, qp_loc, S * K_SIM)             # this rank's kernel against this rank's GPU
     achieved_tf = flops / kern_s / 1e12 if kern_s > 0 else 0.0
     d_uk_res = d_rec[:S, 2 * (K_SIM + 1):3 * K_SIM + 2].contiguous()
+    if args.dump_outputs:
+        outs = [d_rec[:S], d_inner[:S], d_qp[:S]]
+        if world > 1:                                                # whole job in scenario order, as the gather delivers it
+            outs = [D.all_gather_scenarios(t, S_job) for t in outs]
+        if rank == 0:
+            dump_outputs(args.dump_outputs, *(t.cpu().numpy() for t in outs))
 
     # ---- e2e: public host API, host buffers, H2D + kernel + D2H every step (pinned, then pageable)
     mpc.reset_stream()

@@ -1,10 +1,15 @@
-"""bench.py contract (CPU part): the reference arm prints ONE JSON line with the keys the driver reads."""
+"""bench.py contract: the reference arm prints ONE JSON line with the keys a caller reads; --dump-outputs writes what the
+timed path returned (-m gpu for the native run)."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+DUMPED = ("xk", "uk", "cost", "status", "inner_iters", "qp_iters", "scenario")
 
 
 def test_reference_arm_prints_one_contract_line():
@@ -64,3 +69,52 @@ def test_committed_traffic_figures_feed_the_roofline_objects():
     assert b.hess_traffic(8192, 64) is None
     assert b.ncu_traffic("config3", 65536) == t["closed_loop_kernel"]["dram_bytes_per_launch"]
     assert b.ncu_traffic("config3", 8192) is None
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                         capture_output=True, text=True, timeout=300)
+    assert out.returncode != 0 and "--steps must be at least 1" in out.stderr
+
+
+def test_dump_of_a_large_batch_is_a_fixed_sample_below_64_mb(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    S, K = 100_000, 20                                               # 68 MB of outputs in full
+    rec = np.repeat(np.arange(S, dtype=np.float64)[:, None], 3 * K + 4, axis=1)
+    inner = np.full((S, K), 10, dtype=np.int32)
+    qp = np.repeat(np.arange(S, dtype=np.int32)[:, None] % 4096, K, axis=1)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), rec, inner, qp)
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64_000_000
+    a = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in DUMPED}
+    idx = a["scenario"]
+    assert 0 < idx.size < S and np.all(np.diff(idx) > 0)
+    assert np.array_equal(a["cost"], idx) and np.array_equal(a["xk"][:, 3, 1], idx)    # rows are the sampled scenarios
+    assert np.array_equal(a["qp_iters"][:, 0], idx % 4096) and a["xk"].shape == (idx.size, K + 1, 2)
+    for n in DUMPED:
+        assert a[n].dtype in (np.float32, np.float64), n
+        assert np.array_equal(a[n], np.load(tmp_path / "b" / f"{n}.npy")), n     # same sample every time
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_what_the_timed_path_returns(tmp_path):
+    """The native run's dump equals the host API's closed loop on the same seeded batch, bit for bit."""
+    import ntm_mpc
+    from ntm_mpc import physics
+    S = 3000
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--scenarios", str(S),
+                          "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = {n: np.load(tmp_path / f"{n}.npy") for n in DUMPED}
+    P, x0, N = physics.batch_params(3, S=S)
+    mpc = ntm_mpc.NtmMpc(0)
+    try:
+        ref = mpc.closed_loop(x0, P.T, N=N, profile=ntm_mpc.PROFILE_INNER_FIXED)
+    finally:
+        mpc.close()
+    assert np.array_equal(d["scenario"], np.arange(S))
+    for k in DUMPED[:-1]:
+        assert d[k].dtype in (np.float32, np.float64), k
+        assert np.array_equal(d[k], ref[k]), k
