@@ -212,6 +212,37 @@ int ntm_mpc_closed_loop_sc_dev(ntm_handle *h, int layout, int profile, int S, in
                                const double *xbounds, double *xk, double *uk, double *Uk, double *cost,
                                int *inner_iters, int *qp_iters, int *status);
 
+/* ---- one receding-horizon step of the same controller, no plant (NTM_MPC_Sim.m:94-128): the caller closes the loop ---- *
+ * For S scenarios at their measured states x[2*S] (xk(:,k)), runs the inner re-linearisation loop of one time step and
+ * returns u[S] = uk(k) = U(1) (:107), U[N*S] = Uk(:,k), the last QP solution of the step (:106), inner_iters[S] and
+ * qp_iters[S] as in ntm_mpc_closed_loop, and status[S]: the worst QP status of this step, NTM_SCN_NONFINITE if x or u is
+ * not finite.  U, inner_iters, qp_iters and status may be NULL.  x, u and U follow `layout`.
+ * state holds NTM_CTRL_DOUBLES(N) doubles per scenario, one contiguous record per scenario in both layouts, read and
+ * written in place (host entry: copied in and back; _dev entry: resident on the device).  An ALL-ZERO record is a fresh
+ * controller: its first step runs the offline build (:63-73) from rho(x) and x becomes the script's x0.  There is no
+ * init call -- memset is the reset, and zeroing single records restarts single scenarios.  A record carries everything
+ * that crosses a time step of the fused loop:
+ *   [0, N)   a11   [N, 2N) a21   [2N, 3N) b      stage entries of the last re-scheduling (:114-117)
+ *   [3N, 4N) Uold (:86,127, D13)                 [4N, 5N) and [5N, 6N): the last two QP solutions (warm starts)
+ *   [6N, 7N) their partition states, (s1 + 1) + 4 (s2 + 1), s in {-1 lower, 0 free, +1 upper}
+ *   [7N, 7N+2) the last state this controller saw: the state the G, F on hand were built from under NTM_PROFILE_F_XK
+ *   [7N+2, 7N+4) x0 (G, F of the literal profile)   [7N+4] cost (two-phase fused loop only)
+ *   [7N+5] status + 4 first_qp + 8 n (n = warm-start history length, 3 = sticky "a warm QP ran long")
+ *   [7N+6] steps this record has run (0 = fresh)
+ * Preconditions (not checked by the kernel): every call for a record passes the same N, profile and params.
+ * profile: every bit of the fused loop's box-QP instantiations (RHO1_SQ, GAMMA_I, DENSE_G, F_XK, INNER_FIXED); the
+ * plant-only bits PLANT_C and PLANT_RK4 are accepted and ignored, so that one profile word drives both this entry and
+ * ntm_plant_step; NTM_PROFILE_TAUE_W is rejected (NTM_ERR_INVALID).  1 <= N <= NTM_MAX_HORIZON, i_sim >= 1.  One step is
+ * one kernel launch.  Stepped with ntm_plant_step under the same profile, k_sim steps reproduce ntm_mpc_closed_loop
+ * bit for bit. */
+#define NTM_CTRL_DOUBLES(N) (7 * (N) + 7)
+int ntm_mpc_step(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                 const double *params, int params_count, double *state, double *u, double *U, int *inner_iters,
+                 int *qp_iters, int *status);
+int ntm_mpc_step_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                     const double *params, int params_count, double *state, double *u, double *U, int *inner_iters,
+                     int *qp_iters, int *status);
+
 /* ---- the loop on EVERY visible GPU from ONE host process (what a MEX gateway can reach; SURVEY 8e) ------------- *
  * Replaces the same lines as ntm_mpc_closed_loop[_sc] (NTM_MPC_Sim.m:63-73,80-131); host pointers, same argument
  * meaning, no handle: the library keeps one pooled handle per device.  Scenarios never interact (:93-131 has no

@@ -15,6 +15,8 @@
  *   9   getWLc                   getWLc.m:1-63                 [W,L,c] = getWLc(xmax,xmin,umax,umin,Gamma,Phi,Lambda)
  *   10  quadprog                 quadprog call NTM_MPC_Sim.m:97 [U,fval,exitflag] = quadprog(H,f,A,b,[],[],lb,ub,x0,options)
  *                                (shadows the Optimization Toolbox function: input-box rows become bounds, state rows stay)
+ *   11  ntm_mpc_step             one step NTM_MPC_Sim.m:94-128  [u,state,U,inner,status] = ntm_mpc_step(state,x,params,N,i_sim,eps,profile)
+ *                                (no plant: the script's `for k` loop keeps its own plant code and passes state back in)
  *
  * The short forms are the ones NTM_MPC_Sim.m actually uses (:63-66,:113-119,:130); the missing trailing arguments
  * are fetched from the caller's workspace under the script's own variable names (kappa :24, tau_r :9, Ts :31,
@@ -32,7 +34,7 @@
 #include "ntm_mpc.h"
 
 #ifndef NTM_MEX_FN
-#error "compile with -DNTM_MEX_FN=<1..10>"
+#error "compile with -DNTM_MEX_FN=<1..11>"
 #endif
 
 static ntm_handle *g_h = NULL;
@@ -353,6 +355,46 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         plhs[0] = U;
         if (nlhs > 1) plhs[1] = mxCreateDoubleScalar(fval);
         if (nlhs > 2) plhs[2] = mxCreateDoubleScalar(st == NTM_SCN_OK ? 1.0 : (st == NTM_SCN_QP_ITER_CAP ? 0.0 : (st == NTM_SCN_INFEASIBLE ? -2.0 : -3.0)));
+    }
+#elif NTM_MEX_FN == 11
+    {   /* [u, state, U, inner, status] = ntm_mpc_step(state, x (2xS), params (16x1 | 16xS), N, i_sim, eps, profile)
+         * One receding-horizon step at the measured states x; state = [] starts S fresh controllers, otherwise it is the
+         * NTM_CTRL_DOUBLES(N) x S record this gateway returned last time (zeroing a column restarts that scenario).
+         * Pass the same N, params and profile on every call for the same state. */
+        int S, N, i_sim, profile, pc, i;
+        double eps;
+        size_t ld;
+        mxArray *u, *st, *U, *inner, *status;
+        int *ibuf;
+        if (nrhs != 7)
+            mexErrMsgIdAndTxt("ntm:arg", "usage: [u, state, U, inner, status] = ntm_mpc_step(state, x, params, N, i_sim, eps, profile)");
+        S = states_arg(prhs[1]);
+        if (!is_real_double(prhs[2]) || mxGetM(prhs[2]) != NTM_NPARAM || ((int)mxGetN(prhs[2]) != 1 && (int)mxGetN(prhs[2]) != S))
+            mexErrMsgIdAndTxt("ntm:arg", "params must be 16 x 1 or 16 x S (see ntm_mpc.h)");
+        pc = (int)mxGetN(prhs[2]);
+        N = (int)scalar_arg(nrhs, prhs, 3, ""); i_sim = (int)scalar_arg(nrhs, prhs, 4, "");
+        eps = scalar_arg(nrhs, prhs, 5, ""); profile = (int)scalar_arg(nrhs, prhs, 6, "");
+        if (N < 1 || N > NTM_MAX_HORIZON || i_sim < 1) mexErrMsgIdAndTxt("ntm:arg", "N in 1..128, i_sim >= 1");
+        if (profile & NTM_PROFILE_TAUE_W) mexErrMsgIdAndTxt("ntm:arg", "NTM_PROFILE_TAUE_W (128) is not supported by ntm_mpc_step");
+        ld = (size_t)NTM_CTRL_DOUBLES(N);
+        if (!is_real_double(prhs[0]))
+            mexErrMsgIdAndTxt("ntm:arg", "state must be [] or a real double matrix");
+        if (mxGetNumberOfElements(prhs[0]) != 0 && ((size_t)mxGetM(prhs[0]) != ld || (int)mxGetN(prhs[0]) != S))
+            mexErrMsgIdAndTxt("ntm:arg", "state must be [] or NTM_CTRL_DOUBLES(N) = 7N+7 rows by S columns");
+        st = mxCreateDoubleMatrix(ld, S, mxREAL);                  /* zeros: a fresh controller */
+        if (mxGetNumberOfElements(prhs[0]) != 0) memcpy(mxGetPr(st), mxGetPr(prhs[0]), sizeof(double) * ld * (size_t)S);
+        u = mxCreateDoubleMatrix(1, S, mxREAL); U = mxCreateDoubleMatrix(N, S, mxREAL);
+        inner = mxCreateDoubleMatrix(1, S, mxREAL); status = mxCreateDoubleMatrix(1, S, mxREAL);
+        ibuf = (int *)mxMalloc(sizeof(int) * (2 * (size_t)S + 1));
+        check(ntm_mpc_step(handle(), NTM_LAYOUT_MATLAB, profile, S, N, i_sim, eps, mxGetPr(prhs[1]), mxGetPr(prhs[2]), pc,
+                           mxGetPr(st), mxGetPr(u), mxGetPr(U), ibuf, NULL, ibuf + S));
+        for (i = 0; i < S; ++i) { mxGetPr(inner)[i] = (double)ibuf[i]; mxGetPr(status)[i] = (double)ibuf[S + i]; }
+        mxFree(ibuf);
+        plhs[0] = u;
+        if (nlhs > 1) plhs[1] = st; else mxDestroyArray(st);
+        if (nlhs > 2) plhs[2] = U; else mxDestroyArray(U);
+        if (nlhs > 3) plhs[3] = inner; else mxDestroyArray(inner);
+        if (nlhs > 4) plhs[4] = status; else mxDestroyArray(status);
     }
 #else
 #error "unknown NTM_MEX_FN"

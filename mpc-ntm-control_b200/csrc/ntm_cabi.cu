@@ -720,6 +720,61 @@ int ntm_mpc_closed_loop_sc(ntm_handle *h, int layout, int profile, int S, int N,
                                  uk, Uk, cost, inner_iters, qp_iters, status);
 }
 
+// ------------------------------------------------------------------------------------------------ controller step
+// One time step of the fused loop without the plant: k_sim = 1, the caller's records in LoopArgs::sv, ONE launch.
+static int check_step(int profile, int N, int i_sim) {
+    REQUIRE(!(profile & NTM_PROFILE_TAUE_W), "ntm_mpc_step: NTM_PROFILE_TAUE_W is not supported by the controller step");
+    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
+    REQUIRE(i_sim >= 1, "i_sim must be >= 1");
+    return NTM_OK;
+}
+
+int ntm_mpc_step_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                     const double *params, int pc, double *state, double *u, double *U, int *inner_iters, int *qp_iters,
+                     int *status) {
+    TRY(check_common(h, layout, S));
+    TRY(check_step(profile, N, i_sim));
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    REQUIRE(x && state && u, "NULL array");
+    ntm::LoopArgs a = {};
+    a.layout = layout; a.S = S; a.N = N; a.k_sim = 1; a.i_sim = i_sim; a.eps = eps;
+    a.flags = profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4);   // plant-only bits: no effect on the controller
+    a.x0 = x; a.params = params; a.params_count = pc;
+    a.uk = u; a.Uk = U; a.inner = inner_iters; a.qpit = qp_iters; a.status = status;
+    a.counter = h->counter;
+    a.sv = state; a.ctl = 1;
+    TRY(ensure_hscratch(h, N));
+    a.hscratch = h->hscratch;
+    CU(ntm::launch_closed_loop(h->stream, h->props, a, &h->launches));
+    return NTM_OK;
+}
+
+int ntm_mpc_step(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                 const double *params, int pc, double *state, double *u, double *U, int *inner_iters, int *qp_iters,
+                 int *status) {
+    TRY(check_common(h, layout, S));
+    TRY(check_step(profile, N, i_sim));
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    REQUIRE(x && state && u, "NULL array");
+    const size_t s = (size_t)S, n = (size_t)N, ld = (size_t)NTM_CTRL_DOUBLES(N);
+    Arena A(h);
+    A.want(2 * s * 8); A.want((size_t)pc * NTM_NPARAM * 8); A.want(ld * s * 8); A.want(s * 8);
+    if (U) A.want(n * s * 8);
+    A.want(s * 4); A.want(s * 4); A.want(s * 4);
+    TRY(A.reserve());
+    double *dx = A.take<double>(2 * s), *dp = A.take<double>((size_t)pc * NTM_NPARAM), *dst = A.take<double>(ld * s);
+    double *du = A.take<double>(s), *dU = U ? A.take<double>(n * s) : nullptr;
+    int *din = A.take<int>(s), *dqp = A.take<int>(s), *dstat = A.take<int>(s);
+    TRY(h2d(h, dx, x, 2 * s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM)); TRY(h2d(h, dst, state, ld * s));
+    TRY(ntm_mpc_step_dev(h, layout, profile, S, N, i_sim, eps, dx, dp, pc, dst, du, dU, din, dqp, dstat));
+    TRY(d2h(h, state, dst, ld * s)); TRY(d2h(h, u, du, s)); TRY(d2h(h, U, dU, n * s));
+    TRY(d2h(h, inner_iters, din, s)); TRY(d2h(h, qp_iters, dqp, s)); TRY(d2h(h, status, dstat, s));
+    CU(cudaStreamSynchronize(h->stream));
+    return NTM_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ getWLc
 int ntm_getWLc_dev(ntm_handle *h, int layout, int S, int N, const double *bounds, const double *Gamma, const double *Phi,
                    const double *Lambda, double *W, double *L, double *c) {

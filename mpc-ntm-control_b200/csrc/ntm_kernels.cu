@@ -1582,7 +1582,7 @@ size_t lpt_doubles(const DeviceProps &dp, const LoopArgs &a) {
     if (a.S > (1 << 18)) return 0;                                 // 0.5 GB of saved state at most; beyond that the tail is < 1 %
     static const bool quad = getenv("NTM_QUAD") != nullptr;
     if (quad && a.N <= NTM_QUAD_MAX_N) return 0;
-    return (size_t)a.S * NTM_SV_DOUBLES;
+    return (size_t)a.S * NTM_CTRL_DOUBLES(a.N);
 }
 
 cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches) {
@@ -1639,12 +1639,13 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
         else if (dense) { if (ext) NTM_LAUNCH_LOOP1(GWV, true, 1, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, true, 0, BLOCK, SMEM, GPB); } \
         else { if (ext) NTM_LAUNCH_LOOP1(GWV, false, 1, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 0, BLOCK, SMEM, GPB); }         \
     } while (0)
+#define NTM_CTL_EXT 0, 0, true                             // EXT = 0, LV = 0, CTL: multi-warp controller-step instantiation
     // Four lanes per scenario (ntm_quad.cuh) is an EXPERIMENT that lost: half the instructions of the one-warp kernel
     // (741 against 1,510 per re-linearisation) but 255 registers and 3.4 KB of shared memory per scenario leave 8 warps
     // per SM, whose mostly straight-line code stalls on instruction fetch (profiles/README.md, round 2): 53.9 ms
     // against 27.0 ms on config 3.  It stays selectable (NTM_QUAD=1) and parity-tested; the default is the one-warp kernel.
     static const bool use_quad = getenv("NTM_QUAD") != nullptr;
-    if (gw == 1 && !dense && ext != 2 && a.N <= NTM_QUAD_MAX_N && use_quad && !(a.flags & NTM_PROFILE_TAUE_W)) {
+    if (gw == 1 && !dense && ext != 2 && a.N <= NTM_QUAD_MAX_N && use_quad && !(a.flags & NTM_PROFILE_TAUE_W) && !a.ctl) {
         return launch_closed_loop_quad(st, dp, aa, launches);
     } else if (gw == 1) {
         const int wpb = wpb1;
@@ -1669,14 +1670,17 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
     } else if (gw == 2) {
         if (ext == 2) NTM_LAUNCH_LOOP1(2, false, 2, 64, gbytes, 1);
         else if (ext) NTM_LAUNCH_LOOP1(2, true, 1, 64, gbytes, 1);
+        else if (a.ctl) NTM_LAUNCH_LOOP1(2, true, NTM_CTL_EXT, 64, gbytes, 1);   // controller step
         else NTM_LAUNCH_LOOP1(2, true, 0, 64, gbytes, 1);
     } else {
         if (ext == 2) NTM_LAUNCH_LOOP1(4, false, 2, 128, gbytes, 1);
         else if (ext) NTM_LAUNCH_LOOP1(4, true, 1, 128, gbytes, 1);
+        else if (a.ctl) NTM_LAUNCH_LOOP1(4, true, NTM_CTL_EXT, 128, gbytes, 1);
         else NTM_LAUNCH_LOOP1(4, true, 0, 128, gbytes, 1);
     }
 #undef NTM_LAUNCH_LOOP1
 #undef NTM_LAUNCH_LOOP
+#undef NTM_CTL_EXT
     ++*launches;
     return cudaGetLastError();
 }

@@ -27,18 +27,21 @@ struct LoopArgs {
     int rec_ld;
     double *rec_status;                  // record mode: the status word as a double (0..3), or NULL
     // Two-phase launch with a longest-first work queue (one-warp box loop, see lpt_doubles): phase A runs time step 0 of
-    // every scenario, saves its loop state (NTM_SV_DOUBLES per scenario in sv) and a cost key (how many of the step's QPs
-    // missed the vertex test); a counting sort turns the keys into the order in which phase B pops the scenarios for the
-    // remaining steps.  A launch is as long as its slowest scenario STARTED LAST, and the slow scenarios are slow in every
-    // step.  lpt / sv: buffers from the C ABI layer (NULL = one launch in natural order); the rest is set by the launcher.
+    // every scenario, saves its loop state (one controller record per scenario in sv) and a cost key (how many of the
+    // step's QPs missed the vertex test); a counting sort turns the keys into the order in which phase B pops the
+    // scenarios for the remaining steps.  A launch is as long as its slowest scenario STARTED LAST, and the slow scenarios
+    // are slow in every step.  lpt / sv: buffers from the C ABI layer (NULL = one launch in natural order); the rest is
+    // set by the launcher.
     int *lpt;                            // S keys + S positions + NTM_LPT_BINS counters
-    double *sv;
+    double *sv;                          // NTM_CTRL_DOUBLES(N) per scenario (include/ntm_mpc.h), scenario slowest
     int k_begin, k_end;                  // time steps [k_begin, k_end) of this launch
     int *lpt_key;                        // phase A
     const int *perm;                     // phase B
+    // controller step (ntm_mpc_step, EXT = 0 instantiations only): k_sim = 1, x0 is the measured state, sv holds the
+    // caller's records (read at the start, written at the stop rule), no plant; xk and cost are NULL
+    int ctl;
 };
 #define NTM_LPT_BINS 160
-#define NTM_SV_DOUBLES 240
 
 struct DeviceProps {
     int sm_count, cc_major, cc_minor;

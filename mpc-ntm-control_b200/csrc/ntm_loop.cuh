@@ -106,7 +106,10 @@ struct LoopTraits {
 };
 
 // LV (LONG only): 0 = tableau in registers (N + 1 <= 7 * 10 / 7 * 15 for 2 / 4 warps), 1 = tableau in shared memory
-template <int GW, bool DENSE, int EXT, int LV = 0>
+// CTL (multi-warp groups, EXT = 0): the controller-step instantiation (ntm_mpc_step).  The one-warp instantiations run
+// controller steps as a runtime mode (LoopArgs::ctl) at unchanged register counts; in the multi-warp ones that mode cost
+// 2 registers, and 228 bytes of spill stores in closed_loop_kernel<4, false, 0, 0> (DESIGN section 4.8).
+template <int GW, bool DENSE, int EXT, int LV = 0, bool CTL = false>
 __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename LoopTraits<GW, DENSE, EXT>::WorkT &w,
                              unsigned char *gbase, int tI = -1, int tJ = -1) {
     using Gp = Group<GW>;
@@ -119,7 +122,10 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     load_params_shared(w.prm, a.params, layout, a.params_count, s, j);
     Gp::sync();
     const Params &P = *w.prm;
-    const double x01 = __ldg(a.x0 + elem(layout, S, 2, s, 0)), x02 = __ldg(a.x0 + elem(layout, S, 2, s, 1));
+    // controller step (ntm_mpc_step): a.x0 is the measured state, the loop state comes from the caller's record
+    constexpr bool REC = (EXT == 0) && (GW == 1 || CTL);             // instantiations that carry the record code
+    const bool ctl = (GW == 1) ? (EXT == 0 && a.ctl != 0) : CTL;
+    double x01 = __ldg(a.x0 + elem(layout, S, 2, s, 0)), x02 = __ldg(a.x0 + elem(layout, S, 2, s, 1));
     double x1 = x01, x2 = x02;
     // NTM_PROFILE_TAUE_W (EXT instantiations only): the shared parameter block carries the a22 the controller holds over
     // the horizon of the current time step, a22(tau_E(xk(1,k))); the nominal value and c_tauE stay in registers
@@ -169,25 +175,34 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     constexpr bool TWOPH = (GW == 1) && !DENSE && (EXT == 0);
     [[maybe_unused]] int nslow = 0, nqpit = 0;
     bool resumed = false;
-    if constexpr (TWOPH) {
-        if (a.k_begin > 0) {
-            // phase B: the loop state phase A saved after its last plant step.  G and F for the first QP are rebuilt at the
-            // top of the loop from the same stage entries and x0 (no NTM_PROFILE_F_XK here): bit-identical to one launch.
+    if constexpr (REC) {
+        // The loop state a record carries across a time step (layout: NTM_CTRL_DOUBLES in include/ntm_mpc.h), restored
+        // for phase B of a two-phase launch and for a controller step whose record has run before.  G and F for the first
+        // QP are rebuilt at the top of the loop from the same stage entries and from x0 or (NTM_PROFILE_F_XK) the last
+        // state the record saw: bit-identical to one launch.
+        const int N7 = 7 * N;
+        const double *sv = a.sv + (size_t)s * NTM_CTRL_DOUBLES(N);
+        if (a.sv != nullptr && (ctl ? sv[N7 + 6] != 0.0 : a.k_begin > 0)) {
             resumed = true;
-            const double *sv = a.sv + (size_t)s * NTM_SV_DOUBLES;
-            a11 = sv[j]; a21 = sv[32 + j]; bb = sv[64 + j]; Uold = sv[96 + j]; hU1 = sv[128 + j]; hU2 = sv[160 + j];
-            const int pk = reinterpret_cast<const int *>(sv + 192)[j];
-            hs1 = (pk & 3) - 1; hs2 = ((pk >> 2) & 3) - 1;
-            x1 = sv[224]; x2 = sv[225]; cost = sv[226];
-            const int fl = reinterpret_cast<const int *>(sv + 227)[0];
-            status = fl & 3; first_qp = ((fl >> 2) & 1) != 0; hist.n = (fl >> 3) & 3;
-            k = a.k_begin;
+            if (act) {
+                a11 = sv[j]; a21 = sv[N + j]; bb = sv[2 * N + j]; Uold = sv[3 * N + j];
+                const int pk = (int)sv[6 * N + j];
+                if (dense) {                                     // the QP runs in U itself: its own history
+                    hist.u1 = sv[4 * N + j]; hist.u2 = sv[5 * N + j]; hist.s1 = (pk & 3) - 1; hist.s2 = ((pk >> 2) & 3) - 1;
+                } else {
+                    hU1 = sv[4 * N + j]; hU2 = sv[5 * N + j]; hs1 = (pk & 3) - 1; hs2 = ((pk >> 2) & 3) - 1;
+                }
+            }
+            x1 = sv[N7]; x2 = sv[N7 + 1]; x01 = sv[N7 + 2]; x02 = sv[N7 + 3]; cost = sv[N7 + 4];
+            const int fl = (int)sv[N7 + 5];
+            status = ctl ? 0 : (fl & 3); first_qp = ((fl >> 2) & 1) != 0; hist.n = (fl >> 3) & 3;
+            k = ctl ? 0 : a.k_begin;
             Gp::sync();
-            if (act) w.bbs[j] = bb;
+            if (act) { w.bbs[j] = bb; if (GW > 1 || dense) { w.a11s[j] = a11; w.a21s[j] = a21; } }
             Gp::sync();
         }
     }
-    if (lead && !resumed) { a.xk[xk_at(0)] = x1; a.xk[xk_at(1)] = x2; }
+    if (lead && !resumed && !ctl) { a.xk[xk_at(0)] = x1; a.xk[xk_at(1)] = x2; }
 
     // One pass of this loop = [re-]condense (:66,:72-73 / :119-121), the stop rule of the iteration that just
     // finished (:123-127) and, at the end of a time step, the plant (:130); then the next QP + rollout (:97-117).
@@ -207,23 +222,29 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             if (!brk) Uold = Uj;                                                    // :127 (skipped by the break)
             if (stop) {
                 const double u0 = Gp::bcast0(Uj, w.red);                            // :107  uk(:,k) = U(1)
-                double nw, nom;
-                if constexpr (EXT != 0) plant_of(P, flags, a22n, ctau, x1, x2, u0, nw, nom);   // :130, or its RK4 / tau_E(w) refinement
-                else plant_euler(P, flags, x1, x2, u0, nw, nom);                    // :130
-                x1 = nw; x2 = nom;
-                if constexpr (EXT != 0) {
-                    if (taue) {                          // tau_E of the new measured width, held over the next step's horizon
-                        Gp::sync();                      // (G, F just built keep the previous value: a workspace assignment)
-                        if (lead) w.prm->a22 = a22_taue(a22n, ctau, x1);
-                        Gp::sync();
-                        if (GW == 1) { const double a22 = P.a22; sE = 1.0; for (int t = 0; t < j && t < N; ++t) sE *= a22; }
+                if (ctl) {                                                          // the caller runs the plant
+                    if (!isfinite(u0)) status = max(status, (int)NTM_SCN_NONFINITE);
+                } else {
+                    double nw, nom;
+                    if constexpr (EXT != 0) plant_of(P, flags, a22n, ctau, x1, x2, u0, nw, nom);   // :130, or its RK4 / tau_E(w) refinement
+                    else plant_euler(P, flags, x1, x2, u0, nw, nom);                // :130
+                    x1 = nw; x2 = nom;
+                    if constexpr (EXT != 0) {
+                        if (taue) {                      // tau_E of the new measured width, held over the next step's horizon
+                            Gp::sync();                  // (G, F just built keep the previous value: a workspace assignment)
+                            if (lead) w.prm->a22 = a22_taue(a22n, ctau, x1);
+                            Gp::sync();
+                            if (GW == 1) { const double a22 = P.a22; sE = 1.0; for (int t = 0; t < j && t < N; ++t) sE *= a22; }
+                        }
+                    }
+                    const double e1 = x1 - P.r1, e2 = x2 - P.r2;
+                    cost += e1 * (P.q11 * e1 + P.q12 * e2) + e2 * (P.q12 * e1 + P.q22 * e2);
+                    if (lead) {
+                        a.xk[xk_at(2 * (k + 1))] = x1;
+                        a.xk[xk_at(2 * (k + 1) + 1)] = x2;
                     }
                 }
-                const double e1 = x1 - P.r1, e2 = x2 - P.r2;
-                cost += e1 * (P.q11 * e1 + P.q12 * e2) + e2 * (P.q12 * e1 + P.q22 * e2);
                 if (lead) {
-                    a.xk[xk_at(2 * (k + 1))] = x1;
-                    a.xk[xk_at(2 * (k + 1) + 1)] = x2;
                     a.uk[uk_at(k)] = u0;
 #ifdef NTM_DEBUG_NSLOW
                     if (a.inner) a.inner[elem(layout, S, a.k_sim, s, k)] = nslow;     // cumulative count of active-set QPs
@@ -233,22 +254,33 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                     if (a.qpit) a.qpit[elem(layout, S, a.k_sim, s, k)] = qpit;
                 }
                 ++k; it = 0; qpit = 0;
-                if constexpr (TWOPH) {
-                    if (k == a.k_end && k < a.k_sim) {            // phase A ends here: loop state + cost key, then the next scenario
-                        double *sv = a.sv + (size_t)s * NTM_SV_DOUBLES;
-                        sv[j] = a11; sv[32 + j] = a21; sv[64 + j] = bb; sv[96 + j] = Uold; sv[128 + j] = hU1; sv[160 + j] = hU2;
-                        reinterpret_cast<int *>(sv + 192)[j] = (hs1 + 1) | ((hs2 + 1) << 2);
-                        if (lead) {
-                            sv[224] = x1; sv[225] = x2; sv[226] = cost;
-                            reinterpret_cast<int *>(sv + 227)[0] = (status & 3) | ((first_qp ? 1 : 0) << 2) | (hist.n << 3);
-                            a.lpt_key[s] = min(12 * min(nslow, 12) + min(nqpit, 11), NTM_LPT_BINS - 1);
+                if constexpr (REC) {
+                    // the record (see the restore above): end of a controller step, or of phase A (then the next scenario)
+                    if (a.sv != nullptr && (ctl || (k == a.k_end && k < a.k_sim))) {
+                        const int N7 = 7 * N;
+                        double *sv = a.sv + (size_t)s * NTM_CTRL_DOUBLES(N);
+                        if (act) {
+                            sv[j] = a11; sv[N + j] = a21; sv[2 * N + j] = bb; sv[3 * N + j] = Uold;
+                            sv[4 * N + j] = dense ? hist.u1 : hU1; sv[5 * N + j] = dense ? hist.u2 : hU2;
+                            sv[6 * N + j] = dense ? (double)((hist.s1 + 1) | ((hist.s2 + 1) << 2)) : (double)((hs1 + 1) | ((hs2 + 1) << 2));
                         }
-                        return;
+                        if (lead) {
+                            sv[N7] = x1; sv[N7 + 1] = x2; sv[N7 + 2] = x01; sv[N7 + 3] = x02; sv[N7 + 4] = cost;
+                            sv[N7 + 5] = (double)((status & 3) | ((first_qp ? 1 : 0) << 2) | (hist.n << 3));
+                            sv[N7 + 6] = ctl ? sv[N7 + 6] + 1.0 : (double)k;
+                            if constexpr (TWOPH) {
+                                if (!ctl) a.lpt_key[s] = min(12 * min(nslow, 12) + min(nqpit, 11), NTM_LPT_BINS - 1);
+                            }
+                        }
+                        if (!ctl) return;
                     }
                 }
             }
         }
         if (k >= a.k_sim) break;
+        if (ctl && it == 0) {            // G, F on hand are built; the step itself (QP, rollout) starts from the measurement
+            x1 = __ldg(a.x0 + elem(layout, S, 2, s, 0)); x2 = __ldg(a.x0 + elem(layout, S, 2, s, 1));
+        }
         if (!retry) ++it;
         int nit = 0;
         int st = NTM_SCN_OK;
@@ -496,7 +528,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     }
 }
 
-template <int GW, bool DENSE, int EXT, int LV = 0>
+template <int GW, bool DENSE, int EXT, int LV = 0, bool CTL = false>
 __global__ void __launch_bounds__(GW == 1 ? 128 : 32 * GW,
                                   GW == 1 ? (EXT == 0 ? 5 : (EXT == 1 ? 4 : 3)) : (LoopTraits<GW, DENSE, EXT>::LONG ? 3 : 1))
 closed_loop_kernel(LoopArgs a, unsigned int gbytes) {
@@ -524,7 +556,7 @@ closed_loop_kernel(LoopArgs a, unsigned int gbytes) {
         s = Gp::bcast0(s, w.ired);
         if (s >= a.S) break;
         if (a.perm != nullptr) s = __ldg(a.perm + s);       // phase B of a two-phase launch: longest first
-        run_scenario<GW, DENSE, EXT, LV>(a, s, j, w, smem_raw + (size_t)gib * gbytes, tI, tJ);
+        run_scenario<GW, DENSE, EXT, LV, CTL>(a, s, j, w, smem_raw + (size_t)gib * gbytes, tI, tJ);
         Gp::sync();
     }
     // the last group to leave re-arms the work queue for the next launch (saves a memset per call: latency)

@@ -51,6 +51,13 @@ SYMBOLS = {
 def rec_doubles(k_sim: int) -> int:
     """NTM_REC_DOUBLES(k_sim): doubles per scenario of the packed record [xk | uk | cost | status]."""
     return 3 * k_sim + 4
+
+
+def ctrl_doubles(N: int) -> int:
+    """NTM_CTRL_DOUBLES(N): doubles per scenario of a controller record (``ntm_mpc_step``)."""
+    return 7 * N + 7
+
+
 for _sfx in ("", "_dev"):
     SYMBOLS["ntm_rho" + _sfx] = (_i, [_h, _i, _i, _i, _dp, _dp, _i, _dp, _dp, _dp])
     SYMBOLS["ntm_lpv_AB" + _sfx] = (_i, [_h, _i, _i, _dp, _dp, _dp, _dp, _i, _dp, _dp])
@@ -64,6 +71,8 @@ for _sfx in ("", "_dev"):
     SYMBOLS["ntm_plant_step" + _sfx] = (_i, [_h, _i, _i, _i, _dp, _dp, _dp, _i, _dp])
     SYMBOLS["ntm_mpc_closed_loop" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i,
                                                   _dp, _dp, _dp, _dp, _dp, _dp, _dp])
+    SYMBOLS["ntm_mpc_step" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i, _dp, _dp, _dp, _dp,
+                                           _dp, _dp])
     SYMBOLS["ntm_mpc_closed_loop_sc" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i, _i, _dp,
                                                      _dp, _dp, _dp, _dp, _dp, _dp, _dp])
 

@@ -14,7 +14,7 @@ from typing import Dict, Optional
 import numpy as np
 
 from . import _lib
-from ._lib import LAYOUT_MATLAB, LAYOUT_SOA, NPARAM, NtmError, check, load, rec_doubles  # noqa: F401
+from ._lib import LAYOUT_MATLAB, LAYOUT_SOA, NPARAM, NtmError, check, ctrl_doubles, load, rec_doubles  # noqa: F401
 
 MC_NBINS = 32                                   # NTM_MC_NBINS / NTM_MC_NSTAT of include/ntm_mpc.h
 MC_NSTAT = 22 + MC_NBINS
@@ -295,6 +295,11 @@ class NtmMpc:
         check(self._lib.ntm_plant_step(self._h, LAYOUT_MATLAB, profile, S, _ptr(x), _ptr(u), _ptr(p), pc, _ptr(xn)))
         return xn.reshape(S, 2)
 
+    def plant_step_dev(self, S: int, profile: int, layout: int, x_ptr: int, u_ptr: int, params_ptr: int,
+                       params_count: int, xn_ptr: int) -> None:
+        """``plant_step`` on device pointers, asynchronous on the handle's stream (``ntm_plant_step_dev``)."""
+        check(self._lib.ntm_plant_step_dev(self._h, layout, profile, S, x_ptr, u_ptr, params_ptr, params_count, xn_ptr))
+
     # ------------------------------------------------------------------ NTM_MPC_Sim.m:63-131, fused
     def closed_loop(self, x0, params, N: int, k_sim: int = 20, i_sim: int = 10, eps: float = 1e-14,
                     profile: int = 0, want_Uk: bool = False, out: Optional[dict] = None, state_rows: int = 0,
@@ -349,6 +354,43 @@ class NtmMpc:
                                                    params_count, int(state_rows), _ptr(xb), xk_ptr, uk_ptr, Uk_ptr or None,
                                                    cost_ptr or None, inner_ptr or None, qp_ptr or None, status_ptr or None))
 
+    # ------------------------------------------------------------------ NTM_MPC_Sim.m:94-128, one step, no plant
+    def mpc_step(self, state, x, params, N: int, i_sim: int = 10, eps: float = 1e-14, profile: int = 0,
+                 want_U: bool = False):
+        """One receding-horizon step for S scenarios at their measured states ``x`` [S, 2] (``ntm_mpc_step``).
+
+        ``state`` is a C-contiguous float64 array [S, ``ctrl_doubles(N)``] updated in place; an all-zero row is a fresh
+        controller (its first step runs the offline build from ``x``), so ``state[s] = 0`` restarts scenario ``s``.
+        Pass the same N, profile and params on every call for the same records.  Returns a dict with ``u`` [S],
+        ``U`` [S, N] (None unless ``want_U``), ``inner_iters``, ``qp_iters`` and ``status`` [S]."""
+        x = _f64(x).reshape(-1, 2)
+        S = x.shape[0]
+        p, pc = self._params(params, S)
+        if not (isinstance(state, np.ndarray) and state.dtype == np.float64 and state.shape == (S, ctrl_doubles(N))
+                and state.flags.c_contiguous and state.flags.writeable):
+            raise ValueError(f"state must be a writeable C-contiguous float64 array of shape {(S, ctrl_doubles(N))}")
+        u = np.empty(S)
+        U = np.empty((S, N)) if want_U else None
+        inner, qpit, status = (np.empty(S, dtype=np.int32) for _ in range(3))
+        check(self._lib.ntm_mpc_step(self._h, LAYOUT_MATLAB, profile, S, N, i_sim, eps, _ptr(x), _ptr(p), pc, _ptr(state),
+                                     _ptr(u), _ptr(U), _ptr(inner), _ptr(qpit), _ptr(status)))
+        return dict(u=u, U=U, inner_iters=inner, qp_iters=qpit, status=status)
+
+    def mpc_step_dev(self, S: int, N: int, i_sim: int, eps: float, profile: int, layout: int, x_ptr: int,
+                     params_ptr: int, params_count: int, state_ptr: int, u_ptr: int, U_ptr: int = 0, inner_ptr: int = 0,
+                     qp_ptr: int = 0, status_ptr: int = 0) -> None:
+        """``mpc_step`` on device pointers, asynchronous on the handle's stream (``ntm_mpc_step_dev``); the records
+        (``ctrl_doubles(N)`` doubles per scenario, scenario slowest) stay resident."""
+        check(self._lib.ntm_mpc_step_dev(self._h, layout, profile, S, N, i_sim, eps, x_ptr, params_ptr, params_count,
+                                         state_ptr, u_ptr, U_ptr or None, inner_ptr or None, qp_ptr or None,
+                                         status_ptr or None))
+
+    def controller(self, params, N: int, S: Optional[int] = None, i_sim: int = 10, eps: float = 1e-14,
+                   profile: int = 0) -> "Controller":
+        """A ``Controller`` on this handle that owns the records of S scenarios (S from ``params`` [S, NPARAM], or given
+        with one shared [NPARAM] block)."""
+        return Controller(self, params, N, S, i_sim, eps, profile)
+
     # ------------------------------------------------------------------ Monte-Carlo back end (SURVEY 8f-3)
     def mc_stats(self, xk, uk, cost, status, params, bounds=MC_STATE_BOX, w_suppressed: float = 0.06, hist_max: float = 0.2):
         """Reduce a batch of closed-loop results ([S,k_sim+1,2], [S,k_sim], [S], [S]) on the device; returns the
@@ -386,3 +428,39 @@ class NtmMpc:
                      params_ptr: int, params_count: int, phi_ptr: int, gam_ptr: int, lam_ptr: int) -> None:
         check(self._lib.ntm_condense_dev(self._h, layout, profile, S, N, r1_ptr, r2_ptr, r3_ptr, params_ptr, params_count,
                                          phi_ptr, gam_ptr, lam_ptr))
+
+
+class Controller:
+    """The receding-horizon controller of NTM_MPC_Sim.m for S scenarios, in front of a plant the caller runs::
+
+        ctl = NtmMpc(0).controller(params, N=20)
+        for k in range(k_sim):
+            u = ctl.step(x)              # x: measured states [S, 2]
+            x = my_plant(x, u)
+
+    Holds the per-scenario records of ``ntm_mpc_step`` (host memory) and the fixed arguments every call for them must
+    repeat.  ``reset(mask)`` restarts the selected scenarios: their next step is a first step from the state it gets."""
+
+    def __init__(self, mpc: NtmMpc, params, N: int, S: Optional[int] = None, i_sim: int = 10, eps: float = 1e-14,
+                 profile: int = 0):
+        p = _f64(params)
+        if S is None:
+            if p.ndim != 2:
+                raise ValueError("S is needed with one shared parameter block")
+            S = p.shape[0]
+        self.mpc, self.N, self.S, self.i_sim, self.eps, self.profile = mpc, int(N), int(S), int(i_sim), float(eps), int(profile)
+        self.params, _ = NtmMpc._params(p, self.S)
+        self.state = np.zeros((self.S, ctrl_doubles(self.N)))
+        self.last = None
+
+    def step(self, x, want_U: bool = False) -> np.ndarray:
+        """u [S] for the measured states ``x`` [S, 2]; the full result dict of ``mpc_step`` is kept in ``last``."""
+        self.last = self.mpc.mpc_step(self.state, x, self.params, self.N, self.i_sim, self.eps, self.profile, want_U)
+        return self.last["u"]
+
+    def reset(self, mask=None) -> None:
+        """Fresh controllers for every scenario (``mask=None``) or for those selected by a boolean / index ``mask``."""
+        if mask is None:
+            self.state[:] = 0.0
+        else:
+            self.state[np.asarray(mask)] = 0.0
