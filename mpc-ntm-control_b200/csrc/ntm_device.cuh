@@ -789,6 +789,9 @@ __device__ int qp_solve(int N, int j, const Work &w, double Fj, double lbj, doub
         }
     }
     if (it > max_iter) it = max_iter;
+    // a pinned variable (lbj == ubj) has one value either way; its state is the side the gradient points to, which is
+    // what the literal kernels map back to U: b * [umin, umax] can round to one y although umin < umax
+    if (pinned) state = (g < 0.0) ? 1 : -1;
     const bool nonfinite = Gp::any(act && !(isfinite(u) && isfinite(g)), w.ired);
     double Uj = (state < 0) ? lbj : ((state > 0) ? ubj : fmin(fmax(u, lbj), ubj));
     if (nonfinite) Uj = nan("");               // IEEE-faithful: a non-finite Hessian/gradient poisons the step

@@ -414,6 +414,9 @@ __device__ int qp_solve_long(int N, int j, const LongWork &w, double Fj, double 
         }
     }
     if (it > max_iter) it = max_iter;
+    // a pinned variable (lbj == ubj) has one value either way; its state is the side the gradient points to, which is
+    // what the literal kernels map back to U: b * [umin, umax] can round to one y although umin < umax
+    if (pinned) state = (g < 0.0) ? 1 : -1;
     const bool nonfinite = Gp::any(act && !(isfinite(u) && isfinite(g)), w.ired);
     double Uj = (state < 0) ? lbj : ((state > 0) ? ubj : fmin(fmax(u, lbj), ubj));
     if (nonfinite) Uj = nan("");
@@ -825,6 +828,9 @@ __device__ int qp_solve_tile(int N, int j, const LongWork &w, const TileWork &tw
         else --nfree;
     }
     if (it > max_iter) it = max_iter;
+    // a pinned variable (lbj == ubj) has one value either way; its state is the side the gradient points to, which is
+    // what the literal kernels map back to U: b * [umin, umax] can round to one y although umin < umax
+    if (pinned) state = (g < 0.0) ? 1 : -1;
     const bool nonfinite = Gp::any(act && !(isfinite(u) && isfinite(g)), w.ired);
     double Uj = (state < 0) ? lbj : ((state > 0) ? ubj : fmin(fmax(u, lbj), ubj));
     if (nonfinite) Uj = nan("");

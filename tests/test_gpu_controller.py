@@ -111,7 +111,8 @@ def _cases():
         c.append((f"config3_16k_p{prof}", 3, 16384, None, prof, 0, False))
     c.append(("config4_4k", 4, 4096, None, FIXED, 0, False))
     c += [("N32_literal", 3, 512, 32, 0, 0, False), ("N32_gamma_i", 3, 512, 32, 2, 0, False),
-          ("N48_gamma_i", 3, 256, 48, 2, 0, False), ("N80_gamma_i", 3, 64, 80, 2, 0, False)]
+          ("N48_gamma_i", 3, 256, 48, 2, 0, False), ("N80_gamma_i", 3, 64, 80, 2, 0, False),
+          ("N64_gamma_i_row_sweep", 3, 64, 64, 2, 0, False), ("N120_gamma_i_row_sweep", 3, 32, 120, 2, 0, False)]
     for N in (40, 64, 100, 110):                              # long literal paths: tableau in registers / shared memory
         c.append((f"config5_N{N}", 5, 512, N, FIXED, 0, False))
     return c
