@@ -714,29 +714,6 @@ __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc) {
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
-// 1-D bulk copy global -> shared (the TMA engine, SASS UBLKCP) completing on an mbarrier: ONE instruction per contiguous
-// piece instead of one cp.async per 16 bytes and lane
-__device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long *bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long *bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void *dst, const void *src, unsigned bytes, unsigned long long *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n" ::"r"(smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(unsigned long long *bar, unsigned parity) {
-    unsigned ok;
-    asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
-                 : "=r"(ok)
-                 : "r"(smem_u32(bar)), "r"(parity)
-                 : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory"); }
 template <int NKEEP>
 __device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;\n" ::"n"(NKEEP) : "memory"); }
 
@@ -756,24 +733,22 @@ __device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.w
 // Measured and rejected (profiles/README.md, round 2): a double buffer with 40-row chunks (2.01 ms against 1.91), Omega
 // applied in registers without the second copy and one barrier per chunk (bulk copies 2.19, cp.async 2.11), a half-period
 // stagger of the two CTAs of an SM (2.25), dealing the super-tiles to the warps by cost (2.05; 1.78 against 1.75 after the
-// predicated DMMAs were gone).
+// predicated DMMAs were gone), 16 warps and one CTA per SM with the raw chunk double buffered (2.22 against 1.89).
 // F rides along: v = Phi x + Lambda - R is staged as column N of the chunk, and row N of the extended product
 // [Gamma v]' Omega [Gamma v] is F / 2.
-// WARPS = 8, NBUF = 1 (default): two CTAs per SM fill each other's copy waits.  WARPS = 16, NBUF = 2 (NTM_HESS_W16=1): one
-// CTA per SM, the raw chunk double buffered -- the cp.async copies of the next chunk (of the next scenario after the last
-// one) fly while the tensor cores work on this one; measured slower (2.22 against 1.89 ms).
-template <int MAXST, int WARPS, int NBUF>   // MAXST super-tiles per warp: ceil(nst (nst + 1) / 2 / WARPS), nst = ceil(ceil8(N + 1) / 16)
-__global__ void __launch_bounds__(32 * WARPS, (WARPS == 8 && MAXST <= 4) ? 2 : 1)
+// 8 warps per CTA: two CTAs per SM fill each other's copy waits.
+template <int MAXST>   // MAXST super-tiles per warp: ceil(nst (nst + 1) / 2 / WARPS), nst = ceil(ceil8(N + 1) / 16)
+__global__ void __launch_bounds__(256, MAXST <= 4 ? 2 : 1)
 hessian_grad_dmma_kernel(int layout, int S, int N, const double *__restrict__ Phi, const double *__restrict__ Gam,
                          const double *__restrict__ Lam, const double *__restrict__ x, const double *__restrict__ params,
                          int pc, double *__restrict__ G, double *__restrict__ F) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    constexpr int T = 32 * WARPS, KC = NTM_DMMA_KC, ldc = KC, KH = KC / 2;
+    constexpr int WARPS = 8, T = 32 * WARPS, KC = NTM_DMMA_KC, ldc = KC, KH = KC / 2;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const int Np = (N + 1 + 7) & ~7;                       // at least one spare column: column N carries v
     const int K2 = 2 * N, VP = K2 + 4;                     // a Vs buffer: v (2N), then q11, q12, q22 of its scenario
-    double *Ga = reinterpret_cast<double *>(smem_raw);     // NBUF raw chunks: column c at Ga[b*Np*ldc + c*ldc + k], k < KC
-    double *Qs = Ga + NBUF * (size_t)Np * ldc;             // the current chunk times Omega
+    double *Ga = reinterpret_cast<double *>(smem_raw);     // the raw chunk: column c at Ga[c*ldc + k], k < KC
+    double *Qs = Ga + (size_t)Np * ldc;                    // the current chunk times Omega
     double *Vs = Qs + (size_t)Np * ldc;                    // two buffers (this scenario / the next one)
     unsigned char *stab = reinterpret_cast<unsigned char *>(Vs + 2 * VP);   // super-tile t -> (sm, sn)
     const int EG = 2 * N * N;
@@ -832,8 +807,6 @@ hessian_grad_dmma_kernel(int layout, int S, int N, const double *__restrict__ Ph
             if (h >= KH) { h -= KH; off += wrap; }
         }
     };
-    int par = 0;
-    if (NBUF == 2) issue(s, 0, Ga);
     for (; s < S; s += gridDim.x) {
         const int sn = s + gridDim.x;
         const double *vs = Vs + vp * VP;
@@ -847,24 +820,15 @@ hessian_grad_dmma_kernel(int layout, int S, int N, const double *__restrict__ Ph
             const int kend = (rows + 7) & ~7;               // rows [rows, kend) are zero, the rest of the chunk is not read
             const bool last = kc + KC >= K2;
             double nv0 = 0.0, nv1 = 0.0;
-            double *Gs = Ga + (NBUF == 2 ? (size_t)par * Np * ldc : 0);
-            if (NBUF == 2) {
-                cp_async_wait_all();                        // this thread's pairs of the chunk have landed
-                __syncthreads();                            // everyone is done with the previous chunk (Qs, the other raw buffer); Vs visible
-                if (!last) issue(s, kc + KC, Ga + (size_t)(par ^ 1) * Np * ldc);
-                else if (sn < S) issue(sn, 0, Ga + (size_t)(par ^ 1) * Np * ldc);
-                if (last && sn < S && tid < N) vpair(sn, nv0, nv1);      // loads in flight across the Omega pass
-            } else {
-                __syncthreads();                            // everyone is done with the previous chunk; Vs visible
-                issue(s, kc, Gs);
-                if (last && sn < S && tid < N) vpair(sn, nv0, nv1);
-                cp_async_wait_all();
-            }
+            __syncthreads();                                // everyone is done with the previous chunk; Vs visible
+            issue(s, kc, Ga);
+            if (last && sn < S && tid < N) vpair(sn, nv0, nv1);
+            cp_async_wait_all();
             const double q11 = vs[K2], q12 = vs[K2 + 1], q22 = vs[K2 + 2];
             // Omega image of the pairs this thread copied itself (visible to it after the wait)
 #pragma unroll 4
             for (int p = tid; p < N * KH; p += T) {
-                const double2 gg = *reinterpret_cast<const double2 *>(Gs + 2 * p);
+                const double2 gg = *reinterpret_cast<const double2 *>(Ga + 2 * p);
                 *reinterpret_cast<double2 *>(Qs + 2 * p) = make_double2(fma(q11, gg.x, q12 * gg.y), fma(q22, gg.y, q12 * gg.x));
             }
             // the v column and the padding columns: plain stores, both images
@@ -872,7 +836,7 @@ hessian_grad_dmma_kernel(int layout, int S, int N, const double *__restrict__ Ph
                 const int c = p / KH, k = 2 * (p - c * KH);
                 const bool vcol = (c == N) && (k < rows);
                 const double g0 = vcol ? vs[kc + k] : 0.0, g1 = vcol ? vs[kc + k + 1] : 0.0;
-                *reinterpret_cast<double2 *>(Gs + 2 * p) = make_double2(g0, g1);
+                *reinterpret_cast<double2 *>(Ga + 2 * p) = make_double2(g0, g1);
                 *reinterpret_cast<double2 *>(Qs + 2 * p) = make_double2(fma(q11, g0, q12 * g1), fma(q22, g1, q12 * g0));
             }
             if (last && sn < S) {
@@ -889,7 +853,7 @@ hessian_grad_dmma_kernel(int layout, int S, int N, const double *__restrict__ Ph
                     const bool diag = sm == sn2;
                     const bool row1 = 2 * sm + 1 < nt;      // the super-tile has a second tile row / column
                     const bool col1 = 2 * sn2 + 1 < nt;
-                    const double *r0 = Gs + (size_t)(16 * sm + g) * ldc + 2 * t4;
+                    const double *r0 = Ga + (size_t)(16 * sm + g) * ldc + 2 * t4;
                     const double *c0 = Qs + (size_t)(16 * sn2 + g) * ldc + 2 * t4;
                     const double *r1 = row1 ? r0 + 8 * ldc : r0;
                     const double *c1 = col1 ? c0 + 8 * ldc : c0;
@@ -942,7 +906,6 @@ hessian_grad_dmma_kernel(int layout, int S, int N, const double *__restrict__ Ph
                     }
                 }
             }
-            par ^= 1;
         }
         vp ^= 1;
         // results: element e of this scenario sits at base + e * es in either layout (one multiply per store instead of the
@@ -991,8 +954,8 @@ template <int NT>                                                  // NT = ceil(
 __global__ void __launch_bounds__(128, NT <= 3 ? 3 : 1)
 hessian_grad_dmma_warp_kernel(int S, int N, int ld, const double *__restrict__ Phi, const double *__restrict__ Gam,
                               const double *__restrict__ Lam, const double *__restrict__ x, const double *__restrict__ params,
-                              int pc, double *__restrict__ G, double *__restrict__ F, int vec_ok) {
-    // MATLAB layout only (the launcher falls back to the scalar kernel otherwise)
+                              int pc, double *__restrict__ G, double *__restrict__ F, int aligned16) {
+    // MATLAB layout only (the launcher falls back to the scalar kernel otherwise); aligned16: Gam and G are 16-byte aligned
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, wpb = blockDim.x >> 5;
     constexpr int Np = NT * 8;
@@ -1001,7 +964,7 @@ hessian_grad_dmma_warp_kernel(int S, int N, int ld, const double *__restrict__ P
     double *buf0 = reinterpret_cast<double *>(smem_raw) + (size_t)wid * 2 * slice;     // column c at buf[c*ld + k]
     const int EG = 2 * N * N;
     const int g = lane >> 2, t4 = lane & 3;
-    const bool vec = (vec_ok & 1) && !(N & 1);
+    const bool vec = aligned16 && !(N & 1);
     const int stride = gridDim.x * wpb;
 
     // asynchronous copy of Gamma(:,:,s) into columns 0..N-1 of dst (one commit group per scenario).  A lane's element
@@ -1039,31 +1002,13 @@ hessian_grad_dmma_warp_kernel(int S, int N, int ld, const double *__restrict__ P
         buf0[(size_t)b * slice + (size_t)(N + 1) * ld + r] = 0.0;
     }
 
-    // OPT-IN (NTM_HESS_BULK=1; measured and lost, profiles/README.md round 2): each column of a 16-byte aligned Gamma (2N
-    // contiguous doubles) comes in by ONE bulk copy issued by lane c (TMA engine, SASS UBLKCP) and lands on the buffer's
-    // mbarrier -- 1 instruction per lane and scenario instead of ~13 cp.async + their index arithmetic.  At N = 20 the
-    // pieces are 320 bytes: 0.194 ms against 0.176 ms for the cp.async staging (55 % against 61 % of the copy peak).
-    __shared__ unsigned long long bars[4][2];
-    unsigned phase[2] = {0u, 0u};
-    const bool bulk = (vec_ok & 2) != 0 && wpb <= 4;
-    if (bulk && lane == 0) { mbar_init(&bars[wid][0], 1); mbar_init(&bars[wid][1], 1); }
-    if (bulk) { asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory"); __syncwarp(); }
-    auto stage_bulk = [&](int sc, int b) {
-        double *dst = buf0 + (size_t)b * slice;
-        fence_proxy_async();                                       // this warp's plain accesses to the slice come first
-        __syncwarp();
-        if (lane == 0) mbar_expect_tx(&bars[wid][b], (unsigned)(N * 2 * N * sizeof(double)));
-        __syncwarp();
-        if (lane < N) bulk_g2s(dst + lane * ld, Gam + (size_t)sc * EG + (size_t)lane * 2 * N, (unsigned)(2 * N * sizeof(double)), &bars[wid][b]);
-    };
-
     int s = blockIdx.x * wpb + wid;
     int cur = 0;
-    if (s < S) { if (bulk) stage_bulk(s, 0); else stage(s, buf0); }
+    if (s < S) stage(s, buf0);
     for (; s < S; s += stride, cur ^= 1) {
         double *Gs = buf0 + (size_t)cur * slice;
         const int sn = s + stride;
-        if (sn < S) { if (bulk) stage_bulk(sn, cur ^ 1); else stage(sn, buf0 + (size_t)(cur ^ 1) * slice); }   // the other buffer was drained in the previous pass
+        if (sn < S) stage(sn, buf0 + (size_t)(cur ^ 1) * slice);   // the other buffer was drained in the previous pass
         const Params P = load_params(params, NTM_LAYOUT_MATLAB, pc, s);
         {
             // v (column N) and zero rows 2N..Kp-1 of the Gamma columns: the slice doubles as the G staging area, so those
@@ -1082,10 +1027,7 @@ hessian_grad_dmma_warp_kernel(int S, int N, int ld, const double *__restrict__ P
             for (int k = 2 * N + lane; k < Kp; k += 32)           // Kp - 2N <= 2 padding rows of the Gamma columns
                 for (int c = 0; c < N; ++c) Gs[c * ld + k] = 0.0;
         }
-        if (bulk) {
-            while (!mbar_try_wait(&bars[wid][cur], phase[cur])) {}
-            phase[cur] ^= 1u;
-        } else if (sn < S) cp_async_wait_group<1>(); else cp_async_wait_group<0>();     // this scenario's Gamma has landed
+        if (sn < S) cp_async_wait_group<1>(); else cp_async_wait_group<0>();     // this scenario's Gamma has landed
         __syncwarp();
         const double qs = (t4 & 1) ? P.q22 : P.q11;
         double acc[NT * (NT + 1) / 2][2];                          // kept in registers until Gamma is dead
@@ -1470,12 +1412,7 @@ size_t state_rows_dense_smem(int N, int srows) {
 }
 
 size_t hscratch_bytes(const DeviceProps &dp, int N) {
-    size_t b = (size_t)max_groups(dp, N) * N * odd_ld(N) * sizeof(double);
-    if (N <= NTM_QUAD_MAX_N) {                             // the quad kernel keeps one N x N slab per resident quad
-        const size_t q = (size_t)quad_max_groups(dp) * N * N * sizeof(double);
-        if (q > b) b = q;
-    }
-    return b;
+    return (size_t)max_groups(dp, N) * N * odd_ld(N) * sizeof(double);
 }
 
 cudaError_t launch_rho(cudaStream_t st, int layout, int flags, int S, const double *x, const double *params, int pc,
@@ -1576,12 +1513,8 @@ size_t lpt_doubles(const DeviceProps &dp, const LoopArgs &a) {
     // (2.8 rounds of resident warps) it is a wash -- the eight 8,192-scenario shards of config 3 take 4.7-7.2 ms (mean 5.54)
     // as one launch and 4.7-7.0 ms (mean 5.39) in two phases: step 0 does not see the scenarios that turn slow later, and
     // one scenario that needs 2.6 ms ALONE bounds its shard either way.  So: from 2.5 rounds of resident warps.
-    static const char *env_min = getenv("NTM_LPT_MIN");            // diagnostic: another threshold (scenarios)
-    const long long smin = env_min ? atoll(env_min) : (long long)dp.sm_count * 20 * 5 / 2;
-    if ((long long)a.S < smin) return 0;
+    if ((long long)a.S < (long long)dp.sm_count * 20 * 5 / 2) return 0;
     if (a.S > (1 << 18)) return 0;                                 // 0.5 GB of saved state at most; beyond that the tail is < 1 %
-    static const bool quad = getenv("NTM_QUAD") != nullptr;
-    if (quad && a.N <= NTM_QUAD_MAX_N) return 0;
     return (size_t)a.S * NTM_CTRL_DOUBLES(a.N);
 }
 
@@ -1608,7 +1541,7 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
     size_t gbytes = work_bytes(a.N, aa.hcap, aa.gam);
     {
         static const char *env = getenv("NTM_ROWS_WARM");  // diagnostic: 0 = every state-row QP starts cold
-        aa.rows_warm = env ? atoi(env) : 1;
+        aa.rows_warm = (env == nullptr || atoi(env) != 0) ? 1 : 0;
     }
     int wpb1 = 4;                                          // warps (= scenarios) per CTA of the one-warp instantiations
     if (a.srows != 0) {
@@ -1640,14 +1573,7 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
         else { if (ext) NTM_LAUNCH_LOOP1(GWV, false, 1, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 0, BLOCK, SMEM, GPB); }         \
     } while (0)
 #define NTM_CTL_EXT 0, 0, true                             // EXT = 0, LV = 0, CTL: multi-warp controller-step instantiation
-    // Four lanes per scenario (ntm_quad.cuh) is an EXPERIMENT that lost: half the instructions of the one-warp kernel
-    // (741 against 1,510 per re-linearisation) but 255 registers and 3.4 KB of shared memory per scenario leave 8 warps
-    // per SM, whose mostly straight-line code stalls on instruction fetch (profiles/README.md, round 2): 53.9 ms
-    // against 27.0 ms on config 3.  It stays selectable (NTM_QUAD=1) and parity-tested; the default is the one-warp kernel.
-    static const bool use_quad = getenv("NTM_QUAD") != nullptr;
-    if (gw == 1 && !dense && ext != 2 && a.N <= NTM_QUAD_MAX_N && use_quad && !(a.flags & NTM_PROFILE_TAUE_W) && !a.ctl) {
-        return launch_closed_loop_quad(st, dp, aa, launches);
-    } else if (gw == 1) {
+    if (gw == 1) {
         const int wpb = wpb1;
         const size_t smem = gbytes * wpb;
         if (a.lpt != nullptr && a.sv != nullptr && lpt_doubles(dp, a) != 0) {
@@ -1897,21 +1823,17 @@ cudaError_t launch_hessian_grad(cudaStream_t st, const DeviceProps &dp, int layo
     cudaError_t e;
     if (N > 32) {                                            // FP64 tensor-core path
         const int Np = (N + 1 + 7) & ~7, nt = Np >> 3, nst = (nt + 1) >> 1, nsuper = nst * (nst + 1) / 2;
-        // 16 warps + double-buffered chunk, one CTA per SM: measured 2.22 ms against 1.89 ms for 8 warps, two CTAs per SM
-        // (N = 100, 16,384 scenarios) -- kept selectable for the record (NTM_HESS_W16=1), not the default
-        static const bool w16 = getenv("NTM_HESS_W16") != nullptr && atoi(getenv("NTM_HESS_W16")) != 0;
-        const int nbuf = w16 ? 2 : 1, warps = w16 ? 16 : 8;
-        const size_t smem_d = ((nbuf + 1) * (size_t)Np * NTM_DMMA_KC + 2 * (2 * N + 4)) * sizeof(double) + 2 * (size_t)nsuper + 16;
-        const int maxst = (nsuper + warps - 1) / warps;
-#define NTM_LAUNCH_HD(M, W, B)                                                                               \
+        // the raw chunk and its Omega image, two v buffers, the super-tile table
+        const size_t smem_d = (2 * (size_t)Np * NTM_DMMA_KC + 2 * (2 * N + 4)) * sizeof(double) + 2 * (size_t)nsuper + 16;
+        const int maxst = (nsuper + 7) / 8;                  // 8 warps per CTA
+#define NTM_LAUNCH_HD(M)                                                                                     \
     do {                                                                                                     \
-        e = persistent_geometry(hessian_grad_dmma_kernel<M, W, B>, dp, 32 * W, smem_d, S, 1, &grid);         \
+        e = persistent_geometry(hessian_grad_dmma_kernel<M>, dp, 256, smem_d, S, 1, &grid);                  \
         if (e != cudaSuccess) return e;                                                                      \
-        hessian_grad_dmma_kernel<M, W, B><<<grid, 32 * W, smem_d, st>>>(layout, S, N, Phi, Gam, Lam, x, params, pc, G, F); \
+        hessian_grad_dmma_kernel<M><<<grid, 256, smem_d, st>>>(layout, S, N, Phi, Gam, Lam, x, params, pc, G, F); \
     } while (0)
-        if (w16) { if (maxst <= 1) NTM_LAUNCH_HD(1, 16, 2); else if (maxst == 2) NTM_LAUNCH_HD(2, 16, 2); else NTM_LAUNCH_HD(3, 16, 2); }
-        else if (maxst <= 2) NTM_LAUNCH_HD(2, 8, 1); else if (maxst <= 4) NTM_LAUNCH_HD(4, 8, 1); else if (maxst == 5) NTM_LAUNCH_HD(5, 8, 1);
-        else NTM_LAUNCH_HD(6, 8, 1);
+        if (maxst <= 2) NTM_LAUNCH_HD(2); else if (maxst <= 4) NTM_LAUNCH_HD(4); else if (maxst == 5) NTM_LAUNCH_HD(5);
+        else NTM_LAUNCH_HD(6);
 #undef NTM_LAUNCH_HD
         ++*launches;
         return cudaGetLastError();
@@ -1925,15 +1847,13 @@ cudaError_t launch_hessian_grad(cudaStream_t st, const DeviceProps &dp, int layo
         (void)slice;
         const int wpb = 4;                                       // warps per CTA, each with a double-buffered slice
         const size_t smem_w = (size_t)wpb * 2 * ((size_t)Np * ld) * sizeof(double);
-        static const bool use_bulk = getenv("NTM_HESS_BULK") != nullptr;
         const int aligned = ((reinterpret_cast<uintptr_t>(Gam) | reinterpret_cast<uintptr_t>(G)) & 15) == 0;
-        const int vec_ok = aligned ? (use_bulk ? 3 : 1) : 0;     // bit 0: 16-byte pieces, bit 1: bulk copies (UBLKCP)
         const int NT = Np >> 3;
 #define NTM_LAUNCH_HW(T)                                                                                              \
     do {                                                                                                              \
         e = persistent_geometry(hessian_grad_dmma_warp_kernel<T>, dp, 32 * wpb, smem_w, S, wpb, &grid);               \
         if (e != cudaSuccess) return e;                                                                               \
-        hessian_grad_dmma_warp_kernel<T><<<grid, 32 * wpb, smem_w, st>>>(S, N, ld, Phi, Gam, Lam, x, params, pc, G, F, vec_ok); \
+        hessian_grad_dmma_warp_kernel<T><<<grid, 32 * wpb, smem_w, st>>>(S, N, ld, Phi, Gam, Lam, x, params, pc, G, F, aligned); \
     } while (0)
         if (NT == 1) NTM_LAUNCH_HW(1); else if (NT == 2) NTM_LAUNCH_HW(2); else if (NT == 3) NTM_LAUNCH_HW(3);
         else if (NT == 4) NTM_LAUNCH_HW(4); else NTM_LAUNCH_HW(5);

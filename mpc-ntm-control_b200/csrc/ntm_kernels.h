@@ -20,8 +20,8 @@ struct LoopArgs {
     int srows;
     double xmin1, xmax1, xmin2, xmax2;   // NTM_MPC_Sim.m:44-45
     unsigned int wbytes, qbytes;         // offsets of the IneqWork / ExtWork areas in a group's shared memory (launcher)
-    int rows_warm;                       // state-row QPs start from an earlier active set: bit 0 literal Gamma (default on),
-                                         // bit 1 dense Gamma (default off); set by the launcher, NTM_ROWS_WARM=<bits> overrides
+    int rows_warm;                       // 1: state-row QPs on the literal Gamma start from an earlier active set (the dense
+                                         // Gamma always starts cold); set by the launcher, NTM_ROWS_WARM=0 turns it off
     // packed-record output (the multi-GPU gather wants ONE contiguous block per scenario): when rec_ld > 0, xk / uk /
     // cost / rec_status point INTO one array of rec_ld doubles per scenario (scenario slowest) instead of three arrays
     int rec_ld;
@@ -89,10 +89,6 @@ cudaError_t launch_mc_stats(cudaStream_t st, const DeviceProps &dp, int layout, 
 cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches);
 // N > 32, literal Gamma, box QP (ntm_loop_long.cu); called by launch_closed_loop
 cudaError_t launch_closed_loop_long(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches);
-// N <= NTM_QUAD_MAX_N, literal Gamma, box QP: four lanes per scenario (ntm_loop_quad.cu); called by launch_closed_loop
-#define NTM_QUAD_MAX_N 24
-cudaError_t launch_closed_loop_quad(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches);
-inline int quad_max_groups(const DeviceProps &dp) { return dp.sm_count * 64; }   // resident quads (one global slab each)
 // raises cudaFuncAttributeMaxDynamicSharedMemorySize of a kernel to the device maximum, once per (kernel, device)
 cudaError_t raise_smem_attribute(const void *fn, int dev, size_t smem_optin);
 cudaError_t launch_fp64_peak(cudaStream_t st, const DeviceProps &dp, int iters, double *out, long long *launches);

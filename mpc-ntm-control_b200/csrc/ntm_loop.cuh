@@ -165,8 +165,9 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     [[maybe_unused]] bool rows_built = false;
     int hs1 = -1, hs2 = -1;
     bool first_qp = true;
-    // EXT == 2: active sets of the last two state-row QPs of this scenario, offered to the next one as a warm start
-    // (per thread: (vst + 1) | mask of this state's four rows << 2), and the "warm start failed, run this QP again cold" flag
+    // EXT == 2, literal Gamma: active sets of the last two state-row QPs of this scenario, offered to the next one as a
+    // warm start (per thread: (vst + 1) | mask of this state's four rows << 2), and the "warm start failed, run this QP
+    // again cold" flag
     [[maybe_unused]] int hw1 = 0, hw2 = 0, hwn = 0;
     [[maybe_unused]] bool retry = false;
     int status = 0, inner = 0, qpit = 0, k = 0, it = 0;
@@ -285,29 +286,15 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
         int nit = 0;
         int st = NTM_SCN_OK;
         if constexpr (DENSE) {
-            [[maybe_unused]] bool try_warm = false;       // state rows: warm start from an earlier active set (see the literal branch)
-            [[maybe_unused]] int wv = 0, wm = -1;
-            [[maybe_unused]] bool x0bad = false;
-            if constexpr (EXT == 2 && GW == 1) {
-                if (a.srows != 0) {
-                    x0bad = x1 < a.xmin1 || x1 > a.xmax1 || x2 < a.xmin2 || x2 > a.xmax2;   // getWLc.m:30
-                    // (a.rows_warm & 2: the warm start is OFF by default on this path -- on the consistent profile, whose
-                    // closed loop is chaotic at the 1e-4 level, one scenario of the parity sample moved by 2 % in one input)
-                    if ((a.rows_warm & 2) && !retry && hwn > 0 && !x0bad) {
-                        const int hh = (hwn >= 2) ? hw2 : hw1;
-                        wv = (hh & 3) - 1; wm = hh >> 2;
-                        try_warm = Gp::any(act && wm != 0, w.ired);
-                    }
-                    if (!try_warm) wm = -1;
-                }
-                retry = false;
-            }
-            if (!try_warm) st = qp_solve<GW>(N, j, w, Fj, P.umin, P.umax, hist, Uj, qp_cap, nit);   // :97
+            st = qp_solve<GW>(N, j, w, Fj, P.umin, P.umax, hist, Uj, qp_cap, nit);   // :97
             if constexpr (EXT == 2 && GW == 1) {
                 if (a.srows != 0) {
                     // NTM_MPC_Sim.m:97 as written, ANY Gamma index: the state rows of getWLc.m:57 (L = Mcal*Gamma + Ecal)
                     // are read from the dense Gamma tile the tensor-core Hessian build left in shared memory (DenseRows);
-                    // frozen rows (:74) keep a copy of the offline tile.  QP variables are U itself here.
+                    // frozen rows (:74) keep a copy of the offline tile.  QP variables are U itself here.  Every QP starts
+                    // cold from the box minimiser: the literal branch's warm start, tried here, moved one scenario of the
+                    // parity sample by 2 % in one input on the consistent profile (chaotic at the 1e-4 level).
+                    const bool x0bad = x1 < a.xmin1 || x1 > a.xmax1 || x2 < a.xmin2 || x2 > a.xmax2;   // getWLc.m:30
                     const IneqWork q = carve_ineq(gbase + a.wbytes, N, 4 * N);
                     const ExtWork xw = carve_ext(gbase + a.qbytes, N);
                     double *Gam0 = reinterpret_cast<double *>(gbase + a.qbytes + ext_bytes(N));
@@ -342,20 +329,10 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                         });
                         st = x0bad ? (int)NTM_SCN_INFEASIBLE
                                    : qp_ineq_continue<GW>(N, rows, j, w, q, Fj, P.umin, P.umax, Uc, nit + 100 * N + 50, nit,
-                                                          &vs, regen, wv, wm);
-                        if (st == NTM_QP_WARM_FAILED) { retry = true; continue; }   // this QP again, from the box minimiser
-                        if (try_warm || st != NTM_SCN_OK || nit != nit0) {
+                                                          &vs, regen);
+                        if (st != NTM_SCN_OK || nit != nit0) {
                             Uj = (vs < 0) ? P.umin : ((vs > 0) ? P.umax : fmin(fmax(Uc, P.umin), P.umax));
                             if (!(Uc == Uc)) Uj = Uc;
-                        }
-                        if (st == NTM_SCN_OK) {                        // remember the active set this QP ended on
-                            Gp::sync();
-                            int hnew = vs + 1;
-                            if (act) {
-#pragma unroll
-                                for (int qq = 0; qq < 4; ++qq) hnew |= (q.gact[4 * j + qq] ? 1 : 0) << (2 + qq);
-                            }
-                            hw2 = hw1; hw1 = hnew; hwn = min(hwn + 1, 2);
                         }
                     }
                 }

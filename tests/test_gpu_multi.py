@@ -159,31 +159,3 @@ def test_mex_batch_gateway_uses_every_gpu():
     # the pooled handles of the other devices have launched kernels
     from ntm_mpc import _lib
     assert _lib.load().ntm_pool_launch_count(nd - 1) > 0
-
-
-def test_four_lanes_per_scenario_experiment_stays_in_parity():
-    """ntm_quad.cuh (NTM_QUAD=1: four lanes per scenario, eight scenarios per warp) lost on speed and is off by default,
-    but it is compiled into the library: keep it honest against the C oracle (separate process: the switch is read once)."""
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = (
-        "import sys, numpy as np\n"
-        f"sys.path.insert(0, {root!r}); sys.path.insert(0, {os.path.join(root, 'mpc-ntm-control_b200')!r})\n"
-        "import ntm_mpc\nfrom ntm_mpc import physics\nfrom oracle import c_oracle, ntm_oracle as o\n"
-        "mpc = ntm_mpc.NtmMpc(0)\nworst = 0.0\n"
-        "for cfg, N, S, flags in ((3, 20, 513, 16), (4, 20, 257, 0), (2, 10, 129, 16), (3, 3, 33, 0), (3, 24, 65, 16), (3, 17, 65, 80)):\n"
-        "    phys, x0, _ = o.make_batch(cfg, S=S)\n"
-        "    P = physics.params_from_physics(phys).reshape(16, -1)\n"
-        "    g = mpc.closed_loop(x0, np.ascontiguousarray(P.T), N, 8, 10, 1e-14, flags)\n"
-        "    c = c_oracle.closed_loop_batch(phys, x0, N, 8, 10, 1e-14, flags & (31 | 64), 4)\n"
-        "    du = np.max(np.abs(g['uk'] - c['uk']) / np.broadcast_to(np.asarray(phys['umax'], dtype=float), (S,))[:, None])\n"
-        "    w = c['xk'][:, :, 0]\n"
-        "    dw = np.max(np.abs(g['xk'][:, :, 0] - w) / np.maximum(np.max(np.abs(w), axis=1, keepdims=True), 1e-3))\n"
-        "    assert g['status'].max() == 0 and np.mean(g['inner_iters'] == c['inner_iters']) > 0.99\n"
-        "    worst = max(worst, du, dw)\n"
-        "print('WORST', worst)\n")
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=dict(os.environ, NTM_QUAD="1"), timeout=600)
-    assert out.returncode == 0, out.stderr[-3000:]
-    worst = float(out.stdout.strip().split("WORST")[-1])
-    assert worst <= 1e-6, worst
