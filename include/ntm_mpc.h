@@ -225,9 +225,11 @@ int ntm_mpc_closed_loop_sc_dev(ntm_handle *h, int layout, int profile, int S, in
  *   [0, N)   a11   [N, 2N) a21   [2N, 3N) b      stage entries of the last re-scheduling (:114-117)
  *   [3N, 4N) Uold (:86,127, D13)                 [4N, 5N) and [5N, 6N): the last two QP solutions (warm starts)
  *   [6N, 7N) their partition states, (s1 + 1) + 4 (s2 + 1), s in {-1 lower, 0 free, +1 upper}
+ *            (ntm_mpc_step_sc, literal Gamma: + 16 hw1 + 1024 hw2, see there)
  *   [7N, 7N+2) the last state this controller saw: the state the G, F on hand were built from under NTM_PROFILE_F_XK
  *   [7N+2, 7N+4) x0 (G, F of the literal profile)   [7N+4] cost (two-phase fused loop only)
  *   [7N+5] status + 4 first_qp + 8 n (n = warm-start history length, 3 = sticky "a warm QP ran long")
+ *          (ntm_mpc_step_sc, literal Gamma: + 32 hwn, see there)
  *   [7N+6] steps this record has run (0 = fresh)
  * Preconditions (not checked by the kernel): every call for a record passes the same N, profile and params.
  * profile: every bit of the fused loop's box-QP instantiations (RHO1_SQ, GAMMA_I, DENSE_G, F_XK, INNER_FIXED); the
@@ -242,6 +244,28 @@ int ntm_mpc_step(ntm_handle *h, int layout, int profile, int S, int N, int i_sim
 int ntm_mpc_step_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
                      const double *params, int params_count, double *state, double *u, double *U, int *inner_iters,
                      int *qp_iters, int *status);
+
+/* ---- the same step with getWLc's state rows kept in every QP: the controller NTM_MPC_Sim.m:97 solves ------------- *
+ * ntm_mpc_step with state_rows and xbounds as in ntm_mpc_closed_loop_sc (xbounds on the HOST for both entries).
+ * NTM_STATE_ROWS_OFF is ntm_mpc_step: the same launch and the same bits.  Stepped with ntm_plant_step under the same
+ * profile, k_sim steps reproduce ntm_mpc_closed_loop_sc bit for bit, up to the step at which a scenario turns infeasible.
+ * Infeasible step (quadprog exitflag -2, :100-101): u and U are NaN, status = NTM_SCN_INFEASIBLE, inner_iters and
+ * qp_iters count that step as the fused loop does, and the record is NOT written: it still holds the controller as it
+ * was before the call.  The caller decides: zero the record to restart, or call again with a new measurement.
+ * Preconditions (not checked by the kernel): every call for a record passes the same N, profile, params, state_rows
+ * and xbounds.  Record words beyond ntm_mpc_step's (literal Gamma; zero on every other path, so NTM_CTRL_DOUBLES(N)
+ * is unchanged): the active sets of the last two state-row QPs, offered to the next QP as a warm start, per stage j
+ * hw = (v + 1) + 4 m with v the variable's bound state and bit q of m = row 4j + q active; [6N + j] carries
+ * 16 hw1 + 1024 hw2 and [7N+5] carries 32 hwn (hwn = how many of hw1, hw2 are valid, 0..2).  Frozen rows (:74) are
+ * not stored: each resumed step rebuilds them from rho(x0) with x0 from [7N+2, 7N+4), one extra G, F build.
+ * NTM_ERR_INVALID, nothing launched: NTM_PROFILE_TAUE_W, state_rows outside 0..2, NULL or inverted xbounds,
+ * GAMMA_I / DENSE_G with N > 32, a horizon whose factors do not fit shared memory. */
+int ntm_mpc_step_sc(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                    const double *params, int params_count, int state_rows, const double *xbounds, double *state,
+                    double *u, double *U, int *inner_iters, int *qp_iters, int *status);
+int ntm_mpc_step_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                        const double *params, int params_count, int state_rows, const double *xbounds, double *state,
+                        double *u, double *U, int *inner_iters, int *qp_iters, int *status);
 
 /* ---- the loop on EVERY visible GPU from ONE host process (what a MEX gateway can reach; SURVEY 8e) ------------- *
  * Replaces the same lines as ntm_mpc_closed_loop[_sc] (NTM_MPC_Sim.m:63-73,80-131); host pointers, same argument

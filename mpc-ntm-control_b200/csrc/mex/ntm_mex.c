@@ -15,7 +15,7 @@
  *   9   getWLc                   getWLc.m:1-63                 [W,L,c] = getWLc(xmax,xmin,umax,umin,Gamma,Phi,Lambda)
  *   10  quadprog                 quadprog call NTM_MPC_Sim.m:97 [U,fval,exitflag] = quadprog(H,f,A,b,[],[],lb,ub,x0,options)
  *                                (shadows the Optimization Toolbox function: input-box rows become bounds, state rows stay)
- *   11  ntm_mpc_step             one step NTM_MPC_Sim.m:94-128  [u,state,U,inner,status] = ntm_mpc_step(state,x,params,N,i_sim,eps,profile)
+ *   11  ntm_mpc_step             one step NTM_MPC_Sim.m:94-128  [u,state,U,inner,status] = ntm_mpc_step(state,x,params,N,i_sim,eps,profile[,state_rows,xmin,xmax])
  *                                (no plant: the script's `for k` loop keeps its own plant code and passes state back in)
  *
  * The short forms are the ones NTM_MPC_Sim.m actually uses (:63-66,:113-119,:130); the missing trailing arguments
@@ -357,17 +357,29 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         if (nlhs > 2) plhs[2] = mxCreateDoubleScalar(st == NTM_SCN_OK ? 1.0 : (st == NTM_SCN_QP_ITER_CAP ? 0.0 : (st == NTM_SCN_INFEASIBLE ? -2.0 : -3.0)));
     }
 #elif NTM_MEX_FN == 11
-    {   /* [u, state, U, inner, status] = ntm_mpc_step(state, x (2xS), params (16x1 | 16xS), N, i_sim, eps, profile)
+    {   /* [u, state, U, inner, status] = ntm_mpc_step(state, x (2xS), params (16x1 | 16xS), N, i_sim, eps, profile
+         *                                              [, state_rows, xmin (2x1), xmax (2x1)])
          * One receding-horizon step at the measured states x; state = [] starts S fresh controllers, otherwise it is the
          * NTM_CTRL_DOUBLES(N) x S record this gateway returned last time (zeroing a column restarts that scenario).
-         * Pass the same N, params and profile on every call for the same state. */
-        int S, N, i_sim, profile, pc, i;
-        double eps;
+         * state_rows / xmin / xmax as in ntm_mpc_batch (ntm_mpc_step_sc): an infeasible QP returns NaN u and U, status 3
+         * and the record as it was.  Pass the same N, params, profile, state_rows and bounds on every call for the same
+         * state. */
+        int S, N, i_sim, profile, pc, i, srows = 0;
+        double eps, xb[4] = {0.0, 0.0, 0.0, 0.0};
         size_t ld;
         mxArray *u, *st, *U, *inner, *status;
         int *ibuf;
-        if (nrhs != 7)
-            mexErrMsgIdAndTxt("ntm:arg", "usage: [u, state, U, inner, status] = ntm_mpc_step(state, x, params, N, i_sim, eps, profile)");
+        if (nrhs != 7 && nrhs != 10)
+            mexErrMsgIdAndTxt("ntm:arg", "usage: [u, state, U, inner, status] = ntm_mpc_step(state, x, params, N, i_sim, eps, profile [, state_rows, xmin, xmax])");
+        if (nrhs == 10) {
+            srows = (int)scalar_arg(nrhs, prhs, 7, "");
+            if (srows < 0 || srows > 2) mexErrMsgIdAndTxt("ntm:arg", "state_rows must be 0, 1 or 2");
+            if (!is_real_double(prhs[8]) || !is_real_double(prhs[9]) || mxGetNumberOfElements(prhs[8]) != 2 ||
+                mxGetNumberOfElements(prhs[9]) != 2)
+                mexErrMsgIdAndTxt("ntm:arg", "xmin and xmax must be real double 2-vectors");
+            xb[0] = mxGetPr(prhs[8])[0]; xb[1] = mxGetPr(prhs[9])[0]; xb[2] = mxGetPr(prhs[8])[1]; xb[3] = mxGetPr(prhs[9])[1];
+            if (!(xb[0] <= xb[1] && xb[2] <= xb[3])) mexErrMsgIdAndTxt("ntm:arg", "xmin must be <= xmax");
+        }
         S = states_arg(prhs[1]);
         if (!is_real_double(prhs[2]) || mxGetM(prhs[2]) != NTM_NPARAM || ((int)mxGetN(prhs[2]) != 1 && (int)mxGetN(prhs[2]) != S))
             mexErrMsgIdAndTxt("ntm:arg", "params must be 16 x 1 or 16 x S (see ntm_mpc.h)");
@@ -376,6 +388,8 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         eps = scalar_arg(nrhs, prhs, 5, ""); profile = (int)scalar_arg(nrhs, prhs, 6, "");
         if (N < 1 || N > NTM_MAX_HORIZON || i_sim < 1) mexErrMsgIdAndTxt("ntm:arg", "N in 1..128, i_sim >= 1");
         if (profile & NTM_PROFILE_TAUE_W) mexErrMsgIdAndTxt("ntm:arg", "NTM_PROFILE_TAUE_W (128) is not supported by ntm_mpc_step");
+        if (srows != 0 && (profile & (NTM_PROFILE_GAMMA_I | NTM_PROFILE_DENSE_G)) && N > 32)
+            mexErrMsgIdAndTxt("ntm:arg", "state rows with NTM_PROFILE_GAMMA_I / DENSE_G need N <= 32");
         ld = (size_t)NTM_CTRL_DOUBLES(N);
         if (!is_real_double(prhs[0]))
             mexErrMsgIdAndTxt("ntm:arg", "state must be [] or a real double matrix");
@@ -386,8 +400,8 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         u = mxCreateDoubleMatrix(1, S, mxREAL); U = mxCreateDoubleMatrix(N, S, mxREAL);
         inner = mxCreateDoubleMatrix(1, S, mxREAL); status = mxCreateDoubleMatrix(1, S, mxREAL);
         ibuf = (int *)mxMalloc(sizeof(int) * (2 * (size_t)S + 1));
-        check(ntm_mpc_step(handle(), NTM_LAYOUT_MATLAB, profile, S, N, i_sim, eps, mxGetPr(prhs[1]), mxGetPr(prhs[2]), pc,
-                           mxGetPr(st), mxGetPr(u), mxGetPr(U), ibuf, NULL, ibuf + S));
+        check(ntm_mpc_step_sc(handle(), NTM_LAYOUT_MATLAB, profile, S, N, i_sim, eps, mxGetPr(prhs[1]), mxGetPr(prhs[2]), pc,
+                              srows, xb, mxGetPr(st), mxGetPr(u), mxGetPr(U), ibuf, NULL, ibuf + S));
         for (i = 0; i < S; ++i) { mxGetPr(inner)[i] = (double)ibuf[i]; mxGetPr(status)[i] = (double)ibuf[S + i]; }
         mxFree(ibuf);
         plhs[0] = u;

@@ -519,21 +519,9 @@ static int check_loop(int N, int k_sim, int i_sim, const double *x0, double *xk,
     return NTM_OK;
 }
 
-static int closed_loop_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
-                                const double *x0, const double *params, int pc, int state_rows, const double *xb,
-                                double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
-                                int *status, int rec_ld = 0, double *rec_status = nullptr) {
-    TRY(check_common(h, layout, S));
-    if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    TRY(check_loop(N, k_sim, i_sim, x0, xk, uk));
+// state_rows / xbounds of ntm_mpc_closed_loop_sc and ntm_mpc_step_sc (N already checked) into a.srows and a.xmin1..xmax2
+static int set_state_rows(const ntm_handle *h, int profile, int N, int state_rows, const double *xb, ntm::LoopArgs &a) {
     REQUIRE(state_rows >= NTM_STATE_ROWS_OFF && state_rows <= NTM_STATE_ROWS_FROZEN, "unknown state_rows mode");
-    ntm::LoopArgs a = {};
-    a.layout = layout; a.flags = profile; a.S = S; a.N = N; a.k_sim = k_sim; a.i_sim = i_sim; a.eps = eps;
-    a.x0 = x0; a.params = params; a.params_count = pc;
-    a.xk = xk; a.uk = uk; a.Uk = Uk; a.cost = cost; a.inner = inner_iters; a.qpit = qp_iters; a.status = status;
-    a.counter = h->counter;
-    a.rec_ld = rec_ld; a.rec_status = rec_status;
     a.srows = state_rows;
     if (state_rows != NTM_STATE_ROWS_OFF) {
         REQUIRE(xb, "NULL state bounds");
@@ -550,6 +538,24 @@ static int closed_loop_dev_impl(ntm_handle *h, int layout, int profile, int S, i
             REQUIRE(need <= h->props.smem_optin, "horizon too long for the state rows in shared memory");
         }
     }
+    return NTM_OK;
+}
+
+static int closed_loop_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
+                                const double *x0, const double *params, int pc, int state_rows, const double *xb,
+                                double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
+                                int *status, int rec_ld = 0, double *rec_status = nullptr) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    TRY(check_loop(N, k_sim, i_sim, x0, xk, uk));
+    ntm::LoopArgs a = {};
+    a.layout = layout; a.flags = profile; a.S = S; a.N = N; a.k_sim = k_sim; a.i_sim = i_sim; a.eps = eps;
+    a.x0 = x0; a.params = params; a.params_count = pc;
+    a.xk = xk; a.uk = uk; a.Uk = Uk; a.cost = cost; a.inner = inner_iters; a.qpit = qp_iters; a.status = status;
+    a.counter = h->counter;
+    a.rec_ld = rec_ld; a.rec_status = rec_status;
+    TRY(set_state_rows(h, profile, N, state_rows, xb, a));
     TRY(ensure_hscratch(h, N));
     a.hscratch = h->hscratch;
     const size_t svd = ntm::lpt_doubles(h->props, a);      // two-phase launch with a longest-first queue (ntm_kernels.h)
@@ -729,15 +735,16 @@ static int check_step(int profile, int N, int i_sim) {
     return NTM_OK;
 }
 
-int ntm_mpc_step_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
-                     const double *params, int pc, double *state, double *u, double *U, int *inner_iters, int *qp_iters,
-                     int *status) {
+static int step_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                         const double *params, int pc, int state_rows, const double *xb, double *state, double *u,
+                         double *U, int *inner_iters, int *qp_iters, int *status) {
     TRY(check_common(h, layout, S));
     TRY(check_step(profile, N, i_sim));
+    ntm::LoopArgs a = {};
+    TRY(set_state_rows(h, profile, N, state_rows, xb, a));
     if (S == 0) return NTM_OK;
     TRY(check_params(params, pc, S));
     REQUIRE(x && state && u, "NULL array");
-    ntm::LoopArgs a = {};
     a.layout = layout; a.S = S; a.N = N; a.k_sim = 1; a.i_sim = i_sim; a.eps = eps;
     a.flags = profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4);   // plant-only bits: no effect on the controller
     a.x0 = x; a.params = params; a.params_count = pc;
@@ -750,11 +757,13 @@ int ntm_mpc_step_dev(ntm_handle *h, int layout, int profile, int S, int N, int i
     return NTM_OK;
 }
 
-int ntm_mpc_step(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
-                 const double *params, int pc, double *state, double *u, double *U, int *inner_iters, int *qp_iters,
-                 int *status) {
+static int step_host_impl(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                          const double *params, int pc, int state_rows, const double *xb, double *state, double *u,
+                          double *U, int *inner_iters, int *qp_iters, int *status) {
     TRY(check_common(h, layout, S));
     TRY(check_step(profile, N, i_sim));
+    ntm::LoopArgs rows = {};
+    TRY(set_state_rows(h, profile, N, state_rows, xb, rows));   // before any copy
     if (S == 0) return NTM_OK;
     TRY(check_params(params, pc, S));
     REQUIRE(x && state && u, "NULL array");
@@ -768,11 +777,39 @@ int ntm_mpc_step(ntm_handle *h, int layout, int profile, int S, int N, int i_sim
     double *du = A.take<double>(s), *dU = U ? A.take<double>(n * s) : nullptr;
     int *din = A.take<int>(s), *dqp = A.take<int>(s), *dstat = A.take<int>(s);
     TRY(h2d(h, dx, x, 2 * s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM)); TRY(h2d(h, dst, state, ld * s));
-    TRY(ntm_mpc_step_dev(h, layout, profile, S, N, i_sim, eps, dx, dp, pc, dst, du, dU, din, dqp, dstat));
+    TRY(step_dev_impl(h, layout, profile, S, N, i_sim, eps, dx, dp, pc, state_rows, xb, dst, du, dU, din, dqp, dstat));
     TRY(d2h(h, state, dst, ld * s)); TRY(d2h(h, u, du, s)); TRY(d2h(h, U, dU, n * s));
     TRY(d2h(h, inner_iters, din, s)); TRY(d2h(h, qp_iters, dqp, s)); TRY(d2h(h, status, dstat, s));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
+}
+
+int ntm_mpc_step_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                     const double *params, int pc, double *state, double *u, double *U, int *inner_iters, int *qp_iters,
+                     int *status) {
+    return step_dev_impl(h, layout, profile, S, N, i_sim, eps, x, params, pc, NTM_STATE_ROWS_OFF, nullptr, state, u, U,
+                         inner_iters, qp_iters, status);
+}
+
+int ntm_mpc_step(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                 const double *params, int pc, double *state, double *u, double *U, int *inner_iters, int *qp_iters,
+                 int *status) {
+    return step_host_impl(h, layout, profile, S, N, i_sim, eps, x, params, pc, NTM_STATE_ROWS_OFF, nullptr, state, u, U,
+                          inner_iters, qp_iters, status);
+}
+
+int ntm_mpc_step_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                        const double *params, int pc, int state_rows, const double *xbounds, double *state, double *u,
+                        double *U, int *inner_iters, int *qp_iters, int *status) {
+    return step_dev_impl(h, layout, profile, S, N, i_sim, eps, x, params, pc, state_rows, xbounds, state, u, U,
+                         inner_iters, qp_iters, status);
+}
+
+int ntm_mpc_step_sc(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                    const double *params, int pc, int state_rows, const double *xbounds, double *state, double *u,
+                    double *U, int *inner_iters, int *qp_iters, int *status) {
+    return step_host_impl(h, layout, profile, S, N, i_sim, eps, x, params, pc, state_rows, xbounds, state, u, U,
+                          inner_iters, qp_iters, status);
 }
 
 // ------------------------------------------------------------------------------------------------ getWLc

@@ -1568,11 +1568,13 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
     } while (0)
 #define NTM_LAUNCH_LOOP(GWV, BLOCK, SMEM, GPB)                                                              \
     do {                                                                                                    \
-        if (ext == 2) { if (dense) NTM_LAUNCH_LOOP1(GWV, true, 2, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 2, BLOCK, SMEM, GPB); } \
+        if (ext == 2 && a.ctl) { if (dense) NTM_LAUNCH_LOOP1(GWV, true, NTM_CTL_SC, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, NTM_CTL_SC, BLOCK, SMEM, GPB); } \
+        else if (ext == 2) { if (dense) NTM_LAUNCH_LOOP1(GWV, true, 2, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 2, BLOCK, SMEM, GPB); } \
         else if (dense) { if (ext) NTM_LAUNCH_LOOP1(GWV, true, 1, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, true, 0, BLOCK, SMEM, GPB); } \
         else { if (ext) NTM_LAUNCH_LOOP1(GWV, false, 1, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 0, BLOCK, SMEM, GPB); }         \
     } while (0)
 #define NTM_CTL_EXT 0, 0, true                             // EXT = 0, LV = 0, CTL: multi-warp controller-step instantiation
+#define NTM_CTL_SC 2, 0, true                              // EXT = 2, LV = 0, CTL: state-row controller-step instantiation
     if (gw == 1) {
         const int wpb = wpb1;
         const size_t smem = gbytes * wpb;
@@ -1594,12 +1596,14 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
         // long horizons, literal Gamma, box QP: the sweep-tableau instantiations live in ntm_loop_long.cu
         return launch_closed_loop_long(st, dp, aa, launches);
     } else if (gw == 2) {
-        if (ext == 2) NTM_LAUNCH_LOOP1(2, false, 2, 64, gbytes, 1);
+        if (ext == 2 && a.ctl) NTM_LAUNCH_LOOP1(2, false, NTM_CTL_SC, 64, gbytes, 1);   // controller step, state rows
+        else if (ext == 2) NTM_LAUNCH_LOOP1(2, false, 2, 64, gbytes, 1);
         else if (ext) NTM_LAUNCH_LOOP1(2, true, 1, 64, gbytes, 1);
         else if (a.ctl) NTM_LAUNCH_LOOP1(2, true, NTM_CTL_EXT, 64, gbytes, 1);   // controller step
         else NTM_LAUNCH_LOOP1(2, true, 0, 64, gbytes, 1);
     } else {
-        if (ext == 2) NTM_LAUNCH_LOOP1(4, false, 2, 128, gbytes, 1);
+        if (ext == 2 && a.ctl) NTM_LAUNCH_LOOP1(4, false, NTM_CTL_SC, 128, gbytes, 1);
+        else if (ext == 2) NTM_LAUNCH_LOOP1(4, false, 2, 128, gbytes, 1);
         else if (ext) NTM_LAUNCH_LOOP1(4, true, 1, 128, gbytes, 1);
         else if (a.ctl) NTM_LAUNCH_LOOP1(4, true, NTM_CTL_EXT, 128, gbytes, 1);
         else NTM_LAUNCH_LOOP1(4, true, 0, 128, gbytes, 1);
@@ -1607,6 +1611,7 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
 #undef NTM_LAUNCH_LOOP1
 #undef NTM_LAUNCH_LOOP
 #undef NTM_CTL_EXT
+#undef NTM_CTL_SC
     ++*launches;
     return cudaGetLastError();
 }

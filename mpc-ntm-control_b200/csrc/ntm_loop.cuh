@@ -106,9 +106,10 @@ struct LoopTraits {
 };
 
 // LV (LONG only): 0 = tableau in registers (N + 1 <= 7 * 10 / 7 * 15 for 2 / 4 warps), 1 = tableau in shared memory
-// CTL (multi-warp groups, EXT = 0): the controller-step instantiation (ntm_mpc_step).  The one-warp instantiations run
-// controller steps as a runtime mode (LoopArgs::ctl) at unchanged register counts; in the multi-warp ones that mode cost
-// 2 registers, and 228 bytes of spill stores in closed_loop_kernel<4, false, 0, 0> (DESIGN section 4.8).
+// CTL (multi-warp groups with EXT = 0, every group size with EXT = 2): the controller-step instantiation (ntm_mpc_step,
+// ntm_mpc_step_sc).  The one-warp box instantiations run controller steps as a runtime mode (LoopArgs::ctl) at unchanged
+// register counts; in the multi-warp ones that mode cost 2 registers, and 228 bytes of spill stores in
+// closed_loop_kernel<4, false, 0, 0>; the state-row ones sit at their register caps (DESIGN section 4.8).
 template <int GW, bool DENSE, int EXT, int LV = 0, bool CTL = false>
 __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename LoopTraits<GW, DENSE, EXT>::WorkT &w,
                              unsigned char *gbase, int tI = -1, int tJ = -1) {
@@ -122,9 +123,9 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     load_params_shared(w.prm, a.params, layout, a.params_count, s, j);
     Gp::sync();
     const Params &P = *w.prm;
-    // controller step (ntm_mpc_step): a.x0 is the measured state, the loop state comes from the caller's record
-    constexpr bool REC = (EXT == 0) && (GW == 1 || CTL);             // instantiations that carry the record code
-    const bool ctl = (GW == 1) ? (EXT == 0 && a.ctl != 0) : CTL;
+    // controller step (ntm_mpc_step[_sc]): a.x0 is the measured state, the loop state comes from the caller's record
+    constexpr bool REC = (EXT == 0 && (GW == 1 || CTL)) || (EXT == 2 && CTL);   // instantiations that carry the record code
+    const bool ctl = (GW == 1 && EXT == 0) ? (a.ctl != 0) : CTL;
     double x01 = __ldg(a.x0 + elem(layout, S, 2, s, 0)), x02 = __ldg(a.x0 + elem(layout, S, 2, s, 1));
     double x1 = x01, x2 = x02;
     // NTM_PROFILE_TAUE_W (EXT instantiations only): the shared parameter block carries the a22 the controller holds over
@@ -170,6 +171,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     // again cold" flag
     [[maybe_unused]] int hw1 = 0, hw2 = 0, hwn = 0;
     [[maybe_unused]] bool retry = false;
+    [[maybe_unused]] bool regen_rows = false;            // EXT == 2, CTL: rebuild the frozen rows of a resumed record first
     int status = 0, inner = 0, qpit = 0, k = 0, it = 0;
     const int qp_cap = 10 * N + 20;
     // two-phase launch (headline instantiation only): this launch runs the time steps [k_begin, k_end) of the scenario
@@ -192,12 +194,23 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                     hist.u1 = sv[4 * N + j]; hist.u2 = sv[5 * N + j]; hist.s1 = (pk & 3) - 1; hist.s2 = ((pk >> 2) & 3) - 1;
                 } else {
                     hU1 = sv[4 * N + j]; hU2 = sv[5 * N + j]; hs1 = (pk & 3) - 1; hs2 = ((pk >> 2) & 3) - 1;
+                    if constexpr (EXT == 2) { hw1 = (pk >> 4) & 63; hw2 = (pk >> 10) & 63; }
                 }
             }
             x1 = sv[N7]; x2 = sv[N7 + 1]; x01 = sv[N7 + 2]; x02 = sv[N7 + 3]; cost = sv[N7 + 4];
             const int fl = (int)sv[N7 + 5];
             status = ctl ? 0 : (fl & 3); first_qp = ((fl >> 2) & 1) != 0; hist.n = (fl >> 3) & 3;
             k = ctl ? 0 : a.k_begin;
+            if constexpr (EXT == 2) {
+                hwn = (fl >> 5) & 3;
+                // Frozen rows (:74) are a function of x0 alone and are not stored: the first pass of the loop builds
+                // G, F from rho(x0) on every stage, exactly as the offline build did, copies the rows out and then
+                // reloads the record's stage entries (below, after build_GF).
+                if (a.srows == 2) {
+                    regen_rows = true;
+                    schedule(P, flags, x01, x02, a11, a21, bb);
+                }
+            }
             Gp::sync();
             if (act) { w.bbs[j] = bb; if (GW > 1 || dense) { w.a11s[j] = a11; w.a21s[j] = a21; } }
             Gp::sync();
@@ -212,6 +225,32 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
         double Fj;
         if constexpr (LONG) Fj = build_GF_toeplitz_packed<GW>(N, j, w, P, fxk ? x1 : x01, fxk ? x2 : x02);
         else Fj = build_GF<GW, DENSE>(N, j, w, P, flags, a11, a21, sE, fxk ? x1 : x01, fxk ? x2 : x02);
+        if constexpr (EXT == 2 && CTL) {
+            if (regen_rows) {                            // the offline build of a resumed frozen record: keep its rows
+                const ExtWork xw = carve_ext(gbase + a.qbytes, N);
+                double pa, pc, k1, k2;
+                stage_prefix<GW>(N, j, w, P, a11, a21, pa, pc, s22, k1, k2);
+                if (act) {
+                    xw.Phi0[j] = make_double2(pa, pc); xw.Lam0[j] = make_double2(k1, k2);
+                    if constexpr (DENSE) {
+                        double *Gam0 = reinterpret_cast<double *>(gbase + a.qbytes + ext_bytes(N));
+                        const double2 *src = reinterpret_cast<const double2 *>(w.GamS + (size_t)j * w.ldgam);
+                        double2 *dst = reinterpret_cast<double2 *>(Gam0 + (size_t)j * w.ldgam);
+                        for (int i = 0; i < N; ++i) dst[i] = src[i];
+                    } else {
+                        xw.P0[j] = w.P12[j];
+                    }
+                }
+                b0 = bb;
+                rows_built = true; regen_rows = false;
+                const double *sv = a.sv + (size_t)s * NTM_CTRL_DOUBLES(N);
+                if (act) { a11 = sv[j]; a21 = sv[N + j]; bb = sv[2 * N + j]; }
+                Gp::sync();
+                if (act) { w.bbs[j] = bb; if (GW > 1 || dense) { w.a11s[j] = a11; w.a21s[j] = a21; } }
+                Gp::sync();
+                continue;                                // now G, F of the record's stage entries
+            }
+        }
         if (it > 0 && !retry) {
             inner = it;
             bool brk = false;
@@ -263,11 +302,18 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                         if (act) {
                             sv[j] = a11; sv[N + j] = a21; sv[2 * N + j] = bb; sv[3 * N + j] = Uold;
                             sv[4 * N + j] = dense ? hist.u1 : hU1; sv[5 * N + j] = dense ? hist.u2 : hU2;
-                            sv[6 * N + j] = dense ? (double)((hist.s1 + 1) | ((hist.s2 + 1) << 2)) : (double)((hs1 + 1) | ((hs2 + 1) << 2));
+                            if constexpr (EXT == 2)          // + the active sets of the last two state-row QPs (literal)
+                                sv[6 * N + j] = dense ? (double)((hist.s1 + 1) | ((hist.s2 + 1) << 2))
+                                                      : (double)((hs1 + 1) | ((hs2 + 1) << 2) | (hw1 << 4) | (hw2 << 10));
+                            else
+                                sv[6 * N + j] = dense ? (double)((hist.s1 + 1) | ((hist.s2 + 1) << 2)) : (double)((hs1 + 1) | ((hs2 + 1) << 2));
                         }
                         if (lead) {
                             sv[N7] = x1; sv[N7 + 1] = x2; sv[N7 + 2] = x01; sv[N7 + 3] = x02; sv[N7 + 4] = cost;
-                            sv[N7 + 5] = (double)((status & 3) | ((first_qp ? 1 : 0) << 2) | (hist.n << 3));
+                            if constexpr (EXT == 2)
+                                sv[N7 + 5] = (double)((status & 3) | ((first_qp ? 1 : 0) << 2) | (hist.n << 3) | (hwn << 5));
+                            else
+                                sv[N7 + 5] = (double)((status & 3) | ((first_qp ? 1 : 0) << 2) | (hist.n << 3));
                             sv[N7 + 6] = ctl ? sv[N7 + 6] + 1.0 : (double)k;
                             if constexpr (TWOPH) {
                                 if (!ctl) a.lpt_key[s] = min(12 * min(nslow, 12) + min(nqpit, 11), NTM_LPT_BINS - 1);
@@ -448,14 +494,17 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
         if constexpr (EXT == 2) {
             if (st == NTM_SCN_INFEASIBLE) {
                 // quadprog exitflag -2 (:100-101) returns no U and the script cannot continue: the scenario ends here,
-                // everything it has not produced yet is NaN
+                // everything it has not produced yet is NaN.  A controller step (k_sim = 1) returns NaN u and U and
+                // leaves its record as it was before the step: the save sits on the stop-rule path, not on this one.
                 const double nan = __longlong_as_double(0x7ff8000000000000LL);
                 status = max(status, st);
                 for (int kk = k; kk < a.k_sim; ++kk) {
                     if (lead) {
                         a.uk[uk_at(kk)] = nan;
-                        a.xk[xk_at(2 * (kk + 1))] = nan;
-                        a.xk[xk_at(2 * (kk + 1) + 1)] = nan;
+                        if (!ctl) {                      // a controller step has no xk
+                            a.xk[xk_at(2 * (kk + 1))] = nan;
+                            a.xk[xk_at(2 * (kk + 1) + 1)] = nan;
+                        }
                         if (a.inner) a.inner[elem(layout, S, a.k_sim, s, kk)] = (kk == k) ? it : 0;
                         if (a.qpit) a.qpit[elem(layout, S, a.k_sim, s, kk)] = (kk == k) ? qpit + nit : 0;
                     }

@@ -356,13 +356,17 @@ class NtmMpc:
 
     # ------------------------------------------------------------------ NTM_MPC_Sim.m:94-128, one step, no plant
     def mpc_step(self, state, x, params, N: int, i_sim: int = 10, eps: float = 1e-14, profile: int = 0,
-                 want_U: bool = False):
+                 want_U: bool = False, state_rows: int = 0, xbounds=None):
         """One receding-horizon step for S scenarios at their measured states ``x`` [S, 2] (``ntm_mpc_step``).
 
         ``state`` is a C-contiguous float64 array [S, ``ctrl_doubles(N)``] updated in place; an all-zero row is a fresh
         controller (its first step runs the offline build from ``x``), so ``state[s] = 0`` restarts scenario ``s``.
-        Pass the same N, profile and params on every call for the same records.  Returns a dict with ``u`` [S],
-        ``U`` [S, N] (None unless ``want_U``), ``inner_iters``, ``qp_iters`` and ``status`` [S]."""
+        Pass the same N, profile, params, state_rows and xbounds on every call for the same records.  Returns a dict
+        with ``u`` [S], ``U`` [S, N] (None unless ``want_U``), ``inner_iters``, ``qp_iters`` and ``status`` [S].
+
+        ``state_rows`` (``STATE_ROWS_REFRESH`` / ``STATE_ROWS_FROZEN``) keeps getWLc's state rows in every QP
+        (``ntm_mpc_step_sc``); ``xbounds = (xmin1, xmax1, xmin2, xmax2)``, default the script's own state box.  A
+        scenario whose QP is infeasible gets NaN ``u`` / ``U``, status 3, and its record row is left as it was."""
         x = _f64(x).reshape(-1, 2)
         S = x.shape[0]
         p, pc = self._params(params, S)
@@ -372,24 +376,37 @@ class NtmMpc:
         u = np.empty(S)
         U = np.empty((S, N)) if want_U else None
         inner, qpit, status = (np.empty(S, dtype=np.int32) for _ in range(3))
-        check(self._lib.ntm_mpc_step(self._h, LAYOUT_MATLAB, profile, S, N, i_sim, eps, _ptr(x), _ptr(p), pc, _ptr(state),
-                                     _ptr(u), _ptr(U), _ptr(inner), _ptr(qpit), _ptr(status)))
+        if state_rows:
+            xb = _f64(MC_STATE_BOX if xbounds is None else xbounds).reshape(4)
+            check(self._lib.ntm_mpc_step_sc(self._h, LAYOUT_MATLAB, profile, S, N, i_sim, eps, _ptr(x), _ptr(p), pc,
+                                            int(state_rows), _ptr(xb), _ptr(state), _ptr(u), _ptr(U), _ptr(inner),
+                                            _ptr(qpit), _ptr(status)))
+        else:
+            check(self._lib.ntm_mpc_step(self._h, LAYOUT_MATLAB, profile, S, N, i_sim, eps, _ptr(x), _ptr(p), pc,
+                                         _ptr(state), _ptr(u), _ptr(U), _ptr(inner), _ptr(qpit), _ptr(status)))
         return dict(u=u, U=U, inner_iters=inner, qp_iters=qpit, status=status)
 
     def mpc_step_dev(self, S: int, N: int, i_sim: int, eps: float, profile: int, layout: int, x_ptr: int,
                      params_ptr: int, params_count: int, state_ptr: int, u_ptr: int, U_ptr: int = 0, inner_ptr: int = 0,
-                     qp_ptr: int = 0, status_ptr: int = 0) -> None:
-        """``mpc_step`` on device pointers, asynchronous on the handle's stream (``ntm_mpc_step_dev``); the records
-        (``ctrl_doubles(N)`` doubles per scenario, scenario slowest) stay resident."""
+                     qp_ptr: int = 0, status_ptr: int = 0, state_rows: int = 0, xbounds=None) -> None:
+        """``mpc_step`` on device pointers, asynchronous on the handle's stream (``ntm_mpc_step_dev``, or
+        ``ntm_mpc_step_sc_dev`` with ``state_rows``; ``xbounds`` is a host 4-vector); the records (``ctrl_doubles(N)``
+        doubles per scenario, scenario slowest) stay resident."""
+        if state_rows:
+            xb = _f64(MC_STATE_BOX if xbounds is None else xbounds).reshape(4)
+            check(self._lib.ntm_mpc_step_sc_dev(self._h, layout, profile, S, N, i_sim, eps, x_ptr, params_ptr,
+                                                params_count, int(state_rows), _ptr(xb), state_ptr, u_ptr, U_ptr or None,
+                                                inner_ptr or None, qp_ptr or None, status_ptr or None))
+            return
         check(self._lib.ntm_mpc_step_dev(self._h, layout, profile, S, N, i_sim, eps, x_ptr, params_ptr, params_count,
                                          state_ptr, u_ptr, U_ptr or None, inner_ptr or None, qp_ptr or None,
                                          status_ptr or None))
 
     def controller(self, params, N: int, S: Optional[int] = None, i_sim: int = 10, eps: float = 1e-14,
-                   profile: int = 0) -> "Controller":
+                   profile: int = 0, state_rows: int = 0, xbounds=None) -> "Controller":
         """A ``Controller`` on this handle that owns the records of S scenarios (S from ``params`` [S, NPARAM], or given
-        with one shared [NPARAM] block)."""
-        return Controller(self, params, N, S, i_sim, eps, profile)
+        with one shared [NPARAM] block); ``state_rows`` / ``xbounds`` as in ``mpc_step``."""
+        return Controller(self, params, N, S, i_sim, eps, profile, state_rows, xbounds)
 
     # ------------------------------------------------------------------ Monte-Carlo back end (SURVEY 8f-3)
     def mc_stats(self, xk, uk, cost, status, params, bounds=MC_STATE_BOX, w_suppressed: float = 0.06, hist_max: float = 0.2):
@@ -442,7 +459,7 @@ class Controller:
     repeat.  ``reset(mask)`` restarts the selected scenarios: their next step is a first step from the state it gets."""
 
     def __init__(self, mpc: NtmMpc, params, N: int, S: Optional[int] = None, i_sim: int = 10, eps: float = 1e-14,
-                 profile: int = 0):
+                 profile: int = 0, state_rows: int = 0, xbounds=None):
         p = _f64(params)
         if S is None:
             if p.ndim != 2:
@@ -450,12 +467,14 @@ class Controller:
             S = p.shape[0]
         self.mpc, self.N, self.S, self.i_sim, self.eps, self.profile = mpc, int(N), int(S), int(i_sim), float(eps), int(profile)
         self.params, _ = NtmMpc._params(p, self.S)
+        self.state_rows, self.xbounds = int(state_rows), xbounds
         self.state = np.zeros((self.S, ctrl_doubles(self.N)))
         self.last = None
 
     def step(self, x, want_U: bool = False) -> np.ndarray:
         """u [S] for the measured states ``x`` [S, 2]; the full result dict of ``mpc_step`` is kept in ``last``."""
-        self.last = self.mpc.mpc_step(self.state, x, self.params, self.N, self.i_sim, self.eps, self.profile, want_U)
+        self.last = self.mpc.mpc_step(self.state, x, self.params, self.N, self.i_sim, self.eps, self.profile, want_U,
+                                      self.state_rows, self.xbounds)
         return self.last["u"]
 
     def reset(self, mask=None) -> None:
