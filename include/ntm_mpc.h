@@ -267,6 +267,34 @@ int ntm_mpc_step_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, in
                         const double *params, int params_count, int state_rows, const double *xbounds, double *state,
                         double *u, double *U, int *inner_iters, int *qp_iters, int *status);
 
+/* ---- the fused loop against a perturbed plant: the nominal controller, a plant it does not know exactly ---------- *
+ * For k = 0 .. k_sim-1, with y_k the state the controller sees:
+ *   y_k = x_k + v_k                          (measurement noise; v NULL: y_k = x_k)
+ *   u_k, U_k = one ntm_mpc_step of the controller (profile, params, its own record) at y_k
+ *   x_{k+1} = ntm_plant_step(x_k, u_k; plant_params, plant_profile) + d_k   (process disturbance; w NULL: none)
+ * bit for bit, in ONE launch on the handle's stream.  xk(:,0) = x0 is the true initial state; the controller's offline
+ * build (:63-73) runs from y_0.  xk holds the TRUE states, cost sums (x-r)'Q(x-r) over the true states k = 1..k_sim with
+ * r and Q from the controller's block, status is the worst over the run (NTM_SCN_NONFINITE for a non-finite y, u or x).
+ * Outputs as in ntm_mpc_closed_loop.  w (the disturbances d_k) and v: 2*k_sim doubles per scenario in `layout`, element
+ * 2k + i, or NULL.  plant_params: NTM_NPARAM doubles per block in `layout`, plant_params_count 1 or S; NULL = params.
+ * profile: what ntm_mpc_step takes (PLANT_C and PLANT_RK4 are ignored, TAUE_W is rejected).  plant_profile: exactly the
+ * bits ntm_plant_step honours, RHO1_SQ | PLANT_C | PLANT_RK4 | TAUE_W (c_tauE from plant_params[15]).  With
+ * plant_params = params, plant_profile = the plant bits of profile and w = v = NULL, every output is bit-identical to
+ * ntm_mpc_closed_loop.  Box QP only: getWLc's state rows under a perturbed plant are not offered (ntm_mpc_step_sc +
+ * ntm_plant_step cover them), nor is a controller-side tau_E(w).
+ * NTM_ERR_INVALID, nothing copied or launched: bad sizes, NULL x0 / xk / uk / params, plant_params_count not 1 or S,
+ * a controller profile with TAUE_W, a plant_profile bit outside the four above. */
+int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
+                                  const double *x0, const double *params, int params_count, const double *plant_params,
+                                  int plant_params_count, int plant_profile, const double *w, const double *v,
+                                  double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
+                                  int *status);
+int ntm_mpc_closed_loop_perturbed_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
+                                      double eps, const double *x0, const double *params, int params_count,
+                                      const double *plant_params, int plant_params_count, int plant_profile,
+                                      const double *w, const double *v, double *xk, double *uk, double *Uk,
+                                      double *cost, int *inner_iters, int *qp_iters, int *status);
+
 /* ---- the loop on EVERY visible GPU from ONE host process (what a MEX gateway can reach; SURVEY 8e) ------------- *
  * Replaces the same lines as ntm_mpc_closed_loop[_sc] (NTM_MPC_Sim.m:63-73,80-131); host pointers, same argument
  * meaning, no handle: the library keeps one pooled handle per device.  Scenarios never interact (:93-131 has no

@@ -17,6 +17,7 @@
  *                                (shadows the Optimization Toolbox function: input-box rows become bounds, state rows stay)
  *   11  ntm_mpc_step             one step NTM_MPC_Sim.m:94-128  [u,state,U,inner,status] = ntm_mpc_step(state,x,params,N,i_sim,eps,profile[,state_rows,xmin,xmax])
  *                                (no plant: the script's `for k` loop keeps its own plant code and passes state back in)
+ *   12  ntm_mpc_batch_perturbed  the loop vs a perturbed plant  [xk,uk,cost,inner,status] = ntm_mpc_batch_perturbed(x0,params,N,k_sim,i_sim,eps,profile,plant_params,plant_profile,w,v)
  *
  * The short forms are the ones NTM_MPC_Sim.m actually uses (:63-66,:113-119,:130); the missing trailing arguments
  * are fetched from the caller's workspace under the script's own variable names (kappa :24, tau_r :9, Ts :31,
@@ -34,7 +35,7 @@
 #include "ntm_mpc.h"
 
 #ifndef NTM_MEX_FN
-#error "compile with -DNTM_MEX_FN=<1..11>"
+#error "compile with -DNTM_MEX_FN=<1..12>"
 #endif
 
 static ntm_handle *g_h = NULL;
@@ -407,6 +408,58 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         plhs[0] = u;
         if (nlhs > 1) plhs[1] = st; else mxDestroyArray(st);
         if (nlhs > 2) plhs[2] = U; else mxDestroyArray(U);
+        if (nlhs > 3) plhs[3] = inner; else mxDestroyArray(inner);
+        if (nlhs > 4) plhs[4] = status; else mxDestroyArray(status);
+    }
+#elif NTM_MEX_FN == 12
+    {   /* [xk, uk, cost, inner, status] = ntm_mpc_batch_perturbed(x0 (2xS), params (16x1 | 16xS), N, k_sim, i_sim, eps,
+         *                                                           profile, plant_params, plant_profile, w, v)
+         * The fused loop against a perturbed plant (ntm_mpc_closed_loop_perturbed), one device: the controller of
+         * ntm_mpc_batch sees y_k = x_k + v_k; the plant runs on plant_params (16x1 | 16xS, [] = params) under
+         * plant_profile, plus the disturbance w_k.  w, v: 2 x k_sim x S (or 2k_sim x S), [] = none.  xk holds the
+         * true states. */
+        int S, N, k_sim, i_sim, profile, pprofile, pc, ppc, i;
+        double eps;
+        const double *pp = NULL, *w = NULL, *v = NULL;
+        mxArray *xk, *uk, *cost, *inner, *status;
+        int *ibuf;
+        if (nrhs != 11)
+            mexErrMsgIdAndTxt("ntm:arg", "usage: [xk,uk,cost,inner,status] = ntm_mpc_batch_perturbed(x0, params, N, k_sim, i_sim, eps, profile, plant_params, plant_profile, w, v)");
+        S = states_arg(prhs[0]);
+        if (!is_real_double(prhs[1]) || mxGetM(prhs[1]) != NTM_NPARAM || ((int)mxGetN(prhs[1]) != 1 && (int)mxGetN(prhs[1]) != S))
+            mexErrMsgIdAndTxt("ntm:arg", "params must be 16 x 1 or 16 x S (see ntm_mpc.h)");
+        pc = (int)mxGetN(prhs[1]);
+        N = (int)scalar_arg(nrhs, prhs, 2, ""); k_sim = (int)scalar_arg(nrhs, prhs, 3, ""); i_sim = (int)scalar_arg(nrhs, prhs, 4, "");
+        eps = scalar_arg(nrhs, prhs, 5, ""); profile = (int)scalar_arg(nrhs, prhs, 6, "");
+        pprofile = (int)scalar_arg(nrhs, prhs, 8, "");
+        if (N < 1 || N > NTM_MAX_HORIZON || k_sim < 0 || i_sim < 1) mexErrMsgIdAndTxt("ntm:arg", "N in 1..128, k_sim >= 0, i_sim >= 1");
+        if (profile & NTM_PROFILE_TAUE_W) mexErrMsgIdAndTxt("ntm:arg", "NTM_PROFILE_TAUE_W (128) is not supported on the controller side");
+        if (pprofile & ~(NTM_PROFILE_RHO1_SQ | NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W))
+            mexErrMsgIdAndTxt("ntm:arg", "plant_profile: only RHO1_SQ, PLANT_C, PLANT_RK4 and TAUE_W (1, 8, 64, 128) act on the plant");
+        ppc = pc;
+        if (mxGetNumberOfElements(prhs[7]) != 0) {
+            if (!is_real_double(prhs[7]) || mxGetM(prhs[7]) != NTM_NPARAM || ((int)mxGetN(prhs[7]) != 1 && (int)mxGetN(prhs[7]) != S))
+                mexErrMsgIdAndTxt("ntm:arg", "plant_params must be [], 16 x 1 or 16 x S");
+            pp = mxGetPr(prhs[7]); ppc = (int)mxGetN(prhs[7]);
+        }
+        for (i = 9; i <= 10; ++i) {
+            if (mxGetNumberOfElements(prhs[i]) == 0) continue;
+            if (!is_real_double(prhs[i]) || mxGetNumberOfElements(prhs[i]) != 2 * (size_t)k_sim * S)
+                mexErrMsgIdAndTxt("ntm:arg", "w and v must be [] or real doubles of 2 x k_sim x S");
+            if (i == 9) w = mxGetPr(prhs[i]); else v = mxGetPr(prhs[i]);
+        }
+        xk = mxCreateDoubleMatrix(2 * (k_sim + 1), S, mxREAL); uk = mxCreateDoubleMatrix(k_sim, S, mxREAL);
+        cost = mxCreateDoubleMatrix(1, S, mxREAL); inner = mxCreateDoubleMatrix(k_sim, S, mxREAL); status = mxCreateDoubleMatrix(1, S, mxREAL);
+        ibuf = (int *)mxMalloc(sizeof(int) * ((size_t)k_sim * S + S + 1));
+        check(ntm_mpc_closed_loop_perturbed(handle(), NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, mxGetPr(prhs[0]),
+                                            mxGetPr(prhs[1]), pc, pp, ppc, pprofile, w, v, mxGetPr(xk), mxGetPr(uk), NULL,
+                                            mxGetPr(cost), ibuf, NULL, ibuf + (size_t)k_sim * S));
+        for (i = 0; i < k_sim * S; ++i) mxGetPr(inner)[i] = (double)ibuf[i];
+        for (i = 0; i < S; ++i) mxGetPr(status)[i] = (double)ibuf[(size_t)k_sim * S + i];
+        mxFree(ibuf);
+        plhs[0] = xk;
+        if (nlhs > 1) plhs[1] = uk; else mxDestroyArray(uk);
+        if (nlhs > 2) plhs[2] = cost; else mxDestroyArray(cost);
         if (nlhs > 3) plhs[3] = inner; else mxDestroyArray(inner);
         if (nlhs > 4) plhs[4] = status; else mxDestroyArray(status);
     }

@@ -812,6 +812,81 @@ int ntm_mpc_step_sc(ntm_handle *h, int layout, int profile, int S, int N, int i_
                           inner_iters, qp_iters, status);
 }
 
+// ------------------------------------------------------------------------------------------------ perturbed plant
+// The fused loop with the plant of ntm_plant_step on its own block and profile bits, d_k and v_k (EXT = 3, ONE launch).
+static int check_perturbed(int profile, int S, int N, int k_sim, int i_sim, const double *x0, const double *params,
+                           int pc, int ppc, int plant_profile, double *xk, double *uk) {
+    TRY(check_step(profile, N, i_sim));
+    TRY(check_params(params, pc, S));
+    TRY(check_loop(N, k_sim, i_sim, x0, xk, uk));
+    REQUIRE(ppc == 1 || ppc == S, "plant_params_count must be 1 or S");
+    REQUIRE(!(plant_profile & ~(NTM_PROFILE_RHO1_SQ | NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)),
+            "plant_profile: only RHO1_SQ, PLANT_C, PLANT_RK4 and TAUE_W act on the plant");
+    return NTM_OK;
+}
+
+int ntm_mpc_closed_loop_perturbed_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
+                                      double eps, const double *x0, const double *params, int pc,
+                                      const double *plant_params, int ppc, int plant_profile, const double *w,
+                                      const double *v, double *xk, double *uk, double *Uk, double *cost,
+                                      int *inner_iters, int *qp_iters, int *status) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    if (plant_params == nullptr) { plant_params = params; ppc = pc; }
+    TRY(check_perturbed(profile, S, N, k_sim, i_sim, x0, params, pc, ppc, plant_profile, xk, uk));
+    ntm::LoopArgs a = {};
+    a.layout = layout; a.S = S; a.N = N; a.k_sim = k_sim; a.i_sim = i_sim; a.eps = eps;
+    a.flags = profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4);   // plant-only bits: no effect on the controller
+    a.x0 = x0; a.params = params; a.params_count = pc;
+    a.xk = xk; a.uk = uk; a.Uk = Uk; a.cost = cost; a.inner = inner_iters; a.qpit = qp_iters; a.status = status;
+    a.counter = h->counter;
+    a.pert = 1; a.pp.pparams = plant_params; a.pp.pparams_count = ppc; a.pp.pflags = plant_profile;
+    a.pp.dist = w; a.pp.noise = v;
+    TRY(ensure_hscratch(h, N));
+    a.hscratch = h->hscratch;
+    CU(ntm::launch_closed_loop(h->stream, h->props, a, &h->launches));
+    return NTM_OK;
+}
+
+int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
+                                  double eps, const double *x0, const double *params, int pc,
+                                  const double *plant_params, int ppc, int plant_profile, const double *w,
+                                  const double *v, double *xk, double *uk, double *Uk, double *cost, int *inner_iters,
+                                  int *qp_iters, int *status) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    if (plant_params == nullptr) ppc = pc;
+    TRY(check_perturbed(profile, S, N, k_sim, i_sim, x0, params, pc, ppc, plant_profile, xk, uk));
+    const size_t s = (size_t)S, n = (size_t)N, ks = (size_t)k_sim;
+    Arena A(h);
+    A.want(2 * s * 8); A.want((size_t)pc * NTM_NPARAM * 8);
+    if (plant_params) A.want((size_t)ppc * NTM_NPARAM * 8);
+    if (w) A.want(2 * ks * s * 8);
+    if (v) A.want(2 * ks * s * 8);
+    A.want(2 * (ks + 1) * s * 8); A.want(ks * s * 8);
+    if (Uk) A.want(n * ks * s * 8);
+    A.want(s * 8); A.want(ks * s * 4); A.want(ks * s * 4); A.want(s * 4);
+    TRY(A.reserve());
+    double *dx0 = A.take<double>(2 * s), *dp = A.take<double>((size_t)pc * NTM_NPARAM);
+    double *dpp = plant_params ? A.take<double>((size_t)ppc * NTM_NPARAM) : nullptr;
+    double *dw = w ? A.take<double>(2 * ks * s) : nullptr, *dv = v ? A.take<double>(2 * ks * s) : nullptr;
+    double *dxk = A.take<double>(2 * (ks + 1) * s), *duk = A.take<double>(ks * s);
+    double *dUk = Uk ? A.take<double>(n * ks * s) : nullptr;
+    double *dcost = A.take<double>(s);
+    int *din = A.take<int>(ks * s), *dqp = A.take<int>(ks * s), *dst = A.take<int>(s);
+    TRY(h2d(h, dx0, x0, 2 * s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
+    if (dpp) TRY(h2d(h, dpp, plant_params, (size_t)ppc * NTM_NPARAM));
+    if (dw) TRY(h2d(h, dw, w, 2 * ks * s));
+    if (dv) TRY(h2d(h, dv, v, 2 * ks * s));
+    TRY(ntm_mpc_closed_loop_perturbed_dev(h, layout, profile, S, N, k_sim, i_sim, eps, dx0, dp, pc, dpp, ppc,
+                                          plant_profile, dw, dv, dxk, duk, dUk, dcost, din, dqp, dst));
+    TRY(d2h(h, xk, dxk, 2 * (ks + 1) * s)); TRY(d2h(h, uk, duk, ks * s)); TRY(d2h(h, Uk, dUk, n * ks * s));
+    TRY(d2h(h, cost, dcost, s)); TRY(d2h(h, inner_iters, din, ks * s)); TRY(d2h(h, qp_iters, dqp, ks * s));
+    TRY(d2h(h, status, dst, s));
+    CU(cudaStreamSynchronize(h->stream));
+    return NTM_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ getWLc
 int ntm_getWLc_dev(ntm_handle *h, int layout, int S, int N, const double *bounds, const double *Gamma, const double *Phi,
                    const double *Lambda, double *W, double *L, double *c) {

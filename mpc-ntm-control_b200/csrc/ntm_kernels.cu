@@ -64,7 +64,7 @@ plant_kernel(int layout, int flags, int S, const double *__restrict__ x, const d
     if constexpr (RK4) {                                 // the cold options: RK4 and / or tau_E(w)
         const double ctau = (flags & NTM_PROFILE_TAUE_W)
                                 ? __ldg(params + elem(layout, pc == 1 ? 1 : pc, NTM_NPARAM, pc == 1 ? 0 : s, 15)) : 0.0;
-        plant_of(P, flags, P.a22, ctau, w, om, u[s], nw, nom);
+        plant_exact(P, flags, P.a22, ctau, w, om, u[s], nw, nom);   // the fused loop's rounding (ntm_loop.cuh)
     } else plant_euler(P, flags, w, om, u[s], nw, nom);
     xn[elem(layout, S, 2, s, 0)] = nw;
     xn[elem(layout, S, 2, s, 1)] = nom;
@@ -1536,8 +1536,8 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
     }
     aa.hcap = hcap_loop(dp, a.N, aa.gam);
     // EXT = the instantiation that also carries the cold options (RK4 plant, state rows); the headline kernels carry
-    // none of that code
-    const int ext = a.srows != 0 ? 2 : ((a.flags & (NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)) ? 1 : 0);
+    // none of that code; EXT = 3 (perturbed plant, box QP) has its own instantiations
+    const int ext = a.pert ? 3 : (a.srows != 0 ? 2 : ((a.flags & (NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)) ? 1 : 0));
     size_t gbytes = work_bytes(a.N, aa.hcap, aa.gam);
     {
         static const char *env = getenv("NTM_ROWS_WARM");  // diagnostic: 0 = every state-row QP starts cold
@@ -1570,6 +1570,7 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
     do {                                                                                                    \
         if (ext == 2 && a.ctl) { if (dense) NTM_LAUNCH_LOOP1(GWV, true, NTM_CTL_SC, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, NTM_CTL_SC, BLOCK, SMEM, GPB); } \
         else if (ext == 2) { if (dense) NTM_LAUNCH_LOOP1(GWV, true, 2, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 2, BLOCK, SMEM, GPB); } \
+        else if (ext == 3) { if (dense) NTM_LAUNCH_LOOP1(GWV, true, 3, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 3, BLOCK, SMEM, GPB); } \
         else if (dense) { if (ext) NTM_LAUNCH_LOOP1(GWV, true, 1, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, true, 0, BLOCK, SMEM, GPB); } \
         else { if (ext) NTM_LAUNCH_LOOP1(GWV, false, 1, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 0, BLOCK, SMEM, GPB); }         \
     } while (0)
@@ -1598,12 +1599,14 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
     } else if (gw == 2) {
         if (ext == 2 && a.ctl) NTM_LAUNCH_LOOP1(2, false, NTM_CTL_SC, 64, gbytes, 1);   // controller step, state rows
         else if (ext == 2) NTM_LAUNCH_LOOP1(2, false, 2, 64, gbytes, 1);
+        else if (ext == 3) NTM_LAUNCH_LOOP1(2, true, 3, 64, gbytes, 1);      // perturbed plant
         else if (ext) NTM_LAUNCH_LOOP1(2, true, 1, 64, gbytes, 1);
         else if (a.ctl) NTM_LAUNCH_LOOP1(2, true, NTM_CTL_EXT, 64, gbytes, 1);   // controller step
         else NTM_LAUNCH_LOOP1(2, true, 0, 64, gbytes, 1);
     } else {
         if (ext == 2 && a.ctl) NTM_LAUNCH_LOOP1(4, false, NTM_CTL_SC, 128, gbytes, 1);
         else if (ext == 2) NTM_LAUNCH_LOOP1(4, false, 2, 128, gbytes, 1);
+        else if (ext == 3) NTM_LAUNCH_LOOP1(4, true, 3, 128, gbytes, 1);      // perturbed plant
         else if (ext) NTM_LAUNCH_LOOP1(4, true, 1, 128, gbytes, 1);
         else if (a.ctl) NTM_LAUNCH_LOOP1(4, true, NTM_CTL_EXT, 128, gbytes, 1);
         else NTM_LAUNCH_LOOP1(4, true, 0, 128, gbytes, 1);

@@ -18,7 +18,15 @@ struct LoopArgs {
     // state rows of getWLc.m inside the loop (SURVEY 8f-1): 0 = dropped (box QP), 1 = rebuilt from every
     // re-condensation, 2 = frozen at the offline build as NTM_MPC_Sim.m:74 literally does
     int srows;
-    double xmin1, xmax1, xmin2, xmax2;   // NTM_MPC_Sim.m:44-45
+    // The state box of the state rows (EXT = 2) and the perturbed plant's inputs (EXT = 3) share their bytes: no
+    // instantiation reads both, and LoopArgs keeps its size (the kernels' parameter offsets, and so their SASS).
+    union {
+        struct { double xmin1, xmax1, xmin2, xmax2; };   // NTM_MPC_Sim.m:44-45
+        // perturbed plant: the plant runs on its own parameter block (pparams_count 1 or S, `layout`) and profile bits
+        // pflags; the controller sees x_k + v_k, the plant adds d_k after its step.  dist (d) / noise (v): 2 * k_sim
+        // doubles per scenario in `layout`, element 2k + i (NULL = none)
+        struct { const double *pparams, *dist, *noise; int pparams_count, pflags; } pp;
+    };
     unsigned int wbytes, qbytes;         // offsets of the IneqWork / ExtWork areas in a group's shared memory (launcher)
     int rows_warm;                       // 1: state-row QPs on the literal Gamma start from an earlier active set (the dense
                                          // Gamma always starts cold); set by the launcher, NTM_ROWS_WARM=0 turns it off
@@ -40,7 +48,9 @@ struct LoopArgs {
     // controller step (ntm_mpc_step, EXT = 0 instantiations only): k_sim = 1, x0 is the measured state, sv holds the
     // caller's records (read at the start, written at the stop rule), no plant; xk and cost are NULL
     int ctl;
+    int pert;                            // 1: perturbed plant (ntm_mpc_closed_loop_perturbed, EXT = 3, see `pp` above)
 };
+static_assert(sizeof(LoopArgs) == 248, "LoopArgs is the fused kernels' parameter block: its size fixes their SASS");
 #define NTM_LPT_BINS 160
 
 struct DeviceProps {

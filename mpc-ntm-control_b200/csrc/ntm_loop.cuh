@@ -62,6 +62,48 @@ __device__ __forceinline__ void plant_of(const Params &P, int flags, double a22n
     nom = om + (so + ao) / 6.0;
 }
 
+// The plant of ntm_plant_step and of the perturbed fused loop (EXT = 3), every rounding spelled out.  nvcc contracts
+// the products of plant_euler_a22 / plant_of into FMAs differently depending on where they are inlined: every fused-loop
+// instantiation evaluates a21 w + a22 om as fma(a22, om, a21 w), the RK4 / tau_E(w) plant kernel evaluated it as
+// fma(w, a21, a22 om), and the RK4 stages of the fused loop take w^2 + w_marg^2 (NTM_PROFILE_RHO1_SQ) as one FMA where
+// the Euler map rounds w^2 first.  This function is the fused loop's form, so that stepping a controller with
+// ntm_plant_step reproduces the fused loop bit for bit under every plant profile, and so that the perturbed loop
+// gives ntm_plant_step's bits wherever it is instantiated.  a22n, ctau: as plant_of.
+__device__ __forceinline__ void plant_exact(const Params &P, int flags, double a22n, double ctau, double w, double om,
+                                            double u, double &nw, double &nom) {
+    const bool te = (flags & NTM_PROFILE_TAUE_W) != 0, sq = (flags & NTM_PROFILE_RHO1_SQ) != 0;
+    const bool rk4 = (flags & NTM_PROFILE_PLANT_RK4) != 0, pc = (flags & NTM_PROFILE_PLANT_C) != 0;
+    auto euler = [&](double zw, double zo, double &ew, double &eo) {
+        const double a22 = te ? __dsub_rn(1.0, __ddiv_rn(__dsub_rn(1.0, a22n), __dsub_rn(1.0, __dmul_rn(ctau, zw)))) : a22n;
+        const double ww = __dmul_rn(zw, zw);
+        const double r1 = __drcp_rn(sq ? (rk4 ? __fma_rn(zw, zw, P.wmarg2) : __dadd_rn(ww, P.wmarg2)) : __dadd_rn(zw, P.wmarg2));
+        const double r2 = __ddiv_rn(ww, zo);
+        const double ws = __ddiv_rn(zw, P.w_dep), ws2 = __dmul_rn(ws, ws);
+        const double den = __fma_rn(__dmul_rn(ws, ws2), 0.64, __fma_rn(ws2, 0.43, __fma_rn(ws, 1.5, 1.0)));
+        const double r3 = __ddiv_rn(__fma_rn(ws, 0.24, 0.25), den);
+        const double a11 = __fma_rn(P.c_a11, r1, 1.0), a21 = __dmul_rn(P.c_a21, r2), b = __dmul_rn(P.c_b, r3);
+        ew = __fma_rn(zw, a11, __dmul_rn(b, u));
+        eo = __fma_rn(a22, zo, __dmul_rn(zw, a21));
+        if (pc) { ew = __dadd_rn(ew, P.C1); eo = __dadd_rn(eo, P.C2); }
+    };
+    if (!rk4) { euler(w, om, nw, nom); return; }
+    double yw = w, yo = om, sw = 0.0, so = 0.0, aw = 0.0, ao = 0.0;   // ((k1 + 2 k2) + (2 k3 + k4)) / 6, as plant_of
+#pragma unroll 1
+    for (int st = 0; st < 4; ++st) {
+        double e1, e2;
+        euler(yw, yo, e1, e2);
+        const double kw = __dsub_rn(e1, yw), ko = __dsub_rn(e2, yo);
+        if (st == 0) { sw = kw; so = ko; }
+        else if (st == 1) { sw = __fma_rn(kw, 2.0, sw); so = __fma_rn(ko, 2.0, so); }
+        else if (st == 2) { aw = __dadd_rn(kw, kw); ao = __dadd_rn(ko, ko); }
+        else { aw = __dadd_rn(aw, kw); ao = __dadd_rn(ao, ko); }
+        const double h = (st < 2) ? 0.5 : 1.0;
+        yw = __fma_rn(h, kw, w); yo = __fma_rn(h, ko, om);
+    }
+    nw = __dadd_rn(w, __ddiv_rn(__dadd_rn(sw, aw), 6.0));
+    nom = __dadd_rn(om, __ddiv_rn(__dadd_rn(so, ao), 6.0));
+}
+
 // =================================================================================================
 // fused persistent closed loop
 // =================================================================================================
@@ -97,7 +139,8 @@ __device__ void stage_prefix(int N, int j, const Work &w, const Params &P, doubl
     }
 }
 
-// EXT: 0 = the headline instantiation (Euler plant, box QP), 1 = + the RK4 plant option, 2 = + getWLc's state rows
+// EXT: 0 = the headline instantiation (Euler plant, box QP), 1 = + the RK4 plant option, 2 = + getWLc's state rows,
+// 3 = box QP against a perturbed plant (LoopArgs::pert: its own parameters and profile bits, d_k and v_k)
 // LONG (long horizons, literal Gamma, box QP): the QP runs on the packed sweep tableau of ntm_long.cuh
 template <int GW, bool DENSE, int EXT>
 struct LoopTraits {
@@ -128,11 +171,20 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     const bool ctl = (GW == 1 && EXT == 0) ? (a.ctl != 0) : CTL;
     double x01 = __ldg(a.x0 + elem(layout, S, 2, s, 0)), x02 = __ldg(a.x0 + elem(layout, S, 2, s, 1));
     double x1 = x01, x2 = x02;
+    // perturbed plant (EXT = 3): (x1, x2) is what the controller sees, y_k = x_k + v_k; the offline build (:63-65) runs
+    // from y_0.  The true state x_k lives in xk only (written by the lead, read back by the group after a barrier), so
+    // no register carries it across the loop.
+    if constexpr (EXT == 3) {
+        if (a.pp.noise != nullptr) {
+            x01 += __ldg(a.pp.noise + elem(layout, S, 2 * a.k_sim, s, 0)); x02 += __ldg(a.pp.noise + elem(layout, S, 2 * a.k_sim, s, 1));
+            x1 = x01; x2 = x02;
+        }
+    }
     // NTM_PROFILE_TAUE_W (EXT instantiations only): the shared parameter block carries the a22 the controller holds over
     // the horizon of the current time step, a22(tau_E(xk(1,k))); the nominal value and c_tauE stay in registers
     [[maybe_unused]] double a22n = 0.0, ctau = 0.0;
     [[maybe_unused]] bool taue = false;
-    if constexpr (EXT != 0) {
+    if constexpr (EXT == 1 || EXT == 2) {
         taue = (flags & NTM_PROFILE_TAUE_W) != 0;
         a22n = P.a22;
         if (taue) {
@@ -216,7 +268,11 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             Gp::sync();
         }
     }
-    if (lead && !resumed && !ctl) { a.xk[xk_at(0)] = x1; a.xk[xk_at(1)] = x2; }
+    if constexpr (EXT == 3) {
+        if (lead) { a.xk[xk_at(0)] = __ldg(a.x0 + elem(layout, S, 2, s, 0)); a.xk[xk_at(1)] = __ldg(a.x0 + elem(layout, S, 2, s, 1)); }
+    } else {
+        if (lead && !resumed && !ctl) { a.xk[xk_at(0)] = x1; a.xk[xk_at(1)] = x2; }
+    }
 
     // One pass of this loop = [re-]condense (:66,:72-73 / :119-121), the stop rule of the iteration that just
     // finished (:123-127) and, at the end of a time step, the plant (:130); then the next QP + rollout (:97-117).
@@ -262,7 +318,27 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             if (!brk) Uold = Uj;                                                    // :127 (skipped by the break)
             if (stop) {
                 const double u0 = Gp::bcast0(Uj, w.red);                            // :107  uk(:,k) = U(1)
-                if (ctl) {                                                          // the caller runs the plant
+                if constexpr (EXT == 3) {
+                    // the plant's own block and profile bits, read here (once per time step, no shared copy), then + d_k
+                    if (!isfinite(u0)) status = max(status, (int)NTM_SCN_NONFINITE);
+                    const Params Q = load_params(a.pp.pparams, layout, a.pp.pparams_count, s);
+                    const int pf = a.pp.pflags;
+                    const double qtau = (pf & NTM_PROFILE_TAUE_W)
+                        ? __ldg(a.pp.pparams + elem(layout, a.pp.pparams_count, NTM_NPARAM, a.pp.pparams_count == 1 ? 0 : s, 15)) : 0.0;
+                    const double t1 = a.xk[xk_at(2 * k)], t2 = a.xk[xk_at(2 * k + 1)];   // x_k, written by the lead
+                    double nw, nom;
+                    plant_exact(Q, pf, Q.a22, qtau, t1, t2, u0, nw, nom);              // = ntm_plant_step
+                    if (a.pp.dist != nullptr) {
+                        nw += __ldg(a.pp.dist + elem(layout, S, 2 * a.k_sim, s, 2 * k));
+                        nom += __ldg(a.pp.dist + elem(layout, S, 2 * a.k_sim, s, 2 * k + 1));
+                    }
+                    const double e1 = nw - P.r1, e2 = nom - P.r2;                     // judged on the true state
+                    cost += e1 * (P.q11 * e1 + P.q12 * e2) + e2 * (P.q12 * e1 + P.q22 * e2);
+                    if (lead) {
+                        a.xk[xk_at(2 * (k + 1))] = nw;
+                        a.xk[xk_at(2 * (k + 1) + 1)] = nom;
+                    }
+                } else if (ctl) {                                                   // the caller runs the plant
                     if (!isfinite(u0)) status = max(status, (int)NTM_SCN_NONFINITE);
                 } else {
                     double nw, nom;
@@ -325,7 +401,16 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             }
         }
         if (k >= a.k_sim) break;
-        if (ctl && it == 0) {            // G, F on hand are built; the step itself (QP, rollout) starts from the measurement
+        if constexpr (EXT == 3) {
+            if (it == 0) {               // as for a controller step: the measurement y_k = x_k + v_k
+                Gp::sync();              // the lead has just written x_k
+                x1 = a.xk[xk_at(2 * k)]; x2 = a.xk[xk_at(2 * k + 1)];
+                if (a.pp.noise != nullptr) {
+                    x1 += __ldg(a.pp.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k)); x2 += __ldg(a.pp.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k + 1));
+                }
+                if (!(isfinite(x1) && isfinite(x2))) status = max(status, (int)NTM_SCN_NONFINITE);
+            }
+        } else if (ctl && it == 0) {     // G, F on hand are built; the step itself (QP, rollout) starts from the measurement
             x1 = __ldg(a.x0 + elem(layout, S, 2, s, 0)); x2 = __ldg(a.x0 + elem(layout, S, 2, s, 1));
         }
         if (!retry) ++it;
@@ -547,7 +632,12 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
         Gp::sync();
     }
     if (lead) {
-        if (!(isfinite(x1) && isfinite(x2) && isfinite(cost))) status = max(status, (int)NTM_SCN_NONFINITE);
+        if constexpr (EXT == 3) {
+            const double t1 = a.xk[xk_at(2 * a.k_sim)], t2 = a.xk[xk_at(2 * a.k_sim + 1)];
+            if (!(isfinite(t1) && isfinite(t2) && isfinite(cost))) status = max(status, (int)NTM_SCN_NONFINITE);
+        } else {
+            if (!(isfinite(x1) && isfinite(x2) && isfinite(cost))) status = max(status, (int)NTM_SCN_NONFINITE);
+        }
         if (a.cost) a.cost[rec ? rbase : (size_t)s] = cost;
         if (a.status) a.status[s] = status;
         if (rec && a.rec_status) a.rec_status[rbase] = (double)status;
@@ -556,7 +646,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
 
 template <int GW, bool DENSE, int EXT, int LV = 0, bool CTL = false>
 __global__ void __launch_bounds__(GW == 1 ? 128 : 32 * GW,
-                                  GW == 1 ? (EXT == 0 ? 5 : (EXT == 1 ? 4 : 3)) : (LoopTraits<GW, DENSE, EXT>::LONG ? 3 : 1))
+                                  GW == 1 ? (EXT == 0 ? 5 : ((EXT == 1 || EXT == 3) ? 4 : 3)) : (LoopTraits<GW, DENSE, EXT>::LONG ? 3 : 1))
 closed_loop_kernel(LoopArgs a, unsigned int gbytes) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     using Gp = Group<GW>;

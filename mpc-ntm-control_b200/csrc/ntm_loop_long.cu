@@ -1,5 +1,5 @@
 // ntm_loop_long.cu -- long-horizon (33 <= N <= 128) instantiations of the fused closed loop, literal Gamma, EC-power box
-// QP: closed_loop_kernel<GW, false, 0|1> on the packed sweep tableau (ntm_long.cuh).  One CTA of GW warps per scenario,
+// QP: closed_loop_kernel<GW, false, 0|1|3> on the packed sweep tableau (ntm_long.cuh).  One CTA of GW warps per scenario,
 // ~60 KB of shared memory at N = 100, three CTAs per SM (round 1: 178 KB, one CTA per SM).
 #include "ntm_loop.cuh"
 
@@ -32,7 +32,11 @@ cudaError_t launch_closed_loop_long(cudaStream_t st, const DeviceProps &dp, cons
     const bool rk4 = (a.flags & (NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)) != 0;   // the EXT = 1 instantiations: cold plant options
     cudaError_t e;
     // tableau in registers: 7 x 7 blocks, thread I(I+1)/2 + J owns block (I, J): N + 1 <= 70 (2 warps) / 105 (4 warps)
-    if (a.ctl) {                                           // controller step (EXT = 0): its own instantiations
+    if (a.pert) {                                          // perturbed plant (EXT = 3): its own instantiations
+        if (a.N <= 64) e = launch_long<2, 3, 0>(st, dp, a);
+        else if (a.N + 1 <= NTM_TS * 15) e = launch_long<4, 3, 0>(st, dp, a);
+        else e = launch_long<4, 3, 1>(st, dp, a);
+    } else if (a.ctl) {                                           // controller step (EXT = 0): its own instantiations
         if (a.N <= 64) e = launch_long<2, 0, 0, true>(st, dp, a);
         else if (a.N + 1 <= NTM_TS * 15) e = launch_long<4, 0, 0, true>(st, dp, a);
         else e = launch_long<4, 0, 1, true>(st, dp, a);

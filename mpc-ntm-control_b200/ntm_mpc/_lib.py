@@ -75,6 +75,8 @@ for _sfx in ("", "_dev"):
                                            _dp, _dp])
     SYMBOLS["ntm_mpc_step_sc" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i, _i, _dp, _dp, _dp,
                                               _dp, _dp, _dp, _dp])
+    SYMBOLS["ntm_mpc_closed_loop_perturbed" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i,
+                                                            _dp, _i, _i, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp])
     SYMBOLS["ntm_mpc_closed_loop_sc" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i, _i, _dp,
                                                      _dp, _dp, _dp, _dp, _dp, _dp, _dp])
 

@@ -71,6 +71,32 @@ def _loop_outputs(out, S: int, N: int, k_sim: int, want_Uk: bool):
     return res
 
 
+PLANT_PROFILE_BITS = _lib.PROFILE_RHO1_SQ | _lib.PROFILE_PLANT_C | _lib.PROFILE_PLANT_RK4 | _lib.PROFILE_TAUE_W   # ntm_plant_step's bits
+
+
+def perturbed_inputs(x0, params, plant_params, plant_profile, w, v, k_sim: int, profile: int):
+    """Checks and flattens the inputs of ``NtmMpc.closed_loop_perturbed`` (no device needed): returns ``(x0 [S, 2],
+    params, params_count, plant_params or None, plant_params_count, plant_profile, w or None, v or None)`` with
+    ``w`` / ``v`` in MATLAB layout (element 2k + i of scenario s at ``[s, k, i]``)."""
+    x0 = _f64(x0).reshape(-1, 2)
+    S = x0.shape[0]
+    p, pc = NtmMpc._params(params, S)
+    if profile & _lib.PROFILE_TAUE_W:
+        raise ValueError("profile: PROFILE_TAUE_W is not supported on the controller side")
+    pf = (profile & PLANT_PROFILE_BITS) if plant_profile is None else int(plant_profile)
+    if pf & ~PLANT_PROFILE_BITS:
+        raise ValueError("plant_profile: only PROFILE_RHO1_SQ, PLANT_C, PLANT_RK4 and TAUE_W act on the plant")
+    pp, ppc = (None, pc) if plant_params is None else NtmMpc._params(plant_params, S)
+    ext = []
+    for name, a in (("w", w), ("v", v)):
+        if a is not None:
+            a = _f64(a)
+            if a.shape != (S, k_sim, 2):
+                raise ValueError(f"{name} must be [S, k_sim, 2] = {(S, k_sim, 2)} (got {a.shape})")
+        ext.append(a)
+    return x0, p, pc, pp, ppc, pf, ext[0], ext[1]
+
+
 def device_count() -> int:
     """Number of CUDA devices the library can see (``ntm_device_count``)."""
     n = ctypes.c_int(0)
@@ -353,6 +379,36 @@ class NtmMpc:
         check(self._lib.ntm_mpc_closed_loop_sc_dev(self._h, layout, profile, S, N, k_sim, i_sim, eps, x0_ptr, params_ptr,
                                                    params_count, int(state_rows), _ptr(xb), xk_ptr, uk_ptr, Uk_ptr or None,
                                                    cost_ptr or None, inner_ptr or None, qp_ptr or None, status_ptr or None))
+
+    def closed_loop_perturbed(self, x0, params, N: int, plant_params=None, plant_profile: Optional[int] = None, w=None,
+                              v=None, k_sim: int = 20, i_sim: int = 10, eps: float = 1e-14, profile: int = 0,
+                              want_Uk: bool = False, out: Optional[dict] = None):
+        """The fused loop against a perturbed plant (``ntm_mpc_closed_loop_perturbed``): the controller (``params``,
+        ``profile``) sees ``y_k = x_k + v[:, k]``; the plant is ``plant_step`` on ``plant_params`` (default ``params``)
+        under ``plant_profile`` (default: the plant bits of ``profile``), plus ``w[:, k]``.  ``w`` and ``v`` are
+        ``[S, k_sim, 2]`` or None.  Returns the dict of ``closed_loop``; ``xk`` holds the true states and ``cost`` is
+        judged on them."""
+        x0, p, pc, pp, ppc, pf, wf, vf = perturbed_inputs(x0, params, plant_params, plant_profile, w, v, k_sim, profile)
+        S = x0.shape[0]
+        xk, uk, Uk, cost, inner, qpit, status = _loop_outputs(out, S, N, k_sim, want_Uk)
+        check(self._lib.ntm_mpc_closed_loop_perturbed(self._h, LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, _ptr(x0),
+                                                      _ptr(p), pc, _ptr(pp), ppc, pf, _ptr(wf), _ptr(vf), _ptr(xk),
+                                                      _ptr(uk), _ptr(Uk) if want_Uk else None, _ptr(cost), _ptr(inner),
+                                                      _ptr(qpit), _ptr(status)))
+        return dict(xk=xk, uk=uk, Uk=Uk if want_Uk else None, cost=cost, inner_iters=inner, qp_iters=qpit, status=status)
+
+    def closed_loop_perturbed_dev(self, S: int, N: int, k_sim: int, i_sim: int, eps: float, profile: int, layout: int,
+                                  x0_ptr: int, params_ptr: int, params_count: int, plant_params_ptr: int,
+                                  plant_params_count: int, plant_profile: int, w_ptr: int, v_ptr: int, xk_ptr: int,
+                                  uk_ptr: int, Uk_ptr: int = 0, cost_ptr: int = 0, inner_ptr: int = 0, qp_ptr: int = 0,
+                                  status_ptr: int = 0) -> None:
+        """``closed_loop_perturbed`` on device pointers (0 = NULL for ``plant_params_ptr``, ``w_ptr``, ``v_ptr`` and the
+        optional outputs); asynchronous on the handle's stream (``ntm_mpc_closed_loop_perturbed_dev``)."""
+        check(self._lib.ntm_mpc_closed_loop_perturbed_dev(self._h, layout, profile, S, N, k_sim, i_sim, eps, x0_ptr,
+                                                          params_ptr, params_count, plant_params_ptr or None,
+                                                          plant_params_count, plant_profile, w_ptr or None, v_ptr or None,
+                                                          xk_ptr, uk_ptr, Uk_ptr or None, cost_ptr or None,
+                                                          inner_ptr or None, qp_ptr or None, status_ptr or None))
 
     # ------------------------------------------------------------------ NTM_MPC_Sim.m:94-128, one step, no plant
     def mpc_step(self, state, x, params, N: int, i_sim: int = 10, eps: float = 1e-14, profile: int = 0,
