@@ -37,7 +37,7 @@ struct ntm_handle {
     cudaStream_t stream = nullptr;
     ntm::DeviceProps props{};
     unsigned char *arena = nullptr;
-    size_t arena_bytes = 0, arena_used = 0;
+    size_t arena_bytes = 0;
     unsigned int *counter = nullptr;
     double *hscratch = nullptr;      // global LDL' slabs for horizons whose G + H exceed shared memory
     size_t hscratch_bytes = 0;
@@ -76,30 +76,40 @@ int check_params(const double *params, int pc, int S) {
 }
 
 // ---- arena -------------------------------------------------------------------------------------
-struct Arena {
-    ntm_handle *h;
-    size_t need = 0;
+// The buffers of one host-pointer call, carved from the handle's grow-only device arena.  A call declares them once, in a
+// layout callback of take<T>(count) calls; reserve runs it twice, to size the arena and to hand the buffers out, so the
+// size cannot disagree with what is handed out.
+class Arena {
+  public:
     explicit Arena(ntm_handle *hh) : h(hh) {}
-    static size_t pad(size_t b) { return (b + 255) & ~(size_t)255; }
-    void want(size_t bytes) { need += pad(bytes); }
-    int reserve() {
-        h->arena_used = 0;
-        if (need <= h->arena_bytes) return NTM_OK;
-        CU(cudaStreamSynchronize(h->stream));
-        if (h->arena) CU(cudaFree(h->arena));
-        h->arena = nullptr; h->arena_bytes = 0;
-        const size_t want_bytes = need + need / 4;
-        cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&h->arena), want_bytes);
-        if (e != cudaSuccess) return fail(NTM_ERR_ALLOC, "cudaMalloc(%zu): %s", want_bytes, cudaGetErrorString(e));
-        h->arena_bytes = want_bytes;
+    template <typename F>
+    int reserve(F layout) {
+        base = nullptr; used = 0;                        // sizing pass: take() returns NULL
+        layout(*this);
+        if (used > h->arena_bytes) {
+            CU(cudaStreamSynchronize(h->stream));
+            if (h->arena) CU(cudaFree(h->arena));
+            h->arena = nullptr; h->arena_bytes = 0;
+            const size_t want_bytes = used + used / 4;
+            cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&h->arena), want_bytes);
+            if (e != cudaSuccess) return fail(NTM_ERR_ALLOC, "cudaMalloc(%zu): %s", want_bytes, cudaGetErrorString(e));
+            h->arena_bytes = want_bytes;
+        }
+        base = h->arena; used = 0;
+        layout(*this);
         return NTM_OK;
     }
     template <typename T>
     T *take(size_t count) {
-        T *p = reinterpret_cast<T *>(h->arena + h->arena_used);
-        h->arena_used += pad(count * sizeof(T));
+        T *p = base ? reinterpret_cast<T *>(base + used) : nullptr;
+        used += (count * sizeof(T) + 255) & ~(size_t)255;
         return p;
     }
+
+  private:
+    ntm_handle *h;
+    unsigned char *base = nullptr;
+    size_t used = 0;
 };
 
 int ensure_hscratch(ntm_handle *h, int N) {
@@ -170,6 +180,79 @@ int d2h_shard(ntm_handle *h, int layout, T *dst, const T *src, size_t E, size_t 
         CU(cudaMemcpyAsync(dst + (layout == NTM_LAYOUT_MATLAB ? s_off * E : 0), src, E * S * sizeof(T), cudaMemcpyDeviceToHost, h->stream));
     else
         CU(cudaMemcpy2DAsync(dst + s_off, S_total * sizeof(T), src, S * sizeof(T), S * sizeof(T), E, cudaMemcpyDeviceToHost, h->stream));
+    return NTM_OK;
+}
+
+// Arrays of a fused call (closed loop, perturbed loop, controller step), the caller's or their device copies; NULL = not
+// passed.  x0 is the measured state of a controller step, state its records.
+struct Fused {
+    const double *x0, *params, *pparams, *w, *v;
+    double *state, *xk, *uk, *Uk, *cost;
+    int *inner, *qpit, *status;
+};
+
+// Fills the LoopArgs fields every fused call shares and launches it.  The entry has set its own mode fields (srows and the
+// state box, sv and ctl, pp and pert, rec_ld and rec_status) and checked its arguments.
+static int launch_fused(ntm_handle *h, ntm::LoopArgs &a, int layout, int flags, int S, int N, int k_sim, int i_sim,
+                        double eps, int pc, const Fused &d) {
+    a.layout = layout; a.flags = flags; a.S = S; a.N = N; a.k_sim = k_sim; a.i_sim = i_sim; a.eps = eps;
+    a.x0 = d.x0; a.params = d.params; a.params_count = pc;
+    a.xk = d.xk; a.uk = d.uk; a.Uk = d.Uk; a.cost = d.cost; a.inner = d.inner; a.qpit = d.qpit; a.status = d.status;
+    a.counter = h->counter;
+    TRY(ensure_hscratch(h, N));
+    a.hscratch = h->hscratch;
+    const size_t svd = ntm::lpt_doubles(h->props, a);      // two-phase launch with a longest-first queue (ntm_kernels.h)
+    if (svd != 0) {
+        TRY(ensure_lpt(h, svd, 2 * (size_t)S + NTM_LPT_BINS));
+        a.sv = h->sv; a.lpt = h->lpt;
+    }
+    CU(ntm::launch_closed_loop(h->stream, h->props, a, &h->launches));
+    return NTM_OK;
+}
+
+// Host-pointer fused call for the scenarios [s_off, s_off + S) of caller arrays that hold S_total scenarios: copies every
+// array the caller passed to the arena, runs `launch` on the device copies, copies the outputs back and waits.  MATLAB
+// layout: a shard is a contiguous slice of every array.  SoA layout (scenario fastest): a shard is a column band, moved
+// with 2-D copies.  S_total == S, s_off == 0 is the plain single-device call.  A parameter count of 1 is one block for
+// every scenario.
+template <typename F>
+static int fused_host(ntm_handle *h, int layout, int S, int S_total, int s_off, int N, int k_sim, int pc, int ppc,
+                      const Fused &in, F launch) {
+    const size_t s = (size_t)S, n = (size_t)N, ks = (size_t)k_sim, st = (size_t)S_total, so = (size_t)s_off;
+    const size_t ld = (size_t)NTM_CTRL_DOUBLES(N);
+    double *x0, *prm, *pprm, *w, *v, *state, *xk, *uk, *Uk, *cost;
+    int *inner, *qpit, *status;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        x0 = A.take<double>(2 * s);
+        prm = A.take<double>((pc == 1 ? 1 : s) * NTM_NPARAM);
+        pprm = in.pparams ? A.take<double>((ppc == 1 ? 1 : s) * NTM_NPARAM) : nullptr;
+        w = in.w ? A.take<double>(2 * ks * s) : nullptr;
+        v = in.v ? A.take<double>(2 * ks * s) : nullptr;
+        state = in.state ? A.take<double>(ld * s) : nullptr;
+        xk = in.xk ? A.take<double>(2 * (ks + 1) * s) : nullptr;
+        uk = in.uk ? A.take<double>(ks * s) : nullptr;
+        Uk = in.Uk ? A.take<double>(n * ks * s) : nullptr;
+        cost = in.cost ? A.take<double>(s) : nullptr;
+        inner = in.inner ? A.take<int>(ks * s) : nullptr;
+        qpit = in.qpit ? A.take<int>(ks * s) : nullptr;
+        status = in.status ? A.take<int>(s) : nullptr;
+    }));
+    auto blocks = [&](double *dst, const double *src, int count) {
+        return count == 1 ? h2d(h, dst, src, (size_t)NTM_NPARAM) : h2d_shard(h, layout, dst, src, NTM_NPARAM, s, st, so);
+    };
+    TRY(h2d_shard(h, layout, x0, in.x0, 2, s, st, so));
+    TRY(blocks(prm, in.params, pc));
+    if (pprm) TRY(blocks(pprm, in.pparams, ppc));
+    if (w) TRY(h2d_shard(h, layout, w, in.w, 2 * ks, s, st, so));
+    if (v) TRY(h2d_shard(h, layout, v, in.v, 2 * ks, s, st, so));
+    if (state) TRY(h2d_shard(h, layout, state, in.state, ld, s, st, so));
+    TRY(launch(Fused{x0, prm, pprm, w, v, state, xk, uk, Uk, cost, inner, qpit, status}));
+    TRY(d2h_shard(h, layout, in.state, state, ld, s, st, so));
+    TRY(d2h_shard(h, layout, in.xk, xk, 2 * (ks + 1), s, st, so)); TRY(d2h_shard(h, layout, in.uk, uk, ks, s, st, so));
+    TRY(d2h_shard(h, layout, in.Uk, Uk, n * ks, s, st, so)); TRY(d2h_shard(h, layout, in.cost, cost, 1, s, st, so));
+    TRY(d2h_shard(h, layout, in.inner, inner, ks, s, st, so)); TRY(d2h_shard(h, layout, in.qpit, qpit, ks, s, st, so));
+    TRY(d2h_shard(h, layout, in.status, status, 1, s, st, so));
+    CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
 }
 
@@ -284,11 +367,11 @@ int ntm_rho(ntm_handle *h, int layout, int profile, int S, const double *x, cons
     TRY(check_params(params, pc, S));
     REQUIRE(x && rho1 && rho2 && rho3, "NULL array");
     const size_t s = (size_t)S;
-    Arena A(h);
-    A.want(2 * s * 8); A.want((size_t)pc * NTM_NPARAM * 8); A.want(s * 8); A.want(s * 8); A.want(s * 8);
-    TRY(A.reserve());
-    double *dx = A.take<double>(2 * s), *dp = A.take<double>((size_t)pc * NTM_NPARAM);
-    double *d1 = A.take<double>(s), *d2 = A.take<double>(s), *d3 = A.take<double>(s);
+    double *dx, *dp, *d1, *d2, *d3;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        dx = A.take<double>(2 * s); dp = A.take<double>((size_t)pc * NTM_NPARAM);
+        d1 = A.take<double>(s); d2 = A.take<double>(s); d3 = A.take<double>(s);
+    }));
     TRY(h2d(h, dx, x, 2 * s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
     TRY(ntm_rho_dev(h, layout, profile, S, dx, dp, pc, d1, d2, d3));
     TRY(d2h(h, rho1, d1, s)); TRY(d2h(h, rho2, d2, s)); TRY(d2h(h, rho3, d3, s));
@@ -314,11 +397,11 @@ int ntm_lpv_AB(ntm_handle *h, int layout, int S, const double *rho1, const doubl
     TRY(check_params(params, pc, S));
     REQUIRE(rho1 && rho2 && rho3 && Aout && Bout, "NULL array");
     const size_t s = (size_t)S;
-    Arena A(h);
-    A.want(s * 8); A.want(s * 8); A.want(s * 8); A.want((size_t)pc * NTM_NPARAM * 8); A.want(4 * s * 8); A.want(2 * s * 8);
-    TRY(A.reserve());
-    double *d1 = A.take<double>(s), *d2 = A.take<double>(s), *d3 = A.take<double>(s);
-    double *dp = A.take<double>((size_t)pc * NTM_NPARAM), *dA = A.take<double>(4 * s), *dB = A.take<double>(2 * s);
+    double *d1, *d2, *d3, *dp, *dA, *dB;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        d1 = A.take<double>(s); d2 = A.take<double>(s); d3 = A.take<double>(s);
+        dp = A.take<double>((size_t)pc * NTM_NPARAM); dA = A.take<double>(4 * s); dB = A.take<double>(2 * s);
+    }));
     TRY(h2d(h, d1, rho1, s)); TRY(h2d(h, d2, rho2, s)); TRY(h2d(h, d3, rho3, s));
     TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
     TRY(ntm_lpv_AB_dev(h, layout, S, d1, d2, d3, dp, pc, dA, dB));
@@ -348,13 +431,12 @@ int ntm_condense(ntm_handle *h, int layout, int profile, int S, int N, const dou
     REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
     REQUIRE(R1 && R2 && R3 && Phi && Gamma && Lambda, "NULL array");
     const size_t s = (size_t)S, n = (size_t)N;
-    Arena A(h);
-    A.want(n * s * 8); A.want(n * s * 8); A.want(n * s * 8); A.want((size_t)pc * NTM_NPARAM * 8);
-    A.want(4 * n * s * 8); A.want(2 * n * n * s * 8); A.want(2 * n * s * 8);
-    TRY(A.reserve());
-    double *d1 = A.take<double>(n * s), *d2 = A.take<double>(n * s), *d3 = A.take<double>(n * s);
-    double *dp = A.take<double>((size_t)pc * NTM_NPARAM);
-    double *dPhi = A.take<double>(4 * n * s), *dGam = A.take<double>(2 * n * n * s), *dLam = A.take<double>(2 * n * s);
+    double *d1, *d2, *d3, *dp, *dPhi, *dGam, *dLam;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        d1 = A.take<double>(n * s); d2 = A.take<double>(n * s); d3 = A.take<double>(n * s);
+        dp = A.take<double>((size_t)pc * NTM_NPARAM);
+        dPhi = A.take<double>(4 * n * s); dGam = A.take<double>(2 * n * n * s); dLam = A.take<double>(2 * n * s);
+    }));
     TRY(h2d(h, d1, R1, n * s)); TRY(h2d(h, d2, R2, n * s)); TRY(h2d(h, d3, R3, n * s));
     TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
     TRY(ntm_condense_dev(h, layout, profile, S, N, d1, d2, d3, dp, pc, dPhi, dGam, dLam));
@@ -384,13 +466,12 @@ int ntm_hessian_grad(ntm_handle *h, int layout, int S, int N, const double *Phi,
     REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
     REQUIRE(Phi && Gamma && Lambda && x && G && F, "NULL array");
     const size_t s = (size_t)S, n = (size_t)N;
-    Arena A(h);
-    A.want(4 * n * s * 8); A.want(2 * n * n * s * 8); A.want(2 * n * s * 8); A.want(2 * s * 8);
-    A.want((size_t)pc * NTM_NPARAM * 8); A.want(n * n * s * 8); A.want(n * s * 8);
-    TRY(A.reserve());
-    double *dPhi = A.take<double>(4 * n * s), *dGam = A.take<double>(2 * n * n * s), *dLam = A.take<double>(2 * n * s);
-    double *dx = A.take<double>(2 * s), *dp = A.take<double>((size_t)pc * NTM_NPARAM);
-    double *dG = A.take<double>(n * n * s), *dF = A.take<double>(n * s);
+    double *dPhi, *dGam, *dLam, *dx, *dp, *dG, *dF;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        dPhi = A.take<double>(4 * n * s); dGam = A.take<double>(2 * n * n * s); dLam = A.take<double>(2 * n * s);
+        dx = A.take<double>(2 * s); dp = A.take<double>((size_t)pc * NTM_NPARAM);
+        dG = A.take<double>(n * n * s); dF = A.take<double>(n * s);
+    }));
     TRY(h2d(h, dPhi, Phi, 4 * n * s)); TRY(h2d(h, dGam, Gamma, 2 * n * n * s)); TRY(h2d(h, dLam, Lambda, 2 * n * s));
     TRY(h2d(h, dx, x, 2 * s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
     TRY(ntm_hessian_grad_dev(h, layout, S, N, dPhi, dGam, dLam, dx, dp, pc, dG, dF));
@@ -421,13 +502,13 @@ int ntm_qp_box(ntm_handle *h, int layout, int S, int N, const double *G, const d
     REQUIRE(G && F && lb && ub && U, "NULL array");
     REQUIRE(bc == 1 || bc == S, "bounds_count must be 1 or S");
     const size_t s = (size_t)S, n = (size_t)N, b = (size_t)bc;
-    Arena A(h);
-    A.want(n * n * s * 8); A.want(n * s * 8); A.want(n * b * 8); A.want(n * b * 8); A.want(n * s * 8);
-    A.want(s * 4); A.want(s * 4);
-    TRY(A.reserve());
-    double *dG = A.take<double>(n * n * s), *dF = A.take<double>(n * s), *dlb = A.take<double>(n * b);
-    double *dub = A.take<double>(n * b), *dU = A.take<double>(n * s);
-    int *dit = A.take<int>(s), *dst = A.take<int>(s);
+    double *dG, *dF, *dlb, *dub, *dU;
+    int *dit, *dst;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        dG = A.take<double>(n * n * s); dF = A.take<double>(n * s); dlb = A.take<double>(n * b);
+        dub = A.take<double>(n * b); dU = A.take<double>(n * s);
+        dit = A.take<int>(s); dst = A.take<int>(s);
+    }));
     TRY(h2d(h, dG, G, n * n * s)); TRY(h2d(h, dF, F, n * s)); TRY(h2d(h, dlb, lb, n * b)); TRY(h2d(h, dub, ub, n * b));
     TRY(ntm_qp_box_dev(h, layout, S, N, dG, dF, dlb, dub, bc, dU, dit, dst));
     TRY(d2h(h, U, dU, n * s)); TRY(d2h(h, iters, dit, s)); TRY(d2h(h, status, dst, s));
@@ -464,14 +545,14 @@ int ntm_qp_ineq(ntm_handle *h, int layout, int S, int N, int M, const double *G,
     REQUIRE(G && F && lb && ub && U && Lg && bg, "NULL array");
     REQUIRE(bc == 1 || bc == S, "bounds_count must be 1 or S");
     const size_t s = (size_t)S, n = (size_t)N, b = (size_t)bc, m = (size_t)M;
-    Arena A(h);
-    A.want(n * n * s * 8); A.want(n * s * 8); A.want(n * b * 8); A.want(n * b * 8); A.want(n * s * 8);
-    A.want(m * n * s * 8); A.want(m * s * 8); A.want(s * 4); A.want(s * 4);
-    TRY(A.reserve());
-    double *dG = A.take<double>(n * n * s), *dF = A.take<double>(n * s), *dlb = A.take<double>(n * b);
-    double *dub = A.take<double>(n * b), *dU = A.take<double>(n * s);
-    double *dL = A.take<double>(m * n * s), *dbg = A.take<double>(m * s);
-    int *dit = A.take<int>(s), *dst = A.take<int>(s);
+    double *dG, *dF, *dlb, *dub, *dU, *dL, *dbg;
+    int *dit, *dst;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        dG = A.take<double>(n * n * s); dF = A.take<double>(n * s); dlb = A.take<double>(n * b);
+        dub = A.take<double>(n * b); dU = A.take<double>(n * s);
+        dL = A.take<double>(m * n * s); dbg = A.take<double>(m * s);
+        dit = A.take<int>(s); dst = A.take<int>(s);
+    }));
     TRY(h2d(h, dG, G, n * n * s)); TRY(h2d(h, dF, F, n * s)); TRY(h2d(h, dlb, lb, n * b)); TRY(h2d(h, dub, ub, n * b));
     TRY(h2d(h, dL, Lg, m * n * s)); TRY(h2d(h, dbg, bg, m * s));
     TRY(ntm_qp_ineq_dev(h, layout, S, N, M, dG, dF, dlb, dub, bc, dL, dbg, dU, dit, dst));
@@ -498,11 +579,11 @@ int ntm_plant_step(ntm_handle *h, int layout, int profile, int S, const double *
     TRY(check_params(params, pc, S));
     REQUIRE(x && u && xn, "NULL array");
     const size_t s = (size_t)S;
-    Arena A(h);
-    A.want(2 * s * 8); A.want(s * 8); A.want((size_t)pc * NTM_NPARAM * 8); A.want(2 * s * 8);
-    TRY(A.reserve());
-    double *dx = A.take<double>(2 * s), *du = A.take<double>(s), *dp = A.take<double>((size_t)pc * NTM_NPARAM);
-    double *dn = A.take<double>(2 * s);
+    double *dx, *du, *dp, *dn;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        dx = A.take<double>(2 * s); du = A.take<double>(s); dp = A.take<double>((size_t)pc * NTM_NPARAM);
+        dn = A.take<double>(2 * s);
+    }));
     TRY(h2d(h, dx, x, 2 * s)); TRY(h2d(h, du, u, s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
     TRY(ntm_plant_step_dev(h, layout, profile, S, dx, du, dp, pc, dn));
     TRY(d2h(h, xn, dn, 2 * s));
@@ -542,34 +623,20 @@ static int set_state_rows(const ntm_handle *h, int profile, int N, int state_row
 }
 
 static int closed_loop_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
-                                const double *x0, const double *params, int pc, int state_rows, const double *xb,
-                                double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
-                                int *status, int rec_ld = 0, double *rec_status = nullptr) {
+                                int pc, int state_rows, const double *xb, const Fused &d, int rec_ld = 0,
+                                double *rec_status = nullptr) {
     TRY(check_common(h, layout, S));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    TRY(check_loop(N, k_sim, i_sim, x0, xk, uk));
+    TRY(check_params(d.params, pc, S));
+    TRY(check_loop(N, k_sim, i_sim, d.x0, d.xk, d.uk));
     ntm::LoopArgs a = {};
-    a.layout = layout; a.flags = profile; a.S = S; a.N = N; a.k_sim = k_sim; a.i_sim = i_sim; a.eps = eps;
-    a.x0 = x0; a.params = params; a.params_count = pc;
-    a.xk = xk; a.uk = uk; a.Uk = Uk; a.cost = cost; a.inner = inner_iters; a.qpit = qp_iters; a.status = status;
-    a.counter = h->counter;
     a.rec_ld = rec_ld; a.rec_status = rec_status;
     TRY(set_state_rows(h, profile, N, state_rows, xb, a));
-    TRY(ensure_hscratch(h, N));
-    a.hscratch = h->hscratch;
-    const size_t svd = ntm::lpt_doubles(h->props, a);      // two-phase launch with a longest-first queue (ntm_kernels.h)
-    if (svd != 0) {
-        TRY(ensure_lpt(h, svd, 2 * (size_t)S + NTM_LPT_BINS));
-        a.sv = h->sv; a.lpt = h->lpt;
-    }
-    CU(ntm::launch_closed_loop(h->stream, h->props, a, &h->launches));
-    return NTM_OK;
+    return launch_fused(h, a, layout, profile, S, N, k_sim, i_sim, eps, pc, d);
 }
 
-// Host-pointer closed loop for the scenarios [s_off, s_off + S) of a caller array that holds S_total scenarios.
-// MATLAB layout: a shard is a contiguous slice of every array.  SoA layout (scenario fastest): a shard is a column
-// band, moved with 2-D copies.  S_total == S, s_off == 0 is the plain single-device call.
+// Host-pointer closed loop for the scenarios [s_off, s_off + S) of a caller array that holds S_total scenarios (see
+// fused_host).
 static int closed_loop_host_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
                                  const double *x0, const double *params, int pc, int state_rows, const double *xb,
                                  double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
@@ -577,33 +644,14 @@ static int closed_loop_host_impl(ntm_handle *h, int layout, int profile, int S, 
     TRY(check_common(h, layout, S));
     if (S == 0) return NTM_OK;
     if (S_total < 0) S_total = S;
-    const int pc_total = pc;                             // 1 (shared block) or S_total
-    const int pcl = (pc == 1) ? 1 : S;                   // parameter blocks this shard holds
     REQUIRE(params != nullptr, "params is NULL");
-    REQUIRE(pc_total == 1 || pc_total == S_total, "params_count must be 1 or S");
+    REQUIRE(pc == 1 || pc == S_total, "params_count must be 1 or S");   // 1 (shared block) or S_total
     TRY(check_loop(N, k_sim, i_sim, x0, xk, uk));
-    const size_t s = (size_t)S, n = (size_t)N, ks = (size_t)k_sim, st = (size_t)S_total, so = (size_t)s_off;
-    Arena A(h);
-    A.want(2 * s * 8); A.want((size_t)pcl * NTM_NPARAM * 8); A.want(2 * (ks + 1) * s * 8); A.want(ks * s * 8);
-    if (Uk) A.want(n * ks * s * 8);
-    A.want(s * 8); A.want(ks * s * 4); A.want(ks * s * 4); A.want(s * 4);
-    TRY(A.reserve());
-    double *dx0 = A.take<double>(2 * s), *dp = A.take<double>((size_t)pcl * NTM_NPARAM);
-    double *dxk = A.take<double>(2 * (ks + 1) * s), *duk = A.take<double>(ks * s);
-    double *dUk = Uk ? A.take<double>(n * ks * s) : nullptr;
-    double *dcost = A.take<double>(s);
-    int *din = A.take<int>(ks * s), *dqp = A.take<int>(ks * s), *dst = A.take<int>(s);
-    TRY(h2d_shard(h, layout, dx0, x0, 2, s, st, so));
-    if (pc == 1) TRY(h2d(h, dp, params, (size_t)NTM_NPARAM));
-    else TRY(h2d_shard(h, layout, dp, params, NTM_NPARAM, s, st, so));
-    TRY(closed_loop_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, dx0, dp, pcl, state_rows, xb, dxk, duk, dUk,
-                             dcost, din, dqp, dst));
-    TRY(d2h_shard(h, layout, xk, dxk, 2 * (ks + 1), s, st, so)); TRY(d2h_shard(h, layout, uk, duk, ks, s, st, so));
-    if (Uk) TRY(d2h_shard(h, layout, Uk, dUk, n * ks, s, st, so));
-    TRY(d2h_shard(h, layout, cost, dcost, 1, s, st, so)); TRY(d2h_shard(h, layout, inner_iters, din, ks, s, st, so));
-    TRY(d2h_shard(h, layout, qp_iters, dqp, ks, s, st, so)); TRY(d2h_shard(h, layout, status, dst, 1, s, st, so));
-    CU(cudaStreamSynchronize(h->stream));
-    return NTM_OK;
+    const int pcl = (pc == 1) ? 1 : S;                   // parameter blocks this shard holds
+    return fused_host(h, layout, S, S_total, s_off, N, k_sim, pc, pc,
+                      {x0, params, nullptr, nullptr, nullptr, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status},
+                      [&](const Fused &d) { return closed_loop_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pcl,
+                                                                        state_rows, xb, d); });
 }
 
 // ---- one host process, every visible GPU (the MEX gateway ntm_mpc_batch is single-process by construction) ----------
@@ -691,16 +739,17 @@ int ntm_mpc_closed_loop_rec_dev(ntm_handle *h, int profile, int S, int N, int k_
     REQUIRE(rec != nullptr, "rec is NULL");
     TRY(check_loop(N, k_sim, i_sim, x0, rec, rec));
     const int ld = NTM_REC_DOUBLES(k_sim);
-    return closed_loop_dev_impl(h, NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, xbounds,
-                                rec, rec + 2 * (k_sim + 1), nullptr, rec + 3 * k_sim + 2, inner_iters, qp_iters, nullptr,
+    return closed_loop_dev_impl(h, NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, pc, state_rows, xbounds,
+                                {x0, params, nullptr, nullptr, nullptr, nullptr, rec, rec + 2 * (k_sim + 1), nullptr,
+                                 rec + 3 * k_sim + 2, inner_iters, qp_iters, nullptr},
                                 ld, rec + 3 * k_sim + 3);
 }
 
 int ntm_mpc_closed_loop_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
                             const double *x0, const double *params, int pc, double *xk, double *uk, double *Uk,
                             double *cost, int *inner_iters, int *qp_iters, int *status) {
-    return closed_loop_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, NTM_STATE_ROWS_OFF, nullptr,
-                                xk, uk, Uk, cost, inner_iters, qp_iters, status);
+    return closed_loop_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, NTM_STATE_ROWS_OFF, nullptr,
+                                {x0, params, nullptr, nullptr, nullptr, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
 }
 
 int ntm_mpc_closed_loop(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
@@ -714,8 +763,8 @@ int ntm_mpc_closed_loop_sc_dev(ntm_handle *h, int layout, int profile, int S, in
                                const double *x0, const double *params, int pc, int state_rows, const double *xbounds,
                                double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
                                int *status) {
-    return closed_loop_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, xbounds, xk, uk,
-                                Uk, cost, inner_iters, qp_iters, status);
+    return closed_loop_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, state_rows, xbounds,
+                                {x0, params, nullptr, nullptr, nullptr, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
 }
 
 int ntm_mpc_closed_loop_sc(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
@@ -735,26 +784,18 @@ static int check_step(int profile, int N, int i_sim) {
     return NTM_OK;
 }
 
-static int step_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
-                         const double *params, int pc, int state_rows, const double *xb, double *state, double *u,
-                         double *U, int *inner_iters, int *qp_iters, int *status) {
+// d: x0 is the measured state, state the records, uk = u and Uk = U
+static int step_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, int pc,
+                         int state_rows, const double *xb, const Fused &d) {
     TRY(check_common(h, layout, S));
     TRY(check_step(profile, N, i_sim));
     ntm::LoopArgs a = {};
     TRY(set_state_rows(h, profile, N, state_rows, xb, a));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(x && state && u, "NULL array");
-    a.layout = layout; a.S = S; a.N = N; a.k_sim = 1; a.i_sim = i_sim; a.eps = eps;
-    a.flags = profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4);   // plant-only bits: no effect on the controller
-    a.x0 = x; a.params = params; a.params_count = pc;
-    a.uk = u; a.Uk = U; a.inner = inner_iters; a.qpit = qp_iters; a.status = status;
-    a.counter = h->counter;
-    a.sv = state; a.ctl = 1;
-    TRY(ensure_hscratch(h, N));
-    a.hscratch = h->hscratch;
-    CU(ntm::launch_closed_loop(h->stream, h->props, a, &h->launches));
-    return NTM_OK;
+    TRY(check_params(d.params, pc, S));
+    REQUIRE(d.x0 && d.state && d.uk, "NULL array");
+    a.sv = d.state; a.ctl = 1;
+    return launch_fused(h, a, layout, profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4), S, N, 1, i_sim, eps, pc, d);
 }
 
 static int step_host_impl(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
@@ -767,28 +808,16 @@ static int step_host_impl(ntm_handle *h, int layout, int profile, int S, int N, 
     if (S == 0) return NTM_OK;
     TRY(check_params(params, pc, S));
     REQUIRE(x && state && u, "NULL array");
-    const size_t s = (size_t)S, n = (size_t)N, ld = (size_t)NTM_CTRL_DOUBLES(N);
-    Arena A(h);
-    A.want(2 * s * 8); A.want((size_t)pc * NTM_NPARAM * 8); A.want(ld * s * 8); A.want(s * 8);
-    if (U) A.want(n * s * 8);
-    A.want(s * 4); A.want(s * 4); A.want(s * 4);
-    TRY(A.reserve());
-    double *dx = A.take<double>(2 * s), *dp = A.take<double>((size_t)pc * NTM_NPARAM), *dst = A.take<double>(ld * s);
-    double *du = A.take<double>(s), *dU = U ? A.take<double>(n * s) : nullptr;
-    int *din = A.take<int>(s), *dqp = A.take<int>(s), *dstat = A.take<int>(s);
-    TRY(h2d(h, dx, x, 2 * s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM)); TRY(h2d(h, dst, state, ld * s));
-    TRY(step_dev_impl(h, layout, profile, S, N, i_sim, eps, dx, dp, pc, state_rows, xb, dst, du, dU, din, dqp, dstat));
-    TRY(d2h(h, state, dst, ld * s)); TRY(d2h(h, u, du, s)); TRY(d2h(h, U, dU, n * s));
-    TRY(d2h(h, inner_iters, din, s)); TRY(d2h(h, qp_iters, dqp, s)); TRY(d2h(h, status, dstat, s));
-    CU(cudaStreamSynchronize(h->stream));
-    return NTM_OK;
+    return fused_host(h, layout, S, S, 0, N, 1, pc, pc,
+                      {x, params, nullptr, nullptr, nullptr, state, nullptr, u, U, nullptr, inner_iters, qp_iters, status},
+                      [&](const Fused &d) { return step_dev_impl(h, layout, profile, S, N, i_sim, eps, pc, state_rows, xb, d); });
 }
 
 int ntm_mpc_step_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
                      const double *params, int pc, double *state, double *u, double *U, int *inner_iters, int *qp_iters,
                      int *status) {
-    return step_dev_impl(h, layout, profile, S, N, i_sim, eps, x, params, pc, NTM_STATE_ROWS_OFF, nullptr, state, u, U,
-                         inner_iters, qp_iters, status);
+    return step_dev_impl(h, layout, profile, S, N, i_sim, eps, pc, NTM_STATE_ROWS_OFF, nullptr,
+                         {x, params, nullptr, nullptr, nullptr, state, nullptr, u, U, nullptr, inner_iters, qp_iters, status});
 }
 
 int ntm_mpc_step(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
@@ -801,8 +830,8 @@ int ntm_mpc_step(ntm_handle *h, int layout, int profile, int S, int N, int i_sim
 int ntm_mpc_step_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
                         const double *params, int pc, int state_rows, const double *xbounds, double *state, double *u,
                         double *U, int *inner_iters, int *qp_iters, int *status) {
-    return step_dev_impl(h, layout, profile, S, N, i_sim, eps, x, params, pc, state_rows, xbounds, state, u, U,
-                         inner_iters, qp_iters, status);
+    return step_dev_impl(h, layout, profile, S, N, i_sim, eps, pc, state_rows, xbounds,
+                         {x, params, nullptr, nullptr, nullptr, state, nullptr, u, U, nullptr, inner_iters, qp_iters, status});
 }
 
 int ntm_mpc_step_sc(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
@@ -835,17 +864,11 @@ int ntm_mpc_closed_loop_perturbed_dev(ntm_handle *h, int layout, int profile, in
     if (plant_params == nullptr) { plant_params = params; ppc = pc; }
     TRY(check_perturbed(profile, S, N, k_sim, i_sim, x0, params, pc, ppc, plant_profile, xk, uk));
     ntm::LoopArgs a = {};
-    a.layout = layout; a.S = S; a.N = N; a.k_sim = k_sim; a.i_sim = i_sim; a.eps = eps;
-    a.flags = profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4);   // plant-only bits: no effect on the controller
-    a.x0 = x0; a.params = params; a.params_count = pc;
-    a.xk = xk; a.uk = uk; a.Uk = Uk; a.cost = cost; a.inner = inner_iters; a.qpit = qp_iters; a.status = status;
-    a.counter = h->counter;
     a.pert = 1; a.pp.pparams = plant_params; a.pp.pparams_count = ppc; a.pp.pflags = plant_profile;
     a.pp.dist = w; a.pp.noise = v;
-    TRY(ensure_hscratch(h, N));
-    a.hscratch = h->hscratch;
-    CU(ntm::launch_closed_loop(h->stream, h->props, a, &h->launches));
-    return NTM_OK;
+    // plant-only bits have no effect on the controller
+    return launch_fused(h, a, layout, profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4), S, N, k_sim, i_sim, eps, pc,
+                        {x0, params, nullptr, nullptr, nullptr, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
 }
 
 int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
@@ -857,34 +880,13 @@ int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S,
     if (S == 0) return NTM_OK;
     if (plant_params == nullptr) ppc = pc;
     TRY(check_perturbed(profile, S, N, k_sim, i_sim, x0, params, pc, ppc, plant_profile, xk, uk));
-    const size_t s = (size_t)S, n = (size_t)N, ks = (size_t)k_sim;
-    Arena A(h);
-    A.want(2 * s * 8); A.want((size_t)pc * NTM_NPARAM * 8);
-    if (plant_params) A.want((size_t)ppc * NTM_NPARAM * 8);
-    if (w) A.want(2 * ks * s * 8);
-    if (v) A.want(2 * ks * s * 8);
-    A.want(2 * (ks + 1) * s * 8); A.want(ks * s * 8);
-    if (Uk) A.want(n * ks * s * 8);
-    A.want(s * 8); A.want(ks * s * 4); A.want(ks * s * 4); A.want(s * 4);
-    TRY(A.reserve());
-    double *dx0 = A.take<double>(2 * s), *dp = A.take<double>((size_t)pc * NTM_NPARAM);
-    double *dpp = plant_params ? A.take<double>((size_t)ppc * NTM_NPARAM) : nullptr;
-    double *dw = w ? A.take<double>(2 * ks * s) : nullptr, *dv = v ? A.take<double>(2 * ks * s) : nullptr;
-    double *dxk = A.take<double>(2 * (ks + 1) * s), *duk = A.take<double>(ks * s);
-    double *dUk = Uk ? A.take<double>(n * ks * s) : nullptr;
-    double *dcost = A.take<double>(s);
-    int *din = A.take<int>(ks * s), *dqp = A.take<int>(ks * s), *dst = A.take<int>(s);
-    TRY(h2d(h, dx0, x0, 2 * s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
-    if (dpp) TRY(h2d(h, dpp, plant_params, (size_t)ppc * NTM_NPARAM));
-    if (dw) TRY(h2d(h, dw, w, 2 * ks * s));
-    if (dv) TRY(h2d(h, dv, v, 2 * ks * s));
-    TRY(ntm_mpc_closed_loop_perturbed_dev(h, layout, profile, S, N, k_sim, i_sim, eps, dx0, dp, pc, dpp, ppc,
-                                          plant_profile, dw, dv, dxk, duk, dUk, dcost, din, dqp, dst));
-    TRY(d2h(h, xk, dxk, 2 * (ks + 1) * s)); TRY(d2h(h, uk, duk, ks * s)); TRY(d2h(h, Uk, dUk, n * ks * s));
-    TRY(d2h(h, cost, dcost, s)); TRY(d2h(h, inner_iters, din, ks * s)); TRY(d2h(h, qp_iters, dqp, ks * s));
-    TRY(d2h(h, status, dst, s));
-    CU(cudaStreamSynchronize(h->stream));
-    return NTM_OK;
+    return fused_host(h, layout, S, S, 0, N, k_sim, pc, ppc,
+                      {x0, params, plant_params, w, v, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status},
+                      [&](const Fused &d) {
+                          return ntm_mpc_closed_loop_perturbed_dev(h, layout, profile, S, N, k_sim, i_sim, eps, d.x0,
+                                                                   d.params, pc, d.pparams, ppc, plant_profile, d.w, d.v,
+                                                                   d.xk, d.uk, d.Uk, d.cost, d.inner, d.qpit, d.status);
+                      });
 }
 
 // ------------------------------------------------------------------------------------------------ getWLc
@@ -905,12 +907,11 @@ int ntm_getWLc(ntm_handle *h, int layout, int S, int N, const double *bounds, co
     REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
     REQUIRE(bounds && Gamma && Phi && Lambda && W && L && c, "NULL array");
     const size_t s = (size_t)S, n = (size_t)N, r = 6 * n + 4;
-    Arena A(h);
-    A.want(2 * n * n * s * 8); A.want(4 * n * s * 8); A.want(2 * n * s * 8);
-    A.want(r * 2 * s * 8); A.want(r * n * s * 8); A.want(r * s * 8);
-    TRY(A.reserve());
-    double *dGam = A.take<double>(2 * n * n * s), *dPhi = A.take<double>(4 * n * s), *dLam = A.take<double>(2 * n * s);
-    double *dW = A.take<double>(r * 2 * s), *dL = A.take<double>(r * n * s), *dc = A.take<double>(r * s);
+    double *dGam, *dPhi, *dLam, *dW, *dL, *dc;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        dGam = A.take<double>(2 * n * n * s); dPhi = A.take<double>(4 * n * s); dLam = A.take<double>(2 * n * s);
+        dW = A.take<double>(r * 2 * s); dL = A.take<double>(r * n * s); dc = A.take<double>(r * s);
+    }));
     TRY(h2d(h, dGam, Gamma, 2 * n * n * s)); TRY(h2d(h, dPhi, Phi, 4 * n * s)); TRY(h2d(h, dLam, Lambda, 2 * n * s));
     TRY(ntm_getWLc_dev(h, layout, S, N, bounds, dGam, dPhi, dLam, dW, dL, dc));
     TRY(d2h(h, W, dW, r * 2 * s)); TRY(d2h(h, L, dL, r * n * s)); TRY(d2h(h, c, dc, r * s));
@@ -969,13 +970,13 @@ int ntm_mc_stats(ntm_handle *h, int layout, int S, int k_sim, const double *xk, 
         REQUIRE(xk && uk, "NULL array");
     }
     const size_t s = (size_t)S, k = (size_t)k_sim;
-    Arena A(h);
-    A.want(2 * (k + 1) * s * 8 + 8); A.want(k * s * 8 + 8); A.want(s * 8 + 8); A.want(s * 4 + 8);
-    A.want((size_t)pc * NTM_NPARAM * 8 + 8); A.want(NTM_MC_NSTAT * 8);
-    TRY(A.reserve());
-    double *dx = A.take<double>(2 * (k + 1) * s + 1), *du = A.take<double>(k * s + 1), *dc = A.take<double>(s + 1);
-    int *dst = A.take<int>(s + 2);
-    double *dp = A.take<double>((size_t)(S > 0 ? pc : 0) * NTM_NPARAM + 1), *dout = A.take<double>(NTM_MC_NSTAT);
+    double *dx, *du, *dc, *dp, *dout;
+    int *dst;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        dx = A.take<double>(2 * (k + 1) * s + 1); du = A.take<double>(k * s + 1); dc = A.take<double>(s + 1);
+        dst = A.take<int>(s + 2);
+        dp = A.take<double>((size_t)(S > 0 ? pc : 0) * NTM_NPARAM + 1); dout = A.take<double>(NTM_MC_NSTAT);
+    }));
     if (S > 0) {
         TRY(h2d(h, dx, xk, 2 * (k + 1) * s)); TRY(h2d(h, du, uk, k * s));
         if (cost) TRY(h2d(h, dc, cost, s));

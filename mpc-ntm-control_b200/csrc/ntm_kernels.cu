@@ -7,9 +7,12 @@
 //   hessian_grad_kernel<GW>  NTM_MPC_Sim.m:72-73 for arbitrary dense Phi/Gamma/Lambda.
 //   qp_box_kernel<GW>        NTM_MPC_Sim.m:97 (box rows only) for arbitrary SPD G.
 //   rho/lpv/plant kernels    rho1-3.m, A.m, B.m, NTM_MPC_Sim.m:130, one thread per scenario.
+#include <climits>
 #include <cstdint>
 #include <cstdlib>
+#include <map>
 #include <mutex>
+#include <tuple>
 #include <utility>
 #include <vector>
 #include "ntm_device.cuh"
@@ -1462,28 +1465,43 @@ template <typename K>
 static cudaError_t persistent_geometry(K kernel, const DeviceProps &dp, int block, size_t smem, int groups_needed,
                                        int groups_per_block, int *grid) {
     // The occupancy query costs several microseconds of host time -- a visible part of a single-scenario MPC step --
-    // so the answer is cached per kernel instantiation and shared-memory size.
-    static thread_local size_t cached_smem = ~(size_t)0;
-    static thread_local int cached_block = 0, cached_occ = 0, cached_dev = -1;
-    static thread_local const void *cached_fn = nullptr;
+    // so the answers are cached per thread, keyed by (kernel, block, shared memory, device).
+    static thread_local std::map<std::tuple<const void *, int, size_t, int>, int> cache;
+    if (smem > dp.smem_optin) return cudaErrorInvalidConfiguration;
+    const void *fn = reinterpret_cast<const void *>(kernel);
     int dev = 0;
     cudaGetDevice(&dev);
-    int occ = cached_occ;
-    if (smem > dp.smem_optin) return cudaErrorInvalidConfiguration;
-    if (cached_fn != reinterpret_cast<const void *>(kernel) || cached_smem != smem || cached_block != block || cached_dev != dev) {
-        cudaError_t e = raise_smem_attribute(reinterpret_cast<const void *>(kernel), dev, dp.smem_optin);
+    const auto key = std::make_tuple(fn, block, smem, dev);
+    auto hit = cache.find(key);
+    if (hit == cache.end()) {
+        cudaError_t e = raise_smem_attribute(fn, dev, dp.smem_optin);
         if (e != cudaSuccess) return e;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, block, smem);
+        int occ = 0;
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, block, smem);
         if (e != cudaSuccess) return e;
-        cached_fn = reinterpret_cast<const void *>(kernel);
-        cached_smem = smem; cached_block = block; cached_occ = occ; cached_dev = dev;
+        hit = cache.emplace(key, occ).first;
     }
+    const int occ = hit->second;
     if (occ < 1) return cudaErrorInvalidConfiguration;
     const long long cap = (long long)occ * dp.sm_count;
     const long long need = ((long long)groups_needed + groups_per_block - 1) / groups_per_block;
     *grid = (int)(need < cap ? need : cap);
     if (*grid < 1) *grid = 1;
     return cudaSuccess;
+}
+
+// Launch of a persistent kernel whose groups (groups_per_block per CTA) pull work from a queue: as many CTAs as are
+// resident at once, at most those the groups need, and at most group_cap groups (one global LDL' slab each).
+template <typename... P, typename... A>
+static cudaError_t launch_persistent(cudaStream_t st, const DeviceProps &dp, void (*kernel)(P...), int block, size_t smem,
+                                     int groups, int groups_per_block, int group_cap, long long *launches, A... args) {
+    int grid = 1;
+    const cudaError_t e = persistent_geometry(kernel, dp, block, smem, groups, groups_per_block, &grid);
+    if (e != cudaSuccess) return e;
+    if (grid * groups_per_block > group_cap) grid = group_cap / groups_per_block;
+    kernel<<<grid, block, smem, st>>>(args...);
+    ++*launches;
+    return cudaGetLastError();
 }
 
 // ---- two-phase launch: counting sort of the phase-A cost keys, largest key first -----------------------------------
@@ -1507,7 +1525,7 @@ static inline bool lpt_enabled() {
 // Worth it when the launch runs more than one "round" of resident warps and the state fits a sane buffer; one-warp box
 // loop on the literal Gamma with F from x0 (the headline instantiation) only.
 size_t lpt_doubles(const DeviceProps &dp, const LoopArgs &a) {
-    if (!lpt_enabled() || gw_for(a.N) != 1 || a.srows != 0 || a.k_sim < 4) return 0;
+    if (!lpt_enabled() || gw_for(a.N) != 1 || a.srows != 0 || a.ctl || a.pert || a.k_sim < 4) return 0;
     if (a.flags & (NTM_PROFILE_GAMMA_I | NTM_PROFILE_DENSE_G | NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W | NTM_PROFILE_F_XK)) return 0;
     // Measured (profiles/README.md, round 2): -8..9 % at 16 k-64 k scenarios, -20 % with the eps_break stop rule.  At 8,192
     // (2.8 rounds of resident warps) it is a wash -- the eight 8,192-scenario shards of config 3 take 4.7-7.2 ms (mean 5.54)
@@ -1518,105 +1536,130 @@ size_t lpt_doubles(const DeviceProps &dp, const LoopArgs &a) {
     return (size_t)a.S * NTM_CTRL_DOUBLES(a.N);
 }
 
-cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches) {
-    if (a.S <= 0) return cudaSuccess;
-    if (a.hscratch == nullptr) return cudaErrorInvalidValue;
+// Every closed_loop_kernel instantiation of this translation unit; the long-horizon ones are in ntm_loop_long.cu.
+static const LoopKernel kLoopKernels[] = {
+    // one-warp groups (N <= 32); the controller step on the box QP is their runtime mode LoopArgs::ctl
+    {{1, false, EXT_BOX, 0, false}, closed_loop_kernel<1, false, EXT_BOX>},
+    {{1, true, EXT_BOX, 0, false}, closed_loop_kernel<1, true, EXT_BOX>},
+    {{1, false, EXT_COLD_PLANT, 0, false}, closed_loop_kernel<1, false, EXT_COLD_PLANT>},
+    {{1, true, EXT_COLD_PLANT, 0, false}, closed_loop_kernel<1, true, EXT_COLD_PLANT>},
+    {{1, false, EXT_STATE_ROWS, 0, false}, closed_loop_kernel<1, false, EXT_STATE_ROWS>},
+    {{1, true, EXT_STATE_ROWS, 0, false}, closed_loop_kernel<1, true, EXT_STATE_ROWS>},
+    {{1, false, EXT_STATE_ROWS, 0, true}, closed_loop_kernel<1, false, EXT_STATE_ROWS, 0, true>},
+    {{1, true, EXT_STATE_ROWS, 0, true}, closed_loop_kernel<1, true, EXT_STATE_ROWS, 0, true>},
+    {{1, false, EXT_PERTURBED, 0, false}, closed_loop_kernel<1, false, EXT_PERTURBED>},
+    {{1, true, EXT_PERTURBED, 0, false}, closed_loop_kernel<1, true, EXT_PERTURBED>},
+    // multi-warp groups, dense Gamma
+    {{2, true, EXT_BOX, 0, false}, closed_loop_kernel<2, true, EXT_BOX>},
+    {{4, true, EXT_BOX, 0, false}, closed_loop_kernel<4, true, EXT_BOX>},
+    {{2, true, EXT_BOX, 0, true}, closed_loop_kernel<2, true, EXT_BOX, 0, true>},
+    {{4, true, EXT_BOX, 0, true}, closed_loop_kernel<4, true, EXT_BOX, 0, true>},
+    {{2, true, EXT_COLD_PLANT, 0, false}, closed_loop_kernel<2, true, EXT_COLD_PLANT>},
+    {{4, true, EXT_COLD_PLANT, 0, false}, closed_loop_kernel<4, true, EXT_COLD_PLANT>},
+    {{2, true, EXT_PERTURBED, 0, false}, closed_loop_kernel<2, true, EXT_PERTURBED>},
+    {{4, true, EXT_PERTURBED, 0, false}, closed_loop_kernel<4, true, EXT_PERTURBED>},
+    // multi-warp groups, literal Gamma, state rows
+    {{2, false, EXT_STATE_ROWS, 0, false}, closed_loop_kernel<2, false, EXT_STATE_ROWS>},
+    {{4, false, EXT_STATE_ROWS, 0, false}, closed_loop_kernel<4, false, EXT_STATE_ROWS>},
+    {{2, false, EXT_STATE_ROWS, 0, true}, closed_loop_kernel<2, false, EXT_STATE_ROWS, 0, true>},
+    {{4, false, EXT_STATE_ROWS, 0, true}, closed_loop_kernel<4, false, EXT_STATE_ROWS, 0, true>},
+};
+
+// The launch of one fused call: the instantiation and its shape.
+struct LoopRoute {
+    LoopKey key;
+    bool lng;                      // in kLongLoopKernels (ntm_loop_long.cu)
+    int block, groups_per_block, group_cap;
+    size_t smem, gbytes;           // dynamic shared memory per CTA / per group
+};
+
+// Every rule that picks the closed_loop_kernel instantiation of a call, and its launch shape.  Sets the launcher-owned
+// fields of a: hcap, gam, wbytes, qbytes, rows_warm.
+static cudaError_t route_closed_loop(const DeviceProps &dp, LoopArgs &a, LoopRoute &r) {
     const int gw = gw_for(a.N);
-    const int N_ = a.N;
-    LoopArgs aa = a;
-    aa.k_begin = 0; aa.k_end = a.k_sim; aa.lpt_key = nullptr; aa.perm = nullptr;
     const bool dense = (a.flags & (NTM_PROFILE_GAMMA_I | NTM_PROFILE_DENSE_G)) != 0;
+    // the headline instantiations carry none of the cold options
+    const int ext = a.pert ? EXT_PERTURBED
+                  : a.srows != 0 ? EXT_STATE_ROWS
+                  : (a.flags & (NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)) ? EXT_COLD_PLANT : EXT_BOX;
+    // long horizons, literal Gamma, box QP: the sweep tableau, in registers while N + 1 fits 7 x 15 blocks, else in shared
+    // memory (LV = 1)
+    r.lng = gw > 1 && !dense && ext != EXT_STATE_ROWS;
+    // the controller step is a runtime mode of the one-warp box kernels and its own instantiation (CTL) wherever that mode
+    // would cost registers (DESIGN section 4.8)
+    const bool ctl = a.ctl != 0 && (ext == EXT_STATE_ROWS || (gw > 1 && ext == EXT_BOX));
+    r.key = {gw, dense, ext, (r.lng && a.N + 1 > NTM_TS * 15) ? 1 : 0, ctl};
     // dense Gamma on the FP64 tensor cores: a full staging tile per warp (one-warp groups), a 16-row chunk buffer for the
     // multi-warp groups whose ceil8(N + 1) columns fit the group's threads and NTM_DMAXT tiles per warp (N <= 63 / 103)
-    aa.gam = 0;
-    if (dense && gw == 1) aa.gam = 1;
+    a.gam = 0;
+    if (dense && gw == 1) a.gam = 1;
     else if (dense && a.srows == 0) {
         const int Np = (a.N + 1 + 7) & ~7, nt = Np >> 3;
-        if (Np <= 32 * gw && (nt * (nt + 1) / 2 + gw - 1) / gw <= NTM_DMAXT) aa.gam = 2;
+        if (Np <= 32 * gw && (nt * (nt + 1) / 2 + gw - 1) / gw <= NTM_DMAXT) a.gam = 2;
     }
-    aa.hcap = hcap_loop(dp, a.N, aa.gam);
-    // EXT = the instantiation that also carries the cold options (RK4 plant, state rows); the headline kernels carry
-    // none of that code; EXT = 3 (perturbed plant, box QP) has its own instantiations
-    const int ext = a.pert ? 3 : (a.srows != 0 ? 2 : ((a.flags & (NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)) ? 1 : 0));
-    size_t gbytes = work_bytes(a.N, aa.hcap, aa.gam);
+    a.hcap = hcap_loop(dp, a.N, a.gam);
     {
         static const char *env = getenv("NTM_ROWS_WARM");  // diagnostic: 0 = every state-row QP starts cold
-        aa.rows_warm = (env == nullptr || atoi(env) != 0) ? 1 : 0;
+        a.rows_warm = (env == nullptr || atoi(env) != 0) ? 1 : 0;
     }
-    int wpb1 = 4;                                          // warps (= scenarios) per CTA of the one-warp instantiations
+    size_t gbytes = work_bytes(a.N, a.hcap, a.gam);
+    int gpb = gw == 1 ? 4 : 1;                               // groups (= scenarios) per CTA
     if (a.srows != 0) {
         if (a.srows < 0 || a.srows > 2) return cudaErrorInvalidValue;
         if (dense && gw != 1) return cudaErrorInvalidValue;   // rows of a non-literal Gamma are read from the per-warp tile: N <= 32
-        aa.hcap = a.N;                                   // the continuation keeps R in the LDL' buffer: full size
-        aa.gam = dense ? 1 : 0;
-        const size_t wb = work_bytes(a.N, a.N, aa.gam);
-        aa.wbytes = (unsigned int)wb;
-        aa.qbytes = (unsigned int)(wb + ineq_bytes(a.N, 4 * a.N));
-        gbytes = aa.qbytes + ext_bytes(a.N);
+        a.hcap = a.N;                                    // the continuation keeps R in the LDL' buffer: full size
+        a.gam = dense ? 1 : 0;
+        const size_t wb = work_bytes(a.N, a.N, a.gam);
+        a.wbytes = (unsigned int)wb;
+        a.qbytes = (unsigned int)(wb + ineq_bytes(a.N, 4 * a.N));
+        gbytes = a.qbytes + ext_bytes(a.N);
         if (dense && a.srows == 2) gbytes += gam_doubles(a.N, 1) * sizeof(double);   // frozen rows: the offline tile
-        if (gw == 1) while (wpb1 > 1 && gbytes * wpb1 > dp.smem_optin) --wpb1;
-        if (gbytes * (gw == 1 ? wpb1 : 1) > dp.smem_optin) return cudaErrorInvalidValue;
+        while (gpb > 1 && gbytes * gpb > dp.smem_optin) --gpb;
+        if (gbytes * gpb > dp.smem_optin) return cudaErrorInvalidValue;
     }
-    cudaError_t e = cudaSuccess;                       // a.counter[0..1] are zero: armed at creation, re-armed by each launch
-    int grid = 1;
-#define NTM_LAUNCH_LOOP1(GWV, DV, EV, BLOCK, SMEM, GPB)                                                     \
-    do {                                                                                                    \
-        e = persistent_geometry(closed_loop_kernel<GWV, DV, EV>, dp, BLOCK, SMEM, a.S, GPB, &grid);         \
-        if (e != cudaSuccess) return e;                                                                     \
-        if (grid * (GPB) > max_groups(dp, N_)) grid = max_groups(dp, N_) / (GPB);                           \
-        closed_loop_kernel<GWV, DV, EV><<<grid, BLOCK, SMEM, st>>>(aa, (unsigned int)gbytes);                \
-    } while (0)
-#define NTM_LAUNCH_LOOP(GWV, BLOCK, SMEM, GPB)                                                              \
-    do {                                                                                                    \
-        if (ext == 2 && a.ctl) { if (dense) NTM_LAUNCH_LOOP1(GWV, true, NTM_CTL_SC, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, NTM_CTL_SC, BLOCK, SMEM, GPB); } \
-        else if (ext == 2) { if (dense) NTM_LAUNCH_LOOP1(GWV, true, 2, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 2, BLOCK, SMEM, GPB); } \
-        else if (ext == 3) { if (dense) NTM_LAUNCH_LOOP1(GWV, true, 3, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 3, BLOCK, SMEM, GPB); } \
-        else if (dense) { if (ext) NTM_LAUNCH_LOOP1(GWV, true, 1, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, true, 0, BLOCK, SMEM, GPB); } \
-        else { if (ext) NTM_LAUNCH_LOOP1(GWV, false, 1, BLOCK, SMEM, GPB); else NTM_LAUNCH_LOOP1(GWV, false, 0, BLOCK, SMEM, GPB); }         \
-    } while (0)
-#define NTM_CTL_EXT 0, 0, true                             // EXT = 0, LV = 0, CTL: multi-warp controller-step instantiation
-#define NTM_CTL_SC 2, 0, true                              // EXT = 2, LV = 0, CTL: state-row controller-step instantiation
-    if (gw == 1) {
-        const int wpb = wpb1;
-        const size_t smem = gbytes * wpb;
-        if (a.lpt != nullptr && a.sv != nullptr && lpt_doubles(dp, a) != 0) {
-            // phase A: time step 0 of every scenario (state + cost key), counting sort, phase B: the rest, longest first
-            int *key = a.lpt, *perm = a.lpt + a.S, *bins = a.lpt + 2 * (size_t)a.S;
-            e = cudaMemsetAsync(bins, 0, NTM_LPT_BINS * sizeof(int), st);
-            if (e != cudaSuccess) return e;
-            aa.k_begin = 0; aa.k_end = 1; aa.lpt_key = key;
-            NTM_LAUNCH_LOOP1(1, false, 0, 32 * wpb, smem, wpb);
-            lpt_hist_kernel<<<(a.S + 255) / 256, 256, 0, st>>>(a.S, key, bins);
-            lpt_scan_kernel<<<1, 1, 0, st>>>(bins);
-            lpt_scatter_kernel<<<(a.S + 255) / 256, 256, 0, st>>>(a.S, key, bins, perm);
-            *launches += 4;
-            aa.k_begin = 1; aa.k_end = a.k_sim; aa.lpt_key = nullptr; aa.perm = perm;
-        }
-        NTM_LAUNCH_LOOP(1, 32 * wpb, smem, wpb);
-    } else if (!dense && ext != 2) {
-        // long horizons, literal Gamma, box QP: the sweep-tableau instantiations live in ntm_loop_long.cu
-        return launch_closed_loop_long(st, dp, aa, launches);
-    } else if (gw == 2) {
-        if (ext == 2 && a.ctl) NTM_LAUNCH_LOOP1(2, false, NTM_CTL_SC, 64, gbytes, 1);   // controller step, state rows
-        else if (ext == 2) NTM_LAUNCH_LOOP1(2, false, 2, 64, gbytes, 1);
-        else if (ext == 3) NTM_LAUNCH_LOOP1(2, true, 3, 64, gbytes, 1);      // perturbed plant
-        else if (ext) NTM_LAUNCH_LOOP1(2, true, 1, 64, gbytes, 1);
-        else if (a.ctl) NTM_LAUNCH_LOOP1(2, true, NTM_CTL_EXT, 64, gbytes, 1);   // controller step
-        else NTM_LAUNCH_LOOP1(2, true, 0, 64, gbytes, 1);
-    } else {
-        if (ext == 2 && a.ctl) NTM_LAUNCH_LOOP1(4, false, NTM_CTL_SC, 128, gbytes, 1);
-        else if (ext == 2) NTM_LAUNCH_LOOP1(4, false, 2, 128, gbytes, 1);
-        else if (ext == 3) NTM_LAUNCH_LOOP1(4, true, 3, 128, gbytes, 1);      // perturbed plant
-        else if (ext) NTM_LAUNCH_LOOP1(4, true, 1, 128, gbytes, 1);
-        else if (a.ctl) NTM_LAUNCH_LOOP1(4, true, NTM_CTL_EXT, 128, gbytes, 1);
-        else NTM_LAUNCH_LOOP1(4, true, 0, 128, gbytes, 1);
+    r.block = 32 * gw * gpb;
+    r.groups_per_block = gpb;
+    r.group_cap = max_groups(dp, a.N);
+    if (r.lng) {                                           // one CTA per scenario, no global LDL' slabs
+        gbytes = work_bytes_long(a.N);
+        r.group_cap = INT_MAX;
     }
-#undef NTM_LAUNCH_LOOP1
-#undef NTM_LAUNCH_LOOP
-#undef NTM_CTL_EXT
-#undef NTM_CTL_SC
-    ++*launches;
-    return cudaGetLastError();
+    r.gbytes = gbytes;
+    r.smem = gbytes * gpb;
+    return cudaSuccess;
+}
+
+cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches) {
+    if (a.S <= 0) return cudaSuccess;
+    if (a.hscratch == nullptr) return cudaErrorInvalidValue;
+    LoopArgs aa = a;
+    aa.k_begin = 0; aa.k_end = a.k_sim; aa.lpt_key = nullptr; aa.perm = nullptr;
+    LoopRoute r;
+    cudaError_t e = route_closed_loop(dp, aa, r);
+    if (e != cudaSuccess) return e;
+    const LoopKernelFn fn = r.lng ? find_long_loop_kernel(r.key) : find_loop_kernel(kLoopKernels, r.key);
+    if (fn == nullptr) return cudaErrorInvalidDeviceFunction;
+    // a.counter[0..1] are zero: armed at creation, re-armed by each launch
+    auto launch = [&] {
+        return launch_persistent(st, dp, fn, r.block, r.smem, a.S, r.groups_per_block, r.group_cap, launches, aa,
+                                 (unsigned int)r.gbytes);
+    };
+    if (a.lpt != nullptr && a.sv != nullptr && lpt_doubles(dp, a) != 0) {
+        // phase A: time step 0 of every scenario (state + cost key), counting sort, phase B: the rest, longest first.
+        // lpt_doubles admits the headline instantiation <1, false, EXT_BOX> only.
+        int *key = a.lpt, *perm = a.lpt + a.S, *bins = a.lpt + 2 * (size_t)a.S;
+        e = cudaMemsetAsync(bins, 0, NTM_LPT_BINS * sizeof(int), st);
+        if (e != cudaSuccess) return e;
+        aa.k_begin = 0; aa.k_end = 1; aa.lpt_key = key;
+        e = launch();
+        if (e != cudaSuccess) return e;
+        lpt_hist_kernel<<<(a.S + 255) / 256, 256, 0, st>>>(a.S, key, bins);
+        lpt_scan_kernel<<<1, 1, 0, st>>>(bins);
+        lpt_scatter_kernel<<<(a.S + 255) / 256, 256, 0, st>>>(a.S, key, bins, perm);
+        *launches += 3;
+        aa.k_begin = 1; aa.k_end = a.k_sim; aa.lpt_key = nullptr; aa.perm = perm;
+    }
+    return launch();
 }
 
 cudaError_t launch_qp_box(cudaStream_t st, const DeviceProps &dp, int layout, int S, int N, const double *G,
@@ -1624,35 +1667,13 @@ cudaError_t launch_qp_box(cudaStream_t st, const DeviceProps &dp, int layout, in
                           int *status, unsigned int *counter, double *hscratch, long long *launches) {
     if (S <= 0) return cudaSuccess;
     if (hscratch == nullptr) return cudaErrorInvalidValue;
-    const int gw = gw_for(N);
-    const int N_ = N;
+    const int gw = gw_for(N), wpb = gw == 1 ? 4 : 1;
     const int hcap = hcap_qp(dp, N);
     const size_t gbytes = work_bytes(N, hcap);
-    cudaError_t e = cudaSuccess;                       // counter[0..1] are zero: armed at creation, re-armed by each launch
-    int grid = 1;
-    if (gw == 1) {
-        const int wpb = 4;
-        const size_t smem = gbytes * wpb;
-        e = persistent_geometry(qp_box_kernel<1>, dp, 32 * wpb, smem, S, wpb, &grid);
-        if (e != cudaSuccess) return e;
-        if (grid * wpb > max_groups(dp, N_)) grid = max_groups(dp, N_) / wpb;
-        qp_box_kernel<1><<<grid, 32 * wpb, smem, st>>>(layout, S, N, G, F, lb, ub, bc, U, iters, status, counter,
-                                                       (unsigned int)gbytes, hscratch, hcap);
-    } else if (gw == 2) {
-        e = persistent_geometry(qp_box_kernel<2>, dp, 64, gbytes, S, 1, &grid);
-        if (e != cudaSuccess) return e;
-        if (grid > max_groups(dp, N_)) grid = max_groups(dp, N_);
-        qp_box_kernel<2><<<grid, 64, gbytes, st>>>(layout, S, N, G, F, lb, ub, bc, U, iters, status, counter,
-                                                   (unsigned int)gbytes, hscratch, hcap);
-    } else {
-        e = persistent_geometry(qp_box_kernel<4>, dp, 128, gbytes, S, 1, &grid);
-        if (e != cudaSuccess) return e;
-        if (grid > max_groups(dp, N_)) grid = max_groups(dp, N_);
-        qp_box_kernel<4><<<grid, 128, gbytes, st>>>(layout, S, N, G, F, lb, ub, bc, U, iters, status, counter,
-                                                    (unsigned int)gbytes, hscratch, hcap);
-    }
-    ++*launches;
-    return cudaGetLastError();
+    const auto kernel = gw == 1 ? qp_box_kernel<1> : (gw == 2 ? qp_box_kernel<2> : qp_box_kernel<4>);
+    // counter[0..1] are zero: armed at creation, re-armed by each launch
+    return launch_persistent(st, dp, kernel, 32 * gw * wpb, gbytes * wpb, S, wpb, max_groups(dp, N), launches, layout, S,
+                             N, G, F, lb, ub, bc, U, iters, status, counter, (unsigned int)gbytes, hscratch, hcap);
 }
 
 // returns cudaErrorInvalidConfiguration when N x N factor pair + row scales do not fit in shared memory
@@ -1664,30 +1685,12 @@ cudaError_t launch_qp_ineq(cudaStream_t st, const DeviceProps &dp, int layout, i
     const int gw = gw_for(N);
     const size_t wbytes = work_bytes(N, N);
     const size_t gbytes = wbytes + ineq_bytes(N, M);
-    cudaError_t e = cudaSuccess;
-    int grid = 1;
     int wpb = (gw == 1) ? 4 : 1;
     while (wpb > 1 && gbytes * wpb + 1024 > dp.smem_optin) wpb >>= 1;
     if (gbytes * wpb + 1024 > dp.smem_optin) return cudaErrorInvalidConfiguration;
-    if (gw == 1) {
-        const size_t smem = gbytes * wpb;
-        e = persistent_geometry(qp_ineq_kernel<1>, dp, 32 * wpb, smem, S, wpb, &grid);
-        if (e != cudaSuccess) return e;
-        qp_ineq_kernel<1><<<grid, 32 * wpb, smem, st>>>(layout, S, N, M, G, F, lb, ub, bc, Lg, bg, U, iters, status,
-                                                        counter, (unsigned int)gbytes, (unsigned int)wbytes);
-    } else if (gw == 2) {
-        e = persistent_geometry(qp_ineq_kernel<2>, dp, 64, gbytes, S, 1, &grid);
-        if (e != cudaSuccess) return e;
-        qp_ineq_kernel<2><<<grid, 64, gbytes, st>>>(layout, S, N, M, G, F, lb, ub, bc, Lg, bg, U, iters, status,
-                                                    counter, (unsigned int)gbytes, (unsigned int)wbytes);
-    } else {
-        e = persistent_geometry(qp_ineq_kernel<4>, dp, 128, gbytes, S, 1, &grid);
-        if (e != cudaSuccess) return e;
-        qp_ineq_kernel<4><<<grid, 128, gbytes, st>>>(layout, S, N, M, G, F, lb, ub, bc, Lg, bg, U, iters, status,
-                                                     counter, (unsigned int)gbytes, (unsigned int)wbytes);
-    }
-    ++*launches;
-    return cudaGetLastError();
+    const auto kernel = gw == 1 ? qp_ineq_kernel<1> : (gw == 2 ? qp_ineq_kernel<2> : qp_ineq_kernel<4>);
+    return launch_persistent(st, dp, kernel, 32 * gw * wpb, gbytes * wpb, S, wpb, INT_MAX, launches, layout, S, N, M, G,
+                             F, lb, ub, bc, Lg, bg, U, iters, status, counter, (unsigned int)gbytes, (unsigned int)wbytes);
 }
 
 // umin / umax of scenario s are umin[s * ustride] / umax[s * ustride] (ustride 0: one shared pair)

@@ -97,8 +97,32 @@ cudaError_t launch_mc_stats(cudaStream_t st, const DeviceProps &dp, int layout, 
                             const double *uk, const double *cost, const int *status, const double *umin, const double *umax,
                             int ustride, const double *bounds, double w_sup, double hist_max, double *out, long long *launches);
 cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches);
-// N > 32, literal Gamma, box QP (ntm_loop_long.cu); called by launch_closed_loop
-cudaError_t launch_closed_loop_long(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches);
+
+// EXT template argument of closed_loop_kernel (ntm_loop.cuh): the cold code an instantiation carries
+constexpr int EXT_BOX = 0;          // the headline instantiations: Euler plant, box QP
+constexpr int EXT_COLD_PLANT = 1;   // + the RK4 / tau_E(w) plant options
+constexpr int EXT_STATE_ROWS = 2;   // + getWLc's state rows
+constexpr int EXT_PERTURBED = 3;    // box QP against a perturbed plant (LoopArgs::pert)
+// one instantiation closed_loop_kernel<gw, dense, ext, lv, ctl>
+struct LoopKey {
+    int gw;
+    bool dense;
+    int ext, lv;
+    bool ctl;
+};
+using LoopKernelFn = void (*)(LoopArgs, unsigned int);
+struct LoopKernel {
+    LoopKey key;
+    LoopKernelFn fn;
+};
+template <int N>
+inline LoopKernelFn find_loop_kernel(const LoopKernel (&table)[N], const LoopKey &k) {
+    for (const LoopKernel &t : table)
+        if (t.key.gw == k.gw && t.key.dense == k.dense && t.key.ext == k.ext && t.key.lv == k.lv && t.key.ctl == k.ctl) return t.fn;
+    return nullptr;
+}
+// the long-horizon instantiations (N > 32, literal Gamma, box QP), compiled in ntm_loop_long.cu
+LoopKernelFn find_long_loop_kernel(const LoopKey &k);
 // raises cudaFuncAttributeMaxDynamicSharedMemorySize of a kernel to the device maximum, once per (kernel, device)
 cudaError_t raise_smem_attribute(const void *fn, int dev, size_t smem_optin);
 cudaError_t launch_fp64_peak(cudaStream_t st, const DeviceProps &dp, int iters, double *out, long long *launches);

@@ -43,6 +43,19 @@ def _blocks_out(flat: np.ndarray, S: int, rows: int, cols: int) -> np.ndarray:
     return flat.reshape(S, cols, rows).transpose(0, 2, 1)
 
 
+_LOOP_KEYS = ("xk", "uk", "Uk", "cost", "inner_iters", "qp_iters", "status")
+
+
+def _loop_result(arrays) -> dict:
+    """The result dict of a closed-loop call from the arrays ``_loop_outputs`` returned (``Uk`` None unless wanted)."""
+    return dict(zip(_LOOP_KEYS, arrays))
+
+
+def _state_box(state_rows: int, xbounds):
+    """The state box of the ``_sc`` entries: ``xbounds`` (default the script's own), or None with the rows off."""
+    return _f64(MC_STATE_BOX if xbounds is None else xbounds).reshape(4) if state_rows else None
+
+
 def _loop_outputs(out, S: int, N: int, k_sim: int, want_Uk: bool):
     """Output arrays of a closed-loop call: fresh ones, or the caller's preallocated (e.g. pinned) ones from ``out``.
     The C ABI writes through raw addresses, so a supplied array must be exactly what the library expects --
@@ -52,7 +65,7 @@ def _loop_outputs(out, S: int, N: int, k_sim: int, want_Uk: bool):
                 status=((S,), np.int32))
     o = out if out is not None else {}
     res = []
-    for key in ("xk", "uk", "Uk", "cost", "inner_iters", "qp_iters", "status"):
+    for key in _LOOP_KEYS:
         shape, dt = spec[key]
         a = o.get(key)
         if key == "Uk" and not want_Uk:
@@ -118,7 +131,8 @@ def closed_loop_multi(x0, params, N: int, k_sim: int = 20, i_sim: int = 10, eps:
     if p.shape not in ((1, NPARAM), (S, NPARAM)):
         raise ValueError(f"params must be [{NPARAM}] or [S,{NPARAM}], got {p.shape}")
     pc = int(p.shape[0])
-    xk, uk, Uk, cost, inner, qpit, status = _loop_outputs(out, S, N, k_sim, want_Uk)
+    outs = _loop_outputs(out, S, N, k_sim, want_Uk)
+    xk, uk, Uk, cost, inner, qpit, status = outs
     if devices is None:
         nd, dv = 0, None
     elif isinstance(devices, int):
@@ -131,7 +145,7 @@ def closed_loop_multi(x0, params, N: int, k_sim: int = 20, i_sim: int = 10, eps:
                                            i_sim, eps, _ptr(x0), _ptr(p), pc, int(state_rows),
                                            _ptr(xb) if state_rows else None, _ptr(xk), _ptr(uk),
                                            _ptr(Uk) if want_Uk else None, _ptr(cost), _ptr(inner), _ptr(qpit), _ptr(status)))
-    return dict(xk=xk, uk=uk, Uk=Uk if want_Uk else None, cost=cost, inner_iters=inner, qp_iters=qpit, status=status)
+    return _loop_result(outs)
 
 
 
@@ -339,18 +353,12 @@ class NtmMpc:
         x0 = _f64(x0).reshape(-1, 2)
         S = x0.shape[0]
         p, pc = self._params(params, S)
-        xk, uk, Uk, cost, inner, qpit, status = _loop_outputs(out, S, N, k_sim, want_Uk)
-        if state_rows:
-            xb = _f64(MC_STATE_BOX if xbounds is None else xbounds).reshape(4)
-            check(self._lib.ntm_mpc_closed_loop_sc(self._h, LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, _ptr(x0), _ptr(p),
-                                                   pc, int(state_rows), _ptr(xb), _ptr(xk), _ptr(uk),
-                                                   _ptr(Uk) if want_Uk else None, _ptr(cost), _ptr(inner), _ptr(qpit),
-                                                   _ptr(status)))
-            return dict(xk=xk, uk=uk, Uk=Uk if want_Uk else None, cost=cost, inner_iters=inner, qp_iters=qpit, status=status)
-        check(self._lib.ntm_mpc_closed_loop(self._h, LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, _ptr(x0), _ptr(p), pc,
-                                            _ptr(xk), _ptr(uk), _ptr(Uk) if want_Uk else None, _ptr(cost), _ptr(inner),
-                                            _ptr(qpit), _ptr(status)))
-        return dict(xk=xk, uk=uk, Uk=Uk if want_Uk else None, cost=cost, inner_iters=inner, qp_iters=qpit, status=status)
+        outs = _loop_outputs(out, S, N, k_sim, want_Uk)
+        xk, uk, Uk, cost, inner, qpit, status = outs
+        check(self._lib.ntm_mpc_closed_loop_sc(self._h, LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, _ptr(x0), _ptr(p),
+                                               pc, int(state_rows), _ptr(_state_box(state_rows, xbounds)), _ptr(xk),
+                                               _ptr(uk), _ptr(Uk), _ptr(cost), _ptr(inner), _ptr(qpit), _ptr(status)))
+        return _loop_result(outs)
 
     def closed_loop_dev(self, S: int, N: int, k_sim: int, i_sim: int, eps: float, profile: int, layout: int,
                         x0_ptr: int, params_ptr: int, params_count: int, xk_ptr: int, uk_ptr: int, Uk_ptr: int = 0,
@@ -390,12 +398,13 @@ class NtmMpc:
         judged on them."""
         x0, p, pc, pp, ppc, pf, wf, vf = perturbed_inputs(x0, params, plant_params, plant_profile, w, v, k_sim, profile)
         S = x0.shape[0]
-        xk, uk, Uk, cost, inner, qpit, status = _loop_outputs(out, S, N, k_sim, want_Uk)
+        outs = _loop_outputs(out, S, N, k_sim, want_Uk)
+        xk, uk, Uk, cost, inner, qpit, status = outs
         check(self._lib.ntm_mpc_closed_loop_perturbed(self._h, LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, _ptr(x0),
                                                       _ptr(p), pc, _ptr(pp), ppc, pf, _ptr(wf), _ptr(vf), _ptr(xk),
                                                       _ptr(uk), _ptr(Uk) if want_Uk else None, _ptr(cost), _ptr(inner),
                                                       _ptr(qpit), _ptr(status)))
-        return dict(xk=xk, uk=uk, Uk=Uk if want_Uk else None, cost=cost, inner_iters=inner, qp_iters=qpit, status=status)
+        return _loop_result(outs)
 
     def closed_loop_perturbed_dev(self, S: int, N: int, k_sim: int, i_sim: int, eps: float, profile: int, layout: int,
                                   x0_ptr: int, params_ptr: int, params_count: int, plant_params_ptr: int,
@@ -432,31 +441,20 @@ class NtmMpc:
         u = np.empty(S)
         U = np.empty((S, N)) if want_U else None
         inner, qpit, status = (np.empty(S, dtype=np.int32) for _ in range(3))
-        if state_rows:
-            xb = _f64(MC_STATE_BOX if xbounds is None else xbounds).reshape(4)
-            check(self._lib.ntm_mpc_step_sc(self._h, LAYOUT_MATLAB, profile, S, N, i_sim, eps, _ptr(x), _ptr(p), pc,
-                                            int(state_rows), _ptr(xb), _ptr(state), _ptr(u), _ptr(U), _ptr(inner),
-                                            _ptr(qpit), _ptr(status)))
-        else:
-            check(self._lib.ntm_mpc_step(self._h, LAYOUT_MATLAB, profile, S, N, i_sim, eps, _ptr(x), _ptr(p), pc,
-                                         _ptr(state), _ptr(u), _ptr(U), _ptr(inner), _ptr(qpit), _ptr(status)))
+        check(self._lib.ntm_mpc_step_sc(self._h, LAYOUT_MATLAB, profile, S, N, i_sim, eps, _ptr(x), _ptr(p), pc,
+                                        int(state_rows), _ptr(_state_box(state_rows, xbounds)), _ptr(state), _ptr(u),
+                                        _ptr(U), _ptr(inner), _ptr(qpit), _ptr(status)))
         return dict(u=u, U=U, inner_iters=inner, qp_iters=qpit, status=status)
 
     def mpc_step_dev(self, S: int, N: int, i_sim: int, eps: float, profile: int, layout: int, x_ptr: int,
                      params_ptr: int, params_count: int, state_ptr: int, u_ptr: int, U_ptr: int = 0, inner_ptr: int = 0,
                      qp_ptr: int = 0, status_ptr: int = 0, state_rows: int = 0, xbounds=None) -> None:
-        """``mpc_step`` on device pointers, asynchronous on the handle's stream (``ntm_mpc_step_dev``, or
-        ``ntm_mpc_step_sc_dev`` with ``state_rows``; ``xbounds`` is a host 4-vector); the records (``ctrl_doubles(N)``
+        """``mpc_step`` on device pointers, asynchronous on the handle's stream (``ntm_mpc_step_sc_dev``, which is
+        ``ntm_mpc_step_dev`` with the state rows off; ``xbounds`` is a host 4-vector); the records (``ctrl_doubles(N)``
         doubles per scenario, scenario slowest) stay resident."""
-        if state_rows:
-            xb = _f64(MC_STATE_BOX if xbounds is None else xbounds).reshape(4)
-            check(self._lib.ntm_mpc_step_sc_dev(self._h, layout, profile, S, N, i_sim, eps, x_ptr, params_ptr,
-                                                params_count, int(state_rows), _ptr(xb), state_ptr, u_ptr, U_ptr or None,
-                                                inner_ptr or None, qp_ptr or None, status_ptr or None))
-            return
-        check(self._lib.ntm_mpc_step_dev(self._h, layout, profile, S, N, i_sim, eps, x_ptr, params_ptr, params_count,
-                                         state_ptr, u_ptr, U_ptr or None, inner_ptr or None, qp_ptr or None,
-                                         status_ptr or None))
+        check(self._lib.ntm_mpc_step_sc_dev(self._h, layout, profile, S, N, i_sim, eps, x_ptr, params_ptr, params_count,
+                                            int(state_rows), _ptr(_state_box(state_rows, xbounds)), state_ptr, u_ptr,
+                                            U_ptr or None, inner_ptr or None, qp_ptr or None, status_ptr or None))
 
     def controller(self, params, N: int, S: Optional[int] = None, i_sim: int = 10, eps: float = 1e-14,
                    profile: int = 0, state_rows: int = 0, xbounds=None) -> "Controller":
