@@ -100,7 +100,7 @@ __device__ __forceinline__ void wlc_element(int layout, int S, int N, int R, con
     if (col < N) {                                            // L
         double v = (xb >= 0) ? sgn * Gam[elem(layout, S, 2 * N * N, s, col * 2 * N + 2 * xb + comp)] : 0.0;
         if (r < 6 * N && col == i) { if (q == 0) v += -1.0; else if (q == 1) v += 1.0; }   // Ecal
-        L[elem(layout, S, R * N, s, col * R + r)] = v;
+        L[elem(layout, S, R * N, s, col * R + r)] = (v == 0.0) ? 0.0 : v;   // -1 * 0 above the diagonal: +0, like the other kernels
     } else if (col < N + 2) {                                 // W = -Dcal - Mcal*Phi
         const int wc = col - N;
         double v = (xb >= 0) ? -sgn * Phi[elem(layout, S, 4 * N, s, wc * 2 * N + 2 * xb + comp)] : 0.0;
@@ -764,15 +764,19 @@ hessian_grad_dmma_kernel(int layout, int S, int N, const double *__restrict__ Ph
     const int g = lane >> 2, t4 = lane & 3;
     // 16-byte copies: MATLAB layout (a column of Gamma is contiguous), 16-byte aligned base; 2N and the chunk start are even
     const bool vec16 = layout == NTM_LAYOUT_MATLAB && (reinterpret_cast<uintptr_t>(Gam) & 15) == 0;
-    // v = Phi x + Lambda - R of scenario sc, entries 2*tid, 2*tid + 1 (N <= 128 < T)
+    // v = Phi x + Lambda - R of scenario sc, entries 2*tid, 2*tid + 1 (N <= 128 < T).  Two call sites (the first scenario,
+    // and the prefetch of the next one inside the chunk loop): explicitly rounded operations, so that the compiler cannot
+    // contract the two copies into FMAs differently and give a scenario other bits as a CTA's second scenario.
     auto vpair = [&](int sc, double &v0, double &v1) {
         const Params P = load_params(params, layout, pc, sc);
         const double xw = x[elem(layout, S, 2, sc, 0)], xo = x[elem(layout, S, 2, sc, 1)];
         const int i = tid;
-        v0 = Phi[elem(layout, S, 4 * N, sc, 2 * i)] * xw + Phi[elem(layout, S, 4 * N, sc, 2 * N + 2 * i)] * xo +
-             Lam[elem(layout, S, 2 * N, sc, 2 * i)] - P.r1;
-        v1 = Phi[elem(layout, S, 4 * N, sc, 2 * i + 1)] * xw + Phi[elem(layout, S, 4 * N, sc, 2 * N + 2 * i + 1)] * xo +
-             Lam[elem(layout, S, 2 * N, sc, 2 * i + 1)] - P.r2;
+        v0 = __dsub_rn(__dadd_rn(__fma_rn(Phi[elem(layout, S, 4 * N, sc, 2 * i)], xw,
+                                          __dmul_rn(Phi[elem(layout, S, 4 * N, sc, 2 * N + 2 * i)], xo)),
+                                 Lam[elem(layout, S, 2 * N, sc, 2 * i)]), P.r1);
+        v1 = __dsub_rn(__dadd_rn(__fma_rn(Phi[elem(layout, S, 4 * N, sc, 2 * i + 1)], xw,
+                                          __dmul_rn(Phi[elem(layout, S, 4 * N, sc, 2 * N + 2 * i + 1)], xo)),
+                                 Lam[elem(layout, S, 2 * N, sc, 2 * i + 1)]), P.r2);
     };
     auto qstore = [&](int sc, double *vb) {
         if (tid == T - 1) {
