@@ -280,8 +280,8 @@ int ntm_mpc_step_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, in
  * profile: what ntm_mpc_step takes (PLANT_C and PLANT_RK4 are ignored, TAUE_W is rejected).  plant_profile: exactly the
  * bits ntm_plant_step honours, RHO1_SQ | PLANT_C | PLANT_RK4 | TAUE_W (c_tauE from plant_params[15]).  With
  * plant_params = params, plant_profile = the plant bits of profile and w = v = NULL, every output is bit-identical to
- * ntm_mpc_closed_loop.  Box QP only: getWLc's state rows under a perturbed plant are not offered (ntm_mpc_step_sc +
- * ntm_plant_step cover them), nor is a controller-side tau_E(w).
+ * ntm_mpc_closed_loop.  The controller solves the box QP; ntm_mpc_closed_loop_perturbed_sc below keeps getWLc's state
+ * rows.  A controller-side tau_E(w) is not offered.
  * NTM_ERR_INVALID, nothing copied or launched: bad sizes, NULL x0 / xk / uk / params, plant_params_count not 1 or S,
  * a controller profile with TAUE_W, a plant_profile bit outside the four above. */
 int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
@@ -294,6 +294,35 @@ int ntm_mpc_closed_loop_perturbed_dev(ntm_handle *h, int layout, int profile, in
                                       const double *plant_params, int plant_params_count, int plant_profile,
                                       const double *w, const double *v, double *xk, double *uk, double *Uk,
                                       double *cost, int *inner_iters, int *qp_iters, int *status);
+
+/* ---- the same loop with getWLc's state rows kept in every QP: does the TRUE state stay inside the state box? ----- *
+ * ntm_mpc_closed_loop_perturbed with state_rows and xbounds as in ntm_mpc_closed_loop_sc (xbounds on the HOST for both
+ * entries).  For k = 0 .. k_sim-1, in ONE launch:
+ *   y_k = x_k + v_k
+ *   u_k, U_k = one ntm_mpc_step_sc (profile, params, state_rows, xbounds, its own record) at y_k
+ *   x_{k+1} = ntm_plant_step(x_k, u_k; plant_params, plant_profile) + d_k
+ * bit for bit, up to and including the step at which a scenario turns infeasible.  The offline build (:63-73) and the
+ * frozen rows (:74) come from y_0; the x_0 block of getWLc.m:30 tests y_k, so measurement noise alone can make a QP
+ * infeasible.  At the infeasible step u_k and U_k are NaN and inner_iters / qp_iters count the step as ntm_mpc_step_sc
+ * does; from then on the scenario ends as in ntm_mpc_closed_loop_sc: uk, Uk and xk(:, k+1 ..) are NaN, the iteration
+ * counts 0, cost NaN, status NTM_SCN_INFEASIBLE.  xk and cost are the true states, as in ntm_mpc_closed_loop_perturbed.
+ * NTM_STATE_ROWS_OFF is ntm_mpc_closed_loop_perturbed (the same launch and the same bits).  With nothing perturbed
+ * (plant_params NULL, plant_profile = the plant bits of profile, w = v = NULL) every output is bit-identical to
+ * ntm_mpc_closed_loop_sc.  The plant's inputs travel to the kernel through a small device buffer of the handle, copied
+ * on the handle's stream before the launch.
+ * NTM_ERR_INVALID, nothing copied or launched: whatever ntm_mpc_closed_loop_perturbed or ntm_mpc_step_sc rejects. */
+int ntm_mpc_closed_loop_perturbed_sc(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
+                                     double eps, const double *x0, const double *params, int params_count,
+                                     int state_rows, const double *xbounds, const double *plant_params,
+                                     int plant_params_count, int plant_profile, const double *w, const double *v,
+                                     double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
+                                     int *status);
+int ntm_mpc_closed_loop_perturbed_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
+                                         double eps, const double *x0, const double *params, int params_count,
+                                         int state_rows, const double *xbounds, const double *plant_params,
+                                         int plant_params_count, int plant_profile, const double *w, const double *v,
+                                         double *xk, double *uk, double *Uk, double *cost, int *inner_iters,
+                                         int *qp_iters, int *status);
 
 /* ---- the loop on EVERY visible GPU from ONE host process (what a MEX gateway can reach; SURVEY 8e) ------------- *
  * Replaces the same lines as ntm_mpc_closed_loop[_sc] (NTM_MPC_Sim.m:63-73,80-131); host pointers, same argument

@@ -17,7 +17,7 @@
  *                                (shadows the Optimization Toolbox function: input-box rows become bounds, state rows stay)
  *   11  ntm_mpc_step             one step NTM_MPC_Sim.m:94-128  [u,state,U,inner,status] = ntm_mpc_step(state,x,params,N,i_sim,eps,profile[,state_rows,xmin,xmax])
  *                                (no plant: the script's `for k` loop keeps its own plant code and passes state back in)
- *   12  ntm_mpc_batch_perturbed  the loop vs a perturbed plant  [xk,uk,cost,inner,status] = ntm_mpc_batch_perturbed(x0,params,N,k_sim,i_sim,eps,profile,plant_params,plant_profile,w,v)
+ *   12  ntm_mpc_batch_perturbed  the loop vs a perturbed plant  [xk,uk,cost,inner,status] = ntm_mpc_batch_perturbed(x0,params,N,k_sim,i_sim,eps,profile,plant_params,plant_profile,w,v[,state_rows,xmin,xmax])
  *
  * The short forms are the ones NTM_MPC_Sim.m actually uses (:63-66,:113-119,:130); the missing trailing arguments
  * are fetched from the caller's workspace under the script's own variable names (kappa :24, tau_r :9, Ts :31,
@@ -413,18 +413,28 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
     }
 #elif NTM_MEX_FN == 12
     {   /* [xk, uk, cost, inner, status] = ntm_mpc_batch_perturbed(x0 (2xS), params (16x1 | 16xS), N, k_sim, i_sim, eps,
-         *                                                           profile, plant_params, plant_profile, w, v)
-         * The fused loop against a perturbed plant (ntm_mpc_closed_loop_perturbed), one device: the controller of
+         *                                                           profile, plant_params, plant_profile, w, v
+         *                                                           [, state_rows, xmin, xmax])
+         * The fused loop against a perturbed plant (ntm_mpc_closed_loop_perturbed_sc), one device: the controller of
          * ntm_mpc_batch sees y_k = x_k + v_k; the plant runs on plant_params (16x1 | 16xS, [] = params) under
          * plant_profile, plus the disturbance w_k.  w, v: 2 x k_sim x S (or 2k_sim x S), [] = none.  xk holds the
-         * true states. */
-        int S, N, k_sim, i_sim, profile, pprofile, pc, ppc, i;
-        double eps;
+         * true states.  state_rows / xmin / xmax as in ntm_mpc_batch: getWLc's state rows in the controller's QPs. */
+        int S, N, k_sim, i_sim, profile, pprofile, pc, ppc, i, srows = 0;
+        double eps, xb[4] = {0.0, 0.0, 0.0, 0.0};
         const double *pp = NULL, *w = NULL, *v = NULL;
         mxArray *xk, *uk, *cost, *inner, *status;
         int *ibuf;
-        if (nrhs != 11)
-            mexErrMsgIdAndTxt("ntm:arg", "usage: [xk,uk,cost,inner,status] = ntm_mpc_batch_perturbed(x0, params, N, k_sim, i_sim, eps, profile, plant_params, plant_profile, w, v)");
+        if (nrhs != 11 && nrhs != 14)
+            mexErrMsgIdAndTxt("ntm:arg", "usage: [xk,uk,cost,inner,status] = ntm_mpc_batch_perturbed(x0, params, N, k_sim, i_sim, eps, profile, plant_params, plant_profile, w, v [, state_rows, xmin, xmax])");
+        if (nrhs == 14) {
+            srows = (int)scalar_arg(nrhs, prhs, 11, "");
+            if (srows < 0 || srows > 2) mexErrMsgIdAndTxt("ntm:arg", "state_rows must be 0, 1 or 2");
+            if (!is_real_double(prhs[12]) || !is_real_double(prhs[13]) || mxGetNumberOfElements(prhs[12]) != 2 ||
+                mxGetNumberOfElements(prhs[13]) != 2)
+                mexErrMsgIdAndTxt("ntm:arg", "xmin and xmax must be real double 2-vectors");
+            xb[0] = mxGetPr(prhs[12])[0]; xb[1] = mxGetPr(prhs[13])[0]; xb[2] = mxGetPr(prhs[12])[1]; xb[3] = mxGetPr(prhs[13])[1];
+            if (!(xb[0] <= xb[1] && xb[2] <= xb[3])) mexErrMsgIdAndTxt("ntm:arg", "xmin must be <= xmax");
+        }
         S = states_arg(prhs[0]);
         if (!is_real_double(prhs[1]) || mxGetM(prhs[1]) != NTM_NPARAM || ((int)mxGetN(prhs[1]) != 1 && (int)mxGetN(prhs[1]) != S))
             mexErrMsgIdAndTxt("ntm:arg", "params must be 16 x 1 or 16 x S (see ntm_mpc.h)");
@@ -434,6 +444,8 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         pprofile = (int)scalar_arg(nrhs, prhs, 8, "");
         if (N < 1 || N > NTM_MAX_HORIZON || k_sim < 0 || i_sim < 1) mexErrMsgIdAndTxt("ntm:arg", "N in 1..128, k_sim >= 0, i_sim >= 1");
         if (profile & NTM_PROFILE_TAUE_W) mexErrMsgIdAndTxt("ntm:arg", "NTM_PROFILE_TAUE_W (128) is not supported on the controller side");
+        if (srows != 0 && (profile & (NTM_PROFILE_GAMMA_I | NTM_PROFILE_DENSE_G)) && N > 32)
+            mexErrMsgIdAndTxt("ntm:arg", "state rows with NTM_PROFILE_GAMMA_I / DENSE_G need N <= 32");
         if (pprofile & ~(NTM_PROFILE_RHO1_SQ | NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W))
             mexErrMsgIdAndTxt("ntm:arg", "plant_profile: only RHO1_SQ, PLANT_C, PLANT_RK4 and TAUE_W (1, 8, 64, 128) act on the plant");
         ppc = pc;
@@ -451,9 +463,9 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         xk = mxCreateDoubleMatrix(2 * (k_sim + 1), S, mxREAL); uk = mxCreateDoubleMatrix(k_sim, S, mxREAL);
         cost = mxCreateDoubleMatrix(1, S, mxREAL); inner = mxCreateDoubleMatrix(k_sim, S, mxREAL); status = mxCreateDoubleMatrix(1, S, mxREAL);
         ibuf = (int *)mxMalloc(sizeof(int) * ((size_t)k_sim * S + S + 1));
-        check(ntm_mpc_closed_loop_perturbed(handle(), NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, mxGetPr(prhs[0]),
-                                            mxGetPr(prhs[1]), pc, pp, ppc, pprofile, w, v, mxGetPr(xk), mxGetPr(uk), NULL,
-                                            mxGetPr(cost), ibuf, NULL, ibuf + (size_t)k_sim * S));
+        check(ntm_mpc_closed_loop_perturbed_sc(handle(), NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, mxGetPr(prhs[0]),
+                                               mxGetPr(prhs[1]), pc, srows, xb, pp, ppc, pprofile, w, v, mxGetPr(xk), mxGetPr(uk),
+                                               NULL, mxGetPr(cost), ibuf, NULL, ibuf + (size_t)k_sim * S));
         for (i = 0; i < k_sim * S; ++i) mxGetPr(inner)[i] = (double)ibuf[i];
         for (i = 0; i < S; ++i) mxGetPr(status)[i] = (double)ibuf[(size_t)k_sim * S + i];
         mxFree(ibuf);

@@ -45,6 +45,7 @@ struct ntm_handle {
     size_t sv_doubles = 0;
     int *lpt = nullptr;              // ... and keys + order + bins of its longest-first work queue
     size_t lpt_ints = 0;
+    ntm::PlantIn *pin = nullptr;     // the plant's inputs of the perturbed loop with state rows (ntm::LoopArgs::ppd)
     long long launches = 0;
 };
 
@@ -303,6 +304,7 @@ int ntm_destroy(ntm_handle *h) {
     if (h->hscratch) cudaFree(h->hscratch);
     if (h->sv) cudaFree(h->sv);
     if (h->lpt) cudaFree(h->lpt);
+    if (h->pin) cudaFree(h->pin);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
     return NTM_OK;
@@ -842,7 +844,8 @@ int ntm_mpc_step_sc(ntm_handle *h, int layout, int profile, int S, int N, int i_
 }
 
 // ------------------------------------------------------------------------------------------------ perturbed plant
-// The fused loop with the plant of ntm_plant_step on its own block and profile bits, d_k and v_k (EXT = 3, ONE launch).
+// The fused loop with the plant of ntm_plant_step on its own block and profile bits, d_k and v_k (EXT = 3, or 4 with the
+// state rows; ONE launch).
 static int check_perturbed(int profile, int S, int N, int k_sim, int i_sim, const double *x0, const double *params,
                            int pc, int ppc, int plant_profile, double *xk, double *uk) {
     TRY(check_step(profile, N, i_sim));
@@ -854,21 +857,60 @@ static int check_perturbed(int profile, int S, int N, int k_sim, int i_sim, cons
     return NTM_OK;
 }
 
+// The perturbed loop with the box in a.xmin1..xmax2 (state_rows != OFF, EXT = 4) cannot carry the plant's inputs in
+// LoopArgs::pp, which shares those bytes: they go to the handle's device PlantIn, written on the handle's stream ahead of
+// the launch (stream order keeps each launch's copy until it has run).  With the rows off they stay in a.pp (EXT = 3).
+static int perturbed_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
+                              int pc, int state_rows, const double *xb, const double *plant_params, int ppc,
+                              int plant_profile, const Fused &d) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    if (plant_params == nullptr) { plant_params = d.params; ppc = pc; }
+    TRY(check_perturbed(profile, S, N, k_sim, i_sim, d.x0, d.params, pc, ppc, plant_profile, d.xk, d.uk));
+    ntm::LoopArgs a = {};
+    TRY(set_state_rows(h, profile, N, state_rows, xb, a));
+    const ntm::PlantIn pin = {plant_params, d.w, d.v, ppc, plant_profile};
+    a.pert = 1;
+    if (state_rows == NTM_STATE_ROWS_OFF) {
+        a.pp = pin;
+    } else {
+        if (h->pin == nullptr) {
+            cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&h->pin), sizeof(ntm::PlantIn));
+            if (e != cudaSuccess) return fail(NTM_ERR_ALLOC, "cudaMalloc(%zu): %s", sizeof(ntm::PlantIn), cudaGetErrorString(e));
+        }
+        CU(cudaMemcpyAsync(h->pin, &pin, sizeof(pin), cudaMemcpyHostToDevice, h->stream));
+        a.ppd = h->pin;
+    }
+    // plant-only bits have no effect on the controller
+    return launch_fused(h, a, layout, profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4), S, N, k_sim, i_sim, eps, pc, d);
+}
+
+static int perturbed_host_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
+                               const double *x0, const double *params, int pc, int state_rows, const double *xb,
+                               const double *plant_params, int ppc, int plant_profile, const double *w, const double *v,
+                               double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
+                               int *status) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    if (plant_params == nullptr) ppc = pc;
+    TRY(check_perturbed(profile, S, N, k_sim, i_sim, x0, params, pc, ppc, plant_profile, xk, uk));
+    ntm::LoopArgs rows = {};
+    TRY(set_state_rows(h, profile, N, state_rows, xb, rows));   // before any copy
+    return fused_host(h, layout, S, S, 0, N, k_sim, pc, ppc,
+                      {x0, params, plant_params, w, v, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status},
+                      [&](const Fused &d) {
+                          return perturbed_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, state_rows, xb,
+                                                    d.pparams, ppc, plant_profile, d);
+                      });
+}
+
 int ntm_mpc_closed_loop_perturbed_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
                                       double eps, const double *x0, const double *params, int pc,
                                       const double *plant_params, int ppc, int plant_profile, const double *w,
                                       const double *v, double *xk, double *uk, double *Uk, double *cost,
                                       int *inner_iters, int *qp_iters, int *status) {
-    TRY(check_common(h, layout, S));
-    if (S == 0) return NTM_OK;
-    if (plant_params == nullptr) { plant_params = params; ppc = pc; }
-    TRY(check_perturbed(profile, S, N, k_sim, i_sim, x0, params, pc, ppc, plant_profile, xk, uk));
-    ntm::LoopArgs a = {};
-    a.pert = 1; a.pp.pparams = plant_params; a.pp.pparams_count = ppc; a.pp.pflags = plant_profile;
-    a.pp.dist = w; a.pp.noise = v;
-    // plant-only bits have no effect on the controller
-    return launch_fused(h, a, layout, profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4), S, N, k_sim, i_sim, eps, pc,
-                        {x0, params, nullptr, nullptr, nullptr, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
+    return perturbed_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, NTM_STATE_ROWS_OFF, nullptr, plant_params,
+                              ppc, plant_profile, {x0, params, nullptr, w, v, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
 }
 
 int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
@@ -876,17 +918,26 @@ int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S,
                                   const double *plant_params, int ppc, int plant_profile, const double *w,
                                   const double *v, double *xk, double *uk, double *Uk, double *cost, int *inner_iters,
                                   int *qp_iters, int *status) {
-    TRY(check_common(h, layout, S));
-    if (S == 0) return NTM_OK;
-    if (plant_params == nullptr) ppc = pc;
-    TRY(check_perturbed(profile, S, N, k_sim, i_sim, x0, params, pc, ppc, plant_profile, xk, uk));
-    return fused_host(h, layout, S, S, 0, N, k_sim, pc, ppc,
-                      {x0, params, plant_params, w, v, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status},
-                      [&](const Fused &d) {
-                          return ntm_mpc_closed_loop_perturbed_dev(h, layout, profile, S, N, k_sim, i_sim, eps, d.x0,
-                                                                   d.params, pc, d.pparams, ppc, plant_profile, d.w, d.v,
-                                                                   d.xk, d.uk, d.Uk, d.cost, d.inner, d.qpit, d.status);
-                      });
+    return perturbed_host_impl(h, layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, NTM_STATE_ROWS_OFF, nullptr,
+                               plant_params, ppc, plant_profile, w, v, xk, uk, Uk, cost, inner_iters, qp_iters, status);
+}
+
+int ntm_mpc_closed_loop_perturbed_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
+                                         double eps, const double *x0, const double *params, int pc, int state_rows,
+                                         const double *xbounds, const double *plant_params, int ppc, int plant_profile,
+                                         const double *w, const double *v, double *xk, double *uk, double *Uk,
+                                         double *cost, int *inner_iters, int *qp_iters, int *status) {
+    return perturbed_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, state_rows, xbounds, plant_params, ppc,
+                              plant_profile, {x0, params, nullptr, w, v, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
+}
+
+int ntm_mpc_closed_loop_perturbed_sc(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
+                                     double eps, const double *x0, const double *params, int pc, int state_rows,
+                                     const double *xbounds, const double *plant_params, int ppc, int plant_profile,
+                                     const double *w, const double *v, double *xk, double *uk, double *Uk, double *cost,
+                                     int *inner_iters, int *qp_iters, int *status) {
+    return perturbed_host_impl(h, layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, xbounds,
+                               plant_params, ppc, plant_profile, w, v, xk, uk, Uk, cost, inner_iters, qp_iters, status);
 }
 
 // ------------------------------------------------------------------------------------------------ getWLc

@@ -1553,6 +1553,8 @@ static const LoopKernel kLoopKernels[] = {
     {{1, true, EXT_STATE_ROWS, 0, true}, closed_loop_kernel<1, true, EXT_STATE_ROWS, 0, true>},
     {{1, false, EXT_PERTURBED, 0, false}, closed_loop_kernel<1, false, EXT_PERTURBED>},
     {{1, true, EXT_PERTURBED, 0, false}, closed_loop_kernel<1, true, EXT_PERTURBED>},
+    {{1, false, EXT_PERTURBED_ROWS, 0, false}, closed_loop_kernel<1, false, EXT_PERTURBED_ROWS>},
+    {{1, true, EXT_PERTURBED_ROWS, 0, false}, closed_loop_kernel<1, true, EXT_PERTURBED_ROWS>},
     // multi-warp groups, dense Gamma
     {{2, true, EXT_BOX, 0, false}, closed_loop_kernel<2, true, EXT_BOX>},
     {{4, true, EXT_BOX, 0, false}, closed_loop_kernel<4, true, EXT_BOX>},
@@ -1567,7 +1569,10 @@ static const LoopKernel kLoopKernels[] = {
     {{4, false, EXT_STATE_ROWS, 0, false}, closed_loop_kernel<4, false, EXT_STATE_ROWS>},
     {{2, false, EXT_STATE_ROWS, 0, true}, closed_loop_kernel<2, false, EXT_STATE_ROWS, 0, true>},
     {{4, false, EXT_STATE_ROWS, 0, true}, closed_loop_kernel<4, false, EXT_STATE_ROWS, 0, true>},
+    {{2, false, EXT_PERTURBED_ROWS, 0, false}, closed_loop_kernel<2, false, EXT_PERTURBED_ROWS>},
+    {{4, false, EXT_PERTURBED_ROWS, 0, false}, closed_loop_kernel<4, false, EXT_PERTURBED_ROWS>},
 };
+static_assert(sizeof(kLoopKernels) / sizeof(kLoopKernels[0]) == 26, "kLoopKernels: one entry per instantiation");
 
 // The launch of one fused call: the instantiation and its shape.
 struct LoopRoute {
@@ -1583,12 +1588,12 @@ static cudaError_t route_closed_loop(const DeviceProps &dp, LoopArgs &a, LoopRou
     const int gw = gw_for(a.N);
     const bool dense = (a.flags & (NTM_PROFILE_GAMMA_I | NTM_PROFILE_DENSE_G)) != 0;
     // the headline instantiations carry none of the cold options
-    const int ext = a.pert ? EXT_PERTURBED
+    const int ext = a.pert ? (a.srows != 0 ? EXT_PERTURBED_ROWS : EXT_PERTURBED)
                   : a.srows != 0 ? EXT_STATE_ROWS
                   : (a.flags & (NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)) ? EXT_COLD_PLANT : EXT_BOX;
     // long horizons, literal Gamma, box QP: the sweep tableau, in registers while N + 1 fits 7 x 15 blocks, else in shared
     // memory (LV = 1)
-    r.lng = gw > 1 && !dense && ext != EXT_STATE_ROWS;
+    r.lng = gw > 1 && !dense && ext != EXT_STATE_ROWS && ext != EXT_PERTURBED_ROWS;
     // the controller step is a runtime mode of the one-warp box kernels and its own instantiation (CTL) wherever that mode
     // would cost registers (DESIGN section 4.8)
     const bool ctl = a.ctl != 0 && (ext == EXT_STATE_ROWS || (gw > 1 && ext == EXT_BOX));

@@ -1,8 +1,17 @@
 // ntm_kernels.h -- host-side launch interface between the C ABI (ntm_cabi.cu) and the kernels.
 #pragma once
+#include <cstddef>
 #include <cuda_runtime.h>
 
 namespace ntm {
+
+// The perturbed plant's inputs (ntm_mpc_closed_loop_perturbed[_sc]): the plant runs on its own parameter block
+// (pparams_count 1 or S, `layout`) and profile bits pflags; the controller sees x_k + v_k, the plant adds d_k after its
+// step.  dist (d) / noise (v): 2 * k_sim doubles per scenario in `layout`, element 2k + i (NULL = none)
+struct PlantIn {
+    const double *pparams, *dist, *noise;
+    int pparams_count, pflags;
+};
 
 struct LoopArgs {
     int layout, flags, S, N, k_sim, i_sim;
@@ -18,14 +27,12 @@ struct LoopArgs {
     // state rows of getWLc.m inside the loop (SURVEY 8f-1): 0 = dropped (box QP), 1 = rebuilt from every
     // re-condensation, 2 = frozen at the offline build as NTM_MPC_Sim.m:74 literally does
     int srows;
-    // The state box of the state rows (EXT = 2) and the perturbed plant's inputs (EXT = 3) share their bytes: no
-    // instantiation reads both, and LoopArgs keeps its size (the kernels' parameter offsets, and so their SASS).
+    // The state box of the state rows (EXT = 2, 4) and the perturbed plant's inputs (EXT = 3) share their bytes, and
+    // LoopArgs keeps its size (the kernels' parameter offsets, and so their SASS).  EXT = 4 needs both: the box stays
+    // here, the plant's inputs are a PlantIn in device memory that ppd (below) points to.
     union {
         struct { double xmin1, xmax1, xmin2, xmax2; };   // NTM_MPC_Sim.m:44-45
-        // perturbed plant: the plant runs on its own parameter block (pparams_count 1 or S, `layout`) and profile bits
-        // pflags; the controller sees x_k + v_k, the plant adds d_k after its step.  dist (d) / noise (v): 2 * k_sim
-        // doubles per scenario in `layout`, element 2k + i (NULL = none)
-        struct { const double *pparams, *dist, *noise; int pparams_count, pflags; } pp;
+        PlantIn pp;
     };
     unsigned int wbytes, qbytes;         // offsets of the IneqWork / ExtWork areas in a group's shared memory (launcher)
     int rows_warm;                       // 1: state-row QPs on the literal Gamma start from an earlier active set (the dense
@@ -40,7 +47,12 @@ struct LoopArgs {
     // scenarios for the remaining steps.  A launch is as long as its slowest scenario STARTED LAST, and the slow scenarios
     // are slow in every step.  lpt / sv: buffers from the C ABI layer (NULL = one launch in natural order); the rest is
     // set by the launcher.
-    int *lpt;                            // S keys + S positions + NTM_LPT_BINS counters
+    // lpt is read on the host only, and never set for a perturbed call (lpt_doubles is 0 there): its bytes carry the
+    // device pointer to the plant's inputs of the perturbed loop with the state rows (EXT = 4, ntm_mpc_closed_loop_perturbed_sc)
+    union {
+        int *lpt;                        // S keys + S positions + NTM_LPT_BINS counters
+        const PlantIn *ppd;
+    };
     double *sv;                          // NTM_CTRL_DOUBLES(N) per scenario (include/ntm_mpc.h), scenario slowest
     int k_begin, k_end;                  // time steps [k_begin, k_end) of this launch
     int *lpt_key;                        // phase A
@@ -51,6 +63,20 @@ struct LoopArgs {
     int pert;                            // 1: perturbed plant (ntm_mpc_closed_loop_perturbed, EXT = 3, see `pp` above)
 };
 static_assert(sizeof(LoopArgs) == 248, "LoopArgs is the fused kernels' parameter block: its size fixes their SASS");
+// ... and so do the offsets of the fields the kernels read
+static_assert(offsetof(LoopArgs, eps) == 24 && offsetof(LoopArgs, x0) == 32 && offsetof(LoopArgs, params) == 40 &&
+              offsetof(LoopArgs, params_count) == 48 && offsetof(LoopArgs, xk) == 56 && offsetof(LoopArgs, uk) == 64 &&
+              offsetof(LoopArgs, Uk) == 72 && offsetof(LoopArgs, cost) == 80 && offsetof(LoopArgs, inner) == 88 &&
+              offsetof(LoopArgs, qpit) == 96 && offsetof(LoopArgs, status) == 104 && offsetof(LoopArgs, counter) == 112 &&
+              offsetof(LoopArgs, hcap) == 120 && offsetof(LoopArgs, gam) == 124 && offsetof(LoopArgs, hscratch) == 128 &&
+              offsetof(LoopArgs, srows) == 136 && offsetof(LoopArgs, xmin1) == 144 && offsetof(LoopArgs, xmax2) == 168 &&
+              offsetof(LoopArgs, pp) == 144 && offsetof(LoopArgs, wbytes) == 176 && offsetof(LoopArgs, qbytes) == 180 &&
+              offsetof(LoopArgs, rows_warm) == 184 && offsetof(LoopArgs, rec_ld) == 188 &&
+              offsetof(LoopArgs, rec_status) == 192 && offsetof(LoopArgs, lpt) == 200 && offsetof(LoopArgs, ppd) == 200 &&
+              offsetof(LoopArgs, sv) == 208 && offsetof(LoopArgs, k_begin) == 216 && offsetof(LoopArgs, k_end) == 220 &&
+              offsetof(LoopArgs, lpt_key) == 224 && offsetof(LoopArgs, perm) == 232 && offsetof(LoopArgs, ctl) == 240 &&
+              offsetof(LoopArgs, pert) == 244,
+              "LoopArgs field offsets are fixed: the fused kernels' SASS reads them");
 #define NTM_LPT_BINS 160
 
 struct DeviceProps {
@@ -103,6 +129,7 @@ constexpr int EXT_BOX = 0;          // the headline instantiations: Euler plant,
 constexpr int EXT_COLD_PLANT = 1;   // + the RK4 / tau_E(w) plant options
 constexpr int EXT_STATE_ROWS = 2;   // + getWLc's state rows
 constexpr int EXT_PERTURBED = 3;    // box QP against a perturbed plant (LoopArgs::pert)
+constexpr int EXT_PERTURBED_ROWS = 4;   // getWLc's state rows against a perturbed plant (LoopArgs::pert, LoopArgs::ppd)
 // one instantiation closed_loop_kernel<gw, dense, ext, lv, ctl>
 struct LoopKey {
     int gw;

@@ -140,13 +140,24 @@ __device__ void stage_prefix(int N, int j, const Work &w, const Params &P, doubl
 }
 
 // EXT: 0 = the headline instantiation (Euler plant, box QP), 1 = + the RK4 plant option, 2 = + getWLc's state rows,
-// 3 = box QP against a perturbed plant (LoopArgs::pert: its own parameters and profile bits, d_k and v_k)
+// 3 = box QP against a perturbed plant (LoopArgs::pert: its own parameters and profile bits, d_k and v_k),
+// 4 = getWLc's state rows against a perturbed plant (the code of 2 and of 3, without 2's record and tau_E(w) code)
 // LONG (long horizons, literal Gamma, box QP): the QP runs on the packed sweep tableau of ntm_long.cuh
 template <int GW, bool DENSE, int EXT>
 struct LoopTraits {
-    static constexpr bool LONG = (GW > 1) && !DENSE && (EXT != 2);
+    static constexpr bool ROWS = (EXT == 2 || EXT == 4);   // getWLc's state rows
+    static constexpr bool PERT = (EXT == 3 || EXT == 4);   // the perturbed plant
+    static constexpr bool LONG = (GW > 1) && !DENSE && !ROWS;
     using WorkT = typename std::conditional<LONG, LongWork, Work>::type;
 };
+
+// The perturbed plant's inputs: LoopArgs::pp (EXT = 3), or the device copy LoopArgs::ppd points to (EXT = 4, whose
+// LoopArgs union holds the state box)
+template <int EXT>
+__device__ __forceinline__ const PlantIn &plant_in(const LoopArgs &a) {
+    if constexpr (EXT == 4) return *a.ppd;
+    else return a.pp;
+}
 
 // LV (LONG only): 0 = tableau in registers (N + 1 <= 7 * 10 / 7 * 15 for 2 / 4 warps), 1 = tableau in shared memory
 // CTL (multi-warp groups with EXT = 0, every group size with EXT = 2): the controller-step instantiation (ntm_mpc_step,
@@ -158,6 +169,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                              unsigned char *gbase, int tI = -1, int tJ = -1) {
     using Gp = Group<GW>;
     constexpr bool LONG = LoopTraits<GW, DENSE, EXT>::LONG;
+    using LT = LoopTraits<GW, DENSE, EXT>;               // LT::ROWS, LT::PERT (a constexpr local here moves registers)
     const int N = a.N, S = a.S, flags = a.flags, layout = a.layout;
     const bool act = j < N;
     const bool lead = (j == 0);
@@ -171,12 +183,13 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     const bool ctl = (GW == 1 && EXT == 0) ? (a.ctl != 0) : CTL;
     double x01 = __ldg(a.x0 + elem(layout, S, 2, s, 0)), x02 = __ldg(a.x0 + elem(layout, S, 2, s, 1));
     double x1 = x01, x2 = x02;
-    // perturbed plant (EXT = 3): (x1, x2) is what the controller sees, y_k = x_k + v_k; the offline build (:63-65) runs
-    // from y_0.  The true state x_k lives in xk only (written by the lead, read back by the group after a barrier), so
-    // no register carries it across the loop.
-    if constexpr (EXT == 3) {
-        if (a.pp.noise != nullptr) {
-            x01 += __ldg(a.pp.noise + elem(layout, S, 2 * a.k_sim, s, 0)); x02 += __ldg(a.pp.noise + elem(layout, S, 2 * a.k_sim, s, 1));
+    // perturbed plant (EXT = 3, 4): (x1, x2) is what the controller sees, y_k = x_k + v_k; the offline build (:63-65)
+    // and frozen state rows (:74) run from y_0.  The true state x_k lives in xk only (written by the lead, read back by
+    // the group after a barrier), so no register carries it across the loop.
+    if constexpr (LT::PERT) {
+        const PlantIn &pi = plant_in<EXT>(a);
+        if (pi.noise != nullptr) {
+            x01 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 0)); x02 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 1));
             x1 = x01; x2 = x02;
         }
     }
@@ -218,9 +231,9 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     [[maybe_unused]] bool rows_built = false;
     int hs1 = -1, hs2 = -1;
     bool first_qp = true;
-    // EXT == 2, literal Gamma: active sets of the last two state-row QPs of this scenario, offered to the next one as a
-    // warm start (per thread: (vst + 1) | mask of this state's four rows << 2), and the "warm start failed, run this QP
-    // again cold" flag
+    // state rows (EXT 2, 4), literal Gamma: active sets of the last two state-row QPs of this scenario, offered to the
+    // next one as a warm start (per thread: (vst + 1) | mask of this state's four rows << 2), and the "warm start failed,
+    // run this QP again cold" flag
     [[maybe_unused]] int hw1 = 0, hw2 = 0, hwn = 0;
     [[maybe_unused]] bool retry = false;
     [[maybe_unused]] bool regen_rows = false;            // EXT == 2, CTL: rebuild the frozen rows of a resumed record first
@@ -268,7 +281,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             Gp::sync();
         }
     }
-    if constexpr (EXT == 3) {
+    if constexpr (LT::PERT) {
         if (lead) { a.xk[xk_at(0)] = __ldg(a.x0 + elem(layout, S, 2, s, 0)); a.xk[xk_at(1)] = __ldg(a.x0 + elem(layout, S, 2, s, 1)); }
     } else {
         if (lead && !resumed && !ctl) { a.xk[xk_at(0)] = x1; a.xk[xk_at(1)] = x2; }
@@ -318,19 +331,20 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             if (!brk) Uold = Uj;                                                    // :127 (skipped by the break)
             if (stop) {
                 const double u0 = Gp::bcast0(Uj, w.red);                            // :107  uk(:,k) = U(1)
-                if constexpr (EXT == 3) {
+                if constexpr (LT::PERT) {
                     // the plant's own block and profile bits, read here (once per time step, no shared copy), then + d_k
                     if (!isfinite(u0)) status = max(status, (int)NTM_SCN_NONFINITE);
-                    const Params Q = load_params(a.pp.pparams, layout, a.pp.pparams_count, s);
-                    const int pf = a.pp.pflags;
+                    const PlantIn &pi = plant_in<EXT>(a);
+                    const Params Q = load_params(pi.pparams, layout, pi.pparams_count, s);
+                    const int pf = pi.pflags;
                     const double qtau = (pf & NTM_PROFILE_TAUE_W)
-                        ? __ldg(a.pp.pparams + elem(layout, a.pp.pparams_count, NTM_NPARAM, a.pp.pparams_count == 1 ? 0 : s, 15)) : 0.0;
+                        ? __ldg(pi.pparams + elem(layout, pi.pparams_count, NTM_NPARAM, pi.pparams_count == 1 ? 0 : s, 15)) : 0.0;
                     const double t1 = a.xk[xk_at(2 * k)], t2 = a.xk[xk_at(2 * k + 1)];   // x_k, written by the lead
                     double nw, nom;
                     plant_exact(Q, pf, Q.a22, qtau, t1, t2, u0, nw, nom);              // = ntm_plant_step
-                    if (a.pp.dist != nullptr) {
-                        nw += __ldg(a.pp.dist + elem(layout, S, 2 * a.k_sim, s, 2 * k));
-                        nom += __ldg(a.pp.dist + elem(layout, S, 2 * a.k_sim, s, 2 * k + 1));
+                    if (pi.dist != nullptr) {
+                        nw += __ldg(pi.dist + elem(layout, S, 2 * a.k_sim, s, 2 * k));
+                        nom += __ldg(pi.dist + elem(layout, S, 2 * a.k_sim, s, 2 * k + 1));
                     }
                     const double e1 = nw - P.r1, e2 = nom - P.r2;                     // judged on the true state
                     cost += e1 * (P.q11 * e1 + P.q12 * e2) + e2 * (P.q12 * e1 + P.q22 * e2);
@@ -401,12 +415,13 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             }
         }
         if (k >= a.k_sim) break;
-        if constexpr (EXT == 3) {
+        if constexpr (LT::PERT) {
             if (it == 0) {               // as for a controller step: the measurement y_k = x_k + v_k
                 Gp::sync();              // the lead has just written x_k
                 x1 = a.xk[xk_at(2 * k)]; x2 = a.xk[xk_at(2 * k + 1)];
-                if (a.pp.noise != nullptr) {
-                    x1 += __ldg(a.pp.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k)); x2 += __ldg(a.pp.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k + 1));
+                const PlantIn &pi = plant_in<EXT>(a);
+                if (pi.noise != nullptr) {
+                    x1 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k)); x2 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k + 1));
                 }
                 if (!(isfinite(x1) && isfinite(x2))) status = max(status, (int)NTM_SCN_NONFINITE);
             }
@@ -418,7 +433,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
         int st = NTM_SCN_OK;
         if constexpr (DENSE) {
             st = qp_solve<GW>(N, j, w, Fj, P.umin, P.umax, hist, Uj, qp_cap, nit);   // :97
-            if constexpr (EXT == 2 && GW == 1) {
+            if constexpr (LT::ROWS && GW == 1) {
                 if (a.srows != 0) {
                     // NTM_MPC_Sim.m:97 as written, ANY Gamma index: the state rows of getWLc.m:57 (L = Mcal*Gamma + Ecal)
                     // are read from the dense Gamma tile the tensor-core Hessian build left in shared memory (DenseRows);
@@ -479,9 +494,10 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             [[maybe_unused]] bool try_warm = false;
             [[maybe_unused]] int wv = 0, wm = -1;
             [[maybe_unused]] bool x0bad = false;
-            if constexpr (EXT == 2) {
+            if constexpr (LT::ROWS) {
                 if (a.srows != 0) {
-                    // the x_0 block of getWLc.m:30 has no U: it only asks that x_k itself is inside the state box
+                    // the x_0 block of getWLc.m:30 has no U: it only asks that x_k itself (y_k under a perturbed plant:
+                    // the state the controller sees) is inside the state box
                     x0bad = x1 < a.xmin1 || x1 > a.xmax1 || x2 < a.xmin2 || x2 > a.xmax2;
                     if ((a.rows_warm & 1) && !retry && hwn > 0 && !x0bad) {
                         const int hh = (hwn >= 2) ? hw2 : hw1;
@@ -518,7 +534,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                 if (first_qp) { hU2 = Uj; hs2 = sn; first_qp = false; } else { hU2 = hU1; hs2 = hs1; }
                 hU1 = Uj; hs1 = sn;
             }
-            if constexpr (EXT == 2) {
+            if constexpr (LT::ROWS) {
                 if (a.srows != 0) {
                     // NTM_MPC_Sim.m:97 as written: L*U <= c + W*xk(:,k) with getWLc's state rows kept.  The box
                     // minimiser above is the dual-feasible start of the active-set continuation (qp_ineq_continue).
@@ -576,7 +592,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                 }
             }
         }
-        if constexpr (EXT == 2) {
+        if constexpr (LT::ROWS) {
             if (st == NTM_SCN_INFEASIBLE) {
                 // quadprog exitflag -2 (:100-101) returns no U and the script cannot continue: the scenario ends here,
                 // everything it has not produced yet is NaN.  A controller step (k_sim = 1) returns NaN u and U and
@@ -632,7 +648,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
         Gp::sync();
     }
     if (lead) {
-        if constexpr (EXT == 3) {
+        if constexpr (LT::PERT) {
             const double t1 = a.xk[xk_at(2 * a.k_sim)], t2 = a.xk[xk_at(2 * a.k_sim + 1)];
             if (!(isfinite(t1) && isfinite(t2) && isfinite(cost))) status = max(status, (int)NTM_SCN_NONFINITE);
         } else {

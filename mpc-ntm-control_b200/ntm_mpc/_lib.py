@@ -77,6 +77,9 @@ for _sfx in ("", "_dev"):
                                               _dp, _dp, _dp, _dp])
     SYMBOLS["ntm_mpc_closed_loop_perturbed" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i,
                                                             _dp, _i, _i, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp])
+    SYMBOLS["ntm_mpc_closed_loop_perturbed_sc" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp,
+                                                               _i, _i, _dp, _dp, _i, _i, _dp, _dp, _dp, _dp, _dp, _dp,
+                                                               _dp, _dp, _dp])
     SYMBOLS["ntm_mpc_closed_loop_sc" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i, _i, _dp,
                                                      _dp, _dp, _dp, _dp, _dp, _dp, _dp])
 

@@ -56,6 +56,19 @@ def _state_box(state_rows: int, xbounds):
     return _f64(MC_STATE_BOX if xbounds is None else xbounds).reshape(4) if state_rows else None
 
 
+def state_box_inputs(state_rows: int, xbounds):
+    """Checks ``state_rows`` / ``xbounds`` of the perturbed loop (no device needed) and returns the state box as
+    ``_state_box`` does: a float64 4-vector (default the script's own box), or None with the rows off."""
+    if int(state_rows) not in (_lib.STATE_ROWS_OFF, _lib.STATE_ROWS_REFRESH, _lib.STATE_ROWS_FROZEN):
+        raise ValueError(f"state_rows must be STATE_ROWS_OFF, STATE_ROWS_REFRESH or STATE_ROWS_FROZEN (got {state_rows})")
+    if xbounds is not None and np.asarray(xbounds).size != 4:
+        raise ValueError("xbounds must be (xmin1, xmax1, xmin2, xmax2)")
+    xb = _state_box(state_rows, xbounds)
+    if xb is not None and not (xb[0] <= xb[1] and xb[2] <= xb[3]):
+        raise ValueError("xbounds: xmin > xmax (or NaN)")
+    return xb
+
+
 def _loop_outputs(out, S: int, N: int, k_sim: int, want_Uk: bool):
     """Output arrays of a closed-loop call: fresh ones, or the caller's preallocated (e.g. pinned) ones from ``out``.
     The C ABI writes through raw addresses, so a supplied array must be exactly what the library expects --
@@ -390,34 +403,44 @@ class NtmMpc:
 
     def closed_loop_perturbed(self, x0, params, N: int, plant_params=None, plant_profile: Optional[int] = None, w=None,
                               v=None, k_sim: int = 20, i_sim: int = 10, eps: float = 1e-14, profile: int = 0,
-                              want_Uk: bool = False, out: Optional[dict] = None):
+                              want_Uk: bool = False, out: Optional[dict] = None, state_rows: int = 0, xbounds=None):
         """The fused loop against a perturbed plant (``ntm_mpc_closed_loop_perturbed``): the controller (``params``,
         ``profile``) sees ``y_k = x_k + v[:, k]``; the plant is ``plant_step`` on ``plant_params`` (default ``params``)
         under ``plant_profile`` (default: the plant bits of ``profile``), plus ``w[:, k]``.  ``w`` and ``v`` are
         ``[S, k_sim, 2]`` or None.  Returns the dict of ``closed_loop``; ``xk`` holds the true states and ``cost`` is
-        judged on them."""
+        judged on them.
+
+        ``state_rows`` (``STATE_ROWS_REFRESH`` / ``STATE_ROWS_FROZEN``) keeps getWLc's state rows in every QP of the
+        controller (``ntm_mpc_closed_loop_perturbed_sc``); ``xbounds = (xmin1, xmax1, xmin2, xmax2)``, default the
+        script's own state box.  The rows test what the controller sees, ``y_k``; whether the true state stayed inside
+        the box is in ``xk``."""
         x0, p, pc, pp, ppc, pf, wf, vf = perturbed_inputs(x0, params, plant_params, plant_profile, w, v, k_sim, profile)
         S = x0.shape[0]
+        xb = state_box_inputs(state_rows, xbounds)
         outs = _loop_outputs(out, S, N, k_sim, want_Uk)
         xk, uk, Uk, cost, inner, qpit, status = outs
-        check(self._lib.ntm_mpc_closed_loop_perturbed(self._h, LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, _ptr(x0),
-                                                      _ptr(p), pc, _ptr(pp), ppc, pf, _ptr(wf), _ptr(vf), _ptr(xk),
-                                                      _ptr(uk), _ptr(Uk) if want_Uk else None, _ptr(cost), _ptr(inner),
-                                                      _ptr(qpit), _ptr(status)))
+        check(self._lib.ntm_mpc_closed_loop_perturbed_sc(self._h, LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps,
+                                                         _ptr(x0), _ptr(p), pc, int(state_rows), _ptr(xb), _ptr(pp), ppc,
+                                                         pf, _ptr(wf), _ptr(vf), _ptr(xk), _ptr(uk),
+                                                         _ptr(Uk) if want_Uk else None, _ptr(cost), _ptr(inner),
+                                                         _ptr(qpit), _ptr(status)))
         return _loop_result(outs)
 
     def closed_loop_perturbed_dev(self, S: int, N: int, k_sim: int, i_sim: int, eps: float, profile: int, layout: int,
                                   x0_ptr: int, params_ptr: int, params_count: int, plant_params_ptr: int,
                                   plant_params_count: int, plant_profile: int, w_ptr: int, v_ptr: int, xk_ptr: int,
                                   uk_ptr: int, Uk_ptr: int = 0, cost_ptr: int = 0, inner_ptr: int = 0, qp_ptr: int = 0,
-                                  status_ptr: int = 0) -> None:
+                                  status_ptr: int = 0, state_rows: int = 0, xbounds=None) -> None:
         """``closed_loop_perturbed`` on device pointers (0 = NULL for ``plant_params_ptr``, ``w_ptr``, ``v_ptr`` and the
-        optional outputs); asynchronous on the handle's stream (``ntm_mpc_closed_loop_perturbed_dev``)."""
-        check(self._lib.ntm_mpc_closed_loop_perturbed_dev(self._h, layout, profile, S, N, k_sim, i_sim, eps, x0_ptr,
-                                                          params_ptr, params_count, plant_params_ptr or None,
-                                                          plant_params_count, plant_profile, w_ptr or None, v_ptr or None,
-                                                          xk_ptr, uk_ptr, Uk_ptr or None, cost_ptr or None,
-                                                          inner_ptr or None, qp_ptr or None, status_ptr or None))
+        optional outputs); asynchronous on the handle's stream (``ntm_mpc_closed_loop_perturbed_sc_dev``, which is
+        ``ntm_mpc_closed_loop_perturbed_dev`` with the state rows off; ``xbounds`` is a host 4-vector)."""
+        check(self._lib.ntm_mpc_closed_loop_perturbed_sc_dev(self._h, layout, profile, S, N, k_sim, i_sim, eps, x0_ptr,
+                                                             params_ptr, params_count, int(state_rows),
+                                                             _ptr(state_box_inputs(state_rows, xbounds)),
+                                                             plant_params_ptr or None, plant_params_count, plant_profile,
+                                                             w_ptr or None, v_ptr or None, xk_ptr, uk_ptr, Uk_ptr or None,
+                                                             cost_ptr or None, inner_ptr or None, qp_ptr or None,
+                                                             status_ptr or None))
 
     # ------------------------------------------------------------------ NTM_MPC_Sim.m:94-128, one step, no plant
     def mpc_step(self, state, x, params, N: int, i_sim: int = 10, eps: float = 1e-14, profile: int = 0,

@@ -62,14 +62,14 @@ def run(config: int = 3, S: Optional[int] = None, seed: Optional[int] = None, pr
     controller, tau_E(w) in the plant.  ``plant_profile`` defaults to the plant bits of ``profile``.  ``w_std`` /
     ``v_std`` (scalar or per-component pair): Gaussian process disturbances d_k and measurement noise v_k, drawn on the
     device by ``noise`` and never copied to the host.  The reduction runs on the true trajectories with the controller's
-    umin / umax.  Not combined with ``state_rows``."""
+    umin / umax.  With ``state_rows`` the controller keeps getWLc's state rows (box = ``bounds``) against the perturbed
+    plant (``ntm_mpc_closed_loop_perturbed_sc_dev``): the rows test what the controller sees, y_k = x_k + v_k, and the
+    reduction counts how often the TRUE state left the box."""
     import torch                                               # device buffers + stream plumbing only
     h = handle or NtmMpc(device)
     prm, x0, N = physics.batch_params(config, S, seed, sample) # [NPARAM, S] SoA, [S, 2]
     S = x0.shape[0]
     perturbed = plant_sample is not None or plant_profile is not None or w_std is not None or v_std is not None
-    if perturbed and state_rows:
-        raise ValueError("the perturbed plant runs the box-QP controller: state_rows must be 0")
     dev = torch.device(f"cuda:{device}")
     d_prm = torch.from_numpy(prm).to(dev)                      # SoA block: scenario index fastest
     d_x0 = torch.from_numpy(np.ascontiguousarray(x0.T)).to(dev)
@@ -88,7 +88,8 @@ def run(config: int = 3, S: Optional[int] = None, seed: Optional[int] = None, pr
             h.closed_loop_perturbed_dev(S, N, k_sim, i_sim, eps, profile, LAYOUT_SOA, d_x0.data_ptr(), d_prm.data_ptr(), S,
                                         d_pp.data_ptr() if d_pp is not None else 0, S, pf,
                                         d_w.data_ptr() if d_w is not None else 0, d_v.data_ptr() if d_v is not None else 0,
-                                        d_xk.data_ptr(), d_uk.data_ptr(), 0, d_cost.data_ptr(), 0, 0, d_st.data_ptr())
+                                        d_xk.data_ptr(), d_uk.data_ptr(), 0, d_cost.data_ptr(), 0, 0, d_st.data_ptr(),
+                                        state_rows=state_rows, xbounds=bounds)
         elif state_rows:
             h.closed_loop_sc_dev(S, N, k_sim, i_sim, eps, profile, LAYOUT_SOA, d_x0.data_ptr(), d_prm.data_ptr(), S,
                                  state_rows, bounds, d_xk.data_ptr(), d_uk.data_ptr(), 0, d_cost.data_ptr(), 0, 0,
