@@ -308,8 +308,8 @@ int ntm_mpc_closed_loop_perturbed_dev(ntm_handle *h, int layout, int profile, in
  * counts 0, cost NaN, status NTM_SCN_INFEASIBLE.  xk and cost are the true states, as in ntm_mpc_closed_loop_perturbed.
  * NTM_STATE_ROWS_OFF is ntm_mpc_closed_loop_perturbed (the same launch and the same bits).  With nothing perturbed
  * (plant_params NULL, plant_profile = the plant bits of profile, w = v = NULL) every output is bit-identical to
- * ntm_mpc_closed_loop_sc.  The plant's inputs travel to the kernel through a small device buffer of the handle, copied
- * on the handle's stream before the launch.
+ * ntm_mpc_closed_loop_sc.  The plant's inputs travel to the kernel with its launch parameters: the _dev entry queues
+ * the launch and no copy.
  * NTM_ERR_INVALID, nothing copied or launched: whatever ntm_mpc_closed_loop_perturbed or ntm_mpc_step_sc rejects. */
 int ntm_mpc_closed_loop_perturbed_sc(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
                                      double eps, const double *x0, const double *params, int params_count,

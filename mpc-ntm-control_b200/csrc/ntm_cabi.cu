@@ -45,7 +45,6 @@ struct ntm_handle {
     size_t sv_doubles = 0;
     int *lpt = nullptr;              // ... and keys + order + bins of its longest-first work queue
     size_t lpt_ints = 0;
-    ntm::PlantIn *pin = nullptr;     // the plant's inputs of the perturbed loop with state rows (ntm::LoopArgs::ppd)
     long long launches = 0;
 };
 
@@ -203,11 +202,12 @@ static int launch_fused(ntm_handle *h, ntm::LoopArgs &a, int layout, int flags, 
     TRY(ensure_hscratch(h, N));
     a.hscratch = h->hscratch;
     const size_t svd = ntm::lpt_doubles(h->props, a);      // two-phase launch with a longest-first queue (ntm_kernels.h)
+    int *lpt = nullptr;
     if (svd != 0) {
         TRY(ensure_lpt(h, svd, 2 * (size_t)S + NTM_LPT_BINS));
-        a.sv = h->sv; a.lpt = h->lpt;
+        a.sv = h->sv; lpt = h->lpt;
     }
-    CU(ntm::launch_closed_loop(h->stream, h->props, a, &h->launches));
+    CU(ntm::launch_closed_loop(h->stream, h->props, a, lpt, &h->launches));
     return NTM_OK;
 }
 
@@ -304,7 +304,6 @@ int ntm_destroy(ntm_handle *h) {
     if (h->hscratch) cudaFree(h->hscratch);
     if (h->sv) cudaFree(h->sv);
     if (h->lpt) cudaFree(h->lpt);
-    if (h->pin) cudaFree(h->pin);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
     return NTM_OK;
@@ -844,8 +843,8 @@ int ntm_mpc_step_sc(ntm_handle *h, int layout, int profile, int S, int N, int i_
 }
 
 // ------------------------------------------------------------------------------------------------ perturbed plant
-// The fused loop with the plant of ntm_plant_step on its own block and profile bits, d_k and v_k (EXT = 3, or 4 with the
-// state rows; ONE launch).
+// The fused loop with the plant of ntm_plant_step on its own block and profile bits, d_k and v_k, with the box QP or the
+// state rows (ONE launch).
 static int check_perturbed(int profile, int S, int N, int k_sim, int i_sim, const double *x0, const double *params,
                            int pc, int ppc, int plant_profile, double *xk, double *uk) {
     TRY(check_step(profile, N, i_sim));
@@ -857,9 +856,6 @@ static int check_perturbed(int profile, int S, int N, int k_sim, int i_sim, cons
     return NTM_OK;
 }
 
-// The perturbed loop with the box in a.xmin1..xmax2 (state_rows != OFF, EXT = 4) cannot carry the plant's inputs in
-// LoopArgs::pp, which shares those bytes: they go to the handle's device PlantIn, written on the handle's stream ahead of
-// the launch (stream order keeps each launch's copy until it has run).  With the rows off they stay in a.pp (EXT = 3).
 static int perturbed_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
                               int pc, int state_rows, const double *xb, const double *plant_params, int ppc,
                               int plant_profile, const Fused &d) {
@@ -869,18 +865,8 @@ static int perturbed_dev_impl(ntm_handle *h, int layout, int profile, int S, int
     TRY(check_perturbed(profile, S, N, k_sim, i_sim, d.x0, d.params, pc, ppc, plant_profile, d.xk, d.uk));
     ntm::LoopArgs a = {};
     TRY(set_state_rows(h, profile, N, state_rows, xb, a));
-    const ntm::PlantIn pin = {plant_params, d.w, d.v, ppc, plant_profile};
+    a.pp = {plant_params, d.w, d.v, ppc, plant_profile};
     a.pert = 1;
-    if (state_rows == NTM_STATE_ROWS_OFF) {
-        a.pp = pin;
-    } else {
-        if (h->pin == nullptr) {
-            cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&h->pin), sizeof(ntm::PlantIn));
-            if (e != cudaSuccess) return fail(NTM_ERR_ALLOC, "cudaMalloc(%zu): %s", sizeof(ntm::PlantIn), cudaGetErrorString(e));
-        }
-        CU(cudaMemcpyAsync(h->pin, &pin, sizeof(pin), cudaMemcpyHostToDevice, h->stream));
-        a.ppd = h->pin;
-    }
     // plant-only bits have no effect on the controller
     return launch_fused(h, a, layout, profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4), S, N, k_sim, i_sim, eps, pc, d);
 }

@@ -1638,7 +1638,7 @@ static cudaError_t route_closed_loop(const DeviceProps &dp, LoopArgs &a, LoopRou
     return cudaSuccess;
 }
 
-cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches) {
+cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, int *lpt, long long *launches) {
     if (a.S <= 0) return cudaSuccess;
     if (a.hscratch == nullptr) return cudaErrorInvalidValue;
     LoopArgs aa = a;
@@ -1653,10 +1653,10 @@ cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const Loo
         return launch_persistent(st, dp, fn, r.block, r.smem, a.S, r.groups_per_block, r.group_cap, launches, aa,
                                  (unsigned int)r.gbytes);
     };
-    if (a.lpt != nullptr && a.sv != nullptr && lpt_doubles(dp, a) != 0) {
+    if (lpt != nullptr && a.sv != nullptr && lpt_doubles(dp, a) != 0) {
         // phase A: time step 0 of every scenario (state + cost key), counting sort, phase B: the rest, longest first.
         // lpt_doubles admits the headline instantiation <1, false, EXT_BOX> only.
-        int *key = a.lpt, *perm = a.lpt + a.S, *bins = a.lpt + 2 * (size_t)a.S;
+        int *key = lpt, *perm = lpt + a.S, *bins = lpt + 2 * (size_t)a.S;
         e = cudaMemsetAsync(bins, 0, NTM_LPT_BINS * sizeof(int), st);
         if (e != cudaSuccess) return e;
         aa.k_begin = 0; aa.k_end = 1; aa.lpt_key = key;

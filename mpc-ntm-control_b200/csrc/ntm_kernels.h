@@ -27,13 +27,8 @@ struct LoopArgs {
     // state rows of getWLc.m inside the loop (SURVEY 8f-1): 0 = dropped (box QP), 1 = rebuilt from every
     // re-condensation, 2 = frozen at the offline build as NTM_MPC_Sim.m:74 literally does
     int srows;
-    // The state box of the state rows (EXT = 2, 4) and the perturbed plant's inputs (EXT = 3) share their bytes, and
-    // LoopArgs keeps its size (the kernels' parameter offsets, and so their SASS).  EXT = 4 needs both: the box stays
-    // here, the plant's inputs are a PlantIn in device memory that ppd (below) points to.
-    union {
-        struct { double xmin1, xmax1, xmin2, xmax2; };   // NTM_MPC_Sim.m:44-45
-        PlantIn pp;
-    };
+    double xmin1, xmax1, xmin2, xmax2;   // the state box of the state rows, NTM_MPC_Sim.m:44-45
+    PlantIn pp;                          // the perturbed plant's inputs (pert = 1)
     unsigned int wbytes, qbytes;         // offsets of the IneqWork / ExtWork areas in a group's shared memory (launcher)
     int rows_warm;                       // 1: state-row QPs on the literal Gamma start from an earlier active set (the dense
                                          // Gamma always starts cold); set by the launcher, NTM_ROWS_WARM=0 turns it off
@@ -45,38 +40,17 @@ struct LoopArgs {
     // every scenario, saves its loop state (one controller record per scenario in sv) and a cost key (how many of the
     // step's QPs missed the vertex test); a counting sort turns the keys into the order in which phase B pops the
     // scenarios for the remaining steps.  A launch is as long as its slowest scenario STARTED LAST, and the slow scenarios
-    // are slow in every step.  lpt / sv: buffers from the C ABI layer (NULL = one launch in natural order); the rest is
-    // set by the launcher.
-    // lpt is read on the host only, and never set for a perturbed call (lpt_doubles is 0 there): its bytes carry the
-    // device pointer to the plant's inputs of the perturbed loop with the state rows (EXT = 4, ntm_mpc_closed_loop_perturbed_sc)
-    union {
-        int *lpt;                        // S keys + S positions + NTM_LPT_BINS counters
-        const PlantIn *ppd;
-    };
+    // are slow in every step.  sv (and launch_closed_loop's lpt): buffers from the C ABI layer (NULL = one launch in
+    // natural order); the rest is set by the launcher.
     double *sv;                          // NTM_CTRL_DOUBLES(N) per scenario (include/ntm_mpc.h), scenario slowest
     int k_begin, k_end;                  // time steps [k_begin, k_end) of this launch
     int *lpt_key;                        // phase A
     const int *perm;                     // phase B
-    // controller step (ntm_mpc_step, EXT = 0 instantiations only): k_sim = 1, x0 is the measured state, sv holds the
-    // caller's records (read at the start, written at the stop rule), no plant; xk and cost are NULL
+    // controller step (ntm_mpc_step[_sc]): k_sim = 1, x0 is the measured state, sv holds the caller's records (read at
+    // the start, written at the stop rule), no plant; xk and cost are NULL
     int ctl;
-    int pert;                            // 1: perturbed plant (ntm_mpc_closed_loop_perturbed, EXT = 3, see `pp` above)
+    int pert;                            // 1: perturbed plant (ntm_mpc_closed_loop_perturbed[_sc], see `pp` above)
 };
-static_assert(sizeof(LoopArgs) == 248, "LoopArgs is the fused kernels' parameter block: its size fixes their SASS");
-// ... and so do the offsets of the fields the kernels read
-static_assert(offsetof(LoopArgs, eps) == 24 && offsetof(LoopArgs, x0) == 32 && offsetof(LoopArgs, params) == 40 &&
-              offsetof(LoopArgs, params_count) == 48 && offsetof(LoopArgs, xk) == 56 && offsetof(LoopArgs, uk) == 64 &&
-              offsetof(LoopArgs, Uk) == 72 && offsetof(LoopArgs, cost) == 80 && offsetof(LoopArgs, inner) == 88 &&
-              offsetof(LoopArgs, qpit) == 96 && offsetof(LoopArgs, status) == 104 && offsetof(LoopArgs, counter) == 112 &&
-              offsetof(LoopArgs, hcap) == 120 && offsetof(LoopArgs, gam) == 124 && offsetof(LoopArgs, hscratch) == 128 &&
-              offsetof(LoopArgs, srows) == 136 && offsetof(LoopArgs, xmin1) == 144 && offsetof(LoopArgs, xmax2) == 168 &&
-              offsetof(LoopArgs, pp) == 144 && offsetof(LoopArgs, wbytes) == 176 && offsetof(LoopArgs, qbytes) == 180 &&
-              offsetof(LoopArgs, rows_warm) == 184 && offsetof(LoopArgs, rec_ld) == 188 &&
-              offsetof(LoopArgs, rec_status) == 192 && offsetof(LoopArgs, lpt) == 200 && offsetof(LoopArgs, ppd) == 200 &&
-              offsetof(LoopArgs, sv) == 208 && offsetof(LoopArgs, k_begin) == 216 && offsetof(LoopArgs, k_end) == 220 &&
-              offsetof(LoopArgs, lpt_key) == 224 && offsetof(LoopArgs, perm) == 232 && offsetof(LoopArgs, ctl) == 240 &&
-              offsetof(LoopArgs, pert) == 244,
-              "LoopArgs field offsets are fixed: the fused kernels' SASS reads them");
 #define NTM_LPT_BINS 160
 
 struct DeviceProps {
@@ -122,14 +96,17 @@ cudaError_t launch_getwlc(cudaStream_t st, const DeviceProps &dp, int layout, in
 cudaError_t launch_mc_stats(cudaStream_t st, const DeviceProps &dp, int layout, int S, int k_sim, const double *xk,
                             const double *uk, const double *cost, const int *status, const double *umin, const double *umax,
                             int ustride, const double *bounds, double w_sup, double hist_max, double *out, long long *launches);
-cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, long long *launches);
+// lpt: the two-phase launch's keys, order and bins (2 S + NTM_LPT_BINS ints; used when a.sv is set and lpt_doubles is
+// not 0), or NULL
+cudaError_t launch_closed_loop(cudaStream_t st, const DeviceProps &dp, const LoopArgs &a, int *lpt, long long *launches);
 
-// EXT template argument of closed_loop_kernel (ntm_loop.cuh): the cold code an instantiation carries
-constexpr int EXT_BOX = 0;          // the headline instantiations: Euler plant, box QP
-constexpr int EXT_COLD_PLANT = 1;   // + the RK4 / tau_E(w) plant options
-constexpr int EXT_STATE_ROWS = 2;   // + getWLc's state rows
-constexpr int EXT_PERTURBED = 3;    // box QP against a perturbed plant (LoopArgs::pert)
-constexpr int EXT_PERTURBED_ROWS = 4;   // getWLc's state rows against a perturbed plant (LoopArgs::pert, LoopArgs::ppd)
+// EXT template argument of closed_loop_kernel: the instantiation key; what each one carries is spelled out by the
+// members of LoopTraits (ntm_loop.cuh)
+constexpr int EXT_BOX = 0;
+constexpr int EXT_COLD_PLANT = 1;
+constexpr int EXT_STATE_ROWS = 2;
+constexpr int EXT_PERTURBED = 3;
+constexpr int EXT_PERTURBED_ROWS = 4;
 // one instantiation closed_loop_kernel<gw, dense, ext, lv, ctl>
 struct LoopKey {
     int gw;

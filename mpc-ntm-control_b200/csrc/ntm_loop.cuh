@@ -34,8 +34,8 @@ __device__ __forceinline__ double a22_taue(double a22n, double ctau, double w) {
 // RK4: the Euler map is x + g(x,u) with g = Ts * (dx/dt) of the GRE model, so the classical RK4 step over one sample
 // needs no extra parameter: k1 = g(x), k2 = g(x + k1/2), k3 = g(x + k2/2), k4 = g(x + k3),
 // x+ = x + (k1 + 2 k2 + 2 k3 + k4)/6, summed as ((k1 + 2 k2) + (2 k3 + k4)) / 6 (the order the tests' CPU checker uses).
-// The fused kernel carries this code only in its EXT instantiations: inlined into the literal hot kernel it cost
-// 44 bytes of spills at the 96-register budget, out of line 84.
+// The fused kernel carries this code only in its LoopTraits::COLD instantiations: inlined into the literal hot kernel
+// it cost 44 bytes of spills at the 96-register budget, out of line 84.
 __device__ __forceinline__ void plant_of(const Params &P, int flags, double a22n, double ctau, double w, double om,
                                          double u, double &nw, double &nom) {
     const bool te = (flags & NTM_PROFILE_TAUE_W) != 0;
@@ -62,10 +62,10 @@ __device__ __forceinline__ void plant_of(const Params &P, int flags, double a22n
     nom = om + (so + ao) / 6.0;
 }
 
-// The plant of ntm_plant_step and of the perturbed fused loop (EXT = 3), every rounding spelled out.  nvcc contracts
-// the products of plant_euler_a22 / plant_of into FMAs differently depending on where they are inlined: every fused-loop
-// instantiation evaluates a21 w + a22 om as fma(a22, om, a21 w), the RK4 / tau_E(w) plant kernel evaluated it as
-// fma(w, a21, a22 om), and the RK4 stages of the fused loop take w^2 + w_marg^2 (NTM_PROFILE_RHO1_SQ) as one FMA where
+// The plant of ntm_plant_step and of the perturbed fused loop (LoopTraits::PERT), every rounding spelled out.  nvcc
+// contracts the products of plant_euler_a22 / plant_of into FMAs differently depending on where they are inlined: every
+// fused-loop instantiation evaluates a21 w + a22 om as fma(a22, om, a21 w), the RK4 / tau_E(w) plant kernel evaluated
+// it as fma(w, a21, a22 om), and the RK4 stages of the fused loop take w^2 + w_marg^2 (NTM_PROFILE_RHO1_SQ) as one FMA where
 // the Euler map rounds w^2 first.  This function is the fused loop's form, so that stepping a controller with
 // ntm_plant_step reproduces the fused loop bit for bit under every plant profile, and so that the perturbed loop
 // gives ntm_plant_step's bits wherever it is instantiated.  a22n, ctau: as plant_of.
@@ -107,7 +107,7 @@ __device__ __forceinline__ void plant_exact(const Params &P, int flags, double a
 // =================================================================================================
 // fused persistent closed loop
 // =================================================================================================
-// Inclusive composition of the stage maps up to this thread's stage j (cold path of the EXT instantiation):
+// Inclusive composition of the stage maps up to this thread's stage j (cold path of the state rows):
 // (pa, pc) = first column of Phi's block j, s22 = its (2,2) entry a22^(j+1), (k1, k2) = Lambda's block j
 // (Rho_to_PhiGammaLambda.m:17-23,47-52), so that Phi_j*x + Lambda_j = (pa*x1 + k1, pc*x1 + s22*x2 + k2).
 template <int GW>
@@ -139,37 +139,79 @@ __device__ void stage_prefix(int N, int j, const Work &w, const Params &P, doubl
     }
 }
 
-// EXT: 0 = the headline instantiation (Euler plant, box QP), 1 = + the RK4 plant option, 2 = + getWLc's state rows,
-// 3 = box QP against a perturbed plant (LoopArgs::pert: its own parameters and profile bits, d_k and v_k),
-// 4 = getWLc's state rows against a perturbed plant (the code of 2 and of 3, without 2's record and tau_E(w) code)
-// LONG (long horizons, literal Gamma, box QP): the QP runs on the packed sweep tableau of ntm_long.cuh
-template <int GW, bool DENSE, int EXT>
+// What the instantiation closed_loop_kernel<GW, DENSE, EXT, LV, CTL> carries.  EXT (EXT_* in ntm_kernels.h) is only the
+// key: run_scenario and closed_loop_kernel test these members, never EXT itself.  (They are read through a type alias:
+// function-scope constexpr locals for the same conditions changed the register assignment of the literal state-row
+// kernels.)  CTL: the controller-step instantiation (ntm_mpc_step, ntm_mpc_step_sc) of a box instantiation with
+// multi-warp groups or of a state-row one; the one-warp box instantiations run controller steps as a runtime mode
+// (LoopArgs::ctl) at unchanged register counts, in the multi-warp ones that mode cost 2 registers, and 228 bytes of
+// spill stores in closed_loop_kernel<4, false, 0, 0>; the state-row ones sit at their register caps (DESIGN section 4.8).
+template <int GW, bool DENSE, int EXT, bool CTL = false>
 struct LoopTraits {
     static constexpr bool ROWS = (EXT == 2 || EXT == 4);   // getWLc's state rows
-    static constexpr bool PERT = (EXT == 3 || EXT == 4);   // the perturbed plant
+    static constexpr bool PERT = (EXT == 3 || EXT == 4);   // the perturbed plant (LoopArgs::pp: its own parameters and
+                                                           // profile bits, d_k and v_k)
+    static constexpr bool COLD = (EXT == 1 || EXT == 2);   // the controller's plant with the RK4 / tau_E(w) options, and
+                                                           // the controller-side tau_E(w)
+    // long horizons, literal Gamma, box QP: the QP runs on the packed sweep tableau of ntm_long.cuh
     static constexpr bool LONG = (GW > 1) && !DENSE && !ROWS;
+    static constexpr bool CTL_MODE = (GW == 1 && EXT == 0);   // LoopArgs::ctl selects the controller step at run time
+    // the record code (NTM_CTRL_DOUBLES): controller steps and the two-phase launch
+    static constexpr bool REC = (EXT == 0 && (GW == 1 || CTL)) || (EXT == 2 && CTL);
+    static constexpr bool REGEN = ROWS && CTL;   // a resumed frozen record rebuilds its rows (they are not stored)
+    // two-phase launch (headline instantiation only): a launch runs the time steps [k_begin, k_end) of the scenario
+    static constexpr bool TWOPH = (GW == 1) && !DENSE && (EXT == 0);
+    // __launch_bounds__ minimum blocks per SM
+    static constexpr int MIN_BLOCKS = GW == 1 ? (EXT == 0 ? 5 : ((EXT == 1 || EXT == 3) ? 4 : 3)) : (LONG ? 3 : 1);
     using WorkT = typename std::conditional<LONG, LongWork, Work>::type;
 };
 
-// The perturbed plant's inputs: LoopArgs::pp (EXT = 3), or the device copy LoopArgs::ppd points to (EXT = 4, whose
-// LoopArgs union holds the state box)
-template <int EXT>
-__device__ __forceinline__ const PlantIn &plant_in(const LoopArgs &a) {
-    if constexpr (EXT == 4) return *a.ppd;
-    else return a.pp;
+// getWLc's frozen rows (NTM_MPC_Sim.m:74, rho(x0) on every stage), kept at the offline build: Phi0, Lam0 from
+// stage_prefix, and the Gamma tile the Hessian build left in shared memory (dense Gamma, to Gam0) or P12 (literal),
+// and b0 = b of this build
+template <bool DENSE>
+__device__ __forceinline__ void freeze_rows(int N, int j, const Work &w, const ExtWork &xw, double *Gam0, double pa,
+                                            double pc, double k1, double k2, double bb, double &b0) {
+    if (j < N) {
+        xw.Phi0[j] = make_double2(pa, pc); xw.Lam0[j] = make_double2(k1, k2);
+        if constexpr (DENSE) {
+            const double2 *src = reinterpret_cast<const double2 *>(w.GamS + (size_t)j * w.ldgam);
+            double2 *dst = reinterpret_cast<double2 *>(Gam0 + (size_t)j * w.ldgam);
+            for (int i = 0; i < N; ++i) dst[i] = src[i];
+        } else {
+            xw.P0[j] = w.P12[j];
+        }
+    }
+    b0 = bb;
+}
+
+// The state rows of the QP at hand: the free response fs = Phi x + Lam of this stage, from the G, F just built
+// (srows = 1) or from the frozen rows, built at the first QP (srows = 2; literal Gamma: + the column scale cs = b0 / b)
+template <int GW, bool DENSE>
+__device__ __forceinline__ void state_rows_setup(int N, int j, const Work &w, const Params &P, const ExtWork &xw,
+                                                 double *Gam0, bool frozen, bool &built, double a11, double a21,
+                                                 double bb, double x1, double x2, double &s22, double &b0) {
+    const bool act = j < N;
+    if (!frozen || !built) {
+        double pa, pc, k1, k2;
+        stage_prefix<GW>(N, j, w, P, a11, a21, pa, pc, s22, k1, k2);
+        if (frozen) freeze_rows<DENSE>(N, j, w, xw, Gam0, pa, pc, k1, k2, bb, b0);
+        else if (act) xw.fs[j] = make_double2(fma(pa, x1, k1), fma(pc, x1, fma(s22, x2, k2)));
+        built = true;
+    }
+    if (frozen && act) {
+        const double2 ph = xw.Phi0[j], lm = xw.Lam0[j];
+        xw.fs[j] = make_double2(fma(ph.x, x1, lm.x), fma(ph.y, x1, fma(s22, x2, lm.y)));
+        if constexpr (!DENSE) xw.cs[j] = b0 / bb;
+    }
 }
 
 // LV (LONG only): 0 = tableau in registers (N + 1 <= 7 * 10 / 7 * 15 for 2 / 4 warps), 1 = tableau in shared memory
-// CTL (multi-warp groups with EXT = 0, every group size with EXT = 2): the controller-step instantiation (ntm_mpc_step,
-// ntm_mpc_step_sc).  The one-warp box instantiations run controller steps as a runtime mode (LoopArgs::ctl) at unchanged
-// register counts; in the multi-warp ones that mode cost 2 registers, and 228 bytes of spill stores in
-// closed_loop_kernel<4, false, 0, 0>; the state-row ones sit at their register caps (DESIGN section 4.8).
 template <int GW, bool DENSE, int EXT, int LV = 0, bool CTL = false>
-__device__ void run_scenario(const LoopArgs &a, int s, int j, const typename LoopTraits<GW, DENSE, EXT>::WorkT &w,
+__device__ void run_scenario(const LoopArgs &a, int s, int j, const typename LoopTraits<GW, DENSE, EXT, CTL>::WorkT &w,
                              unsigned char *gbase, int tI = -1, int tJ = -1) {
     using Gp = Group<GW>;
-    constexpr bool LONG = LoopTraits<GW, DENSE, EXT>::LONG;
-    using LT = LoopTraits<GW, DENSE, EXT>;               // LT::ROWS, LT::PERT (a constexpr local here moves registers)
+    using LT = LoopTraits<GW, DENSE, EXT, CTL>;
     const int N = a.N, S = a.S, flags = a.flags, layout = a.layout;
     const bool act = j < N;
     const bool lead = (j == 0);
@@ -179,25 +221,24 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     Gp::sync();
     const Params &P = *w.prm;
     // controller step (ntm_mpc_step[_sc]): a.x0 is the measured state, the loop state comes from the caller's record
-    constexpr bool REC = (EXT == 0 && (GW == 1 || CTL)) || (EXT == 2 && CTL);   // instantiations that carry the record code
-    const bool ctl = (GW == 1 && EXT == 0) ? (a.ctl != 0) : CTL;
+    const bool ctl = LT::CTL_MODE ? (a.ctl != 0) : CTL;
     double x01 = __ldg(a.x0 + elem(layout, S, 2, s, 0)), x02 = __ldg(a.x0 + elem(layout, S, 2, s, 1));
     double x1 = x01, x2 = x02;
-    // perturbed plant (EXT = 3, 4): (x1, x2) is what the controller sees, y_k = x_k + v_k; the offline build (:63-65)
+    // perturbed plant: (x1, x2) is what the controller sees, y_k = x_k + v_k; the offline build (:63-65)
     // and frozen state rows (:74) run from y_0.  The true state x_k lives in xk only (written by the lead, read back by
     // the group after a barrier), so no register carries it across the loop.
     if constexpr (LT::PERT) {
-        const PlantIn &pi = plant_in<EXT>(a);
+        const PlantIn &pi = a.pp;
         if (pi.noise != nullptr) {
             x01 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 0)); x02 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 1));
             x1 = x01; x2 = x02;
         }
     }
-    // NTM_PROFILE_TAUE_W (EXT instantiations only): the shared parameter block carries the a22 the controller holds over
+    // NTM_PROFILE_TAUE_W (COLD only): the shared parameter block carries the a22 the controller holds over
     // the horizon of the current time step, a22(tau_E(xk(1,k))); the nominal value and c_tauE stay in registers
     [[maybe_unused]] double a22n = 0.0, ctau = 0.0;
     [[maybe_unused]] bool taue = false;
-    if constexpr (EXT == 1 || EXT == 2) {
+    if constexpr (LT::COLD) {
         taue = (flags & NTM_PROFILE_TAUE_W) != 0;
         a22n = P.a22;
         if (taue) {
@@ -227,23 +268,21 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     double Uj = 0.0, cost = 0.0;
     QpHist hist = {0.0, 0.0, -1, -1, 0};                 // previous two QP solutions (warm-start candidates)
     double hU1 = 0.0, hU2 = 0.0;                         // the same in U-space (literal path: the QP runs in y = b .* U)
-    [[maybe_unused]] double b0 = bb, s22 = 0.0;          // EXT, frozen state rows: b and a22^(j+1) of the offline build
+    [[maybe_unused]] double b0 = bb, s22 = 0.0;          // frozen state rows: b and a22^(j+1) of the offline build
     [[maybe_unused]] bool rows_built = false;
     int hs1 = -1, hs2 = -1;
     bool first_qp = true;
-    // state rows (EXT 2, 4), literal Gamma: active sets of the last two state-row QPs of this scenario, offered to the
+    // state rows, literal Gamma: active sets of the last two state-row QPs of this scenario, offered to the
     // next one as a warm start (per thread: (vst + 1) | mask of this state's four rows << 2), and the "warm start failed,
     // run this QP again cold" flag
     [[maybe_unused]] int hw1 = 0, hw2 = 0, hwn = 0;
     [[maybe_unused]] bool retry = false;
-    [[maybe_unused]] bool regen_rows = false;            // EXT == 2, CTL: rebuild the frozen rows of a resumed record first
+    [[maybe_unused]] bool regen_rows = false;            // REGEN: rebuild the frozen rows of a resumed record first
     int status = 0, inner = 0, qpit = 0, k = 0, it = 0;
     const int qp_cap = 10 * N + 20;
-    // two-phase launch (headline instantiation only): this launch runs the time steps [k_begin, k_end) of the scenario
-    constexpr bool TWOPH = (GW == 1) && !DENSE && (EXT == 0);
     [[maybe_unused]] int nslow = 0, nqpit = 0;
     bool resumed = false;
-    if constexpr (REC) {
+    if constexpr (LT::REC) {
         // The loop state a record carries across a time step (layout: NTM_CTRL_DOUBLES in include/ntm_mpc.h), restored
         // for phase B of a two-phase launch and for a controller step whose record has run before.  G and F for the first
         // QP are rebuilt at the top of the loop from the same stage entries and from x0 or (NTM_PROFILE_F_XK) the last
@@ -259,14 +298,14 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                     hist.u1 = sv[4 * N + j]; hist.u2 = sv[5 * N + j]; hist.s1 = (pk & 3) - 1; hist.s2 = ((pk >> 2) & 3) - 1;
                 } else {
                     hU1 = sv[4 * N + j]; hU2 = sv[5 * N + j]; hs1 = (pk & 3) - 1; hs2 = ((pk >> 2) & 3) - 1;
-                    if constexpr (EXT == 2) { hw1 = (pk >> 4) & 63; hw2 = (pk >> 10) & 63; }
+                    if constexpr (LT::ROWS) { hw1 = (pk >> 4) & 63; hw2 = (pk >> 10) & 63; }
                 }
             }
             x1 = sv[N7]; x2 = sv[N7 + 1]; x01 = sv[N7 + 2]; x02 = sv[N7 + 3]; cost = sv[N7 + 4];
             const int fl = (int)sv[N7 + 5];
             status = ctl ? 0 : (fl & 3); first_qp = ((fl >> 2) & 1) != 0; hist.n = (fl >> 3) & 3;
             k = ctl ? 0 : a.k_begin;
-            if constexpr (EXT == 2) {
+            if constexpr (LT::REGEN) {
                 hwn = (fl >> 5) & 3;
                 // Frozen rows (:74) are a function of x0 alone and are not stored: the first pass of the loop builds
                 // G, F from rho(x0) on every stage, exactly as the offline build did, copies the rows out and then
@@ -292,25 +331,14 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
     // Written as a single loop so that build_GF and qp_solve are instantiated once (instruction-cache footprint).
     for (;;) {
         double Fj;
-        if constexpr (LONG) Fj = build_GF_toeplitz_packed<GW>(N, j, w, P, fxk ? x1 : x01, fxk ? x2 : x02);
+        if constexpr (LT::LONG) Fj = build_GF_toeplitz_packed<GW>(N, j, w, P, fxk ? x1 : x01, fxk ? x2 : x02);
         else Fj = build_GF<GW, DENSE>(N, j, w, P, flags, a11, a21, sE, fxk ? x1 : x01, fxk ? x2 : x02);
-        if constexpr (EXT == 2 && CTL) {
+        if constexpr (LT::REGEN) {
             if (regen_rows) {                            // the offline build of a resumed frozen record: keep its rows
-                const ExtWork xw = carve_ext(gbase + a.qbytes, N);
                 double pa, pc, k1, k2;
                 stage_prefix<GW>(N, j, w, P, a11, a21, pa, pc, s22, k1, k2);
-                if (act) {
-                    xw.Phi0[j] = make_double2(pa, pc); xw.Lam0[j] = make_double2(k1, k2);
-                    if constexpr (DENSE) {
-                        double *Gam0 = reinterpret_cast<double *>(gbase + a.qbytes + ext_bytes(N));
-                        const double2 *src = reinterpret_cast<const double2 *>(w.GamS + (size_t)j * w.ldgam);
-                        double2 *dst = reinterpret_cast<double2 *>(Gam0 + (size_t)j * w.ldgam);
-                        for (int i = 0; i < N; ++i) dst[i] = src[i];
-                    } else {
-                        xw.P0[j] = w.P12[j];
-                    }
-                }
-                b0 = bb;
+                freeze_rows<DENSE>(N, j, w, carve_ext(gbase + a.qbytes, N),
+                                   reinterpret_cast<double *>(gbase + a.qbytes + ext_bytes(N)), pa, pc, k1, k2, bb, b0);
                 rows_built = true; regen_rows = false;
                 const double *sv = a.sv + (size_t)s * NTM_CTRL_DOUBLES(N);
                 if (act) { a11 = sv[j]; a21 = sv[N + j]; bb = sv[2 * N + j]; }
@@ -334,7 +362,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                 if constexpr (LT::PERT) {
                     // the plant's own block and profile bits, read here (once per time step, no shared copy), then + d_k
                     if (!isfinite(u0)) status = max(status, (int)NTM_SCN_NONFINITE);
-                    const PlantIn &pi = plant_in<EXT>(a);
+                    const PlantIn &pi = a.pp;
                     const Params Q = load_params(pi.pparams, layout, pi.pparams_count, s);
                     const int pf = pi.pflags;
                     const double qtau = (pf & NTM_PROFILE_TAUE_W)
@@ -356,10 +384,10 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                     if (!isfinite(u0)) status = max(status, (int)NTM_SCN_NONFINITE);
                 } else {
                     double nw, nom;
-                    if constexpr (EXT != 0) plant_of(P, flags, a22n, ctau, x1, x2, u0, nw, nom);   // :130, or its RK4 / tau_E(w) refinement
+                    if constexpr (LT::COLD) plant_of(P, flags, a22n, ctau, x1, x2, u0, nw, nom);   // :130, or its RK4 / tau_E(w) refinement
                     else plant_euler(P, flags, x1, x2, u0, nw, nom);                // :130
                     x1 = nw; x2 = nom;
-                    if constexpr (EXT != 0) {
+                    if constexpr (LT::COLD) {
                         if (taue) {                      // tau_E of the new measured width, held over the next step's horizon
                             Gp::sync();                  // (G, F just built keep the previous value: a workspace assignment)
                             if (lead) w.prm->a22 = a22_taue(a22n, ctau, x1);
@@ -384,7 +412,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                     if (a.qpit) a.qpit[elem(layout, S, a.k_sim, s, k)] = qpit;
                 }
                 ++k; it = 0; qpit = 0;
-                if constexpr (REC) {
+                if constexpr (LT::REC) {
                     // the record (see the restore above): end of a controller step, or of phase A (then the next scenario)
                     if (a.sv != nullptr && (ctl || (k == a.k_end && k < a.k_sim))) {
                         const int N7 = 7 * N;
@@ -392,20 +420,15 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                         if (act) {
                             sv[j] = a11; sv[N + j] = a21; sv[2 * N + j] = bb; sv[3 * N + j] = Uold;
                             sv[4 * N + j] = dense ? hist.u1 : hU1; sv[5 * N + j] = dense ? hist.u2 : hU2;
-                            if constexpr (EXT == 2)          // + the active sets of the last two state-row QPs (literal)
-                                sv[6 * N + j] = dense ? (double)((hist.s1 + 1) | ((hist.s2 + 1) << 2))
-                                                      : (double)((hs1 + 1) | ((hs2 + 1) << 2) | (hw1 << 4) | (hw2 << 10));
-                            else
-                                sv[6 * N + j] = dense ? (double)((hist.s1 + 1) | ((hist.s2 + 1) << 2)) : (double)((hs1 + 1) | ((hs2 + 1) << 2));
+                            // + the active sets of the last two state-row QPs (literal Gamma; 0 outside ROWS)
+                            sv[6 * N + j] = dense ? (double)((hist.s1 + 1) | ((hist.s2 + 1) << 2))
+                                                  : (double)((hs1 + 1) | ((hs2 + 1) << 2) | (hw1 << 4) | (hw2 << 10));
                         }
                         if (lead) {
                             sv[N7] = x1; sv[N7 + 1] = x2; sv[N7 + 2] = x01; sv[N7 + 3] = x02; sv[N7 + 4] = cost;
-                            if constexpr (EXT == 2)
-                                sv[N7 + 5] = (double)((status & 3) | ((first_qp ? 1 : 0) << 2) | (hist.n << 3) | (hwn << 5));
-                            else
-                                sv[N7 + 5] = (double)((status & 3) | ((first_qp ? 1 : 0) << 2) | (hist.n << 3));
+                            sv[N7 + 5] = (double)((status & 3) | ((first_qp ? 1 : 0) << 2) | (hist.n << 3) | (hwn << 5));
                             sv[N7 + 6] = ctl ? sv[N7 + 6] + 1.0 : (double)k;
-                            if constexpr (TWOPH) {
+                            if constexpr (LT::TWOPH) {
                                 if (!ctl) a.lpt_key[s] = min(12 * min(nslow, 12) + min(nqpit, 11), NTM_LPT_BINS - 1);
                             }
                         }
@@ -419,7 +442,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             if (it == 0) {               // as for a controller step: the measurement y_k = x_k + v_k
                 Gp::sync();              // the lead has just written x_k
                 x1 = a.xk[xk_at(2 * k)]; x2 = a.xk[xk_at(2 * k + 1)];
-                const PlantIn &pi = plant_in<EXT>(a);
+                const PlantIn &pi = a.pp;
                 if (pi.noise != nullptr) {
                     x1 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k)); x2 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k + 1));
                 }
@@ -431,6 +454,10 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
         if (!retry) ++it;
         int nit = 0;
         int st = NTM_SCN_OK;
+        // the x_0 block of getWLc.m:30 has no U: it only asks that x_k itself (y_k under a perturbed plant: the state the
+        // controller sees) is inside the state box
+        [[maybe_unused]] bool x0bad = false;
+        if constexpr (LT::ROWS) x0bad = x1 < a.xmin1 || x1 > a.xmax1 || x2 < a.xmin2 || x2 > a.xmax2;
         if constexpr (DENSE) {
             st = qp_solve<GW>(N, j, w, Fj, P.umin, P.umax, hist, Uj, qp_cap, nit);   // :97
             if constexpr (LT::ROWS && GW == 1) {
@@ -440,30 +467,11 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                     // frozen rows (:74) keep a copy of the offline tile.  QP variables are U itself here.  Every QP starts
                     // cold from the box minimiser: the literal branch's warm start, tried here, moved one scenario of the
                     // parity sample by 2 % in one input on the consistent profile (chaotic at the 1e-4 level).
-                    const bool x0bad = x1 < a.xmin1 || x1 > a.xmax1 || x2 < a.xmin2 || x2 > a.xmax2;   // getWLc.m:30
                     const IneqWork q = carve_ineq(gbase + a.wbytes, N, 4 * N);
                     const ExtWork xw = carve_ext(gbase + a.qbytes, N);
                     double *Gam0 = reinterpret_cast<double *>(gbase + a.qbytes + ext_bytes(N));
                     const bool frozen = a.srows == 2;
-                    if (!frozen || !rows_built) {
-                        double pa, pc, k1, k2;
-                        stage_prefix<GW>(N, j, w, P, a11, a21, pa, pc, s22, k1, k2);
-                        if (frozen) {
-                            if (act) {
-                                xw.Phi0[j] = make_double2(pa, pc); xw.Lam0[j] = make_double2(k1, k2);
-                                const double2 *src = reinterpret_cast<const double2 *>(w.GamS + (size_t)j * w.ldgam);
-                                double2 *dst = reinterpret_cast<double2 *>(Gam0 + (size_t)j * w.ldgam);
-                                for (int i = 0; i < N; ++i) dst[i] = src[i];
-                            }
-                        } else if (act) {
-                            xw.fs[j] = make_double2(fma(pa, x1, k1), fma(pc, x1, fma(s22, x2, k2)));
-                        }
-                        rows_built = true;
-                    }
-                    if (frozen && act) {
-                        const double2 ph = xw.Phi0[j], lm = xw.Lam0[j];
-                        xw.fs[j] = make_double2(fma(ph.x, x1, lm.x), fma(ph.y, x1, fma(s22, x2, lm.y)));
-                    }
+                    state_rows_setup<GW, true>(N, j, w, P, xw, Gam0, frozen, rows_built, a11, a21, bb, x1, x2, s22, b0);
                     Gp::sync();
                     if (st == NTM_SCN_OK) {
                         const DenseRows rows = {frozen ? Gam0 : w.GamS, w.ldgam, xw.fs, a.xmin1, a.xmax1, a.xmin2, a.xmax2, N};
@@ -493,12 +501,8 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             // state rows: offer the active set of the QP before last (or the last one) instead of solving the box QP first
             [[maybe_unused]] bool try_warm = false;
             [[maybe_unused]] int wv = 0, wm = -1;
-            [[maybe_unused]] bool x0bad = false;
             if constexpr (LT::ROWS) {
                 if (a.srows != 0) {
-                    // the x_0 block of getWLc.m:30 has no U: it only asks that x_k itself (y_k under a perturbed plant:
-                    // the state the controller sees) is inside the state box
-                    x0bad = x1 < a.xmin1 || x1 > a.xmax1 || x2 < a.xmin2 || x2 > a.xmax2;
                     if ((a.rows_warm & 1) && !retry && hwn > 0 && !x0bad) {
                         const int hh = (hwn >= 2) ? hw2 : hw1;
                         wv = (hh & 3) - 1; wm = hh >> 2;
@@ -511,16 +515,16 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
             if (!try_warm) {
                 hist.u1 = bb * hU1; hist.u2 = bb * hU2;
                 hist.s1 = neg ? -hs1 : hs1; hist.s2 = neg ? -hs2 : hs2;
-                if constexpr (LONG && LV == 0) {
+                if constexpr (LT::LONG && LV == 0) {
                     const TileWork tw = {w.tpcb, w.tybuf, w.tgbuf, w.tpcn};
                     st = qp_solve_tile<GW>(N, j, w, tw, tI, tJ, Fj, fmin(yl, yh), fmax(yl, yh), hist, yj, qp_cap, nit);
-                } else if constexpr (LONG) {
+                } else if constexpr (LT::LONG) {
                     const auto regen = make_regen([&]() {      // the tableau is rebuilt from the stage entries (same values)
                         build_GF_toeplitz_packed<GW>(N, j, w, P, fxk ? x1 : x01, fxk ? x2 : x02);
                     });
                     st = qp_solve_long<GW>(N, j, w, Fj, fmin(yl, yh), fmax(yl, yh), hist, yj, qp_cap, nit, regen);
                 } else {
-                    if constexpr (TWOPH) {
+                    if constexpr (LT::TWOPH) {
                         st = qp_solve<GW>(N, j, w, Fj, fmin(yl, yh), fmax(yl, yh), hist, yj, qp_cap, nit, &nslow);
                         nqpit += nit - 1;
                     } else {
@@ -541,22 +545,7 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                     const IneqWork q = carve_ineq(gbase + a.wbytes, N, 4 * N);
                     const ExtWork xw = carve_ext(gbase + a.qbytes, N);
                     const bool frozen = a.srows == 2;
-                    if (!frozen || !rows_built) {
-                        double pa, pc, k1, k2;
-                        stage_prefix<GW>(N, j, w, P, a11, a21, pa, pc, s22, k1, k2);
-                        if (frozen) {                                  // :74 sits outside the loops: rho(x0) on every stage
-                            if (act) { xw.P0[j] = w.P12[j]; xw.Phi0[j] = make_double2(pa, pc); xw.Lam0[j] = make_double2(k1, k2); }
-                            b0 = bb;
-                        } else if (act) {
-                            xw.fs[j] = make_double2(fma(pa, x1, k1), fma(pc, x1, fma(s22, x2, k2)));
-                        }
-                        rows_built = true;
-                    }
-                    if (frozen && act) {
-                        const double2 ph = xw.Phi0[j], lm = xw.Lam0[j];
-                        xw.fs[j] = make_double2(fma(ph.x, x1, lm.x), fma(ph.y, x1, fma(s22, x2, lm.y)));
-                        xw.cs[j] = b0 / bb;
-                    }
+                    state_rows_setup<GW, false>(N, j, w, P, xw, nullptr, frozen, rows_built, a11, a21, bb, x1, x2, s22, b0);
                     Gp::sync();
                     if (st == NTM_SCN_OK) {
                         const StateRows rows = {frozen ? xw.P0 : w.P12, xw.fs, frozen ? xw.cs : nullptr,
@@ -661,24 +650,23 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
 }
 
 template <int GW, bool DENSE, int EXT, int LV = 0, bool CTL = false>
-__global__ void __launch_bounds__(GW == 1 ? 128 : 32 * GW,
-                                  GW == 1 ? (EXT == 0 ? 5 : ((EXT == 1 || EXT == 3) ? 4 : 3)) : (LoopTraits<GW, DENSE, EXT>::LONG ? 3 : 1))
+__global__ void __launch_bounds__(GW == 1 ? 128 : 32 * GW, (LoopTraits<GW, DENSE, EXT, CTL>::MIN_BLOCKS))
 closed_loop_kernel(LoopArgs a, unsigned int gbytes) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     using Gp = Group<GW>;
     const int gib = (GW == 1) ? (int)(threadIdx.x >> 5) : 0;
     const int j = (GW == 1) ? (int)(threadIdx.x & 31) : (int)threadIdx.x;
     const int gpb = (GW == 1) ? (int)(blockDim.x >> 5) : 1;
-    using WorkT = typename LoopTraits<GW, DENSE, EXT>::WorkT;
-    WorkT w;
-    if constexpr (LoopTraits<GW, DENSE, EXT>::LONG) {
+    using LT = LoopTraits<GW, DENSE, EXT, CTL>;
+    typename LT::WorkT w;
+    if constexpr (LT::LONG) {
         w = carve_long(smem_raw, a.N);
     } else {
         double *hbig = a.hscratch + ((size_t)blockIdx.x * gpb + gib) * a.N * odd_ld(a.N);
         w = carve(smem_raw + (size_t)gib * gbytes, a.N, a.hcap, hbig, a.gam);
     }
     int tI = -1, tJ = -1;
-    if constexpr (LoopTraits<GW, DENSE, EXT>::LONG && LV == 0) tile_coords(j, (a.N + 1 + NTM_TS - 1) / NTM_TS, tI, tJ);
+    if constexpr (LT::LONG && LV == 0) tile_coords(j, (a.N + 1 + NTM_TS - 1) / NTM_TS, tI, tJ);
     if (w.GamS) for (int i = j; i < (int)gam_doubles(a.N, a.gam); i += Gp::T) w.GamS[i] = 0.0;
     for (int i = j; i < 2 * a.N; i += Gp::T) { w.QP12[i] = make_double2(0.0, 0.0); w.QE12[i] = make_double2(0.0, 0.0); }
     Gp::sync();
