@@ -6,6 +6,8 @@
  * message of the last failure on the calling thread.  A handle owns one CUDA device, one stream and
  * its scratch buffers; it is not thread-safe (one handle per host thread / per GPU).
  *
+ * An argument error returns NTM_ERR_INVALID before anything is allocated, copied or launched.
+ *
  * There is NO CPU fallback: every compute entry point launches hand-written sm_100a kernels and
  * fails with NTM_ERR_CUDA when no CUDA device is usable.
  *
@@ -258,8 +260,8 @@ int ntm_mpc_step_dev(ntm_handle *h, int layout, int profile, int S, int N, int i
  * hw = (v + 1) + 4 m with v the variable's bound state and bit q of m = row 4j + q active; [6N + j] carries
  * 16 hw1 + 1024 hw2 and [7N+5] carries 32 hwn (hwn = how many of hw1, hw2 are valid, 0..2).  Frozen rows (:74) are
  * not stored: each resumed step rebuilds them from rho(x0) with x0 from [7N+2, 7N+4), one extra G, F build.
- * NTM_ERR_INVALID, nothing launched: NTM_PROFILE_TAUE_W, state_rows outside 0..2, NULL or inverted xbounds,
- * GAMMA_I / DENSE_G with N > 32, a horizon whose factors do not fit shared memory. */
+ * NTM_ERR_INVALID: NTM_PROFILE_TAUE_W, state_rows outside 0..2, NULL or inverted xbounds, GAMMA_I / DENSE_G with
+ * N > 32, a horizon whose factors do not fit shared memory. */
 int ntm_mpc_step_sc(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
                     const double *params, int params_count, int state_rows, const double *xbounds, double *state,
                     double *u, double *U, int *inner_iters, int *qp_iters, int *status);
@@ -282,8 +284,8 @@ int ntm_mpc_step_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, in
  * plant_params = params, plant_profile = the plant bits of profile and w = v = NULL, every output is bit-identical to
  * ntm_mpc_closed_loop.  The controller solves the box QP; ntm_mpc_closed_loop_perturbed_sc below keeps getWLc's state
  * rows.  A controller-side tau_E(w) is not offered.
- * NTM_ERR_INVALID, nothing copied or launched: bad sizes, NULL x0 / xk / uk / params, plant_params_count not 1 or S,
- * a controller profile with TAUE_W, a plant_profile bit outside the four above. */
+ * NTM_ERR_INVALID: bad sizes, NULL x0 / xk / uk / params, plant_params_count not 1 or S, a controller profile with
+ * TAUE_W, a plant_profile bit outside the four above. */
 int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
                                   const double *x0, const double *params, int params_count, const double *plant_params,
                                   int plant_params_count, int plant_profile, const double *w, const double *v,
@@ -310,7 +312,7 @@ int ntm_mpc_closed_loop_perturbed_dev(ntm_handle *h, int layout, int profile, in
  * (plant_params NULL, plant_profile = the plant bits of profile, w = v = NULL) every output is bit-identical to
  * ntm_mpc_closed_loop_sc.  The plant's inputs travel to the kernel with its launch parameters: the _dev entry queues
  * the launch and no copy.
- * NTM_ERR_INVALID, nothing copied or launched: whatever ntm_mpc_closed_loop_perturbed or ntm_mpc_step_sc rejects. */
+ * NTM_ERR_INVALID: whatever ntm_mpc_closed_loop_perturbed or ntm_mpc_step_sc rejects. */
 int ntm_mpc_closed_loop_perturbed_sc(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
                                      double eps, const double *x0, const double *params, int params_count,
                                      int state_rows, const double *xbounds, const double *plant_params,
@@ -331,7 +333,8 @@ int ntm_mpc_closed_loop_perturbed_sc_dev(ntm_handle *h, int layout, int profile,
  * moves it straight between the caller's arrays and its own HBM on its own host thread and stream -- no collective,
  * the D2H copy of each shard IS the gather.  devices = NULL: ordinals 0..n_devices-1; n_devices = 0: every visible
  * device.  params_count is 1 or S.  state_rows / xbounds as in ntm_mpc_closed_loop_sc (NTM_STATE_ROWS_OFF, NULL for
- * the EC-power box only).  Results are bit-identical to the single-device call for every n_devices. */
+ * the EC-power box only).  Results are bit-identical to the single-device call for every n_devices.  The pooled
+ * handles are created on first use, before the arguments of that call are checked against each device. */
 int ntm_device_count(int *count);
 long long ntm_pool_launch_count(int device);   /* kernels launched so far by the pooled handle of `device`, -1 if none */
 int ntm_mpc_closed_loop_multi(int n_devices, const int *devices, int layout, int profile, int S, int N, int k_sim,

@@ -2,8 +2,10 @@
 //
 // Host-pointer entry points stage through a grow-only device arena owned by the handle:
 // H2D copies, kernel launch and D2H copies are all enqueued on the handle's stream, then the
-// call blocks on the stream.  *_dev entry points only enqueue.  No exceptions leave this file
+// call blocks on the stream.  *_dev entry points only enqueue.  Every entry checks all of its
+// arguments before it allocates, copies or launches anything.  No exceptions leave this file
 // and there is no CPU fallback: without a usable CUDA device ntm_create fails with NTM_ERR_CUDA.
+#include <algorithm>
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
@@ -12,6 +14,7 @@
 #include <new>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/ntm_mpc.h"
@@ -42,9 +45,9 @@ struct ntm_handle {
     double *hscratch = nullptr;      // global LDL' slabs for horizons whose G + H exceed shared memory
     size_t hscratch_bytes = 0;
     double *sv = nullptr;            // two-phase launch: saved loop state (ntm::LoopArgs::sv) ...
-    size_t sv_doubles = 0;
+    size_t sv_bytes = 0;
     int *lpt = nullptr;              // ... and keys + order + bins of its longest-first work queue
-    size_t lpt_ints = 0;
+    size_t lpt_bytes = 0;
     long long launches = 0;
 };
 
@@ -61,6 +64,12 @@ namespace {
         if (!(cond)) return fail(NTM_ERR_INVALID, "%s", msg); \
     } while (0)
 
+#define TRY(expr)                      \
+    do {                               \
+        int rc__ = (expr);             \
+        if (rc__ != NTM_OK) return rc__; \
+    } while (0)
+
 int check_common(ntm_handle *h, int layout, int S) {
     REQUIRE(h != nullptr, "handle is NULL");
     REQUIRE(layout == NTM_LAYOUT_MATLAB || layout == NTM_LAYOUT_SOA, "unknown layout");
@@ -75,6 +84,22 @@ int check_params(const double *params, int pc, int S) {
     return NTM_OK;
 }
 
+// Grows a handle-owned device buffer to `bytes` unless it already holds `need`; it never shrinks.  Work still queued on
+// the handle's stream may use the old buffer, so the stream is drained before it is freed.
+template <typename T>
+int grow(ntm_handle *h, T *&buf, size_t &have, size_t need, size_t bytes) {
+    if (need <= have) return NTM_OK;
+    CU(cudaStreamSynchronize(h->stream));
+    if (buf) CU(cudaFree(buf));
+    buf = nullptr; have = 0;
+    cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&buf), bytes);
+    if (e != cudaSuccess) return fail(NTM_ERR_ALLOC, "cudaMalloc(%zu): %s", bytes, cudaGetErrorString(e));
+    have = bytes;
+    return NTM_OK;
+}
+template <typename T>
+int grow(ntm_handle *h, T *&buf, size_t &have, size_t bytes) { return grow(h, buf, have, bytes, bytes); }
+
 // ---- arena -------------------------------------------------------------------------------------
 // The buffers of one host-pointer call, carved from the handle's grow-only device arena.  A call declares them once, in a
 // layout callback of take<T>(count) calls; reserve runs it twice, to size the arena and to hand the buffers out, so the
@@ -86,15 +111,7 @@ class Arena {
     int reserve(F layout) {
         base = nullptr; used = 0;                        // sizing pass: take() returns NULL
         layout(*this);
-        if (used > h->arena_bytes) {
-            CU(cudaStreamSynchronize(h->stream));
-            if (h->arena) CU(cudaFree(h->arena));
-            h->arena = nullptr; h->arena_bytes = 0;
-            const size_t want_bytes = used + used / 4;
-            cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&h->arena), want_bytes);
-            if (e != cudaSuccess) return fail(NTM_ERR_ALLOC, "cudaMalloc(%zu): %s", want_bytes, cudaGetErrorString(e));
-            h->arena_bytes = want_bytes;
-        }
+        TRY(grow(h, h->arena, h->arena_bytes, used, used + used / 4));
         base = h->arena; used = 0;
         layout(*this);
         return NTM_OK;
@@ -112,38 +129,6 @@ class Arena {
     size_t used = 0;
 };
 
-int ensure_hscratch(ntm_handle *h, int N) {
-    const size_t need = ntm::hscratch_bytes(h->props, N);
-    if (need <= h->hscratch_bytes) return NTM_OK;
-    CU(cudaStreamSynchronize(h->stream));
-    if (h->hscratch) CU(cudaFree(h->hscratch));
-    h->hscratch = nullptr; h->hscratch_bytes = 0;
-    cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&h->hscratch), need);
-    if (e != cudaSuccess) return fail(NTM_ERR_ALLOC, "cudaMalloc(%zu): %s", need, cudaGetErrorString(e));
-    h->hscratch_bytes = need;
-    return NTM_OK;
-}
-
-int ensure_lpt(ntm_handle *h, size_t doubles, size_t ints) {
-    if (doubles <= h->sv_doubles && ints <= h->lpt_ints) return NTM_OK;
-    CU(cudaStreamSynchronize(h->stream));
-    if (doubles > h->sv_doubles) {
-        if (h->sv) CU(cudaFree(h->sv));
-        h->sv = nullptr; h->sv_doubles = 0;
-        cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&h->sv), doubles * sizeof(double));
-        if (e != cudaSuccess) return fail(NTM_ERR_ALLOC, "cudaMalloc(%zu): %s", doubles * sizeof(double), cudaGetErrorString(e));
-        h->sv_doubles = doubles;
-    }
-    if (ints > h->lpt_ints) {
-        if (h->lpt) CU(cudaFree(h->lpt));
-        h->lpt = nullptr; h->lpt_ints = 0;
-        cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&h->lpt), ints * sizeof(int));
-        if (e != cudaSuccess) return fail(NTM_ERR_ALLOC, "cudaMalloc(%zu): %s", ints * sizeof(int), cudaGetErrorString(e));
-        h->lpt_ints = ints;
-    }
-    return NTM_OK;
-}
-
 template <typename T>
 int h2d(ntm_handle *h, T *dst, const T *src, size_t count) {
     if (count == 0) return NTM_OK;
@@ -157,13 +142,7 @@ int d2h(ntm_handle *h, T *dst, const T *src, size_t count) {
     return NTM_OK;
 }
 
-#define TRY(expr)                      \
-    do {                               \
-        int rc__ = (expr);             \
-        if (rc__ != NTM_OK) return rc__; \
-    } while (0)
-
-// shard copies: see closed_loop_host_impl
+// shard copies: see fused_host
 template <typename T>
 int h2d_shard(ntm_handle *h, int layout, T *dst, const T *src, size_t E, size_t S, size_t S_total, size_t s_off) {
     if (S == 0 || E == 0) return NTM_OK;
@@ -183,77 +162,300 @@ int d2h_shard(ntm_handle *h, int layout, T *dst, const T *src, size_t E, size_t 
     return NTM_OK;
 }
 
-// Arrays of a fused call (closed loop, perturbed loop, controller step), the caller's or their device copies; NULL = not
-// passed.  x0 is the measured state of a controller step, state its records.
-struct Fused {
-    const double *x0, *params, *pparams, *w, *v;
-    double *state, *xk, *uk, *Uk, *cost;
-    int *inner, *qpit, *status;
-};
+// ---- fused calls: closed loop, perturbed loop, controller step -------------------------------------------------------
+// A fused call is the ntm::LoopArgs of its launch.  Its entry fills in the caller's arrays (NULL = not passed) and its
+// mode: srows, ctl with the controller records in sv, pert with the plant in pp, rec_ld and rec_status.  check_fused
+// checks it, then the dev path launches it as it is and the host path stages its arrays first.
 
-// Fills the LoopArgs fields every fused call shares and launches it.  The entry has set its own mode fields (srows and the
-// state box, sv and ctl, pp and pert, rec_ld and rec_status) and checked its arguments.
-static int launch_fused(ntm_handle *h, ntm::LoopArgs &a, int layout, int flags, int S, int N, int k_sim, int i_sim,
-                        double eps, int pc, const Fused &d) {
-    a.layout = layout; a.flags = flags; a.S = S; a.N = N; a.k_sim = k_sim; a.i_sim = i_sim; a.eps = eps;
-    a.x0 = d.x0; a.params = d.params; a.params_count = pc;
-    a.xk = d.xk; a.uk = d.uk; a.Uk = d.Uk; a.cost = d.cost; a.inner = d.inner; a.qpit = d.qpit; a.status = d.status;
+ntm::LoopArgs loop_args(int layout, int profile, int S, int N, int k_sim, int i_sim, double eps, const double *x0,
+                        const double *params, int pc, int state_rows, double *xk, double *uk, double *Uk, double *cost,
+                        int *inner, int *qpit, int *status) {
+    ntm::LoopArgs a = {};
+    a.layout = layout; a.flags = profile; a.S = S; a.N = N; a.k_sim = k_sim; a.i_sim = i_sim; a.eps = eps;
+    a.x0 = x0; a.params = params; a.params_count = pc; a.srows = state_rows;
+    a.xk = xk; a.uk = uk; a.Uk = Uk; a.cost = cost; a.inner = inner; a.qpit = qpit; a.status = status;
+    return a;
+}
+
+// One time step of the fused loop without the plant: k_sim = 1, x the measured state, the caller's records in sv, u and U
+// in uk and Uk.
+ntm::LoopArgs step_args(int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
+                        const double *params, int pc, int state_rows, double *state, double *u, double *U, int *inner,
+                        int *qpit, int *status) {
+    ntm::LoopArgs a = loop_args(layout, profile, S, N, 1, i_sim, eps, x, params, pc, state_rows, nullptr, u, U, nullptr,
+                                inner, qpit, status);
+    a.sv = state; a.ctl = 1;
+    return a;
+}
+
+// The fused loop with the plant of ntm_plant_step on its own block and profile bits, d_k and v_k.
+ntm::LoopArgs perturbed_args(int layout, int profile, int S, int N, int k_sim, int i_sim, double eps, const double *x0,
+                             const double *params, int pc, int state_rows, const double *plant_params, int ppc,
+                             int plant_profile, const double *w, const double *v, double *xk, double *uk, double *Uk,
+                             double *cost, int *inner, int *qpit, int *status) {
+    ntm::LoopArgs a = loop_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, xk, uk, Uk, cost,
+                                inner, qpit, status);
+    a.pp = {plant_params, w, v, ppc, plant_profile};
+    a.pert = 1;
+    return a;
+}
+
+// Every rule of a fused call.  It also sets what the rules decide: the state box from xb (on the host), the profile the
+// controller runs (a step and the perturbed loop ignore the plant-only bits) and the plant's parameter count when
+// plant_params is NULL (the controller's block).  At S == 0 a loop checks nothing beyond handle, layout and S; a
+// controller step checks everything but its parameters and arrays.  params_count (and plant_params_count) is 1 or
+// S_total, the scenarios of the caller's arrays, of which `a` may be a shard.
+int check_fused(ntm_handle *h, ntm::LoopArgs &a, const double *xb, int S_total) {
+    TRY(check_common(h, a.layout, a.S));
+    if (a.S == 0 && !a.ctl) return NTM_OK;
+    if (a.ctl || a.pert) {
+        REQUIRE(!(a.flags & NTM_PROFILE_TAUE_W), "ntm_mpc_step: NTM_PROFILE_TAUE_W is not supported by the controller step");
+        a.flags &= ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4);
+    }
+    REQUIRE(a.N >= 1 && a.N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
+    REQUIRE(a.k_sim >= 0, "k_sim must be >= 0");
+    REQUIRE(a.i_sim >= 1, "i_sim must be >= 1");
+    REQUIRE(a.srows >= NTM_STATE_ROWS_OFF && a.srows <= NTM_STATE_ROWS_FROZEN, "unknown state_rows mode");
+    if (a.srows != NTM_STATE_ROWS_OFF) {
+        REQUIRE(xb, "NULL state bounds");
+        a.xmin1 = xb[0]; a.xmax1 = xb[1]; a.xmin2 = xb[2]; a.xmax2 = xb[3];
+        REQUIRE(a.xmin1 <= a.xmax1 && a.xmin2 <= a.xmax2, "state bounds: xmin > xmax (or NaN)");
+        // The rows of a non-literal Gamma are read from the per-warp dense Gamma tile of the tensor-core Hessian build;
+        // with the literal Gamma both N x N factors of the continuation + 4N rows of bookkeeping live in shared memory.
+        const bool dense = a.flags & (NTM_PROFILE_GAMMA_I | NTM_PROFILE_DENSE_G);
+        REQUIRE(!dense || a.N <= 32, "state rows inside the loop with NTM_PROFILE_GAMMA_I / DENSE_G: N <= 32");
+        REQUIRE((dense ? ntm::state_rows_dense_smem(a.N, a.srows) : ntm::state_rows_smem(a.N)) <= h->props.smem_optin,
+                "horizon too long for the state rows in shared memory");
+    }
+    if (a.S == 0) return NTM_OK;
+    TRY(check_params(a.params, a.params_count, S_total));
+    REQUIRE(a.rec_ld == 0 || a.xk, "rec is NULL");
+    REQUIRE(a.x0 && (a.ctl ? a.sv : a.xk) && (a.uk || a.k_sim == 0), "NULL array");
+    if (a.pert) {
+        if (!a.pp.pparams) a.pp.pparams_count = a.params_count;
+        REQUIRE(a.pp.pparams_count == 1 || a.pp.pparams_count == S_total, "plant_params_count must be 1 or S");
+        REQUIRE(!(a.pp.pflags & ~(NTM_PROFILE_RHO1_SQ | NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)),
+                "plant_profile: only RHO1_SQ, PLANT_C, PLANT_RK4 and TAUE_W act on the plant");
+    }
+    return NTM_OK;
+}
+
+// Launches a checked fused call on device arrays, with the handle's work-queue counter, LDL' scratch and, when the launch
+// runs in two phases, its saved loop state and longest-first queue.
+int launch_fused(ntm_handle *h, ntm::LoopArgs a) {
+    if (a.pert && !a.pp.pparams) a.pp.pparams = a.params;
     a.counter = h->counter;
-    TRY(ensure_hscratch(h, N));
+    TRY(grow(h, h->hscratch, h->hscratch_bytes, ntm::hscratch_bytes(h->props, a.N)));
     a.hscratch = h->hscratch;
     const size_t svd = ntm::lpt_doubles(h->props, a);      // two-phase launch with a longest-first queue (ntm_kernels.h)
     int *lpt = nullptr;
     if (svd != 0) {
-        TRY(ensure_lpt(h, svd, 2 * (size_t)S + NTM_LPT_BINS));
+        TRY(grow(h, h->sv, h->sv_bytes, svd * sizeof(double)));
+        TRY(grow(h, h->lpt, h->lpt_bytes, (2 * (size_t)a.S + NTM_LPT_BINS) * sizeof(int)));
         a.sv = h->sv; lpt = h->lpt;
     }
     CU(ntm::launch_closed_loop(h->stream, h->props, a, lpt, &h->launches));
     return NTM_OK;
 }
 
-// Host-pointer fused call for the scenarios [s_off, s_off + S) of caller arrays that hold S_total scenarios: copies every
-// array the caller passed to the arena, runs `launch` on the device copies, copies the outputs back and waits.  MATLAB
-// layout: a shard is a contiguous slice of every array.  SoA layout (scenario fastest): a shard is a column band, moved
-// with 2-D copies.  S_total == S, s_off == 0 is the plain single-device call.  A parameter count of 1 is one block for
-// every scenario.
+enum Dir { IN, OUT, INOUT };
+
+// The arrays a host-pointer fused call stages, the caller's in `a` beside their device copies in `d`:
+// f(caller's, copy, elements per scenario, direction, one block for every scenario).  The only place their sizes are
+// written.
 template <typename F>
-static int fused_host(ntm_handle *h, int layout, int S, int S_total, int s_off, int N, int k_sim, int pc, int ppc,
-                      const Fused &in, F launch) {
-    const size_t s = (size_t)S, n = (size_t)N, ks = (size_t)k_sim, st = (size_t)S_total, so = (size_t)s_off;
-    const size_t ld = (size_t)NTM_CTRL_DOUBLES(N);
-    double *x0, *prm, *pprm, *w, *v, *state, *xk, *uk, *Uk, *cost;
-    int *inner, *qpit, *status;
+void fused_arrays(const ntm::LoopArgs &a, ntm::LoopArgs &d, F f) {
+    const size_t n = (size_t)a.N, ks = (size_t)a.k_sim;
+    f(a.x0, d.x0, 2, IN, false);
+    f(a.params, d.params, NTM_NPARAM, IN, a.params_count == 1);
+    f(a.pp.pparams, d.pp.pparams, NTM_NPARAM, IN, a.pp.pparams_count == 1);
+    f(a.pp.dist, d.pp.dist, 2 * ks, IN, false);
+    f(a.pp.noise, d.pp.noise, 2 * ks, IN, false);
+    f(a.sv, d.sv, (size_t)NTM_CTRL_DOUBLES(a.N), INOUT, false);
+    f(a.xk, d.xk, 2 * (ks + 1), OUT, false);
+    f(a.uk, d.uk, ks, OUT, false);
+    f(a.Uk, d.Uk, n * ks, OUT, false);
+    f(a.cost, d.cost, 1, OUT, false);
+    f(a.inner, d.inner, ks, OUT, false);
+    f(a.qpit, d.qpit, ks, OUT, false);
+    f(a.status, d.status, 1, OUT, false);
+}
+
+// Host-pointer fused call for the scenarios [s_off, s_off + a.S) of caller arrays that hold S_total scenarios, `a`
+// checked: copies every array the caller passed to the arena, launches on the copies, copies the outputs back and waits.
+// MATLAB layout: a shard is a contiguous slice of every array.  SoA layout (scenario fastest): a shard is a column band,
+// moved with 2-D copies.  A parameter count of 1 is one block for every scenario.
+int fused_host(ntm_handle *h, const ntm::LoopArgs &a, int S_total, int s_off) {
+    const size_t s = (size_t)a.S, st = (size_t)S_total, so = (size_t)s_off;
+    ntm::LoopArgs d = a;
     TRY(Arena(h).reserve([&](Arena &A) {
-        x0 = A.take<double>(2 * s);
-        prm = A.take<double>((pc == 1 ? 1 : s) * NTM_NPARAM);
-        pprm = in.pparams ? A.take<double>((ppc == 1 ? 1 : s) * NTM_NPARAM) : nullptr;
-        w = in.w ? A.take<double>(2 * ks * s) : nullptr;
-        v = in.v ? A.take<double>(2 * ks * s) : nullptr;
-        state = in.state ? A.take<double>(ld * s) : nullptr;
-        xk = in.xk ? A.take<double>(2 * (ks + 1) * s) : nullptr;
-        uk = in.uk ? A.take<double>(ks * s) : nullptr;
-        Uk = in.Uk ? A.take<double>(n * ks * s) : nullptr;
-        cost = in.cost ? A.take<double>(s) : nullptr;
-        inner = in.inner ? A.take<int>(ks * s) : nullptr;
-        qpit = in.qpit ? A.take<int>(ks * s) : nullptr;
-        status = in.status ? A.take<int>(s) : nullptr;
+        fused_arrays(a, d, [&](auto src, auto &dst, size_t E, Dir, bool shared) {
+            if (src) dst = A.take<std::remove_pointer_t<decltype(src)>>(shared ? E : E * s);
+        });
     }));
-    auto blocks = [&](double *dst, const double *src, int count) {
-        return count == 1 ? h2d(h, dst, src, (size_t)NTM_NPARAM) : h2d_shard(h, layout, dst, src, NTM_NPARAM, s, st, so);
-    };
-    TRY(h2d_shard(h, layout, x0, in.x0, 2, s, st, so));
-    TRY(blocks(prm, in.params, pc));
-    if (pprm) TRY(blocks(pprm, in.pparams, ppc));
-    if (w) TRY(h2d_shard(h, layout, w, in.w, 2 * ks, s, st, so));
-    if (v) TRY(h2d_shard(h, layout, v, in.v, 2 * ks, s, st, so));
-    if (state) TRY(h2d_shard(h, layout, state, in.state, ld, s, st, so));
-    TRY(launch(Fused{x0, prm, pprm, w, v, state, xk, uk, Uk, cost, inner, qpit, status}));
-    TRY(d2h_shard(h, layout, in.state, state, ld, s, st, so));
-    TRY(d2h_shard(h, layout, in.xk, xk, 2 * (ks + 1), s, st, so)); TRY(d2h_shard(h, layout, in.uk, uk, ks, s, st, so));
-    TRY(d2h_shard(h, layout, in.Uk, Uk, n * ks, s, st, so)); TRY(d2h_shard(h, layout, in.cost, cost, 1, s, st, so));
-    TRY(d2h_shard(h, layout, in.inner, inner, ks, s, st, so)); TRY(d2h_shard(h, layout, in.qpit, qpit, ks, s, st, so));
-    TRY(d2h_shard(h, layout, in.status, status, 1, s, st, so));
+    int rc = NTM_OK;
+    fused_arrays(a, d, [&](auto src, auto dst, size_t E, Dir dir, bool shared) {
+        using T = std::remove_const_t<std::remove_pointer_t<decltype(src)>>;
+        T *to = const_cast<T *>(dst);                      // the arena copy of an input
+        if (rc == NTM_OK && src && dir != OUT)
+            rc = shared ? h2d(h, to, src, E) : h2d_shard(h, a.layout, to, src, E, s, st, so);
+    });
+    TRY(rc);
+    if (d.params_count == S_total) d.params_count = a.S;   // the blocks of this shard
+    if (d.pp.pparams_count == S_total) d.pp.pparams_count = a.S;
+    TRY(launch_fused(h, d));
+    fused_arrays(a, d, [&](auto src, auto dst, size_t E, Dir dir, bool) {
+        if constexpr (!std::is_const_v<std::remove_pointer_t<decltype(src)>>)   // inputs are const
+            if (rc == NTM_OK && dir != IN) rc = d2h_shard(h, a.layout, src, dst, E, s, st, so);
+    });
+    TRY(rc);
     CU(cudaStreamSynchronize(h->stream));
+    return NTM_OK;
+}
+
+int fused_dev_call(ntm_handle *h, ntm::LoopArgs a, const double *xb) {
+    TRY(check_fused(h, a, xb, a.S));
+    return a.S == 0 ? NTM_OK : launch_fused(h, a);
+}
+
+int fused_host_call(ntm_handle *h, ntm::LoopArgs a, const double *xb) {
+    TRY(check_fused(h, a, xb, a.S));
+    return a.S == 0 ? NTM_OK : fused_host(h, a, a.S, 0);
+}
+
+// ---- per-call operations: one check each, called by its host and its device entry ------------------------------------
+
+int check_rho(ntm_handle *h, int layout, int S, const double *x, const double *params, int pc, const double *rho1,
+              const double *rho2, const double *rho3) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    REQUIRE(x && rho1 && rho2 && rho3, "NULL array");
+    return NTM_OK;
+}
+
+int check_lpv(ntm_handle *h, int layout, int S, const double *rho1, const double *rho2, const double *rho3,
+              const double *params, int pc, const double *A, const double *B) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    REQUIRE(rho1 && rho2 && rho3 && A && B, "NULL array");
+    return NTM_OK;
+}
+
+int check_condense(ntm_handle *h, int layout, int S, int N, const double *R1, const double *R2, const double *R3,
+                   const double *params, int pc, const double *Phi, const double *Gamma, const double *Lambda) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
+    REQUIRE(R1 && R2 && R3 && Phi && Gamma && Lambda, "NULL array");
+    return NTM_OK;
+}
+
+int check_hessian_grad(ntm_handle *h, int layout, int S, int N, const double *Phi, const double *Gamma,
+                       const double *Lambda, const double *x, const double *params, int pc, const double *G,
+                       const double *F) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
+    REQUIRE(Phi && Gamma && Lambda && x && G && F, "NULL array");
+    return NTM_OK;
+}
+
+int check_qp_box(ntm_handle *h, int layout, int S, int N, const double *G, const double *F, const double *lb,
+                 const double *ub, int bc, const double *U) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
+    REQUIRE(G && F && lb && ub && U, "NULL array");
+    REQUIRE(bc == 1 || bc == S, "bounds_count must be 1 or S");
+    return NTM_OK;
+}
+
+// M == 0 passes here and is ntm_qp_box's to check
+int check_qp_ineq(ntm_handle *h, int layout, int S, int N, int M, const double *G, const double *F, const double *lb,
+                  const double *ub, int bc, const double *Lg, const double *bg, const double *U) {
+    TRY(check_common(h, layout, S));
+    REQUIRE(M >= 0, "M must be >= 0");
+    if (M == 0 || S == 0) return NTM_OK;
+    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
+    REQUIRE(G && F && lb && ub && U && Lg && bg, "NULL array");
+    REQUIRE(bc == 1 || bc == S, "bounds_count must be 1 or S");
+    REQUIRE((long long)M * N <= 0x7fffffffLL, "M*N overflows int");
+    REQUIRE(ntm::qp_ineq_groups(h->props, N, M) > 0, "ntm_qp_ineq: N, M too large for the shared-memory factor pair");
+    return NTM_OK;
+}
+
+int check_plant(ntm_handle *h, int layout, int S, const double *x, const double *u, const double *params, int pc,
+                const double *xn) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    REQUIRE(x && u && xn, "NULL array");
+    return NTM_OK;
+}
+
+int check_getwlc(ntm_handle *h, int layout, int S, int N, const double *bounds, const double *Gamma, const double *Phi,
+                 const double *Lambda, const double *W, const double *L, const double *c) {
+    TRY(check_common(h, layout, S));
+    if (S == 0) return NTM_OK;
+    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
+    REQUIRE(bounds && Gamma && Phi && Lambda && W && L && c, "NULL array");
+    return NTM_OK;
+}
+
+// S == 0 passes here and still reduces (to empty statistics)
+int check_mc_stats(ntm_handle *h, int layout, int S, int k_sim, const double *xk, const double *uk, const double *params,
+                   int pc, const double *bounds, const double *out) {
+    TRY(check_common(h, layout, S));
+    REQUIRE(k_sim >= 1, "k_sim must be >= 1");
+    REQUIRE(bounds && out, "NULL array");
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    REQUIRE(xk && uk, "NULL array");
+    return NTM_OK;
+}
+
+// launch_mc_stats with umin / umax read where they live (slots 8 and 9 of the parameter block) in the caller's layout
+int mc_stats_launch(ntm_handle *h, int layout, int S, int k_sim, const double *xk, const double *uk, const double *cost,
+                    const int *status, const double *params, int pc, const double *bounds, double w_sup, double hist_max,
+                    double *out) {
+    const double *umin = nullptr, *umax = nullptr;
+    int ustride = 0;
+    if (S > 0) {
+        if (pc == 1) { umin = params + 8; umax = params + 9; ustride = 0; }
+        else if (layout == NTM_LAYOUT_MATLAB) { umin = params + 8; umax = params + 9; ustride = NTM_NPARAM; }
+        else { umin = params + 8 * (size_t)S; umax = params + 9 * (size_t)S; ustride = 1; }
+    }
+    CU(ntm::launch_mc_stats(h->stream, h->props, layout, S, k_sim, xk, uk, cost, status, umin, umax, ustride, bounds, w_sup,
+                            hist_max, out, &h->launches));
+    return NTM_OK;
+}
+
+// Times `launch` (after a warm-up of an eighth of its iterations) with events on the handle's stream; `flops` per
+// iteration and SM.
+int time_peak(ntm_handle *h, int iters, cudaError_t (*launch)(cudaStream_t, const ntm::DeviceProps &, int, double *, long long *),
+              double flops, double *tflops, double *ms_out) {
+    REQUIRE(h != nullptr, "handle is NULL");
+    REQUIRE(iters > 0, "iters must be > 0");
+    CU(cudaSetDevice(h->device));
+    cudaEvent_t e0, e1;
+    CU(cudaEventCreate(&e0));
+    CU(cudaEventCreate(&e1));
+    double *out = reinterpret_cast<double *>(h->counter) + 8;
+    CU(launch(h->stream, h->props, iters / 8 + 1, out, &h->launches));   // warm-up
+    CU(cudaEventRecord(e0, h->stream));
+    CU(launch(h->stream, h->props, iters, out, &h->launches));
+    CU(cudaEventRecord(e1, h->stream));
+    CU(cudaEventSynchronize(e1));
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, e0, e1));
+    cudaEventDestroy(e0);
+    cudaEventDestroy(e1);
+    if (tflops) *tflops = flops * (double)iters * (double)h->props.sm_count / (ms * 1e-3) / 1e12;
+    if (ms_out) *ms_out = ms;
     return NTM_OK;
 }
 
@@ -353,20 +555,16 @@ long long ntm_launch_count(ntm_handle *h) { return h ? h->launches : -1; }
 // ------------------------------------------------------------------------------------------------ rho
 int ntm_rho_dev(ntm_handle *h, int layout, int profile, int S, const double *x, const double *params, int pc,
                 double *rho1, double *rho2, double *rho3) {
-    TRY(check_common(h, layout, S));
+    TRY(check_rho(h, layout, S, x, params, pc, rho1, rho2, rho3));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(x && rho1 && rho2 && rho3, "NULL array");
     CU(ntm::launch_rho(h->stream, layout, profile, S, x, params, pc, rho1, rho2, rho3, &h->launches));
     return NTM_OK;
 }
 
 int ntm_rho(ntm_handle *h, int layout, int profile, int S, const double *x, const double *params, int pc,
             double *rho1, double *rho2, double *rho3) {
-    TRY(check_common(h, layout, S));
+    TRY(check_rho(h, layout, S, x, params, pc, rho1, rho2, rho3));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(x && rho1 && rho2 && rho3, "NULL array");
     const size_t s = (size_t)S;
     double *dx, *dp, *d1, *d2, *d3;
     TRY(Arena(h).reserve([&](Arena &A) {
@@ -374,7 +572,7 @@ int ntm_rho(ntm_handle *h, int layout, int profile, int S, const double *x, cons
         d1 = A.take<double>(s); d2 = A.take<double>(s); d3 = A.take<double>(s);
     }));
     TRY(h2d(h, dx, x, 2 * s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
-    TRY(ntm_rho_dev(h, layout, profile, S, dx, dp, pc, d1, d2, d3));
+    CU(ntm::launch_rho(h->stream, layout, profile, S, dx, dp, pc, d1, d2, d3, &h->launches));
     TRY(d2h(h, rho1, d1, s)); TRY(d2h(h, rho2, d2, s)); TRY(d2h(h, rho3, d3, s));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
@@ -383,20 +581,16 @@ int ntm_rho(ntm_handle *h, int layout, int profile, int S, const double *x, cons
 // ------------------------------------------------------------------------------------------------ A, B
 int ntm_lpv_AB_dev(ntm_handle *h, int layout, int S, const double *rho1, const double *rho2, const double *rho3,
                    const double *params, int pc, double *Aout, double *Bout) {
-    TRY(check_common(h, layout, S));
+    TRY(check_lpv(h, layout, S, rho1, rho2, rho3, params, pc, Aout, Bout));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(rho1 && rho2 && rho3 && Aout && Bout, "NULL array");
     CU(ntm::launch_lpv(h->stream, layout, S, rho1, rho2, rho3, params, pc, Aout, Bout, &h->launches));
     return NTM_OK;
 }
 
 int ntm_lpv_AB(ntm_handle *h, int layout, int S, const double *rho1, const double *rho2, const double *rho3,
                const double *params, int pc, double *Aout, double *Bout) {
-    TRY(check_common(h, layout, S));
+    TRY(check_lpv(h, layout, S, rho1, rho2, rho3, params, pc, Aout, Bout));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(rho1 && rho2 && rho3 && Aout && Bout, "NULL array");
     const size_t s = (size_t)S;
     double *d1, *d2, *d3, *dp, *dA, *dB;
     TRY(Arena(h).reserve([&](Arena &A) {
@@ -405,7 +599,7 @@ int ntm_lpv_AB(ntm_handle *h, int layout, int S, const double *rho1, const doubl
     }));
     TRY(h2d(h, d1, rho1, s)); TRY(h2d(h, d2, rho2, s)); TRY(h2d(h, d3, rho3, s));
     TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
-    TRY(ntm_lpv_AB_dev(h, layout, S, d1, d2, d3, dp, pc, dA, dB));
+    CU(ntm::launch_lpv(h->stream, layout, S, d1, d2, d3, dp, pc, dA, dB, &h->launches));
     TRY(d2h(h, Aout, dA, 4 * s)); TRY(d2h(h, Bout, dB, 2 * s));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
@@ -414,11 +608,8 @@ int ntm_lpv_AB(ntm_handle *h, int layout, int S, const double *rho1, const doubl
 // ------------------------------------------------------------------------------------------------ condense
 int ntm_condense_dev(ntm_handle *h, int layout, int profile, int S, int N, const double *R1, const double *R2,
                      const double *R3, const double *params, int pc, double *Phi, double *Gamma, double *Lambda) {
-    TRY(check_common(h, layout, S));
+    TRY(check_condense(h, layout, S, N, R1, R2, R3, params, pc, Phi, Gamma, Lambda));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(R1 && R2 && R3 && Phi && Gamma && Lambda, "NULL array");
     CU(ntm::launch_condense(h->stream, h->props, layout, profile, S, N, R1, R2, R3, params, pc, Phi, Gamma, Lambda,
                             &h->launches));
     return NTM_OK;
@@ -426,11 +617,8 @@ int ntm_condense_dev(ntm_handle *h, int layout, int profile, int S, int N, const
 
 int ntm_condense(ntm_handle *h, int layout, int profile, int S, int N, const double *R1, const double *R2,
                  const double *R3, const double *params, int pc, double *Phi, double *Gamma, double *Lambda) {
-    TRY(check_common(h, layout, S));
+    TRY(check_condense(h, layout, S, N, R1, R2, R3, params, pc, Phi, Gamma, Lambda));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(R1 && R2 && R3 && Phi && Gamma && Lambda, "NULL array");
     const size_t s = (size_t)S, n = (size_t)N;
     double *d1, *d2, *d3, *dp, *dPhi, *dGam, *dLam;
     TRY(Arena(h).reserve([&](Arena &A) {
@@ -440,7 +628,8 @@ int ntm_condense(ntm_handle *h, int layout, int profile, int S, int N, const dou
     }));
     TRY(h2d(h, d1, R1, n * s)); TRY(h2d(h, d2, R2, n * s)); TRY(h2d(h, d3, R3, n * s));
     TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
-    TRY(ntm_condense_dev(h, layout, profile, S, N, d1, d2, d3, dp, pc, dPhi, dGam, dLam));
+    CU(ntm::launch_condense(h->stream, h->props, layout, profile, S, N, d1, d2, d3, dp, pc, dPhi, dGam, dLam,
+                            &h->launches));
     TRY(d2h(h, Phi, dPhi, 4 * n * s)); TRY(d2h(h, Gamma, dGam, 2 * n * n * s)); TRY(d2h(h, Lambda, dLam, 2 * n * s));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
@@ -449,11 +638,8 @@ int ntm_condense(ntm_handle *h, int layout, int profile, int S, int N, const dou
 // ------------------------------------------------------------------------------------------------ G, F
 int ntm_hessian_grad_dev(ntm_handle *h, int layout, int S, int N, const double *Phi, const double *Gamma,
                          const double *Lambda, const double *x, const double *params, int pc, double *G, double *F) {
-    TRY(check_common(h, layout, S));
+    TRY(check_hessian_grad(h, layout, S, N, Phi, Gamma, Lambda, x, params, pc, G, F));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(Phi && Gamma && Lambda && x && G && F, "NULL array");
     CU(ntm::launch_hessian_grad(h->stream, h->props, layout, S, N, Phi, Gamma, Lambda, x, params, pc, G, F,
                                 &h->launches));
     return NTM_OK;
@@ -461,11 +647,8 @@ int ntm_hessian_grad_dev(ntm_handle *h, int layout, int S, int N, const double *
 
 int ntm_hessian_grad(ntm_handle *h, int layout, int S, int N, const double *Phi, const double *Gamma,
                      const double *Lambda, const double *x, const double *params, int pc, double *G, double *F) {
-    TRY(check_common(h, layout, S));
+    TRY(check_hessian_grad(h, layout, S, N, Phi, Gamma, Lambda, x, params, pc, G, F));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(Phi && Gamma && Lambda && x && G && F, "NULL array");
     const size_t s = (size_t)S, n = (size_t)N;
     double *dPhi, *dGam, *dLam, *dx, *dp, *dG, *dF;
     TRY(Arena(h).reserve([&](Arena &A) {
@@ -475,7 +658,7 @@ int ntm_hessian_grad(ntm_handle *h, int layout, int S, int N, const double *Phi,
     }));
     TRY(h2d(h, dPhi, Phi, 4 * n * s)); TRY(h2d(h, dGam, Gamma, 2 * n * n * s)); TRY(h2d(h, dLam, Lambda, 2 * n * s));
     TRY(h2d(h, dx, x, 2 * s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
-    TRY(ntm_hessian_grad_dev(h, layout, S, N, dPhi, dGam, dLam, dx, dp, pc, dG, dF));
+    CU(ntm::launch_hessian_grad(h->stream, h->props, layout, S, N, dPhi, dGam, dLam, dx, dp, pc, dG, dF, &h->launches));
     TRY(d2h(h, G, dG, n * n * s)); TRY(d2h(h, F, dF, n * s));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
@@ -484,12 +667,9 @@ int ntm_hessian_grad(ntm_handle *h, int layout, int S, int N, const double *Phi,
 // ------------------------------------------------------------------------------------------------ box QP
 int ntm_qp_box_dev(ntm_handle *h, int layout, int S, int N, const double *G, const double *F, const double *lb,
                    const double *ub, int bc, double *U, int *iters, int *status) {
-    TRY(check_common(h, layout, S));
+    TRY(check_qp_box(h, layout, S, N, G, F, lb, ub, bc, U));
     if (S == 0) return NTM_OK;
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(G && F && lb && ub && U, "NULL array");
-    REQUIRE(bc == 1 || bc == S, "bounds_count must be 1 or S");
-    TRY(ensure_hscratch(h, N));
+    TRY(grow(h, h->hscratch, h->hscratch_bytes, ntm::hscratch_bytes(h->props, N)));
     CU(ntm::launch_qp_box(h->stream, h->props, layout, S, N, G, F, lb, ub, bc, U, iters, status, h->counter,
                           h->hscratch, &h->launches));
     return NTM_OK;
@@ -497,11 +677,8 @@ int ntm_qp_box_dev(ntm_handle *h, int layout, int S, int N, const double *G, con
 
 int ntm_qp_box(ntm_handle *h, int layout, int S, int N, const double *G, const double *F, const double *lb,
                const double *ub, int bc, double *U, int *iters, int *status) {
-    TRY(check_common(h, layout, S));
+    TRY(check_qp_box(h, layout, S, N, G, F, lb, ub, bc, U));
     if (S == 0) return NTM_OK;
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(G && F && lb && ub && U, "NULL array");
-    REQUIRE(bc == 1 || bc == S, "bounds_count must be 1 or S");
     const size_t s = (size_t)S, n = (size_t)N, b = (size_t)bc;
     double *dG, *dF, *dlb, *dub, *dU;
     int *dit, *dst;
@@ -511,7 +688,9 @@ int ntm_qp_box(ntm_handle *h, int layout, int S, int N, const double *G, const d
         dit = A.take<int>(s); dst = A.take<int>(s);
     }));
     TRY(h2d(h, dG, G, n * n * s)); TRY(h2d(h, dF, F, n * s)); TRY(h2d(h, dlb, lb, n * b)); TRY(h2d(h, dub, ub, n * b));
-    TRY(ntm_qp_box_dev(h, layout, S, N, dG, dF, dlb, dub, bc, dU, dit, dst));
+    TRY(grow(h, h->hscratch, h->hscratch_bytes, ntm::hscratch_bytes(h->props, N)));
+    CU(ntm::launch_qp_box(h->stream, h->props, layout, S, N, dG, dF, dlb, dub, bc, dU, dit, dst, h->counter,
+                          h->hscratch, &h->launches));
     TRY(d2h(h, U, dU, n * s)); TRY(d2h(h, iters, dit, s)); TRY(d2h(h, status, dst, s));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
@@ -521,30 +700,19 @@ int ntm_qp_box(ntm_handle *h, int layout, int S, int N, const double *G, const d
 int ntm_qp_ineq_dev(ntm_handle *h, int layout, int S, int N, int M, const double *G, const double *F,
                     const double *lb, const double *ub, int bc, const double *Lg, const double *bg, double *U,
                     int *iters, int *status) {
-    TRY(check_common(h, layout, S));
-    REQUIRE(M >= 0, "M must be >= 0");
+    TRY(check_qp_ineq(h, layout, S, N, M, G, F, lb, ub, bc, Lg, bg, U));
     if (M == 0) return ntm_qp_box_dev(h, layout, S, N, G, F, lb, ub, bc, U, iters, status);
     if (S == 0) return NTM_OK;
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(G && F && lb && ub && U && Lg && bg, "NULL array");
-    REQUIRE(bc == 1 || bc == S, "bounds_count must be 1 or S");
-    REQUIRE((long long)M * N <= 0x7fffffffLL, "M*N overflows int");
-    const cudaError_t e = ntm::launch_qp_ineq(h->stream, h->props, layout, S, N, M, G, F, lb, ub, bc, Lg, bg, U, iters,
-                                              status, h->counter, &h->launches);
-    REQUIRE(e != cudaErrorInvalidConfiguration, "ntm_qp_ineq: N, M too large for the shared-memory factor pair");
-    CU(e);
+    CU(ntm::launch_qp_ineq(h->stream, h->props, layout, S, N, M, G, F, lb, ub, bc, Lg, bg, U, iters, status, h->counter,
+                           &h->launches));
     return NTM_OK;
 }
 
 int ntm_qp_ineq(ntm_handle *h, int layout, int S, int N, int M, const double *G, const double *F, const double *lb,
                 const double *ub, int bc, const double *Lg, const double *bg, double *U, int *iters, int *status) {
-    TRY(check_common(h, layout, S));
-    REQUIRE(M >= 0, "M must be >= 0");
+    TRY(check_qp_ineq(h, layout, S, N, M, G, F, lb, ub, bc, Lg, bg, U));
     if (M == 0) return ntm_qp_box(h, layout, S, N, G, F, lb, ub, bc, U, iters, status);
     if (S == 0) return NTM_OK;
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(G && F && lb && ub && U && Lg && bg, "NULL array");
-    REQUIRE(bc == 1 || bc == S, "bounds_count must be 1 or S");
     const size_t s = (size_t)S, n = (size_t)N, b = (size_t)bc, m = (size_t)M;
     double *dG, *dF, *dlb, *dub, *dU, *dL, *dbg;
     int *dit, *dst;
@@ -556,7 +724,8 @@ int ntm_qp_ineq(ntm_handle *h, int layout, int S, int N, int M, const double *G,
     }));
     TRY(h2d(h, dG, G, n * n * s)); TRY(h2d(h, dF, F, n * s)); TRY(h2d(h, dlb, lb, n * b)); TRY(h2d(h, dub, ub, n * b));
     TRY(h2d(h, dL, Lg, m * n * s)); TRY(h2d(h, dbg, bg, m * s));
-    TRY(ntm_qp_ineq_dev(h, layout, S, N, M, dG, dF, dlb, dub, bc, dL, dbg, dU, dit, dst));
+    CU(ntm::launch_qp_ineq(h->stream, h->props, layout, S, N, M, dG, dF, dlb, dub, bc, dL, dbg, dU, dit, dst, h->counter,
+                           &h->launches));
     TRY(d2h(h, U, dU, n * s)); TRY(d2h(h, iters, dit, s)); TRY(d2h(h, status, dst, s));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
@@ -565,20 +734,16 @@ int ntm_qp_ineq(ntm_handle *h, int layout, int S, int N, int M, const double *G,
 // ------------------------------------------------------------------------------------------------ plant
 int ntm_plant_step_dev(ntm_handle *h, int layout, int profile, int S, const double *x, const double *u,
                        const double *params, int pc, double *xn) {
-    TRY(check_common(h, layout, S));
+    TRY(check_plant(h, layout, S, x, u, params, pc, xn));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(x && u && xn, "NULL array");
     CU(ntm::launch_plant(h->stream, layout, profile, S, x, u, params, pc, xn, &h->launches));
     return NTM_OK;
 }
 
 int ntm_plant_step(ntm_handle *h, int layout, int profile, int S, const double *x, const double *u,
                    const double *params, int pc, double *xn) {
-    TRY(check_common(h, layout, S));
+    TRY(check_plant(h, layout, S, x, u, params, pc, xn));
     if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(x && u && xn, "NULL array");
     const size_t s = (size_t)S;
     double *dx, *du, *dp, *dn;
     TRY(Arena(h).reserve([&](Arena &A) {
@@ -586,75 +751,13 @@ int ntm_plant_step(ntm_handle *h, int layout, int profile, int S, const double *
         dn = A.take<double>(2 * s);
     }));
     TRY(h2d(h, dx, x, 2 * s)); TRY(h2d(h, du, u, s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
-    TRY(ntm_plant_step_dev(h, layout, profile, S, dx, du, dp, pc, dn));
+    CU(ntm::launch_plant(h->stream, layout, profile, S, dx, du, dp, pc, dn, &h->launches));
     TRY(d2h(h, xn, dn, 2 * s));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
 }
 
 // ------------------------------------------------------------------------------------------------ closed loop
-static int check_loop(int N, int k_sim, int i_sim, const double *x0, double *xk, double *uk) {
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(k_sim >= 0, "k_sim must be >= 0");
-    REQUIRE(i_sim >= 1, "i_sim must be >= 1");
-    REQUIRE(x0 && xk && (uk || k_sim == 0), "NULL array");
-    return NTM_OK;
-}
-
-// state_rows / xbounds of ntm_mpc_closed_loop_sc and ntm_mpc_step_sc (N already checked) into a.srows and a.xmin1..xmax2
-static int set_state_rows(const ntm_handle *h, int profile, int N, int state_rows, const double *xb, ntm::LoopArgs &a) {
-    REQUIRE(state_rows >= NTM_STATE_ROWS_OFF && state_rows <= NTM_STATE_ROWS_FROZEN, "unknown state_rows mode");
-    a.srows = state_rows;
-    if (state_rows != NTM_STATE_ROWS_OFF) {
-        REQUIRE(xb, "NULL state bounds");
-        a.xmin1 = xb[0]; a.xmax1 = xb[1]; a.xmin2 = xb[2]; a.xmax2 = xb[3];
-        REQUIRE(a.xmin1 <= a.xmax1 && a.xmin2 <= a.xmax2, "state bounds: xmin > xmax (or NaN)");
-        if (profile & (NTM_PROFILE_GAMMA_I | NTM_PROFILE_DENSE_G)) {
-            // rows of a non-literal Gamma are read from the per-warp dense Gamma tile of the tensor-core Hessian build
-            REQUIRE(N <= 32, "state rows inside the loop with NTM_PROFILE_GAMMA_I / DENSE_G: N <= 32");
-            REQUIRE(ntm::state_rows_dense_smem(N, state_rows) <= h->props.smem_optin,
-                    "horizon too long for the state rows in shared memory");
-        } else {
-            // both N x N factors of the continuation + 4N rows of bookkeeping live in shared memory
-            const size_t need = (ntm::state_rows_smem(N));
-            REQUIRE(need <= h->props.smem_optin, "horizon too long for the state rows in shared memory");
-        }
-    }
-    return NTM_OK;
-}
-
-static int closed_loop_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
-                                int pc, int state_rows, const double *xb, const Fused &d, int rec_ld = 0,
-                                double *rec_status = nullptr) {
-    TRY(check_common(h, layout, S));
-    if (S == 0) return NTM_OK;
-    TRY(check_params(d.params, pc, S));
-    TRY(check_loop(N, k_sim, i_sim, d.x0, d.xk, d.uk));
-    ntm::LoopArgs a = {};
-    a.rec_ld = rec_ld; a.rec_status = rec_status;
-    TRY(set_state_rows(h, profile, N, state_rows, xb, a));
-    return launch_fused(h, a, layout, profile, S, N, k_sim, i_sim, eps, pc, d);
-}
-
-// Host-pointer closed loop for the scenarios [s_off, s_off + S) of a caller array that holds S_total scenarios (see
-// fused_host).
-static int closed_loop_host_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
-                                 const double *x0, const double *params, int pc, int state_rows, const double *xb,
-                                 double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
-                                 int *status, int S_total = -1, int s_off = 0) {
-    TRY(check_common(h, layout, S));
-    if (S == 0) return NTM_OK;
-    if (S_total < 0) S_total = S;
-    REQUIRE(params != nullptr, "params is NULL");
-    REQUIRE(pc == 1 || pc == S_total, "params_count must be 1 or S");   // 1 (shared block) or S_total
-    TRY(check_loop(N, k_sim, i_sim, x0, xk, uk));
-    const int pcl = (pc == 1) ? 1 : S;                   // parameter blocks this shard holds
-    return fused_host(h, layout, S, S_total, s_off, N, k_sim, pc, pc,
-                      {x0, params, nullptr, nullptr, nullptr, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status},
-                      [&](const Fused &d) { return closed_loop_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pcl,
-                                                                        state_rows, xb, d); });
-}
-
 // ---- one host process, every visible GPU (the MEX gateway ntm_mpc_batch is single-process by construction) ----------
 // Scenarios never interact (NTM_MPC_Sim.m:93-131 has no cross-scenario term), so the batch is cut into contiguous
 // shards of ceil(S / G) scenarios, one per device; each device runs on its own pooled handle and host thread and moves
@@ -705,25 +808,31 @@ int ntm_mpc_closed_loop_multi(int n_devices, const int *devices, int layout, int
         for (int q = 0; q < g; ++q) REQUIRE(dev[q] != dev[g], "device listed twice");
     }
     if (S == 0) return NTM_OK;
-    REQUIRE(params != nullptr, "params is NULL");
-    REQUIRE(pc == 1 || pc == S, "params_count must be 1 or S");
-    TRY(check_loop(N, k_sim, i_sim, x0, xk, uk));
     const int per = (S + n_devices - 1) / n_devices;       // SURVEY 8(e): rank g owns [g*per, min(S, (g+1)*per))
-    std::vector<ntm_handle *> hs((size_t)n_devices, nullptr);
-    for (int g = 0; g < n_devices; ++g) if (g * per < S) TRY(pool_handle(dev[g], &hs[g]));
-    std::vector<int> rc((size_t)n_devices, NTM_OK);
-    std::vector<std::string> msg((size_t)n_devices);
-    auto shard = [&](int g) {
-        const int s0 = g * per, sl = (S - s0 < per) ? S - s0 : per;
-        rc[g] = closed_loop_host_impl(hs[g], layout, profile, sl, N, k_sim, i_sim, eps, x0, params, pc, state_rows, xbounds,
-                                      xk, uk, Uk, cost, inner_iters, qp_iters, status, S, s0);
+    const int shards = (S + per - 1) / per;
+    std::vector<ntm_handle *> hs((size_t)shards, nullptr);
+    std::vector<ntm::LoopArgs> as((size_t)shards);
+    for (int g = 0; g < shards; ++g) {                     // every shard is checked before any is copied
+        TRY(pool_handle(dev[g], &hs[g]));
+        as[g] = loop_args(layout, profile, std::min(per, S - g * per), N, k_sim, i_sim, eps, x0, params, pc, state_rows,
+                          xk, uk, Uk, cost, inner_iters, qp_iters, status);
+        TRY(check_fused(hs[g], as[g], xbounds, S));
+    }
+    std::vector<int> rc((size_t)shards, NTM_OK);
+    std::vector<std::string> msg((size_t)shards);
+    auto shard = [&](int g) -> int {
+        CU(cudaSetDevice(hs[g]->device));                  // the current device is per host thread
+        return fused_host(hs[g], as[g], S, g * per);
+    };
+    auto run = [&](int g) {
+        rc[g] = shard(g);
         if (rc[g] != NTM_OK) msg[g] = g_err;               // g_err is thread-local: carry the text to the caller's thread
     };
     std::vector<std::thread> th;
-    for (int g = 1; g < n_devices; ++g) if (hs[g]) th.emplace_back(shard, g);
-    shard(0);
+    for (int g = 1; g < shards; ++g) th.emplace_back(run, g);
+    run(0);
     for (auto &t : th) t.join();
-    for (int g = 0; g < n_devices; ++g)
+    for (int g = 0; g < shards; ++g)
         if (rc[g] != NTM_OK) return fail(rc[g], "device %d: %s", dev[g], msg[g].c_str());
     return NTM_OK;
 }
@@ -734,169 +843,81 @@ int ntm_mpc_closed_loop_multi(int n_devices, const int *devices, int layout, int
 int ntm_mpc_closed_loop_rec_dev(ntm_handle *h, int profile, int S, int N, int k_sim, int i_sim, double eps,
                                 const double *x0, const double *params, int pc, int state_rows, const double *xbounds,
                                 double *rec, int *inner_iters, int *qp_iters) {
-    TRY(check_common(h, NTM_LAYOUT_MATLAB, S));
-    if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(rec != nullptr, "rec is NULL");
-    TRY(check_loop(N, k_sim, i_sim, x0, rec, rec));
-    const int ld = NTM_REC_DOUBLES(k_sim);
-    return closed_loop_dev_impl(h, NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, pc, state_rows, xbounds,
-                                {x0, params, nullptr, nullptr, nullptr, nullptr, rec, rec + 2 * (k_sim + 1), nullptr,
-                                 rec + 3 * k_sim + 2, inner_iters, qp_iters, nullptr},
-                                ld, rec + 3 * k_sim + 3);
+    ntm::LoopArgs a = loop_args(NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, rec,
+                                nullptr, nullptr, nullptr, inner_iters, qp_iters, nullptr);
+    a.rec_ld = NTM_REC_DOUBLES(k_sim);
+    if (rec) { a.uk = rec + 2 * (k_sim + 1); a.cost = rec + 3 * k_sim + 2; a.rec_status = rec + 3 * k_sim + 3; }
+    return fused_dev_call(h, a, xbounds);
 }
 
 int ntm_mpc_closed_loop_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
                             const double *x0, const double *params, int pc, double *xk, double *uk, double *Uk,
                             double *cost, int *inner_iters, int *qp_iters, int *status) {
-    return closed_loop_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, NTM_STATE_ROWS_OFF, nullptr,
-                                {x0, params, nullptr, nullptr, nullptr, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
+    return fused_dev_call(h, loop_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, NTM_STATE_ROWS_OFF, xk,
+                                       uk, Uk, cost, inner_iters, qp_iters, status), nullptr);
 }
 
 int ntm_mpc_closed_loop(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
                         const double *x0, const double *params, int pc, double *xk, double *uk, double *Uk,
                         double *cost, int *inner_iters, int *qp_iters, int *status) {
-    return closed_loop_host_impl(h, layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, NTM_STATE_ROWS_OFF,
-                                 nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status);
+    return fused_host_call(h, loop_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, NTM_STATE_ROWS_OFF, xk,
+                                        uk, Uk, cost, inner_iters, qp_iters, status), nullptr);
 }
 
 int ntm_mpc_closed_loop_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
                                const double *x0, const double *params, int pc, int state_rows, const double *xbounds,
                                double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
                                int *status) {
-    return closed_loop_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, state_rows, xbounds,
-                                {x0, params, nullptr, nullptr, nullptr, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
+    return fused_dev_call(h, loop_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, xk, uk, Uk,
+                                       cost, inner_iters, qp_iters, status), xbounds);
 }
 
 int ntm_mpc_closed_loop_sc(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
                            const double *x0, const double *params, int pc, int state_rows, const double *xbounds,
                            double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
                            int *status) {
-    return closed_loop_host_impl(h, layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, xbounds, xk,
-                                 uk, Uk, cost, inner_iters, qp_iters, status);
+    return fused_host_call(h, loop_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, xk, uk, Uk,
+                                        cost, inner_iters, qp_iters, status), xbounds);
 }
 
 // ------------------------------------------------------------------------------------------------ controller step
-// One time step of the fused loop without the plant: k_sim = 1, the caller's records in LoopArgs::sv, ONE launch.
-static int check_step(int profile, int N, int i_sim) {
-    REQUIRE(!(profile & NTM_PROFILE_TAUE_W), "ntm_mpc_step: NTM_PROFILE_TAUE_W is not supported by the controller step");
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(i_sim >= 1, "i_sim must be >= 1");
-    return NTM_OK;
-}
-
-// d: x0 is the measured state, state the records, uk = u and Uk = U
-static int step_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, int pc,
-                         int state_rows, const double *xb, const Fused &d) {
-    TRY(check_common(h, layout, S));
-    TRY(check_step(profile, N, i_sim));
-    ntm::LoopArgs a = {};
-    TRY(set_state_rows(h, profile, N, state_rows, xb, a));
-    if (S == 0) return NTM_OK;
-    TRY(check_params(d.params, pc, S));
-    REQUIRE(d.x0 && d.state && d.uk, "NULL array");
-    a.sv = d.state; a.ctl = 1;
-    return launch_fused(h, a, layout, profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4), S, N, 1, i_sim, eps, pc, d);
-}
-
-static int step_host_impl(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
-                          const double *params, int pc, int state_rows, const double *xb, double *state, double *u,
-                          double *U, int *inner_iters, int *qp_iters, int *status) {
-    TRY(check_common(h, layout, S));
-    TRY(check_step(profile, N, i_sim));
-    ntm::LoopArgs rows = {};
-    TRY(set_state_rows(h, profile, N, state_rows, xb, rows));   // before any copy
-    if (S == 0) return NTM_OK;
-    TRY(check_params(params, pc, S));
-    REQUIRE(x && state && u, "NULL array");
-    return fused_host(h, layout, S, S, 0, N, 1, pc, pc,
-                      {x, params, nullptr, nullptr, nullptr, state, nullptr, u, U, nullptr, inner_iters, qp_iters, status},
-                      [&](const Fused &d) { return step_dev_impl(h, layout, profile, S, N, i_sim, eps, pc, state_rows, xb, d); });
-}
-
 int ntm_mpc_step_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
                      const double *params, int pc, double *state, double *u, double *U, int *inner_iters, int *qp_iters,
                      int *status) {
-    return step_dev_impl(h, layout, profile, S, N, i_sim, eps, pc, NTM_STATE_ROWS_OFF, nullptr,
-                         {x, params, nullptr, nullptr, nullptr, state, nullptr, u, U, nullptr, inner_iters, qp_iters, status});
+    return fused_dev_call(h, step_args(layout, profile, S, N, i_sim, eps, x, params, pc, NTM_STATE_ROWS_OFF, state, u, U,
+                                       inner_iters, qp_iters, status), nullptr);
 }
 
 int ntm_mpc_step(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
                  const double *params, int pc, double *state, double *u, double *U, int *inner_iters, int *qp_iters,
                  int *status) {
-    return step_host_impl(h, layout, profile, S, N, i_sim, eps, x, params, pc, NTM_STATE_ROWS_OFF, nullptr, state, u, U,
-                          inner_iters, qp_iters, status);
+    return fused_host_call(h, step_args(layout, profile, S, N, i_sim, eps, x, params, pc, NTM_STATE_ROWS_OFF, state, u, U,
+                                        inner_iters, qp_iters, status), nullptr);
 }
 
 int ntm_mpc_step_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
                         const double *params, int pc, int state_rows, const double *xbounds, double *state, double *u,
                         double *U, int *inner_iters, int *qp_iters, int *status) {
-    return step_dev_impl(h, layout, profile, S, N, i_sim, eps, pc, state_rows, xbounds,
-                         {x, params, nullptr, nullptr, nullptr, state, nullptr, u, U, nullptr, inner_iters, qp_iters, status});
+    return fused_dev_call(h, step_args(layout, profile, S, N, i_sim, eps, x, params, pc, state_rows, state, u, U,
+                                       inner_iters, qp_iters, status), xbounds);
 }
 
 int ntm_mpc_step_sc(ntm_handle *h, int layout, int profile, int S, int N, int i_sim, double eps, const double *x,
                     const double *params, int pc, int state_rows, const double *xbounds, double *state, double *u,
                     double *U, int *inner_iters, int *qp_iters, int *status) {
-    return step_host_impl(h, layout, profile, S, N, i_sim, eps, x, params, pc, state_rows, xbounds, state, u, U,
-                          inner_iters, qp_iters, status);
+    return fused_host_call(h, step_args(layout, profile, S, N, i_sim, eps, x, params, pc, state_rows, state, u, U,
+                                        inner_iters, qp_iters, status), xbounds);
 }
 
 // ------------------------------------------------------------------------------------------------ perturbed plant
-// The fused loop with the plant of ntm_plant_step on its own block and profile bits, d_k and v_k, with the box QP or the
-// state rows (ONE launch).
-static int check_perturbed(int profile, int S, int N, int k_sim, int i_sim, const double *x0, const double *params,
-                           int pc, int ppc, int plant_profile, double *xk, double *uk) {
-    TRY(check_step(profile, N, i_sim));
-    TRY(check_params(params, pc, S));
-    TRY(check_loop(N, k_sim, i_sim, x0, xk, uk));
-    REQUIRE(ppc == 1 || ppc == S, "plant_params_count must be 1 or S");
-    REQUIRE(!(plant_profile & ~(NTM_PROFILE_RHO1_SQ | NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)),
-            "plant_profile: only RHO1_SQ, PLANT_C, PLANT_RK4 and TAUE_W act on the plant");
-    return NTM_OK;
-}
-
-static int perturbed_dev_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
-                              int pc, int state_rows, const double *xb, const double *plant_params, int ppc,
-                              int plant_profile, const Fused &d) {
-    TRY(check_common(h, layout, S));
-    if (S == 0) return NTM_OK;
-    if (plant_params == nullptr) { plant_params = d.params; ppc = pc; }
-    TRY(check_perturbed(profile, S, N, k_sim, i_sim, d.x0, d.params, pc, ppc, plant_profile, d.xk, d.uk));
-    ntm::LoopArgs a = {};
-    TRY(set_state_rows(h, profile, N, state_rows, xb, a));
-    a.pp = {plant_params, d.w, d.v, ppc, plant_profile};
-    a.pert = 1;
-    // plant-only bits have no effect on the controller
-    return launch_fused(h, a, layout, profile & ~(NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4), S, N, k_sim, i_sim, eps, pc, d);
-}
-
-static int perturbed_host_impl(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
-                               const double *x0, const double *params, int pc, int state_rows, const double *xb,
-                               const double *plant_params, int ppc, int plant_profile, const double *w, const double *v,
-                               double *xk, double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters,
-                               int *status) {
-    TRY(check_common(h, layout, S));
-    if (S == 0) return NTM_OK;
-    if (plant_params == nullptr) ppc = pc;
-    TRY(check_perturbed(profile, S, N, k_sim, i_sim, x0, params, pc, ppc, plant_profile, xk, uk));
-    ntm::LoopArgs rows = {};
-    TRY(set_state_rows(h, profile, N, state_rows, xb, rows));   // before any copy
-    return fused_host(h, layout, S, S, 0, N, k_sim, pc, ppc,
-                      {x0, params, plant_params, w, v, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status},
-                      [&](const Fused &d) {
-                          return perturbed_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, state_rows, xb,
-                                                    d.pparams, ppc, plant_profile, d);
-                      });
-}
-
 int ntm_mpc_closed_loop_perturbed_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
                                       double eps, const double *x0, const double *params, int pc,
                                       const double *plant_params, int ppc, int plant_profile, const double *w,
                                       const double *v, double *xk, double *uk, double *Uk, double *cost,
                                       int *inner_iters, int *qp_iters, int *status) {
-    return perturbed_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, NTM_STATE_ROWS_OFF, nullptr, plant_params,
-                              ppc, plant_profile, {x0, params, nullptr, w, v, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
+    return fused_dev_call(h, perturbed_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, NTM_STATE_ROWS_OFF,
+                                            plant_params, ppc, plant_profile, w, v, xk, uk, Uk, cost, inner_iters,
+                                            qp_iters, status), nullptr);
 }
 
 int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
@@ -904,8 +925,9 @@ int ntm_mpc_closed_loop_perturbed(ntm_handle *h, int layout, int profile, int S,
                                   const double *plant_params, int ppc, int plant_profile, const double *w,
                                   const double *v, double *xk, double *uk, double *Uk, double *cost, int *inner_iters,
                                   int *qp_iters, int *status) {
-    return perturbed_host_impl(h, layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, NTM_STATE_ROWS_OFF, nullptr,
-                               plant_params, ppc, plant_profile, w, v, xk, uk, Uk, cost, inner_iters, qp_iters, status);
+    return fused_host_call(h, perturbed_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, NTM_STATE_ROWS_OFF,
+                                             plant_params, ppc, plant_profile, w, v, xk, uk, Uk, cost, inner_iters,
+                                             qp_iters, status), nullptr);
 }
 
 int ntm_mpc_closed_loop_perturbed_sc_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
@@ -913,8 +935,9 @@ int ntm_mpc_closed_loop_perturbed_sc_dev(ntm_handle *h, int layout, int profile,
                                          const double *xbounds, const double *plant_params, int ppc, int plant_profile,
                                          const double *w, const double *v, double *xk, double *uk, double *Uk,
                                          double *cost, int *inner_iters, int *qp_iters, int *status) {
-    return perturbed_dev_impl(h, layout, profile, S, N, k_sim, i_sim, eps, pc, state_rows, xbounds, plant_params, ppc,
-                              plant_profile, {x0, params, nullptr, w, v, nullptr, xk, uk, Uk, cost, inner_iters, qp_iters, status});
+    return fused_dev_call(h, perturbed_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows,
+                                            plant_params, ppc, plant_profile, w, v, xk, uk, Uk, cost, inner_iters,
+                                            qp_iters, status), xbounds);
 }
 
 int ntm_mpc_closed_loop_perturbed_sc(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
@@ -922,27 +945,24 @@ int ntm_mpc_closed_loop_perturbed_sc(ntm_handle *h, int layout, int profile, int
                                      const double *xbounds, const double *plant_params, int ppc, int plant_profile,
                                      const double *w, const double *v, double *xk, double *uk, double *Uk, double *cost,
                                      int *inner_iters, int *qp_iters, int *status) {
-    return perturbed_host_impl(h, layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, xbounds,
-                               plant_params, ppc, plant_profile, w, v, xk, uk, Uk, cost, inner_iters, qp_iters, status);
+    return fused_host_call(h, perturbed_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows,
+                                             plant_params, ppc, plant_profile, w, v, xk, uk, Uk, cost, inner_iters,
+                                             qp_iters, status), xbounds);
 }
 
 // ------------------------------------------------------------------------------------------------ getWLc
 int ntm_getWLc_dev(ntm_handle *h, int layout, int S, int N, const double *bounds, const double *Gamma, const double *Phi,
                    const double *Lambda, double *W, double *L, double *c) {
-    TRY(check_common(h, layout, S));
+    TRY(check_getwlc(h, layout, S, N, bounds, Gamma, Phi, Lambda, W, L, c));
     if (S == 0) return NTM_OK;
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(bounds && Gamma && Phi && Lambda && W && L && c, "NULL array");
     CU(ntm::launch_getwlc(h->stream, h->props, layout, S, N, bounds, Gamma, Phi, Lambda, W, L, c, &h->launches));
     return NTM_OK;
 }
 
 int ntm_getWLc(ntm_handle *h, int layout, int S, int N, const double *bounds, const double *Gamma, const double *Phi,
                const double *Lambda, double *W, double *L, double *c) {
-    TRY(check_common(h, layout, S));
+    TRY(check_getwlc(h, layout, S, N, bounds, Gamma, Phi, Lambda, W, L, c));
     if (S == 0) return NTM_OK;
-    REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
-    REQUIRE(bounds && Gamma && Phi && Lambda && W && L && c, "NULL array");
     const size_t s = (size_t)S, n = (size_t)N, r = 6 * n + 4;
     double *dGam, *dPhi, *dLam, *dW, *dL, *dc;
     TRY(Arena(h).reserve([&](Arena &A) {
@@ -950,7 +970,7 @@ int ntm_getWLc(ntm_handle *h, int layout, int S, int N, const double *bounds, co
         dW = A.take<double>(r * 2 * s); dL = A.take<double>(r * n * s); dc = A.take<double>(r * s);
     }));
     TRY(h2d(h, dGam, Gamma, 2 * n * n * s)); TRY(h2d(h, dPhi, Phi, 4 * n * s)); TRY(h2d(h, dLam, Lambda, 2 * n * s));
-    TRY(ntm_getWLc_dev(h, layout, S, N, bounds, dGam, dPhi, dLam, dW, dL, dc));
+    CU(ntm::launch_getwlc(h->stream, h->props, layout, S, N, bounds, dGam, dPhi, dLam, dW, dL, dc, &h->launches));
     TRY(d2h(h, W, dW, r * 2 * s)); TRY(d2h(h, L, dL, r * n * s)); TRY(d2h(h, c, dc, r * s));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
@@ -960,22 +980,8 @@ int ntm_getWLc(ntm_handle *h, int layout, int S, int N, const double *bounds, co
 int ntm_mc_stats_dev(ntm_handle *h, int layout, int S, int k_sim, const double *xk, const double *uk,
                      const double *cost, const int *status, const double *params, int pc, const double *bounds,
                      double w_sup, double hist_max, double *out) {
-    TRY(check_common(h, layout, S));
-    REQUIRE(k_sim >= 1, "k_sim must be >= 1");
-    REQUIRE(bounds && out, "NULL array");
-    const double *umin = nullptr, *umax = nullptr;
-    int ustride = 0;
-    if (S > 0) {
-        TRY(check_params(params, pc, S));
-        REQUIRE(xk && uk, "NULL array");
-        // where umin / umax (slots 8 and 9 of the parameter block) of scenario s live in the caller's layout
-        if (pc == 1) { umin = params + 8; umax = params + 9; ustride = 0; }
-        else if (layout == NTM_LAYOUT_MATLAB) { umin = params + 8; umax = params + 9; ustride = NTM_NPARAM; }
-        else { umin = params + 8 * (size_t)S; umax = params + 9 * (size_t)S; ustride = 1; }
-    }
-    CU(ntm::launch_mc_stats(h->stream, h->props, layout, S, k_sim, xk, uk, cost, status, umin, umax, ustride, bounds, w_sup,
-                            hist_max, out, &h->launches));
-    return NTM_OK;
+    TRY(check_mc_stats(h, layout, S, k_sim, xk, uk, params, pc, bounds, out));
+    return mc_stats_launch(h, layout, S, k_sim, xk, uk, cost, status, params, pc, bounds, w_sup, hist_max, out);
 }
 
 // The same reduction with the EC-power box handed over as two compact arrays umin[S], umax[S] (bounds_count = S) or
@@ -999,13 +1005,7 @@ int ntm_mc_stats_ub_dev(ntm_handle *h, int layout, int S, int k_sim, const doubl
 int ntm_mc_stats(ntm_handle *h, int layout, int S, int k_sim, const double *xk, const double *uk, const double *cost,
                  const int *status, const double *params, int pc, const double *bounds, double w_sup,
                  double hist_max, double *out) {
-    TRY(check_common(h, layout, S));
-    REQUIRE(k_sim >= 1, "k_sim must be >= 1");
-    REQUIRE(bounds && out, "NULL array");
-    if (S > 0) {
-        TRY(check_params(params, pc, S));
-        REQUIRE(xk && uk, "NULL array");
-    }
+    TRY(check_mc_stats(h, layout, S, k_sim, xk, uk, params, pc, bounds, out));
     const size_t s = (size_t)S, k = (size_t)k_sim;
     double *dx, *du, *dc, *dp, *dout;
     int *dst;
@@ -1020,8 +1020,8 @@ int ntm_mc_stats(ntm_handle *h, int layout, int S, int k_sim, const double *xk, 
         if (status) TRY(h2d(h, dst, status, s));
         TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
     }
-    TRY(ntm_mc_stats_dev(h, layout, S, k_sim, dx, du, cost ? dc : nullptr, status ? dst : nullptr, dp, pc, bounds, w_sup,
-                         hist_max, dout));
+    TRY(mc_stats_launch(h, layout, S, k_sim, dx, du, cost ? dc : nullptr, status ? dst : nullptr, dp, pc, bounds, w_sup,
+                        hist_max, dout));
     TRY(d2h(h, out, dout, (size_t)NTM_MC_NSTAT));
     CU(cudaStreamSynchronize(h->stream));
     return NTM_OK;
@@ -1029,50 +1029,13 @@ int ntm_mc_stats(ntm_handle *h, int layout, int S, int k_sim, const double *xk, 
 
 // ------------------------------------------------------------------------------------------------ fp64 peak
 int ntm_fp64_peak(ntm_handle *h, int iters, double *tflops_dfma, double *ms_out) {
-    REQUIRE(h != nullptr, "handle is NULL");
-    REQUIRE(iters > 0, "iters must be > 0");
-    CU(cudaSetDevice(h->device));
-    cudaEvent_t e0, e1;
-    CU(cudaEventCreate(&e0));
-    CU(cudaEventCreate(&e1));
-    double *out = reinterpret_cast<double *>(h->counter) + 8;
-    CU(ntm::launch_fp64_peak(h->stream, h->props, iters / 8 + 1, out, &h->launches));   // warm-up
-    CU(cudaEventRecord(e0, h->stream));
-    CU(ntm::launch_fp64_peak(h->stream, h->props, iters, out, &h->launches));
-    CU(cudaEventRecord(e1, h->stream));
-    CU(cudaEventSynchronize(e1));
-    float ms = 0.f;
-    CU(cudaEventElapsedTime(&ms, e0, e1));
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    const double flops = 2.0 * 64.0 * (double)iters * 256.0 * (double)h->props.sm_count * 8.0;
-    if (tflops_dfma) *tflops_dfma = flops / (ms * 1e-3) / 1e12;
-    if (ms_out) *ms_out = ms;
-    return NTM_OK;
+    // 64 DFMA (2 flops each) per thread and iteration, 256 threads per CTA, 8 CTAs per SM
+    return time_peak(h, iters, ntm::launch_fp64_peak, 2.0 * 64.0 * 256.0 * 8.0, tflops_dfma, ms_out);
+}
+
+int ntm_dmma_peak(ntm_handle *h, int iters, double *tflops_dmma, double *ms_out) {
+    // 8 DMMA.8x8x4 per warp and iteration, 2*8*8*4 flops each, 8 warps per CTA, 8 CTAs per SM
+    return time_peak(h, iters, ntm::launch_dmma_peak, 512.0 * 8.0 * 8.0 * 8.0, tflops_dmma, ms_out);
 }
 
 }  // extern "C"
-
-int ntm_dmma_peak(ntm_handle *h, int iters, double *tflops_dmma, double *ms_out) {
-    REQUIRE(h != nullptr, "handle is NULL");
-    REQUIRE(iters > 0, "iters must be > 0");
-    CU(cudaSetDevice(h->device));
-    cudaEvent_t e0, e1;
-    CU(cudaEventCreate(&e0));
-    CU(cudaEventCreate(&e1));
-    double *out = reinterpret_cast<double *>(h->counter) + 8;
-    CU(ntm::launch_dmma_peak(h->stream, h->props, iters / 8 + 1, out, &h->launches));   // warm-up
-    CU(cudaEventRecord(e0, h->stream));
-    CU(ntm::launch_dmma_peak(h->stream, h->props, iters, out, &h->launches));
-    CU(cudaEventRecord(e1, h->stream));
-    CU(cudaEventSynchronize(e1));
-    float ms = 0.f;
-    CU(cudaEventElapsedTime(&ms, e0, e1));
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    // 8 DMMA.8x8x4 per warp and iteration, 2*8*8*4 flops each, 8 warps per CTA, 8 CTAs per SM
-    const double flops = 512.0 * 8.0 * (double)iters * 8.0 * (double)h->props.sm_count * 8.0;
-    if (tflops_dmma) *tflops_dmma = flops / (ms * 1e-3) / 1e12;
-    if (ms_out) *ms_out = ms;
-    return NTM_OK;
-}

@@ -1418,6 +1418,13 @@ size_t state_rows_dense_smem(int N, int srows) {
     return work_bytes(N, N, 1) + ineq_bytes(N, 4 * N) + ext_bytes(N) + (srows == 2 ? gam_doubles(N, 1) * sizeof(double) : 0);
 }
 
+int qp_ineq_groups(const DeviceProps &dp, int N, int M) {
+    const size_t gbytes = work_bytes(N, N) + ineq_bytes(N, M);
+    int wpb = (gw_for(N) == 1) ? 4 : 1;
+    while (wpb > 1 && gbytes * wpb + 1024 > dp.smem_optin) wpb >>= 1;
+    return gbytes * wpb + 1024 <= dp.smem_optin ? wpb : 0;
+}
+
 size_t hscratch_bytes(const DeviceProps &dp, int N) {
     return (size_t)max_groups(dp, N) * N * odd_ld(N) * sizeof(double);
 }
@@ -1694,9 +1701,8 @@ cudaError_t launch_qp_ineq(cudaStream_t st, const DeviceProps &dp, int layout, i
     const int gw = gw_for(N);
     const size_t wbytes = work_bytes(N, N);
     const size_t gbytes = wbytes + ineq_bytes(N, M);
-    int wpb = (gw == 1) ? 4 : 1;
-    while (wpb > 1 && gbytes * wpb + 1024 > dp.smem_optin) wpb >>= 1;
-    if (gbytes * wpb + 1024 > dp.smem_optin) return cudaErrorInvalidConfiguration;
+    const int wpb = qp_ineq_groups(dp, N, M);
+    if (wpb == 0) return cudaErrorInvalidConfiguration;
     const auto kernel = gw == 1 ? qp_ineq_kernel<1> : (gw == 2 ? qp_ineq_kernel<2> : qp_ineq_kernel<4>);
     return launch_persistent(st, dp, kernel, 32 * gw * wpb, gbytes * wpb, S, wpb, INT_MAX, launches, layout, S, N, M, G,
                              F, lb, ub, bc, Lg, bg, U, iters, status, counter, (unsigned int)gbytes, (unsigned int)wbytes);

@@ -67,6 +67,9 @@ size_t lpt_doubles(const DeviceProps &dp, const LoopArgs &a);
 size_t state_rows_smem(int N);
 // the same for ONE group with a non-literal Gamma index (NTM_PROFILE_GAMMA_I / DENSE_G; one-warp groups, N <= 32)
 size_t state_rows_dense_smem(int N, int srows);
+// groups per CTA of the general-inequality QP (launch_qp_ineq) whose N x N factor pair + row scales fit in shared memory;
+// 0: not even one fits
+int qp_ineq_groups(const DeviceProps &dp, int N, int M);
 
 // every launcher returns the CUDA error of the launch (cudaSuccess on success) and adds the number of
 // kernels it launched to *launches
