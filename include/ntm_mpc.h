@@ -326,6 +326,59 @@ int ntm_mpc_closed_loop_perturbed_sc_dev(ntm_handle *h, int layout, int profile,
                                          double *xk, double *uk, double *Uk, double *cost, int *inner_iters,
                                          int *qp_iters, int *status);
 
+/* ---- state observer: one step of an LPV Kalman filter on the controller's own model, per scenario ---------------- *
+ * The quasi-LPV Kalman filter: rho is frozen at the estimate, as the condensation (:63-66) freezes it; no Jacobian of
+ * rho1..rho3 (not an EKF).  For S scenarios at the measurements y[2*S] (layout) and the inputs u[S] applied since their
+ * last step, it updates each scenario's record in place and writes the estimate to xhat[2*S] (layout; may be NULL).
+ * state holds NTM_KF_DOUBLES doubles per scenario, one contiguous record per scenario in both layouts:
+ *   [0, 2) xhat   [2, 5) P as p11, p21, p22   [5] steps run (0 = fresh)
+ * An ALL-ZERO record is a fresh filter (memset is the reset, as for NTM_CTRL_DOUBLES).  One step:
+ *   fresh record:  xhat = y, P = Rv, steps = 1 (u is not read)
+ *   otherwise:     xhat- = ntm_plant_step(xhat, u) under profile & (RHO1_SQ | PLANT_C | PLANT_RK4), params
+ *                  F = A(rho(xhat)) of A.m:2 (the Euler-map matrix, also under PLANT_RK4: the quasi-LPV approximation)
+ *                  P- = F P F' + Qw,  K = P- (P- + Rv)^-1 (closed-form 2x2 inverse),  xhat = xhat- + K (y - xhat-)
+ *                  P = (I - K) P- (I - K)' + K Rv K' (Joseph form: P stays symmetric positive semi-definite although
+ *                  w ~ 0.1 m and omega ~ 6e3 rad/s differ in scale by ~1e5),  steps += 1
+ * Non-finite inputs get no special case: they propagate into the record, and zeroing it restarts the filter.
+ * kf_cov = {qw11, qw21, qw22, rv11, rv21, rv22} on the HOST in both variants (shared by all scenarios): Qw the process
+ * and Rv the measurement covariance.  profile: the controller's profile word (the other bits are ignored).  One launch.
+ * host entry: records copied in and back; _dev entry: records resident.  u must be non-NULL for S > 0.
+ * NTM_ERR_INVALID: NULL or non-finite kf_cov, Qw not positive semi-definite (q11 >= 0, q22 >= 0, q11 q22 >= q21^2), Rv
+ * not positive definite (r11 > 0, r11 r22 > r21^2; then P- + Rv is invertible for every reachable P-), NTM_PROFILE_TAUE_W
+ * in profile, bad sizes, NULL arrays, params_count not 1 or S. */
+#define NTM_KF_DOUBLES 6
+int ntm_kf_step(ntm_handle *h, int layout, int profile, int S, const double *y, const double *u, const double *params,
+                int params_count, const double *kf_cov, double *state, double *xhat);
+int ntm_kf_step_dev(ntm_handle *h, int layout, int profile, int S, const double *y, const double *u,
+                    const double *params, int params_count, const double *kf_cov, double *state, double *xhat);
+
+/* ---- the perturbed loop whose controller sees the observer's estimate instead of the raw measurement ------------- *
+ * For k = 0 .. k_sim-1, in ONE launch:
+ *   y_k = x_k + v_k
+ *   xhat_k = ntm_kf_step(y_k, u_{k-1}; profile, params, kf_cov, its own record)   (fresh at k = 0: xhat_0 = y_0)
+ *   u_k, U_k = one ntm_mpc_step_sc (NTM_STATE_ROWS_OFF: ntm_mpc_step) at xhat_k
+ *   x_{k+1} = ntm_plant_step(x_k, u_k; plant_params, plant_profile) + d_k
+ * bit for bit, up to and including the step at which a scenario turns infeasible.  Every other argument and output
+ * means what it means in ntm_mpc_closed_loop_perturbed_sc: xk and cost are the true states, the offline build and the
+ * frozen rows come from xhat_0 = y_0, the x_0 block of getWLc.m:30 tests xhat_k, and after an infeasible step the
+ * scenario ends as there.  xhat: 2*k_sim doubles per scenario in `layout`, element 2k + i (or NULL): the estimate the
+ * controller used at step k, NaN after an infeasible step.  kf_cov is required (the _perturbed entries are the loop
+ * without an observer).  The filter records live in a handle-owned device buffer and every input travels with the
+ * launch: the _dev entry queues one launch and no copy.
+ * NTM_ERR_INVALID: whatever ntm_mpc_closed_loop_perturbed_sc or ntm_kf_step rejects. */
+int ntm_mpc_closed_loop_observed(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
+                                 const double *x0, const double *params, int params_count, int state_rows,
+                                 const double *xbounds, const double *plant_params, int plant_params_count,
+                                 int plant_profile, const double *w, const double *v, const double *kf_cov,
+                                 double *xhat, double *xk, double *uk, double *Uk, double *cost, int *inner_iters,
+                                 int *qp_iters, int *status);
+int ntm_mpc_closed_loop_observed_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
+                                     double eps, const double *x0, const double *params, int params_count,
+                                     int state_rows, const double *xbounds, const double *plant_params,
+                                     int plant_params_count, int plant_profile, const double *w, const double *v,
+                                     const double *kf_cov, double *xhat, double *xk, double *uk, double *Uk,
+                                     double *cost, int *inner_iters, int *qp_iters, int *status);
+
 /* ---- the loop on EVERY visible GPU from ONE host process (what a MEX gateway can reach; SURVEY 8e) ------------- *
  * Replaces the same lines as ntm_mpc_closed_loop[_sc] (NTM_MPC_Sim.m:63-73,80-131); host pointers, same argument
  * meaning, no handle: the library keeps one pooled handle per device.  Scenarios never interact (:93-131 has no

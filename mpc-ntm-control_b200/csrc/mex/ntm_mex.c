@@ -17,7 +17,9 @@
  *                                (shadows the Optimization Toolbox function: input-box rows become bounds, state rows stay)
  *   11  ntm_mpc_step             one step NTM_MPC_Sim.m:94-128  [u,state,U,inner,status] = ntm_mpc_step(state,x,params,N,i_sim,eps,profile[,state_rows,xmin,xmax])
  *                                (no plant: the script's `for k` loop keeps its own plant code and passes state back in)
- *   12  ntm_mpc_batch_perturbed  the loop vs a perturbed plant  [xk,uk,cost,inner,status] = ntm_mpc_batch_perturbed(x0,params,N,k_sim,i_sim,eps,profile,plant_params,plant_profile,w,v[,state_rows,xmin,xmax])
+ *   12  ntm_mpc_batch_perturbed  the loop vs a perturbed plant  [xk,uk,cost,inner,status,xhat] = ntm_mpc_batch_perturbed(x0,params,N,k_sim,i_sim,eps,profile,plant_params,plant_profile,w,v[,state_rows,xmin,xmax[,kf_cov]])
+ *                                (with kf_cov: the controller sees the estimate of the observer, xhat, not y_k)
+ *   13  ntm_kf_step              the state observer, one step   [xhat,state] = ntm_kf_step(y,u,params,kf_cov,state,profile)
  *
  * The short forms are the ones NTM_MPC_Sim.m actually uses (:63-66,:113-119,:130); the missing trailing arguments
  * are fetched from the caller's workspace under the script's own variable names (kappa :24, tau_r :9, Ts :31,
@@ -35,7 +37,7 @@
 #include "ntm_mpc.h"
 
 #ifndef NTM_MEX_FN
-#error "compile with -DNTM_MEX_FN=<1..12>"
+#error "compile with -DNTM_MEX_FN=<1..13>"
 #endif
 
 static ntm_handle *g_h = NULL;
@@ -90,6 +92,21 @@ static void model_params(double *p, double kappa, double taur, double Ts, double
     p[2] = 1 - Ts / TE;
     p[3] = (kappa * Ts * etaCD / wdep);
     p[7] = wdep;
+}
+
+/* kf_cov = {qw11, qw21, qw22, rv11, rv21, rv22}: 6 finite reals, Qw positive semi-definite, Rv positive definite (the
+ * rules of ntm_kf_step, raised here as argument errors before the GPU is touched) */
+static const double *kf_cov_arg(const mxArray *c) {
+    const double *k;
+    int i;
+    if (!is_real_double(c) || mxGetNumberOfElements(c) != 6)
+        mexErrMsgIdAndTxt("ntm:arg", "kf_cov must be a real double 6-vector {qw11, qw21, qw22, rv11, rv21, rv22}");
+    k = mxGetPr(c);
+    for (i = 0; i < 6; ++i)
+        if (!isfinite(k[i])) mexErrMsgIdAndTxt("ntm:arg", "kf_cov: non-finite entry");
+    if (!(k[0] >= 0.0 && k[2] >= 0.0 && k[0] * k[2] >= k[1] * k[1])) mexErrMsgIdAndTxt("ntm:arg", "kf_cov: Qw is not positive semi-definite");
+    if (!(k[3] > 0.0 && k[3] * k[5] > k[4] * k[4])) mexErrMsgIdAndTxt("ntm:arg", "kf_cov: Rv is not positive definite");
+    return k;
 }
 
 static int states_arg(const mxArray *x) {
@@ -418,15 +435,19 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
          * The fused loop against a perturbed plant (ntm_mpc_closed_loop_perturbed_sc), one device: the controller of
          * ntm_mpc_batch sees y_k = x_k + v_k; the plant runs on plant_params (16x1 | 16xS, [] = params) under
          * plant_profile, plus the disturbance w_k.  w, v: 2 x k_sim x S (or 2k_sim x S), [] = none.  xk holds the
-         * true states.  state_rows / xmin / xmax as in ntm_mpc_batch: getWLc's state rows in the controller's QPs. */
+         * true states.  state_rows / xmin / xmax as in ntm_mpc_batch: getWLc's state rows in the controller's QPs.
+         * A trailing kf_cov (6 elements, see ntm_kf_step) puts the state observer between the sensor and the controller
+         * (ntm_mpc_closed_loop_observed); the sixth output xhat (2k_sim x S) is then the estimate it used per step. */
         int S, N, k_sim, i_sim, profile, pprofile, pc, ppc, i, srows = 0;
         double eps, xb[4] = {0.0, 0.0, 0.0, 0.0};
-        const double *pp = NULL, *w = NULL, *v = NULL;
-        mxArray *xk, *uk, *cost, *inner, *status;
+        const double *pp = NULL, *w = NULL, *v = NULL, *kc = NULL;
+        mxArray *xk, *uk, *cost, *inner, *status, *xhat = NULL;
         int *ibuf;
-        if (nrhs != 11 && nrhs != 14)
-            mexErrMsgIdAndTxt("ntm:arg", "usage: [xk,uk,cost,inner,status] = ntm_mpc_batch_perturbed(x0, params, N, k_sim, i_sim, eps, profile, plant_params, plant_profile, w, v [, state_rows, xmin, xmax])");
-        if (nrhs == 14) {
+        if (nrhs != 11 && nrhs != 14 && nrhs != 15)
+            mexErrMsgIdAndTxt("ntm:arg", "usage: [xk,uk,cost,inner,status,xhat] = ntm_mpc_batch_perturbed(x0, params, N, k_sim, i_sim, eps, profile, plant_params, plant_profile, w, v [, state_rows, xmin, xmax [, kf_cov]])");
+        if (nrhs == 15) kc = kf_cov_arg(prhs[14]);
+        if (nlhs > 5 && !kc) mexErrMsgIdAndTxt("ntm:arg", "xhat (the sixth output) needs the kf_cov argument");
+        if (nrhs >= 14) {
             srows = (int)scalar_arg(nrhs, prhs, 11, "");
             if (srows < 0 || srows > 2) mexErrMsgIdAndTxt("ntm:arg", "state_rows must be 0, 1 or 2");
             if (!is_real_double(prhs[12]) || !is_real_double(prhs[13]) || mxGetNumberOfElements(prhs[12]) != 2 ||
@@ -463,9 +484,16 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         xk = mxCreateDoubleMatrix(2 * (k_sim + 1), S, mxREAL); uk = mxCreateDoubleMatrix(k_sim, S, mxREAL);
         cost = mxCreateDoubleMatrix(1, S, mxREAL); inner = mxCreateDoubleMatrix(k_sim, S, mxREAL); status = mxCreateDoubleMatrix(1, S, mxREAL);
         ibuf = (int *)mxMalloc(sizeof(int) * ((size_t)k_sim * S + S + 1));
-        check(ntm_mpc_closed_loop_perturbed_sc(handle(), NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, mxGetPr(prhs[0]),
-                                               mxGetPr(prhs[1]), pc, srows, xb, pp, ppc, pprofile, w, v, mxGetPr(xk), mxGetPr(uk),
-                                               NULL, mxGetPr(cost), ibuf, NULL, ibuf + (size_t)k_sim * S));
+        if (kc) {
+            xhat = mxCreateDoubleMatrix(2 * (size_t)k_sim, S, mxREAL);
+            check(ntm_mpc_closed_loop_observed(handle(), NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, mxGetPr(prhs[0]),
+                                               mxGetPr(prhs[1]), pc, srows, xb, pp, ppc, pprofile, w, v, kc, mxGetPr(xhat),
+                                               mxGetPr(xk), mxGetPr(uk), NULL, mxGetPr(cost), ibuf, NULL, ibuf + (size_t)k_sim * S));
+        } else {
+            check(ntm_mpc_closed_loop_perturbed_sc(handle(), NTM_LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, mxGetPr(prhs[0]),
+                                                   mxGetPr(prhs[1]), pc, srows, xb, pp, ppc, pprofile, w, v, mxGetPr(xk), mxGetPr(uk),
+                                                   NULL, mxGetPr(cost), ibuf, NULL, ibuf + (size_t)k_sim * S));
+        }
         for (i = 0; i < k_sim * S; ++i) mxGetPr(inner)[i] = (double)ibuf[i];
         for (i = 0; i < S; ++i) mxGetPr(status)[i] = (double)ibuf[(size_t)k_sim * S + i];
         mxFree(ibuf);
@@ -474,6 +502,38 @@ void mexFunction(int nlhs, mxArray *plhs[], int nrhs, const mxArray *prhs[]) {
         if (nlhs > 2) plhs[2] = cost; else mxDestroyArray(cost);
         if (nlhs > 3) plhs[3] = inner; else mxDestroyArray(inner);
         if (nlhs > 4) plhs[4] = status; else mxDestroyArray(status);
+        if (nlhs > 5) plhs[5] = xhat; else if (xhat) mxDestroyArray(xhat);
+    }
+#elif NTM_MEX_FN == 13
+    {   /* [xhat, state] = ntm_kf_step(y (2xS), u (1xS), params (16x1 | 16xS), kf_cov (6), state ([] | 6xS), profile)
+         * One step of the state observer (ntm_kf_step): y the measurements, u the inputs applied since each record's last
+         * step (ignored for fresh records), kf_cov = {qw11, qw21, qw22, rv11, rv21, rv22}.  state: NTM_KF_DOUBLES = 6 rows
+         * (xhat, p11, p21, p22, steps) per scenario, [] or a zero column = a fresh filter; pass the returned state back in.
+         * profile: the controller's profile word (its RHO1_SQ, PLANT_C and PLANT_RK4 bits choose the prediction). */
+        int S, pc, profile;
+        const double *kc;
+        mxArray *st, *xhat;
+        if (nrhs != 6) mexErrMsgIdAndTxt("ntm:arg", "usage: [xhat, state] = ntm_kf_step(y, u, params, kf_cov, state, profile)");
+        S = states_arg(prhs[0]);
+        if (!is_real_double(prhs[1]) || (int)mxGetNumberOfElements(prhs[1]) != S)
+            mexErrMsgIdAndTxt("ntm:arg", "u must be a real double vector of S elements");
+        if (!is_real_double(prhs[2]) || mxGetM(prhs[2]) != NTM_NPARAM || ((int)mxGetN(prhs[2]) != 1 && (int)mxGetN(prhs[2]) != S))
+            mexErrMsgIdAndTxt("ntm:arg", "params must be 16 x 1 or 16 x S (see ntm_mpc.h)");
+        pc = (int)mxGetN(prhs[2]);
+        kc = kf_cov_arg(prhs[3]);
+        if (!is_real_double(prhs[4]))
+            mexErrMsgIdAndTxt("ntm:arg", "state must be [] or a real double matrix");
+        if (mxGetNumberOfElements(prhs[4]) != 0 && (mxGetM(prhs[4]) != NTM_KF_DOUBLES || (int)mxGetN(prhs[4]) != S))
+            mexErrMsgIdAndTxt("ntm:arg", "state must be [] or NTM_KF_DOUBLES = 6 rows by S columns");
+        profile = (int)scalar_arg(nrhs, prhs, 5, "");
+        if (profile & NTM_PROFILE_TAUE_W) mexErrMsgIdAndTxt("ntm:arg", "NTM_PROFILE_TAUE_W (128) is not supported by ntm_kf_step");
+        st = mxCreateDoubleMatrix(NTM_KF_DOUBLES, S, mxREAL);       /* zeros: a fresh filter */
+        if (mxGetNumberOfElements(prhs[4]) != 0) memcpy(mxGetPr(st), mxGetPr(prhs[4]), sizeof(double) * NTM_KF_DOUBLES * (size_t)S);
+        xhat = mxCreateDoubleMatrix(2, S, mxREAL);
+        check(ntm_kf_step(handle(), NTM_LAYOUT_MATLAB, profile, S, mxGetPr(prhs[0]), mxGetPr(prhs[1]), mxGetPr(prhs[2]), pc, kc,
+                          mxGetPr(st), mxGetPr(xhat)));
+        plhs[0] = xhat;
+        if (nlhs > 1) plhs[1] = st; else mxDestroyArray(st);
     }
 #else
 #error "unknown NTM_MEX_FN"

@@ -6,6 +6,7 @@
 // arguments before it allocates, copies or launches anything.  No exceptions leave this file
 // and there is no CPU fallback: without a usable CUDA device ntm_create fails with NTM_ERR_CUDA.
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
@@ -48,6 +49,8 @@ struct ntm_handle {
     size_t sv_bytes = 0;
     int *lpt = nullptr;              // ... and keys + order + bins of its longest-first work queue
     size_t lpt_bytes = 0;
+    double *kf = nullptr;            // the observed loop's filter records (ntm::ObsIn::rec)
+    size_t kf_bytes = 0;
     long long launches = 0;
 };
 
@@ -63,6 +66,9 @@ namespace {
     do {                                                    \
         if (!(cond)) return fail(NTM_ERR_INVALID, "%s", msg); \
     } while (0)
+
+// the model bits of a profile word: the plant the observer predicts with (ntm_kf_step)
+constexpr int KF_MODEL_BITS = NTM_PROFILE_RHO1_SQ | NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4;
 
 #define TRY(expr)                      \
     do {                               \
@@ -200,12 +206,36 @@ ntm::LoopArgs perturbed_args(int layout, int profile, int S, int N, int k_sim, i
     return a;
 }
 
+// The perturbed loop whose controller sees the estimate of ntm_kf_step; kf_cov is checked by check_fused.
+ntm::LoopArgs observed_args(int layout, int profile, int S, int N, int k_sim, int i_sim, double eps, const double *x0,
+                            const double *params, int pc, int state_rows, const double *plant_params, int ppc,
+                            int plant_profile, const double *w, const double *v, double *xhat, double *xk, double *uk,
+                            double *Uk, double *cost, int *inner, int *qpit, int *status) {
+    ntm::LoopArgs a = perturbed_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows, plant_params,
+                                     ppc, plant_profile, w, v, xk, uk, Uk, cost, inner, qpit, status);
+    a.obs.on = 1; a.obs.xhat = xhat;
+    a.obs.mflags = profile & KF_MODEL_BITS;             // before check_fused strips the plant bits from a.flags
+    return a;
+}
+
+// The filter's covariances: Qw positive semi-definite, Rv positive definite (so P- + Rv is invertible for every P- the
+// filter can reach), every entry finite.
+int check_kf_cov(const double *c, ntm::KfCov &cov) {
+    REQUIRE(c, "kf_cov is NULL");
+    for (int i = 0; i < 6; ++i) REQUIRE(std::isfinite(c[i]), "kf_cov: non-finite entry");
+    REQUIRE(c[0] >= 0.0 && c[2] >= 0.0 && c[0] * c[2] >= c[1] * c[1], "kf_cov: Qw is not positive semi-definite");
+    REQUIRE(c[3] > 0.0 && c[3] * c[5] > c[4] * c[4], "kf_cov: Rv is not positive definite");
+    cov = {c[0], c[1], c[2], c[3], c[4], c[5]};
+    return NTM_OK;
+}
+
 // Every rule of a fused call.  It also sets what the rules decide: the state box from xb (on the host), the profile the
 // controller runs (a step and the perturbed loop ignore the plant-only bits) and the plant's parameter count when
-// plant_params is NULL (the controller's block).  At S == 0 a loop checks nothing beyond handle, layout and S; a
-// controller step checks everything but its parameters and arrays.  params_count (and plant_params_count) is 1 or
-// S_total, the scenarios of the caller's arrays, of which `a` may be a shard.
-int check_fused(ntm_handle *h, ntm::LoopArgs &a, const double *xb, int S_total) {
+// plant_params is NULL (the controller's block), and the observer's covariances from kf_cov (host).  At S == 0 a loop
+// checks nothing beyond handle, layout and S; a controller step checks everything but its parameters and arrays.
+// params_count (and plant_params_count) is 1 or S_total, the scenarios of the caller's arrays, of which `a` may be a
+// shard.
+int check_fused(ntm_handle *h, ntm::LoopArgs &a, const double *xb, int S_total, const double *kf_cov = nullptr) {
     TRY(check_common(h, a.layout, a.S));
     if (a.S == 0 && !a.ctl) return NTM_OK;
     if (a.ctl || a.pert) {
@@ -237,6 +267,7 @@ int check_fused(ntm_handle *h, ntm::LoopArgs &a, const double *xb, int S_total) 
         REQUIRE(!(a.pp.pflags & ~(NTM_PROFILE_RHO1_SQ | NTM_PROFILE_PLANT_C | NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)),
                 "plant_profile: only RHO1_SQ, PLANT_C, PLANT_RK4 and TAUE_W act on the plant");
     }
+    if (a.obs.on) TRY(check_kf_cov(kf_cov, a.obs.cov));
     return NTM_OK;
 }
 
@@ -247,6 +278,10 @@ int launch_fused(ntm_handle *h, ntm::LoopArgs a) {
     a.counter = h->counter;
     TRY(grow(h, h->hscratch, h->hscratch_bytes, ntm::hscratch_bytes(h->props, a.N)));
     a.hscratch = h->hscratch;
+    if (a.obs.on) {
+        TRY(grow(h, h->kf, h->kf_bytes, (size_t)a.S * NTM_KF_DOUBLES * sizeof(double)));
+        a.obs.rec = h->kf;
+    }
     const size_t svd = ntm::lpt_doubles(h->props, a);      // two-phase launch with a longest-first queue (ntm_kernels.h)
     int *lpt = nullptr;
     if (svd != 0) {
@@ -271,6 +306,7 @@ void fused_arrays(const ntm::LoopArgs &a, ntm::LoopArgs &d, F f) {
     f(a.pp.pparams, d.pp.pparams, NTM_NPARAM, IN, a.pp.pparams_count == 1);
     f(a.pp.dist, d.pp.dist, 2 * ks, IN, false);
     f(a.pp.noise, d.pp.noise, 2 * ks, IN, false);
+    f(a.obs.xhat, d.obs.xhat, 2 * ks, OUT, false);
     f(a.sv, d.sv, (size_t)NTM_CTRL_DOUBLES(a.N), INOUT, false);
     f(a.xk, d.xk, 2 * (ks + 1), OUT, false);
     f(a.uk, d.uk, ks, OUT, false);
@@ -313,13 +349,13 @@ int fused_host(ntm_handle *h, const ntm::LoopArgs &a, int S_total, int s_off) {
     return NTM_OK;
 }
 
-int fused_dev_call(ntm_handle *h, ntm::LoopArgs a, const double *xb) {
-    TRY(check_fused(h, a, xb, a.S));
+int fused_dev_call(ntm_handle *h, ntm::LoopArgs a, const double *xb, const double *kf_cov = nullptr) {
+    TRY(check_fused(h, a, xb, a.S, kf_cov));
     return a.S == 0 ? NTM_OK : launch_fused(h, a);
 }
 
-int fused_host_call(ntm_handle *h, ntm::LoopArgs a, const double *xb) {
-    TRY(check_fused(h, a, xb, a.S));
+int fused_host_call(ntm_handle *h, ntm::LoopArgs a, const double *xb, const double *kf_cov = nullptr) {
+    TRY(check_fused(h, a, xb, a.S, kf_cov));
     return a.S == 0 ? NTM_OK : fused_host(h, a, a.S, 0);
 }
 
@@ -403,6 +439,17 @@ int check_getwlc(ntm_handle *h, int layout, int S, int N, const double *bounds, 
     if (S == 0) return NTM_OK;
     REQUIRE(N >= 1 && N <= NTM_MAX_HORIZON, "N out of range [1, NTM_MAX_HORIZON]");
     REQUIRE(bounds && Gamma && Phi && Lambda && W && L && c, "NULL array");
+    return NTM_OK;
+}
+
+int check_kf(ntm_handle *h, int layout, int profile, int S, const double *y, const double *u, const double *params,
+             int pc, const double *kf_cov, const double *state, ntm::KfCov &cov) {
+    TRY(check_common(h, layout, S));
+    TRY(check_kf_cov(kf_cov, cov));
+    REQUIRE(!(profile & NTM_PROFILE_TAUE_W), "ntm_kf_step: NTM_PROFILE_TAUE_W is not supported by the observer");
+    if (S == 0) return NTM_OK;
+    TRY(check_params(params, pc, S));
+    REQUIRE(y && u && state, "NULL array");
     return NTM_OK;
 }
 
@@ -506,6 +553,7 @@ int ntm_destroy(ntm_handle *h) {
     if (h->hscratch) cudaFree(h->hscratch);
     if (h->sv) cudaFree(h->sv);
     if (h->lpt) cudaFree(h->lpt);
+    if (h->kf) cudaFree(h->kf);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
     return NTM_OK;
@@ -757,6 +805,36 @@ int ntm_plant_step(ntm_handle *h, int layout, int profile, int S, const double *
     return NTM_OK;
 }
 
+// ------------------------------------------------------------------------------------------------ observer
+int ntm_kf_step_dev(ntm_handle *h, int layout, int profile, int S, const double *y, const double *u, const double *params,
+                    int pc, const double *kf_cov, double *state, double *xhat) {
+    ntm::KfCov cov;
+    TRY(check_kf(h, layout, profile, S, y, u, params, pc, kf_cov, state, cov));
+    if (S == 0) return NTM_OK;
+    CU(ntm::launch_kf(h->stream, layout, profile & KF_MODEL_BITS, S, y, u, params, pc, cov, state, xhat, &h->launches));
+    return NTM_OK;
+}
+
+int ntm_kf_step(ntm_handle *h, int layout, int profile, int S, const double *y, const double *u, const double *params,
+                int pc, const double *kf_cov, double *state, double *xhat) {
+    ntm::KfCov cov;
+    TRY(check_kf(h, layout, profile, S, y, u, params, pc, kf_cov, state, cov));
+    if (S == 0) return NTM_OK;
+    const size_t s = (size_t)S;
+    double *dy, *du, *dp, *dr, *dx;
+    TRY(Arena(h).reserve([&](Arena &A) {
+        dy = A.take<double>(2 * s); du = A.take<double>(s); dp = A.take<double>((size_t)pc * NTM_NPARAM);
+        dr = A.take<double>(NTM_KF_DOUBLES * s); dx = A.take<double>(2 * s);
+    }));
+    TRY(h2d(h, dy, y, 2 * s)); TRY(h2d(h, du, u, s)); TRY(h2d(h, dp, params, (size_t)pc * NTM_NPARAM));
+    TRY(h2d(h, dr, state, NTM_KF_DOUBLES * s));
+    CU(ntm::launch_kf(h->stream, layout, profile & KF_MODEL_BITS, S, dy, du, dp, pc, cov, dr, xhat ? dx : nullptr,
+                      &h->launches));
+    TRY(d2h(h, state, dr, NTM_KF_DOUBLES * s)); TRY(d2h(h, xhat, dx, 2 * s));
+    CU(cudaStreamSynchronize(h->stream));
+    return NTM_OK;
+}
+
 // ------------------------------------------------------------------------------------------------ closed loop
 // ---- one host process, every visible GPU (the MEX gateway ntm_mpc_batch is single-process by construction) ----------
 // Scenarios never interact (NTM_MPC_Sim.m:93-131 has no cross-scenario term), so the batch is cut into contiguous
@@ -948,6 +1026,27 @@ int ntm_mpc_closed_loop_perturbed_sc(ntm_handle *h, int layout, int profile, int
     return fused_host_call(h, perturbed_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows,
                                              plant_params, ppc, plant_profile, w, v, xk, uk, Uk, cost, inner_iters,
                                              qp_iters, status), xbounds);
+}
+
+// ------------------------------------------------------------------------------------------------ observed loop
+int ntm_mpc_closed_loop_observed_dev(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim,
+                                     double eps, const double *x0, const double *params, int pc, int state_rows,
+                                     const double *xbounds, const double *plant_params, int ppc, int plant_profile,
+                                     const double *w, const double *v, const double *kf_cov, double *xhat, double *xk,
+                                     double *uk, double *Uk, double *cost, int *inner_iters, int *qp_iters, int *status) {
+    return fused_dev_call(h, observed_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows,
+                                           plant_params, ppc, plant_profile, w, v, xhat, xk, uk, Uk, cost, inner_iters,
+                                           qp_iters, status), xbounds, kf_cov);
+}
+
+int ntm_mpc_closed_loop_observed(ntm_handle *h, int layout, int profile, int S, int N, int k_sim, int i_sim, double eps,
+                                 const double *x0, const double *params, int pc, int state_rows, const double *xbounds,
+                                 const double *plant_params, int ppc, int plant_profile, const double *w,
+                                 const double *v, const double *kf_cov, double *xhat, double *xk, double *uk, double *Uk,
+                                 double *cost, int *inner_iters, int *qp_iters, int *status) {
+    return fused_host_call(h, observed_args(layout, profile, S, N, k_sim, i_sim, eps, x0, params, pc, state_rows,
+                                            plant_params, ppc, plant_profile, w, v, xhat, xk, uk, Uk, cost, inner_iters,
+                                            qp_iters, status), xbounds, kf_cov);
 }
 
 // ------------------------------------------------------------------------------------------------ getWLc

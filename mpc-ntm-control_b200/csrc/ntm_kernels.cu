@@ -73,6 +73,24 @@ plant_kernel(int layout, int flags, int S, const double *__restrict__ x, const d
     xn[elem(layout, S, 2, s, 1)] = nom;
 }
 
+// ntm_kf_step: the observer's step of the fused loop (kf_step_exact, ntm_loop.cuh) on the caller's records
+__global__ void __launch_bounds__(256)
+kf_kernel(int layout, int mflags, int S, const double *__restrict__ y, const double *__restrict__ u,
+          const double *__restrict__ params, int pc, KfCov cov, double *__restrict__ rec, double *__restrict__ xhat) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= S) return;
+    const Params P = load_params(params, layout, pc, s);
+    double *r = rec + (size_t)s * NTM_KF_DOUBLES;
+    const bool fresh = r[5] == 0.0;
+    double h1, h2;
+    kf_step_exact(P, mflags, cov, r, fresh, y[elem(layout, S, 2, s, 0)], y[elem(layout, S, 2, s, 1)],
+                  fresh ? 0.0 : u[s], h1, h2);
+    if (xhat != nullptr) {
+        xhat[elem(layout, S, 2, s, 0)] = h1;
+        xhat[elem(layout, S, 2, s, 1)] = h2;
+    }
+}
+
 // =================================================================================================
 // getWLc.m: L = Mcal*Gamma + Ecal, W = -Dcal - Mcal*Phi, c = Ccal - Mcal*Lambda.  Mcal/Ecal/Dcal are sign/selection
 // matrices, so every output row is +-(one row of Gamma/Phi/Lambda) or a constant: a pure gather, one thread per
@@ -1454,6 +1472,14 @@ cudaError_t launch_plant(cudaStream_t st, int layout, int flags, int S, const do
     return cudaGetLastError();
 }
 
+cudaError_t launch_kf(cudaStream_t st, int layout, int mflags, int S, const double *y, const double *u,
+                      const double *params, int pc, const KfCov &cov, double *rec, double *xhat, long long *launches) {
+    if (S <= 0) return cudaSuccess;
+    kf_kernel<<<(S + 255) / 256, 256, 0, st>>>(layout, mflags, S, y, u, params, pc, cov, rec, xhat);
+    ++*launches;
+    return cudaGetLastError();
+}
+
 // The dynamic-shared-memory attribute is PROCESS-WIDE per kernel and device, so it is only ever raised: once per
 // (kernel, device) to the device's opt-in maximum, under a lock.  (Caching "the last size this thread set" and skipping the
 // call let a second host thread lower the attribute under the first one's feet: its next launch then failed with
@@ -1562,6 +1588,10 @@ static const LoopKernel kLoopKernels[] = {
     {{1, true, EXT_PERTURBED, 0, false}, closed_loop_kernel<1, true, EXT_PERTURBED>},
     {{1, false, EXT_PERTURBED_ROWS, 0, false}, closed_loop_kernel<1, false, EXT_PERTURBED_ROWS>},
     {{1, true, EXT_PERTURBED_ROWS, 0, false}, closed_loop_kernel<1, true, EXT_PERTURBED_ROWS>},
+    {{1, false, EXT_OBSERVED, 0, false}, closed_loop_kernel<1, false, EXT_OBSERVED>},
+    {{1, true, EXT_OBSERVED, 0, false}, closed_loop_kernel<1, true, EXT_OBSERVED>},
+    {{1, false, EXT_OBSERVED_ROWS, 0, false}, closed_loop_kernel<1, false, EXT_OBSERVED_ROWS>},
+    {{1, true, EXT_OBSERVED_ROWS, 0, false}, closed_loop_kernel<1, true, EXT_OBSERVED_ROWS>},
     // multi-warp groups, dense Gamma
     {{2, true, EXT_BOX, 0, false}, closed_loop_kernel<2, true, EXT_BOX>},
     {{4, true, EXT_BOX, 0, false}, closed_loop_kernel<4, true, EXT_BOX>},
@@ -1571,6 +1601,8 @@ static const LoopKernel kLoopKernels[] = {
     {{4, true, EXT_COLD_PLANT, 0, false}, closed_loop_kernel<4, true, EXT_COLD_PLANT>},
     {{2, true, EXT_PERTURBED, 0, false}, closed_loop_kernel<2, true, EXT_PERTURBED>},
     {{4, true, EXT_PERTURBED, 0, false}, closed_loop_kernel<4, true, EXT_PERTURBED>},
+    {{2, true, EXT_OBSERVED, 0, false}, closed_loop_kernel<2, true, EXT_OBSERVED>},
+    {{4, true, EXT_OBSERVED, 0, false}, closed_loop_kernel<4, true, EXT_OBSERVED>},
     // multi-warp groups, literal Gamma, state rows
     {{2, false, EXT_STATE_ROWS, 0, false}, closed_loop_kernel<2, false, EXT_STATE_ROWS>},
     {{4, false, EXT_STATE_ROWS, 0, false}, closed_loop_kernel<4, false, EXT_STATE_ROWS>},
@@ -1578,8 +1610,10 @@ static const LoopKernel kLoopKernels[] = {
     {{4, false, EXT_STATE_ROWS, 0, true}, closed_loop_kernel<4, false, EXT_STATE_ROWS, 0, true>},
     {{2, false, EXT_PERTURBED_ROWS, 0, false}, closed_loop_kernel<2, false, EXT_PERTURBED_ROWS>},
     {{4, false, EXT_PERTURBED_ROWS, 0, false}, closed_loop_kernel<4, false, EXT_PERTURBED_ROWS>},
+    {{2, false, EXT_OBSERVED_ROWS, 0, false}, closed_loop_kernel<2, false, EXT_OBSERVED_ROWS>},
+    {{4, false, EXT_OBSERVED_ROWS, 0, false}, closed_loop_kernel<4, false, EXT_OBSERVED_ROWS>},
 };
-static_assert(sizeof(kLoopKernels) / sizeof(kLoopKernels[0]) == 26, "kLoopKernels: one entry per instantiation");
+static_assert(sizeof(kLoopKernels) / sizeof(kLoopKernels[0]) == 34, "kLoopKernels: one entry per instantiation");
 
 // The launch of one fused call: the instantiation and its shape.
 struct LoopRoute {
@@ -1595,12 +1629,13 @@ static cudaError_t route_closed_loop(const DeviceProps &dp, LoopArgs &a, LoopRou
     const int gw = gw_for(a.N);
     const bool dense = (a.flags & (NTM_PROFILE_GAMMA_I | NTM_PROFILE_DENSE_G)) != 0;
     // the headline instantiations carry none of the cold options
-    const int ext = a.pert ? (a.srows != 0 ? EXT_PERTURBED_ROWS : EXT_PERTURBED)
+    const int ext = a.pert ? (a.obs.on ? (a.srows != 0 ? EXT_OBSERVED_ROWS : EXT_OBSERVED)
+                                       : (a.srows != 0 ? EXT_PERTURBED_ROWS : EXT_PERTURBED))
                   : a.srows != 0 ? EXT_STATE_ROWS
                   : (a.flags & (NTM_PROFILE_PLANT_RK4 | NTM_PROFILE_TAUE_W)) ? EXT_COLD_PLANT : EXT_BOX;
     // long horizons, literal Gamma, box QP: the sweep tableau, in registers while N + 1 fits 7 x 15 blocks, else in shared
     // memory (LV = 1)
-    r.lng = gw > 1 && !dense && ext != EXT_STATE_ROWS && ext != EXT_PERTURBED_ROWS;
+    r.lng = gw > 1 && !dense && ext != EXT_STATE_ROWS && ext != EXT_PERTURBED_ROWS && ext != EXT_OBSERVED_ROWS;
     // the controller step is a runtime mode of the one-warp box kernels and its own instantiation (CTL) wherever that mode
     // would cost registers (DESIGN section 4.8)
     const bool ctl = a.ctl != 0 && (ext == EXT_STATE_ROWS || (gw > 1 && ext == EXT_BOX));

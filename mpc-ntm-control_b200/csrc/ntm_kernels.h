@@ -13,6 +13,22 @@ struct PlantIn {
     int pparams_count, pflags;
 };
 
+// The LPV Kalman filter's covariances (ntm_kf_step, kf_cov of include/ntm_mpc.h): Qw and Rv, lower triangles
+struct KfCov {
+    double q11, q21, q22, r11, r21, r22;
+};
+
+// The observer of ntm_mpc_closed_loop_observed: the controller sees the estimate of one ntm_kf_step per time step.
+// rec: NTM_KF_DOUBLES per scenario, scenario slowest (handle-owned scratch); xhat: 2 * k_sim doubles
+// per scenario in `layout`, element 2k + i (or NULL); mflags: the model bits of the controller's profile word
+// (RHO1_SQ | PLANT_C | PLANT_RK4), taken before check_fused strips the plant bits from `flags`; on (host only): the
+// call has an observer, and the C ABI layer points rec at the handle's scratch.
+struct ObsIn {
+    double *rec, *xhat;
+    KfCov cov;
+    int mflags, on;
+};
+
 struct LoopArgs {
     int layout, flags, S, N, k_sim, i_sim;
     double eps;
@@ -50,6 +66,7 @@ struct LoopArgs {
     // the start, written at the stop rule), no plant; xk and cost are NULL
     int ctl;
     int pert;                            // 1: perturbed plant (ntm_mpc_closed_loop_perturbed[_sc], see `pp` above)
+    ObsIn obs;                           // the observer of ntm_mpc_closed_loop_observed (pert = 1, obs.on = 1)
 };
 #define NTM_LPT_BINS 160
 
@@ -79,6 +96,9 @@ cudaError_t launch_lpv(cudaStream_t st, int layout, int S, const double *r1, con
                        const double *params, int pc, double *A, double *B, long long *launches);
 cudaError_t launch_plant(cudaStream_t st, int layout, int flags, int S, const double *x, const double *u,
                          const double *params, int pc, double *xn, long long *launches);
+// one ntm_kf_step: rec (NTM_KF_DOUBLES per scenario, scenario slowest) in place, xhat[2 * S] in `layout` (or NULL)
+cudaError_t launch_kf(cudaStream_t st, int layout, int mflags, int S, const double *y, const double *u,
+                      const double *params, int pc, const KfCov &cov, double *rec, double *xhat, long long *launches);
 cudaError_t launch_condense(cudaStream_t st, const DeviceProps &dp, int layout, int flags, int S, int N,
                             const double *R1, const double *R2, const double *R3, const double *params, int pc,
                             double *Phi, double *Gam, double *Lam, long long *launches);
@@ -110,6 +130,8 @@ constexpr int EXT_COLD_PLANT = 1;
 constexpr int EXT_STATE_ROWS = 2;
 constexpr int EXT_PERTURBED = 3;
 constexpr int EXT_PERTURBED_ROWS = 4;
+constexpr int EXT_OBSERVED = 5;          // EXT_PERTURBED + the observer (LoopArgs::obs)
+constexpr int EXT_OBSERVED_ROWS = 6;     // EXT_PERTURBED_ROWS + the observer
 // one instantiation closed_loop_kernel<gw, dense, ext, lv, ctl>
 struct LoopKey {
     int gw;

@@ -104,6 +104,55 @@ __device__ __forceinline__ void plant_exact(const Params &P, int flags, double a
     nom = __dadd_rn(om, __ddiv_rn(__dadd_rn(so, ao), 6.0));
 }
 
+// One step of the quasi-LPV Kalman filter on the controller's own model (ntm_kf_step; record layout NTM_KF_DOUBLES in
+// include/ntm_mpc.h), shared by the per-call kernel and the observed fused loop so that the two agree bit for bit; every
+// rounding is spelled out for the reason given at plant_exact.  mflags: RHO1_SQ | PLANT_C | PLANT_RK4 of the profile word.
+// Fresh (a new record): xhat = y, P = Rv, u is not read.  Otherwise predict with the plant of ntm_plant_step and
+// F = A(rho(xhat)) of A.m:2 (rho frozen at the estimate, as the condensation freezes it; the Euler-map matrix even under
+// RK4: the quasi-LPV approximation, no Jacobian of rho), P- = F P F' + Qw, then update with S = P- + Rv, K = P- S^-1 and
+// the Joseph form P = (I - K) P- (I - K)' + K Rv K', which keeps P symmetric positive semi-definite although the two
+// states differ in scale by ~1e5.  Only the lower triangle is stored, so P is symmetric by construction.  Non-finite
+// inputs propagate into the record.
+__device__ __forceinline__ void kf_step_exact(const Params &P, int mflags, const KfCov &c, double *rec, bool fresh,
+                                              double y1, double y2, double u, double &xh1, double &xh2) {
+    double p11, p21, p22, steps;
+    if (fresh) {
+        xh1 = y1; xh2 = y2; p11 = c.r11; p21 = c.r21; p22 = c.r22; steps = 1.0;
+    } else {
+        const double w = rec[0], om = rec[1], o11 = rec[2], o21 = rec[3], o22 = rec[4];
+        steps = __dadd_rn(rec[5], 1.0);
+        double m1, m2;                                   // predicted state
+        plant_exact(P, mflags, P.a22, 0.0, w, om, u, m1, m2);
+        const double ww = __dmul_rn(w, w);
+        const double r1 = __drcp_rn((mflags & NTM_PROFILE_RHO1_SQ) ? __dadd_rn(ww, P.wmarg2) : __dadd_rn(w, P.wmarg2));
+        const double a11 = __fma_rn(P.c_a11, r1, 1.0), a21 = __dmul_rn(P.c_a21, __ddiv_rn(ww, om)), a22 = P.a22;
+        // P- = F P F' + Qw, with F P = [a11 p11, a11 p21; t21, t22]
+        const double t21 = __fma_rn(a22, o21, __dmul_rn(a21, o11)), t22 = __fma_rn(a22, o22, __dmul_rn(a21, o21));
+        const double n11 = __fma_rn(a11, __dmul_rn(a11, o11), c.q11), n21 = __fma_rn(a11, t21, c.q21);
+        const double n22 = __fma_rn(a22, t22, __fma_rn(a21, t21, c.q22));
+        // K = P- (P- + Rv)^-1 by the closed-form inverse
+        const double s11 = __dadd_rn(n11, c.r11), s21 = __dadd_rn(n21, c.r21), s22 = __dadd_rn(n22, c.r22);
+        const double det = __fma_rn(s11, s22, -__dmul_rn(s21, s21));
+        const double k11 = __ddiv_rn(__fma_rn(n11, s22, -__dmul_rn(n21, s21)), det);
+        const double k12 = __ddiv_rn(__fma_rn(n21, s11, -__dmul_rn(n11, s21)), det);
+        const double k21 = __ddiv_rn(__fma_rn(n21, s22, -__dmul_rn(n22, s21)), det);
+        const double k22 = __ddiv_rn(__fma_rn(n22, s11, -__dmul_rn(n21, s21)), det);
+        const double e1 = __dsub_rn(y1, m1), e2 = __dsub_rn(y2, m2);
+        xh1 = __fma_rn(k12, e2, __fma_rn(k11, e1, m1));
+        xh2 = __fma_rn(k22, e2, __fma_rn(k21, e1, m2));
+        // Joseph form: (I - K) P- = [b11 b12; b21 b22], K Rv = [g11 g12; g21 g22]
+        const double i11 = __dsub_rn(1.0, k11), i12 = -k12, i21 = -k21, i22 = __dsub_rn(1.0, k22);
+        const double b11 = __fma_rn(i12, n21, __dmul_rn(i11, n11)), b12 = __fma_rn(i12, n22, __dmul_rn(i11, n21));
+        const double b21 = __fma_rn(i22, n21, __dmul_rn(i21, n11)), b22 = __fma_rn(i22, n22, __dmul_rn(i21, n21));
+        const double g11 = __fma_rn(k12, c.r21, __dmul_rn(k11, c.r11)), g12 = __fma_rn(k12, c.r22, __dmul_rn(k11, c.r21));
+        const double g21 = __fma_rn(k22, c.r21, __dmul_rn(k21, c.r11)), g22 = __fma_rn(k22, c.r22, __dmul_rn(k21, c.r21));
+        p11 = __fma_rn(g12, k12, __fma_rn(g11, k11, __fma_rn(b12, i12, __dmul_rn(b11, i11))));
+        p21 = __fma_rn(g22, k12, __fma_rn(g21, k11, __fma_rn(b22, i12, __dmul_rn(b21, i11))));
+        p22 = __fma_rn(g22, k22, __fma_rn(g21, k21, __fma_rn(b22, i22, __dmul_rn(b21, i21))));
+    }
+    rec[0] = xh1; rec[1] = xh2; rec[2] = p11; rec[3] = p21; rec[4] = p22; rec[5] = steps;
+}
+
 // =================================================================================================
 // fused persistent closed loop
 // =================================================================================================
@@ -148,9 +197,12 @@ __device__ void stage_prefix(int N, int j, const Work &w, const Params &P, doubl
 // spill stores in closed_loop_kernel<4, false, 0, 0>; the state-row ones sit at their register caps (DESIGN section 4.8).
 template <int GW, bool DENSE, int EXT, bool CTL = false>
 struct LoopTraits {
-    static constexpr bool ROWS = (EXT == 2 || EXT == 4);   // getWLc's state rows
-    static constexpr bool PERT = (EXT == 3 || EXT == 4);   // the perturbed plant (LoopArgs::pp: its own parameters and
+    static constexpr bool ROWS = (EXT == 2 || EXT == 4 || EXT == 6);   // getWLc's state rows
+    static constexpr bool PERT = (EXT >= 3 && EXT <= 6);   // the perturbed plant (LoopArgs::pp: its own parameters and
                                                            // profile bits, d_k and v_k)
+    // the observer (LoopArgs::obs): the controller sees the estimate of one ntm_kf_step per time step.  Its own keys:
+    // as a runtime mode of the EXT 3 / 4 instantiations it moved their register and spill figures (DESIGN section 4.10).
+    static constexpr bool OBS = (EXT == 5 || EXT == 6);
     static constexpr bool COLD = (EXT == 1 || EXT == 2);   // the controller's plant with the RK4 / tau_E(w) options, and
                                                            // the controller-side tau_E(w)
     // long horizons, literal Gamma, box QP: the QP runs on the packed sweep tableau of ntm_long.cuh
@@ -162,7 +214,7 @@ struct LoopTraits {
     // two-phase launch (headline instantiation only): a launch runs the time steps [k_begin, k_end) of the scenario
     static constexpr bool TWOPH = (GW == 1) && !DENSE && (EXT == 0);
     // __launch_bounds__ minimum blocks per SM
-    static constexpr int MIN_BLOCKS = GW == 1 ? (EXT == 0 ? 5 : ((EXT == 1 || EXT == 3) ? 4 : 3)) : (LONG ? 3 : 1);
+    static constexpr int MIN_BLOCKS = GW == 1 ? (EXT == 0 ? 5 : ((EXT == 1 || EXT == 3 || EXT == 5) ? 4 : 3)) : (LONG ? 3 : 1);
     using WorkT = typename std::conditional<LONG, LongWork, Work>::type;
 };
 
@@ -446,6 +498,23 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                 if (pi.noise != nullptr) {
                     x1 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k)); x2 += __ldg(pi.noise + elem(layout, S, 2 * a.k_sim, s, 2 * k + 1));
                 }
+                if constexpr (LT::OBS) {
+                    // the observer (ntm_mpc_closed_loop_observed): the controller sees xhat_k = ntm_kf_step(y_k, u_{k-1}),
+                    // a fresh filter at k = 0 (xhat_0 = y_0, the point the offline build already ran from).  The lead
+                    // steps the record and the group reads the estimate back after a barrier: no register carries it.
+                    double *rec = a.obs.rec + (size_t)s * NTM_KF_DOUBLES;
+                    if (lead) {
+                        double h1, h2;
+                        kf_step_exact(P, a.obs.mflags, a.obs.cov, rec, k == 0, x1, x2, k > 0 ? a.uk[uk_at(k - 1)] : 0.0,
+                                      h1, h2);
+                        if (a.obs.xhat != nullptr) {
+                            a.obs.xhat[elem(layout, S, 2 * a.k_sim, s, 2 * k)] = h1;
+                            a.obs.xhat[elem(layout, S, 2 * a.k_sim, s, 2 * k + 1)] = h2;
+                        }
+                    }
+                    Gp::sync();
+                    x1 = rec[0]; x2 = rec[1];
+                }
                 if (!(isfinite(x1) && isfinite(x2))) status = max(status, (int)NTM_SCN_NONFINITE);
             }
         } else if (ctl && it == 0) {     // G, F on hand are built; the step itself (QP, rollout) starts from the measurement
@@ -594,6 +663,10 @@ __device__ void run_scenario(const LoopArgs &a, int s, int j, const typename Loo
                         if (!ctl) {                      // a controller step has no xk
                             a.xk[xk_at(2 * (kk + 1))] = nan;
                             a.xk[xk_at(2 * (kk + 1) + 1)] = nan;
+                        }
+                        if (LT::OBS && kk > k && a.obs.xhat != nullptr) {   // no estimate after the infeasible step
+                            a.obs.xhat[elem(layout, S, 2 * a.k_sim, s, 2 * kk)] = nan;
+                            a.obs.xhat[elem(layout, S, 2 * a.k_sim, s, 2 * kk + 1)] = nan;
                         }
                         if (a.inner) a.inner[elem(layout, S, a.k_sim, s, kk)] = (kk == k) ? it : 0;
                         if (a.qpit) a.qpit[elem(layout, S, a.k_sim, s, kk)] = (kk == k) ? qpit + nit : 0;

@@ -53,6 +53,11 @@ def rec_doubles(k_sim: int) -> int:
     return 3 * k_sim + 4
 
 
+def kf_doubles() -> int:
+    """NTM_KF_DOUBLES: doubles per scenario of an observer record (``ntm_kf_step``): xhat, p11, p21, p22, steps."""
+    return 6
+
+
 def ctrl_doubles(N: int) -> int:
     """NTM_CTRL_DOUBLES(N): doubles per scenario of a controller record (``ntm_mpc_step``)."""
     return 7 * N + 7
@@ -80,6 +85,10 @@ for _sfx in ("", "_dev"):
     SYMBOLS["ntm_mpc_closed_loop_perturbed_sc" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp,
                                                                _i, _i, _dp, _dp, _i, _i, _dp, _dp, _dp, _dp, _dp, _dp,
                                                                _dp, _dp, _dp])
+    SYMBOLS["ntm_kf_step" + _sfx] = (_i, [_h, _i, _i, _i, _dp, _dp, _dp, _i, _dp, _dp, _dp])
+    SYMBOLS["ntm_mpc_closed_loop_observed" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i,
+                                                           _i, _dp, _dp, _i, _i, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
+                                                           _dp, _dp, _dp, _dp])
     SYMBOLS["ntm_mpc_closed_loop_sc" + _sfx] = (_i, [_h, _i, _i, _i, _i, _i, _i, ctypes.c_double, _dp, _dp, _i, _i, _dp,
                                                      _dp, _dp, _dp, _dp, _dp, _dp, _dp])
 

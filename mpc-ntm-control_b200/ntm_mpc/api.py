@@ -14,7 +14,8 @@ from typing import Dict, Optional
 import numpy as np
 
 from . import _lib
-from ._lib import LAYOUT_MATLAB, LAYOUT_SOA, NPARAM, NtmError, check, ctrl_doubles, load, rec_doubles  # noqa: F401
+from ._lib import (LAYOUT_MATLAB, LAYOUT_SOA, NPARAM, NtmError, check, ctrl_doubles, kf_doubles, load,  # noqa: F401
+                   rec_doubles)
 
 MC_NBINS = 32                                   # NTM_MC_NBINS / NTM_MC_NSTAT of include/ntm_mpc.h
 MC_NSTAT = 22 + MC_NBINS
@@ -121,6 +122,30 @@ def perturbed_inputs(x0, params, plant_params, plant_profile, w, v, k_sim: int, 
                 raise ValueError(f"{name} must be [S, k_sim, 2] = {(S, k_sim, 2)} (got {a.shape})")
         ext.append(a)
     return x0, p, pc, pp, ppc, pf, ext[0], ext[1]
+
+
+def kf_cov_input(kf_cov) -> np.ndarray:
+    """Checks the observer's covariances ``kf_cov = (qw11, qw21, qw22, rv11, rv21, rv22)`` (no device needed) and returns
+    them as a float64 6-vector: every entry finite, Qw positive semi-definite, Rv positive definite (``ntm_kf_step``)."""
+    if kf_cov is None:
+        raise ValueError("kf_cov is required: (qw11, qw21, qw22, rv11, rv21, rv22)")
+    c = _f64(kf_cov).ravel()
+    if c.size != 6:
+        raise ValueError(f"kf_cov must have 6 entries (qw11, qw21, qw22, rv11, rv21, rv22), got {c.size}")
+    if not np.all(np.isfinite(c)):
+        raise ValueError("kf_cov: non-finite entry")
+    q11, q21, q22, r11, r21, r22 = c
+    if not (q11 >= 0.0 and q22 >= 0.0 and q11 * q22 >= q21 * q21):
+        raise ValueError("kf_cov: Qw is not positive semi-definite")
+    if not (r11 > 0.0 and r11 * r22 > r21 * r21):
+        raise ValueError("kf_cov: Rv is not positive definite")
+    return c
+
+
+def _kf_state(state, S: int) -> None:
+    if not (isinstance(state, np.ndarray) and state.dtype == np.float64 and state.shape == (S, kf_doubles())
+            and state.flags.c_contiguous and state.flags.writeable):
+        raise ValueError(f"state must be a writeable C-contiguous float64 array of shape {(S, kf_doubles())}")
 
 
 def device_count() -> int:
@@ -442,6 +467,78 @@ class NtmMpc:
                                                              cost_ptr or None, inner_ptr or None, qp_ptr or None,
                                                              status_ptr or None))
 
+    def closed_loop_observed(self, x0, params, N: int, kf_cov, plant_params=None, plant_profile: Optional[int] = None,
+                             w=None, v=None, k_sim: int = 20, i_sim: int = 10, eps: float = 1e-14, profile: int = 0,
+                             want_Uk: bool = False, out: Optional[dict] = None, state_rows: int = 0, xbounds=None):
+        """``closed_loop_perturbed`` with a state observer between the sensor and the controller
+        (``ntm_mpc_closed_loop_observed``): the controller sees ``xhat_k = kf_step(y_k, u_{k-1})``, the estimate of an
+        LPV Kalman filter on its own model with the covariances ``kf_cov = (qw11, qw21, qw22, rv11, rv21, rv22)``,
+        instead of ``y_k``.  Returns the dict of ``closed_loop_perturbed`` plus ``xhat`` [S, k_sim, 2], the estimate the
+        controller used at each step (NaN after an infeasible step)."""
+        x0, p, pc, pp, ppc, pf, wf, vf = perturbed_inputs(x0, params, plant_params, plant_profile, w, v, k_sim, profile)
+        S = x0.shape[0]
+        xb = state_box_inputs(state_rows, xbounds)
+        kc = kf_cov_input(kf_cov)
+        outs = _loop_outputs(out, S, N, k_sim, want_Uk)
+        xk, uk, Uk, cost, inner, qpit, status = outs
+        xhat = np.empty((S, k_sim, 2))
+        check(self._lib.ntm_mpc_closed_loop_observed(self._h, LAYOUT_MATLAB, profile, S, N, k_sim, i_sim, eps, _ptr(x0),
+                                                     _ptr(p), pc, int(state_rows), _ptr(xb), _ptr(pp), ppc, pf, _ptr(wf),
+                                                     _ptr(vf), _ptr(kc), _ptr(xhat), _ptr(xk), _ptr(uk),
+                                                     _ptr(Uk) if want_Uk else None, _ptr(cost), _ptr(inner), _ptr(qpit),
+                                                     _ptr(status)))
+        res = _loop_result(outs)
+        res["xhat"] = xhat
+        return res
+
+    def closed_loop_observed_dev(self, S: int, N: int, k_sim: int, i_sim: int, eps: float, profile: int, layout: int,
+                                 x0_ptr: int, params_ptr: int, params_count: int, plant_params_ptr: int,
+                                 plant_params_count: int, plant_profile: int, w_ptr: int, v_ptr: int, xk_ptr: int,
+                                 uk_ptr: int, Uk_ptr: int = 0, cost_ptr: int = 0, inner_ptr: int = 0, qp_ptr: int = 0,
+                                 status_ptr: int = 0, state_rows: int = 0, xbounds=None, kf_cov=None,
+                                 xhat_ptr: int = 0) -> None:
+        """``closed_loop_observed`` on device pointers (``ntm_mpc_closed_loop_observed_dev``), the arguments of
+        ``closed_loop_perturbed_dev`` plus the host 6-vector ``kf_cov`` and ``xhat_ptr`` (2 * k_sim doubles per
+        scenario in ``layout``, 0 = not wanted); one launch on the handle's stream, no copy."""
+        check(self._lib.ntm_mpc_closed_loop_observed_dev(self._h, layout, profile, S, N, k_sim, i_sim, eps, x0_ptr,
+                                                         params_ptr, params_count, int(state_rows),
+                                                         _ptr(state_box_inputs(state_rows, xbounds)),
+                                                         plant_params_ptr or None, plant_params_count, plant_profile,
+                                                         w_ptr or None, v_ptr or None, _ptr(kf_cov_input(kf_cov)),
+                                                         xhat_ptr or None, xk_ptr, uk_ptr, Uk_ptr or None,
+                                                         cost_ptr or None, inner_ptr or None, qp_ptr or None,
+                                                         status_ptr or None))
+
+    # ------------------------------------------------------------------ state observer (LPV Kalman filter)
+    def kf_step(self, state, y, u, params, kf_cov, profile: int = 0) -> np.ndarray:
+        """One step of the observer for S scenarios (``ntm_kf_step``): measurements ``y`` [S, 2], the inputs ``u`` [S]
+        applied since each record's last step (ignored for fresh records).  ``state`` is a C-contiguous float64 array
+        [S, ``kf_doubles()``] (xhat, p11, p21, p22, steps) updated in place; an all-zero row is a fresh filter.  ``kf_cov
+        = (qw11, qw21, qw22, rv11, rv21, rv22)``; ``profile``: the controller's profile word (its model bits RHO1_SQ,
+        PLANT_C and PLANT_RK4 choose the prediction).  Returns the estimate [S, 2]."""
+        y = _f64(y).reshape(-1, 2)
+        S = y.shape[0]
+        u = _f64(np.broadcast_to(np.asarray(u, dtype=np.float64), (S,)))
+        p, pc = self._params(params, S)
+        kc = kf_cov_input(kf_cov)
+        _kf_state(state, S)
+        xhat = np.empty((S, 2))
+        check(self._lib.ntm_kf_step(self._h, LAYOUT_MATLAB, profile, S, _ptr(y), _ptr(u), _ptr(p), pc, _ptr(kc),
+                                    _ptr(state), _ptr(xhat)))
+        return xhat
+
+    def kf_step_dev(self, S: int, profile: int, layout: int, y_ptr: int, u_ptr: int, params_ptr: int,
+                    params_count: int, kf_cov, state_ptr: int, xhat_ptr: int = 0) -> None:
+        """``kf_step`` on device pointers, asynchronous on the handle's stream (``ntm_kf_step_dev``); the records
+        (``kf_doubles()`` doubles per scenario, scenario slowest) stay resident, ``kf_cov`` is a host 6-vector."""
+        check(self._lib.ntm_kf_step_dev(self._h, layout, profile, S, y_ptr, u_ptr, params_ptr, params_count,
+                                        _ptr(kf_cov_input(kf_cov)), state_ptr, xhat_ptr or None))
+
+    def observer(self, params, kf_cov, S: Optional[int] = None, profile: int = 0) -> "Observer":
+        """An ``Observer`` on this handle that owns the filter records of S scenarios (S from ``params`` [S, NPARAM], or
+        given with one shared [NPARAM] block)."""
+        return Observer(self, params, kf_cov, S, profile)
+
     # ------------------------------------------------------------------ NTM_MPC_Sim.m:94-128, one step, no plant
     def mpc_step(self, state, x, params, N: int, i_sim: int = 10, eps: float = 1e-14, profile: int = 0,
                  want_U: bool = False, state_rows: int = 0, xbounds=None):
@@ -556,6 +653,43 @@ class Controller:
 
     def reset(self, mask=None) -> None:
         """Fresh controllers for every scenario (``mask=None``) or for those selected by a boolean / index ``mask``."""
+        if mask is None:
+            self.state[:] = 0.0
+        else:
+            self.state[np.asarray(mask)] = 0.0
+
+
+class Observer:
+    """The state observer of the controller's model for S scenarios, between a sensor and a ``Controller``::
+
+        obs = mpc.observer(params, kf_cov, S)
+        ctl = mpc.controller(params, N=20, S=S)
+        u = None
+        for k in range(k_sim):
+            u = ctl.step(obs.update(y, u))   # y: measurements [S, 2]
+
+    Holds the per-scenario records of ``ntm_kf_step`` (host memory) and the fixed arguments every call for them must
+    repeat.  ``reset(mask)`` restarts the selected scenarios: their next update returns the measurement itself."""
+
+    def __init__(self, mpc: NtmMpc, params, kf_cov, S: Optional[int] = None, profile: int = 0):
+        p = _f64(params)
+        if S is None:
+            if p.ndim != 2:
+                raise ValueError("S is needed with one shared parameter block")
+            S = p.shape[0]
+        self.mpc, self.S, self.profile = mpc, int(S), int(profile)
+        self.params, _ = NtmMpc._params(p, self.S)
+        self.kf_cov = kf_cov_input(kf_cov)
+        self.state = np.zeros((self.S, kf_doubles()))
+
+    def update(self, y, u_prev=None) -> np.ndarray:
+        """The estimate [S, 2] after the measurements ``y`` [S, 2]; ``u_prev`` [S]: the inputs applied since the last
+        update (None on the first one, when every record is fresh)."""
+        u = np.zeros(self.S) if u_prev is None else u_prev
+        return self.mpc.kf_step(self.state, y, u, self.params, self.kf_cov, self.profile)
+
+    def reset(self, mask=None) -> None:
+        """Fresh filters for every scenario (``mask=None``) or for those selected by a boolean / index ``mask``."""
         if mask is None:
             self.state[:] = 0.0
         else:

@@ -13,7 +13,7 @@ import numpy as np
 
 from . import physics
 from ._lib import LAYOUT_SOA, NPARAM
-from .api import MC_NBINS, MC_NSTAT, MC_STATE_BOX, PLANT_PROFILE_BITS, NtmMpc
+from .api import MC_NBINS, MC_NSTAT, MC_STATE_BOX, PLANT_PROFILE_BITS, NtmMpc, kf_cov_input
 
 
 def describe(stats: np.ndarray, hist_max: float = 0.2) -> Dict[str, object]:
@@ -46,7 +46,7 @@ def run(config: int = 3, S: Optional[int] = None, seed: Optional[int] = None, pr
         i_sim: int = 10, eps: float = 1e-14, bounds=MC_STATE_BOX, w_suppressed: float = 0.06, hist_max: float = 0.2,
         trajectories: bool = False, handle: Optional[NtmMpc] = None, device: int = 0,
         state_rows: int = 0, sample=None, plant_sample=None, plant_profile: Optional[int] = None, w_std=None,
-        v_std=None, noise_seed: Optional[int] = None) -> Dict[str, object]:
+        v_std=None, noise_seed: Optional[int] = None, kf_cov=None) -> Dict[str, object]:
     """One Monte-Carlo batch of BASELINE config ``config`` through the fused loop; returns ``describe(...)`` of the
     on-device reduction, ``N``, ``S`` and -- with ``trajectories`` -- ``xk [S,k_sim+1,2]``, ``uk [S,k_sim]``,
     ``cost [S]``, ``status [S]`` on the host.  ``state_rows`` != 0 keeps getWLc's state rows (box = ``bounds``) in every
@@ -64,12 +64,19 @@ def run(config: int = 3, S: Optional[int] = None, seed: Optional[int] = None, pr
     device by ``noise`` and never copied to the host.  The reduction runs on the true trajectories with the controller's
     umin / umax.  With ``state_rows`` the controller keeps getWLc's state rows (box = ``bounds``) against the perturbed
     plant (``ntm_mpc_closed_loop_perturbed_sc_dev``): the rows test what the controller sees, y_k = x_k + v_k, and the
-    reduction counts how often the TRUE state left the box."""
+    reduction counts how often the TRUE state left the box.
+
+    Observer (``ntm_mpc_closed_loop_observed_dev``): with ``kf_cov = (qw11, qw21, qw22, rv11, rv21, rv22)`` the same
+    plant and noise draws run with an LPV Kalman filter between the sensor and the controller, which then sees the
+    estimate instead of y_k (``kf_cov_from_std`` matches the covariances to ``w_std`` / ``v_std``).  The reduction still
+    judges the true states; ``trajectories`` adds ``xhat [S,k_sim,2]``, the estimates the controller used."""
     import torch                                               # device buffers + stream plumbing only
     h = handle or NtmMpc(device)
     prm, x0, N = physics.batch_params(config, S, seed, sample) # [NPARAM, S] SoA, [S, 2]
     S = x0.shape[0]
-    perturbed = plant_sample is not None or plant_profile is not None or w_std is not None or v_std is not None
+    observed = kf_cov is not None
+    kc = kf_cov_input(kf_cov) if observed else None
+    perturbed = observed or plant_sample is not None or plant_profile is not None or w_std is not None or v_std is not None
     dev = torch.device(f"cuda:{device}")
     d_prm = torch.from_numpy(prm).to(dev)                      # SoA block: scenario index fastest
     d_x0 = torch.from_numpy(np.ascontiguousarray(x0.T)).to(dev)
@@ -78,6 +85,7 @@ def run(config: int = 3, S: Optional[int] = None, seed: Optional[int] = None, pr
     d_cost = torch.empty(S, dtype=torch.float64, device=dev)
     d_st = torch.empty(S, dtype=torch.int32, device=dev)
     d_out = torch.empty(MC_NSTAT, dtype=torch.float64, device=dev)
+    d_xhat = torch.empty(2 * k_sim * S, dtype=torch.float64, device=dev) if observed and trajectories else None
     h.set_stream(torch.cuda.current_stream(dev).cuda_stream or None)
     try:
         if perturbed:
@@ -85,11 +93,15 @@ def run(config: int = 3, S: Optional[int] = None, seed: Optional[int] = None, pr
             d_pp = torch.from_numpy(plant_batch_params(config, S, seed, sample, plant_sample)).to(dev) \
                 if plant_sample else None
             d_w, d_v = noise(S, k_sim, w_std, v_std, noise_seed, dev)
-            h.closed_loop_perturbed_dev(S, N, k_sim, i_sim, eps, profile, LAYOUT_SOA, d_x0.data_ptr(), d_prm.data_ptr(), S,
-                                        d_pp.data_ptr() if d_pp is not None else 0, S, pf,
-                                        d_w.data_ptr() if d_w is not None else 0, d_v.data_ptr() if d_v is not None else 0,
-                                        d_xk.data_ptr(), d_uk.data_ptr(), 0, d_cost.data_ptr(), 0, 0, d_st.data_ptr(),
-                                        state_rows=state_rows, xbounds=bounds)
+            args = (S, N, k_sim, i_sim, eps, profile, LAYOUT_SOA, d_x0.data_ptr(), d_prm.data_ptr(), S,
+                    d_pp.data_ptr() if d_pp is not None else 0, S, pf,
+                    d_w.data_ptr() if d_w is not None else 0, d_v.data_ptr() if d_v is not None else 0,
+                    d_xk.data_ptr(), d_uk.data_ptr(), 0, d_cost.data_ptr(), 0, 0, d_st.data_ptr())
+            if observed:
+                h.closed_loop_observed_dev(*args, state_rows=state_rows, xbounds=bounds, kf_cov=kc,
+                                           xhat_ptr=d_xhat.data_ptr() if d_xhat is not None else 0)
+            else:
+                h.closed_loop_perturbed_dev(*args, state_rows=state_rows, xbounds=bounds)
         elif state_rows:
             h.closed_loop_sc_dev(S, N, k_sim, i_sim, eps, profile, LAYOUT_SOA, d_x0.data_ptr(), d_prm.data_ptr(), S,
                                  state_rows, bounds, d_xk.data_ptr(), d_uk.data_ptr(), 0, d_cost.data_ptr(), 0, 0,
@@ -111,10 +123,14 @@ def run(config: int = 3, S: Optional[int] = None, seed: Optional[int] = None, pr
                    v_std=np.zeros(2) if v_std is None else np.broadcast_to(np.asarray(v_std, float), (2,)))
         if plant_sample:
             res["plant_params"] = d_pp.cpu().numpy()
+        if observed:
+            res["kf_cov"] = kc
     if trajectories:
         res["xk"] = np.ascontiguousarray(d_xk.cpu().numpy().reshape(2 * (k_sim + 1), S).T.reshape(S, k_sim + 1, 2))
         res["uk"] = np.ascontiguousarray(d_uk.cpu().numpy().reshape(k_sim, S).T)
         res["cost"] = d_cost.cpu().numpy(); res["status"] = d_st.cpu().numpy()
+        if d_xhat is not None:
+            res["xhat"] = np.ascontiguousarray(d_xhat.cpu().numpy().reshape(2 * k_sim, S).T.reshape(S, k_sim, 2))
     return res
 
 
@@ -132,6 +148,17 @@ def plant_batch_params(config: int, S: int, seed: Optional[int], sample, plant_s
         lo, hi = plant_sample[key]
         phys[key] = lo + (hi - lo) * u[:, c]
     return np.ascontiguousarray(physics.params_from_physics(phys).reshape(NPARAM, -1))
+
+
+def kf_cov_from_std(w_std, v_std) -> np.ndarray:
+    """The observer's ``kf_cov`` matched to the noise ``run`` draws: the diagonal covariances of independent Gaussian
+    components, Qw = diag(w_std^2) (None: no disturbance, Qw = 0) and Rv = diag(v_std^2).  ``w_std`` / ``v_std``: scalar
+    or per-component pair, as in ``run``; Rv must be positive definite, so both components of ``v_std`` are > 0."""
+    q = np.zeros(2) if w_std is None else np.broadcast_to(np.asarray(w_std, dtype=np.float64), (2,)) ** 2
+    if v_std is None:
+        raise ValueError("kf_cov_from_std: v_std is required (the measurement covariance must be positive definite)")
+    r = np.broadcast_to(np.asarray(v_std, dtype=np.float64), (2,)) ** 2
+    return kf_cov_input((q[0], 0.0, q[1], r[0], 0.0, r[1]))
 
 
 def noise(S: int, k_sim: int, w_std, v_std, seed: Optional[int], device):
